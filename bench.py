@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps 20 --warmup 5            # our arm (libglf_sm100a.so)
     python bench.py --impl reference --steps 3 --warmup 1     # the reference algorithm on the host CPU cores
+    python bench.py --steps 20 --dump-outputs DIR              # + the last timed step's output and gradients as .npy
 
 Workload = BASELINE.json configs[1]: MGFM+MLFM modules only, 4 views x 16 frames x 28x28 tokens, C=256, bf16,
 fwd+bwd, frames-as-batch layout (Global_and_Local, R/models/ours.py:1819-1821): one clip = 16 sequences of
@@ -239,6 +240,27 @@ def bind_to_gpu_numa(index: int, world: int = 1):
     return None, None, None
 
 
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Write each tensor as <path>/<name>.npy in float32, in all at most DUMP_BYTES.  Arrays are served smallest
+    first; one larger than its even share of what is left is replaced by a seeded sample of its flattened (logical,
+    row-major) elements.  The sample depends only on the array's shape, so two builds dump the same positions."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES // 4
+    items = sorted(arrays.items(), key=lambda kv: (kv[1].numel(), kv[0]))
+    for i, (name, t) in enumerate(items):
+        t = t.detach()
+        k = min(t.numel(), left // (len(items) - i))
+        left -= k
+        if k < t.numel():
+            idx = torch.randint(0, t.numel(), (k,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     from glfusion_b200 import dp
     rank, local_rank, world = dp.init_process_group("nccl")
@@ -252,7 +274,8 @@ def run_ours(args):
     for t in f4:
         t.requires_grad_(True)
     B = clips * F
-    dz = torch.randn(B, V, HH, WW, C, device=dev, dtype=torch.bfloat16).permute(0, 4, 1, 2, 3)
+    dz = torch.randn(B, V, HH, WW, C, device=dev, dtype=torch.bfloat16,
+                     generator=torch.Generator(device=dev).manual_seed(0)).permute(0, 4, 1, 2, 3)
     bucket = dp.GradBucket(list(fusion.global_attn._plist()) + list(fusion.local_attn._plist()))
     bucket.bind([fusion.global_attn, fusion.local_attn])   # gradients are written into the all-reduce bucket directly
     # the fusion-weight gradient average as one kernel over NVLink peer memory (NCCL stays the fallback)
@@ -263,6 +286,7 @@ def run_ours(args):
         bucket.overlap_with(fusion)      # the exchange starts before the gate backward, on a side stream
 
     params = [p for p in fusion.parameters() if p.requires_grad]
+    last = {}                            # --dump-outputs: the step's forward output (a graph replay rewrites it in place)
 
     def compute():
         for t in f4:
@@ -271,6 +295,8 @@ def run_ours(args):
             p.grad = None                # optimizer.zero_grad(set_to_none=True): gradients are assigned, not accumulated
         out = fusion.forward_stacked(f4, cls, ctr)
         out.backward(dz)
+        if args.dump_outputs:
+            last["out"] = out.detach()   # without the autograd graph, which must not outlive the step
 
     graph = None
     allreduce_in_graph = False
@@ -344,6 +370,11 @@ def run_ours(args):
         sampler.start()
     ms = timed(args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        arrays = {"out": last["out"]}
+        arrays.update({f"grad_f4_{v}": t.grad for v, t in enumerate(f4)})
+        arrays.update({"grad_" + n: p.grad for n, p in fusion.named_parameters() if p.grad is not None})
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- end-to-end: host (pinned) inputs -> H2D -> fwd+bwd -> D2H of the step's scalar result ----------------------
     hf4, hcls, hctr = make_inputs(clips, C, 100 + rank, dev, pinned=True)
@@ -385,7 +416,7 @@ def run_ours(args):
     if world > 1:
         torch.distributed.barrier()
     e0.record()
-    esteps = max(2, min(args.steps, 10))
+    esteps = args.steps
     for _ in range(esteps):
         e2e_step()
     e1.record()
@@ -931,7 +962,13 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-width2048", action="store_true", help="skip the C=2048 secondary object")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's output and gradients to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -17,17 +17,22 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REF_SRC = "/root/reference/GLfusion/models/TPAVI.py"
 REF_DIR = os.path.join(HERE, "_ref")
 REF_DST = os.path.join(REF_DIR, "models", "TPAVI.py")
+REF_MAIN = os.path.join(REF_DIR, "main.py")          # the trainer, for its cycle-consistency methods
 
 
 def build_ref() -> bool:
     """Stage the reference's ``models/`` package (the fusion block and, for the full-network harness of
-    tests/test_gpu_network.py, the network that calls it); True when oracle/_ref holds it afterwards."""
+    tests/test_gpu_network.py, the network that calls it) and its ``main.py`` (the trainer's cycle-consistency methods,
+    for tests/test_oracle_cycle.py); True when oracle/_ref holds the fusion block afterwards."""
     src_dir = os.path.dirname(REF_SRC)
     if os.path.exists(REF_SRC):
         os.makedirs(os.path.dirname(REF_DST), exist_ok=True)
         for name in sorted(os.listdir(src_dir)):
             if name.endswith(".py"):
                 shutil.copyfile(os.path.join(src_dir, name), os.path.join(os.path.dirname(REF_DST), name))
+        main = os.path.join(os.path.dirname(src_dir), "main.py")
+        if os.path.exists(main):
+            shutil.copyfile(main, REF_MAIN)
     return os.path.exists(REF_DST)
 
 

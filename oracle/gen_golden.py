@@ -7,7 +7,9 @@ Run in the build container only (needs /root/reference):
 It imports ``/root/reference/GLfusion/models/TPAVI.py`` (torch-only; semantically identical to the copy at
 R/models/ours.py:770-917), loads seeded weights into it through ``load_state_dict(strict=True)``, re-randomises
 the zero-initialised BatchNorm gamma/beta and the LayerNorm affine (SURVEY.md F3), runs forward + autograd
-backward on CPU in fp32 and writes ``tests/golden/<case>.npz`` with every input, output, gradient and BN buffer.
+backward on CPU in fp32 and writes ``tests/golden/<case>.npz`` with every input, output, gradient and BN buffer
+(the OUTPUTS_ONLY cases without their seeded inputs and weights, which ``seeded_inputs`` rebuilds).  ``init_dot_c96``
+holds the constructor's own state dict under a fixed seed.
 
 The glue case additionally restates, literally, lines 1802-1834 of R/models/ours.py around two reference
 modules (the enclosing class cannot be constructed offline: it downloads ImageNet weights and imports monai).
@@ -53,19 +55,45 @@ def make_module(TPAVIModule, C, mode, bn_layer, params):
     return m
 
 
-def run_case(TPAVIModule, name, B, C, T, H, W, mode, training, bn_layer, seed):
-    torch.manual_seed(seed)
+GLUE_SEED = 7
+# cases whose .npz holds only what the reference computed: their seeded inputs and weights are rebuilt by
+# seeded_inputs() (keeps every golden file under 1 MB)
+OUTPUTS_ONLY = ("dot_train_c256", "glue_dot_c128")
+
+
+def seeded_inputs(name: str) -> dict:
+    """The seeded inputs and weights of golden case `name`, keyed as in its .npz, as torch tensors."""
+    out = {}
+    if name == "glue_dot_c128":
+        B, C, V, h, w = 2, 128, 3, 6, 6
+        for tag, s in (("g", GLUE_SEED), ("l", GLUE_SEED + 100)):
+            out.update({f"param_{tag}:{k}": v for k, v in O.init_params(C, seed=s, randomize_affine=True).items()})
+        gen = torch.Generator().manual_seed(GLUE_SEED + 2)
+        for key, c in (("f4", C), ("cls", 5), ("ctr", 1), ("d_out", C)):
+            out.update({f"{key}:{v}": torch.randn(B, c, h, w, generator=gen) for v in range(V)})
+        return out
+    B, C, T, H, W, mode, training, bn_layer = CASES[name]
+    seed = 100 + list(CASES).index(name)
     params = O.init_params(C, seed=seed, randomize_affine=True, bn_layer=bn_layer)
     if bn_layer and not training:
         # eval mode reads running stats: make them non-trivial
         g = torch.Generator().manual_seed(seed + 1)
         params["W_z.1.running_mean"] = torch.randn(C, generator=g) * 0.1
         params["W_z.1.running_var"] = torch.rand(C, generator=g) * 0.5 + 0.5
+    out.update({"param:" + k: v for k, v in params.items()})
+    g = torch.Generator().manual_seed(seed + 2)
+    out["x"] = torch.randn(B, C, T, H, W, generator=g)
+    out["dz"] = torch.randn(B, C, T, H, W, generator=g)
+    return out
+
+
+def run_case(TPAVIModule, name, B, C, T, H, W, mode, training, bn_layer, seed):
+    torch.manual_seed(seed)
+    inp = seeded_inputs(name)
+    params = {k[len("param:"):]: v for k, v in inp.items() if k.startswith("param:")}
     m = make_module(TPAVIModule, C, mode, bn_layer, params)
     m.train(training)
-    g = torch.Generator().manual_seed(seed + 2)
-    x = torch.randn(B, C, T, H, W, generator=g)
-    dz = torch.randn(B, C, T, H, W, generator=g)
+    x, dz = inp["x"], inp["dz"]
     x.requires_grad_(True)
     z, audio_temp = m(x)
     assert audio_temp == 0
@@ -86,19 +114,18 @@ def run_case(TPAVIModule, name, B, C, T, H, W, mode, training, bn_layer, seed):
     return out
 
 
-def run_glue_case(TPAVIModule, seed=7):
+def run_glue_case(TPAVIModule):
     """ours.py:1802-1834 restated literally around two reference TPAVIModule instances."""
     from torch import nn
     B, C, V, h, w = 2, 128, 3, 6, 6
-    pg = O.init_params(C, seed=seed, randomize_affine=True)
-    pl = O.init_params(C, seed=seed + 100, randomize_affine=True)
+    inp = seeded_inputs("glue_dot_c128")
+    pg = {k[len("param_g:"):]: v for k, v in inp.items() if k.startswith("param_g:")}
+    pl = {k[len("param_l:"):]: v for k, v in inp.items() if k.startswith("param_l:")}
     global_attn = make_module(TPAVIModule, C, "dot", True, pg)
     local_attn = make_module(TPAVIModule, C, "dot", True, pl)
-    gen = torch.Generator().manual_seed(seed + 2)
-    f4 = [torch.randn(B, C, h, w, generator=gen, requires_grad=True) for _ in range(V)]
-    cls_l = [torch.randn(B, 5, h, w, generator=gen, requires_grad=True) for _ in range(V)]
-    ctr_l = [torch.randn(B, 1, h, w, generator=gen, requires_grad=True) for _ in range(V)]
-    d_out = [torch.randn(B, C, h, w, generator=gen) for _ in range(V)]
+    f4, cls_l, ctr_l, d_out = ([inp[f"{key}:{v}"] for v in range(V)] for key in ("f4", "cls", "ctr", "d_out"))
+    for t in f4 + cls_l + ctr_l:
+        t.requires_grad_(True)
     center_aware_weight = 20
     mask_bb, ctr, f4_local = [], [], []
     for v in range(V):
@@ -137,17 +164,29 @@ def run_glue_case(TPAVIModule, seed=7):
     return out
 
 
+def run_init_case(TPAVIModule, C=96, seed=1234):
+    """The constructor's state dict under torch.manual_seed(seed): the weights its initialisers draw from the global RNG."""
+    torch.manual_seed(seed)
+    return {k: v.numpy() for k, v in TPAVIModule(in_channels=C, mode="dot").state_dict().items()}
+
+
+def save(outdir, name, out):
+    if name in OUTPUTS_ONLY:
+        out = {k: v for k, v in out.items() if k not in seeded_inputs(name)}
+    np.savez_compressed(os.path.join(outdir, name + ".npz"), **out)
+
+
 def main():
     TPAVIModule = load_reference_module()
     outdir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(outdir, exist_ok=True)
     for i, (name, cfg) in enumerate(CASES.items()):
         out = run_case(TPAVIModule, name, *cfg, seed=100 + i)
-        np.savez_compressed(os.path.join(outdir, name + ".npz"), **out)
+        save(outdir, name, out)
         print(name, "z", out["z"].shape, "strides", out["z_strides"])
-    out = run_glue_case(TPAVIModule)
-    np.savez_compressed(os.path.join(outdir, "glue_dot_c128.npz"), **out)
-    print("glue_dot_c128 done")
+    save(outdir, "glue_dot_c128", run_glue_case(TPAVIModule))
+    save(outdir, "init_dot_c96", run_init_case(TPAVIModule))
+    print("glue_dot_c128, init_dot_c96 done")
 
 
 if __name__ == "__main__":

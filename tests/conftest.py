@@ -27,8 +27,9 @@ def pytest_collection_modifyitems(config, items):
 def load_golden(name):
     import numpy as np
     import torch
+    from oracle import gen_golden
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
-    out = {}
+    out = gen_golden.seeded_inputs(name) if name in gen_golden.OUTPUTS_ONLY else {}
     for k in z.files:
         a = z[k]
         out[k] = torch.from_numpy(a) if a.dtype.kind in "fi" and a.ndim > 0 else a

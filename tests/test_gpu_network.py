@@ -64,7 +64,7 @@ def _rel(a, b):
 def test_install_full_network_cfg1_step():
     ours = build_ref.import_reference_network()
     if ours is None:
-        pytest.skip("oracle/_ref was not staged (build() found no /root/reference)")
+        pytest.skip("oracle/_ref was not staged (build() found no upstream GL-Fusion sources)")
     ref = _build(ours, patched=False)
     gen = torch.Generator().manual_seed(3)
     with torch.no_grad():                        # SURVEY F3: BN gamma / beta of the fusion blocks are 0 at init

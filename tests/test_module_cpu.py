@@ -1,16 +1,13 @@
 """Host-side mirror of the reference interface: constructor, state_dict, init, error behaviour (no GPU needed)."""
 import os
-import sys
 
 import pytest
 import torch
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 
 import glfusion_b200
 from glfusion_b200 import GlfError, GlobalLocalFusion, TPAVIModule
-
-REF = "/root/reference/GLfusion"
 
 
 def test_state_dict_keys_shapes_match_reference_contract():
@@ -92,21 +89,26 @@ def test_reference_network_checkpoint_slice_loads():
         GlobalLocalFusion(64).load_reference_checkpoint({"network": broken})
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="live reference only in the build container")
 def test_init_rng_stream_identical_to_reference():
-    sys.path.insert(0, REF)
-    from models.TPAVI import TPAVIModule as RefModule
-    torch.manual_seed(1234)
-    ours = TPAVIModule(in_channels=96, mode='dot')
-    torch.manual_seed(1234)
-    ref = RefModule(in_channels=96, mode='dot')
-    sr, so = ref.state_dict(), ours.state_dict()
-    assert list(sr.keys()) == list(so.keys())
-    for k in sr:
-        assert torch.equal(sr[k], so[k]), k
+    """Under torch.manual_seed the constructor draws the same weights as the reference's (the same nn holders created
+    in the same order): the state dict must equal tests/golden/init_dot_c96.npz (oracle/gen_golden.py::run_init_case)
+    bit for bit, and, when the reference module is staged in oracle/_ref, the reference's own state dict."""
+    import numpy as np
+    from oracle import build_ref
+    from oracle import gen_golden as G
+    golden = np.load(os.path.join(GOLDEN, "init_dot_c96.npz"))
+    so = G.run_init_case(TPAVIModule)
+    assert list(so) == golden.files
+    for k in so:
+        assert so[k].dtype == golden[k].dtype and np.array_equal(so[k], golden[k]), k
+    Ref = build_ref.load_reference_tpavi()
+    if Ref is not None:
+        sr = G.run_init_case(Ref)
+        assert list(sr) == list(so)
+        for k in sr:
+            assert np.array_equal(sr[k], so[k]), k
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="live reference only in the build container")
 def test_install_patches_reference_namespace():
     import types
     fake = types.SimpleNamespace(TPAVIModule=None)

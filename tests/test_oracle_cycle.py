@@ -1,6 +1,6 @@
 """The cycle-consistency oracle (oracle/cycle_oracle.py) against golden vectors produced by the reference's own
 Trainer.seg_cycle / Trainer.dense_seg_cycle (R/main.py:650-798, oracle/gen_golden_cycle.py), and against the live
-reference methods when /root/reference is present.  CPU only."""
+reference methods when they are staged in oracle/_ref.  CPU only."""
 import glob
 import os
 
@@ -24,12 +24,15 @@ def test_golden_fixtures_exist():
     assert len(GOLDEN) == 5
 
 
-@pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
-def test_oracle_matches_reference_golden(path):
-    d = np.load(path)
+def check_oracle(d):
     loss, g = run_oracle(d)
     assert abs(loss - float(d["loss"])) <= 2e-6 * abs(float(d["loss"]))           # the reference ran in fp32
     assert np.abs(g - d["dfeat"]).max() <= 5e-5 * np.abs(d["dfeat"]).max()
+
+
+@pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
+def test_oracle_matches_reference_golden(path):
+    check_oracle(np.load(path))
 
 
 @pytest.mark.parametrize("path", GOLDEN[:2] + GOLDEN[-1:], ids=lambda p: os.path.basename(p)[:-4])
@@ -58,13 +61,19 @@ def test_rejects_too_few_frames():
         CO.seg_cycle(np.zeros((18, 8)), 16, 2, 3, 10.0, 0)          # key region shorter than chunk + offset
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/GLfusion/main.py"), reason="reference tree not present")
 def test_oracle_matches_live_reference_methods():
+    """The oracle against the reference's Trainer.seg_cycle / dense_seg_cycle: on the runs they recorded
+    (tests/golden/cycle_*.npz) and, when the reference's main.py is staged in oracle/_ref, on live runs of them."""
     import types
 
     import torch
+    from oracle import build_ref
     from oracle import gen_golden_cycle as G
-    seg_cycle, dense_seg_cycle = G.load_reference_methods()
+    for path in GOLDEN:
+        check_oracle(np.load(path))
+    if not os.path.exists(build_ref.REF_MAIN):
+        return
+    seg_cycle, dense_seg_cycle = G.load_reference_methods(build_ref.REF_MAIN)
     me = types.SimpleNamespace(device=torch.device("cpu"))
     feat = G.features(34, 48, seed=21)
     for kw in ({"soft_label": False, "is_overlap": True}, {"soft_label": True, "is_overlap": False}):
