@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libglf_sm100a.so")
 
 MODE_DOT, MODE_EMBEDDED = 0, 1
-DTYPE_BF16, DTYPE_F32 = 0, 1
+DTYPE_BF16, DTYPE_F32, DTYPE_F16 = 0, 1, 2
 LAYOUT_NCTHW, LAYOUT_TOKEN = 0, 1
 PRECISION_BF16, PRECISION_F32X3 = 0, 1
 PRECISIONS = {"bf16": PRECISION_BF16, "fp32": PRECISION_F32X3}

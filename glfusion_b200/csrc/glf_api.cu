@@ -85,7 +85,13 @@ int make_dims(const glf_desc* d, Dims* o) {
     return set_error(GLF_ERR_INVALID, "bad precision (GLF_PRECISION_BF16 or GLF_PRECISION_F32X3)");
   if (d->precision == GLF_PRECISION_F32X3 && d->mode != GLF_MODE_DOT)
     return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 is implemented for mode='dot' only");
-  if (d->io_dtype != GLF_DTYPE_BF16 && d->io_dtype != GLF_DTYPE_F32) return set_error(GLF_ERR_INVALID, "bad io_dtype");
+  if (d->io_dtype != GLF_DTYPE_BF16 && d->io_dtype != GLF_DTYPE_F32 && d->io_dtype != GLF_DTYPE_F16)
+    return set_error(GLF_ERR_INVALID, "bad io_dtype (GLF_DTYPE_BF16, GLF_DTYPE_F32 or GLF_DTYPE_F16)");
+  // the exact arm is an fp32 contract: fp16 inputs (11-bit significands, 65504 range) would defeat it
+  if (d->precision == GLF_PRECISION_F32X3 && d->io_dtype == GLF_DTYPE_F16)
+    return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 takes fp32 or bf16 activations, not fp16 (GLF_DTYPE_F16)");
+  if (d->reserved[2] != GLF_DTYPE_BF16 && d->reserved[2] != GLF_DTYPE_F16)
+    return set_error(GLF_ERR_INVALID, "reserved[2] (dtype of the fused LayerNorm's z / dz) must be GLF_DTYPE_BF16 or GLF_DTYPE_F16");
   o->B = d->B;
   o->N = static_cast<long long>(d->T) * d->H * d->W;
   o->rows = o->B * o->N;
@@ -96,9 +102,9 @@ int make_dims(const glf_desc* d, Dims* o) {
   o->tiles_seq = gemm_tiles_m(static_cast<int>(o->N));
   o->tiles_all = gemm_tiles_m(static_cast<int>(o->rows > 0x7fffffff ? 0x7fffffff : o->rows));
   if (o->rows > 0x7fffff00LL) return set_error(GLF_ERR_INVALID, "too many tokens");
-  o->pack_x = !(d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_BF16);
-  if (d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_F32 && o->rows * d->C > 0x7fffffffLL)
-    return set_error(GLF_ERR_INVALID, "token-major fp32 input too large for the cast kernel");
+  o->pack_x = !(d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_BF16);   // fp32 / fp16: a bf16 copy
+  if (d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype != GLF_DTYPE_BF16 && o->rows * d->C > 0x7fffffffLL)
+    return set_error(GLF_ERR_INVALID, "token-major fp32 / fp16 input too large for the cast kernel");
   o->pack_dz = d->dz_layout != GLF_LAYOUT_TOKEN;
   o->dot = d->mode == GLF_MODE_DOT;
   // reserved[1]: 0 = choose, 1 = token-space form (theta/phi/g per token), 2 = Gram form
@@ -309,10 +315,12 @@ GemmOperand opnd(const void* p, int mn, long long ld, long long bs) {
 // reserved[0] = 1: the LayerNorm stage (forward epilogue / first backward kernel) is run for MGFM and MLFM together
 // by glf_fusion_ln_fwd / glf_fusion_ln_bwd instead of per block
 bool defer_ln(const glf_desc* d) { return d->reserved[0] == 1; }
+// reserved[2]: dtype of z / z_global / dz of the fused LayerNorm pass (make_dims admits GLF_DTYPE_BF16 = 0 or F16)
+int pair_z_dtype(const glf_desc* d) { return d->reserved[2]; }
 
 int check_pair(const glf_desc* d, const Dims& m) {
   if (d->precision != GLF_PRECISION_BF16 || d->io_dtype != GLF_DTYPE_BF16 || m.pack_x || d->dz_layout != GLF_LAYOUT_TOKEN)
-    return set_error(GLF_ERR_UNSUPPORTED, "fused LayerNorm pair needs bf16 token-major activations");
+    return set_error(GLF_ERR_UNSUPPORTED, "fused LayerNorm pair needs bf16 token-major x_g / x_l and token-major dz");
   if (!ln_tma_supported(m.C) && !ln_pair_wide_supported(m.C))
     return set_error(GLF_ERR_UNSUPPORTED, "fused LayerNorm pair needs C %% 8 == 0 and C <= 2048");
   return 0;
@@ -1028,10 +1036,10 @@ GLF_API int glf_fusion_ln_fwd_parts(const glf_desc* d, const void* xg, const voi
   float* mu[2] = {sg.ln_mu, sl.ln_mu};
   float* r[2] = {sg.ln_r, sl.ln_r};
   if (!ln_tma_supported(m.C))     // wide rows (256 < C <= 2048): the sliced-row ring kernel, both blocks in one pass
-    return ln_pair_fwd_wide(U, X, a, b, lw, lb, mu, r, reinterpret_cast<bf16*>(z), m.rows, m.C, d->eps_ln, d->accumulate,
-                            stream, reinterpret_cast<bf16*>(z_global));
-  return ln_fwd_tma(2, U, X, a, b, lw, lb, mu, r, reinterpret_cast<bf16*>(z), m.rows, m.C, d->eps_ln, d->accumulate,
-                    stream, reinterpret_cast<bf16*>(z_global));
+    return ln_pair_fwd_wide(U, X, a, b, lw, lb, mu, r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream, z_global,
+                            pair_z_dtype(d));
+  return ln_fwd_tma(2, U, X, a, b, lw, lb, mu, r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream, z_global,
+                    pair_z_dtype(d));
 }
 
 GLF_API int glf_fusion_ln_bwd(const glf_desc* d, const void* dz, const void* xg, const void* xl, const glf_weights* wg,
@@ -1089,12 +1097,12 @@ GLF_API int glf_fusion_ln_bwd_views(const glf_desc* d, const void* dz, const voi
     // the two blocks run the sliced-row ring kernel one after the other
     if (views) return set_error(GLF_ERR_UNSUPPORTED, "per-view dz needs C <= 256");
     for (int k = 0; k < 2; ++k)
-      GLF_TRY(bn_res_ln_bwd(dz, GLF_DTYPE_BF16, U[k], X[k], GLF_DTYPE_BF16, a[k], b[k], mean[k], rstd[k], lw[k], mu[k], r[k],
-                            dV[k], part[k], m.rows, m.C, &nb, stream));
+      GLF_TRY(bn_res_ln_bwd(dz, pair_z_dtype(d), U[k], X[k], GLF_DTYPE_BF16, a[k], b[k], mean[k], rstd[k], lw[k], mu[k],
+                            r[k], dV[k], part[k], m.rows, m.C, &nb, stream));
     return 0;
   }
-  return ln_bwd_tma(2, reinterpret_cast<const bf16*>(dz), U, X, a, b, lw, mean, rstd, mu, r, dV, part, m.rows, m.C, &nb,
-                    stream, views ? d->T : 0, dz_views, reinterpret_cast<const long long*>(dz_stride_b), d->H * d->W);
+  return ln_bwd_tma(2, dz, U, X, a, b, lw, mean, rstd, mu, r, dV, part, m.rows, m.C, &nb, stream, views ? d->T : 0,
+                    dz_views, reinterpret_cast<const long long*>(dz_stride_b), d->H * d->W, pair_z_dtype(d));
 }
 
 GLF_API int glf_gate_concat_fwd(int B, int C, int V, int h, int w, int ncls, float weight, int io_dtype, int x_dtype,

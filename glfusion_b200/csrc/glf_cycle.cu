@@ -10,6 +10,7 @@
 //   sim_i = -a sum_j |K[i+j] - feat[s+j]|^2,  beta = softmax(sim),  w_j = sum_i beta_i K[off+i+j],
 //   z_m = -a sum_j |feat[off+m+j] - w_j|^2,   loss_s = mean_m BCEWithLogits(z_m, y_m)
 #include <cstdint>
+#include <type_traits>
 
 #include "glf_internal.h"
 
@@ -224,16 +225,22 @@ template <typename TIn>
 __device__ __forceinline__ float cy_ld(const TIn* p);
 template <> __device__ __forceinline__ float cy_ld<float>(const float* p) { return *p; }
 template <> __device__ __forceinline__ float cy_ld<bf16>(const bf16* p) { return __bfloat162float(*p); }
+template <> __device__ __forceinline__ float cy_ld<f16>(const f16* p) { return __half2float(*p); }
 
 template <typename TIn, int VEC>
 __device__ __forceinline__ void cy_ld_vec(const TIn* p, float (&f)[VEC]) {
   if constexpr (VEC == 1) {
     f[0] = cy_ld<TIn>(p);
-  } else if constexpr (sizeof(TIn) == 2) {                   // 8 bf16 = 16 bytes
+  } else if constexpr (sizeof(TIn) == 2) {                   // 8 bf16 / fp16 = 16 bytes
     const uint4 q = *reinterpret_cast<const uint4*>(p);
-    const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&q);
+    const uint32_t* u = reinterpret_cast<const uint32_t*>(&q);
 #pragma unroll
-    for (int j = 0; j < 4; ++j) { const float2 t = __bfloat1622float2(h2[j]); f[2 * j] = t.x; f[2 * j + 1] = t.y; }
+    for (int j = 0; j < 4; ++j) {
+      float2 t;
+      if constexpr (std::is_same<TIn, bf16>::value) t = __bfloat1622float2(reinterpret_cast<const __nv_bfloat162*>(u)[j]);
+      else t = __half22float2(reinterpret_cast<const __half2*>(u)[j]);
+      f[2 * j] = t.x; f[2 * j + 1] = t.y;
+    }
   } else {                                                   // 4 fp32 = 16 bytes
     const float4 q = *reinterpret_cast<const float4*>(p);
     f[0] = q.x; f[1] = q.y; f[2] = q.z; f[3] = q.w;
@@ -334,14 +341,18 @@ int cycle_loss(const float* feat, int T, int C, int R, int off, int ch, float te
 int spatial_sums(const void* x, int dtype, int B, int C, int T, long long sb, long long sc, long long st, float* out,
                  cudaStream_t stream) {
   if (B <= 0 || C <= 0 || T <= 0) return set_error(GLF_ERR_INVALID, "spatial_sums: empty input");
-  if (dtype != GLF_DTYPE_BF16 && dtype != GLF_DTYPE_F32) return set_error(GLF_ERR_INVALID, "spatial_sums: bad dtype");
+  if (dtype != GLF_DTYPE_BF16 && dtype != GLF_DTYPE_F16 && dtype != GLF_DTYPE_F32)
+    return set_error(GLF_ERR_INVALID, "spatial_sums: bad dtype");
   if (sc == 1 && B <= 65535) {
-    const int per16 = dtype == GLF_DTYPE_BF16 ? 8 : 4;
+    const int per16 = dtype == GLF_DTYPE_F32 ? 4 : 8;
     const bool vec = C % per16 == 0 && sb % per16 == 0 && st % per16 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0;
     const dim3 grid((C + 32 * (vec ? per16 : 1) - 1) / (32 * (vec ? per16 : 1)), B);
     if (dtype == GLF_DTYPE_BF16) {
       if (vec) spatial_sums_cl_kernel<bf16, 8><<<grid, 256, 0, stream>>>(reinterpret_cast<const bf16*>(x), sb, st, C, T, out);
       else spatial_sums_cl_kernel<bf16, 1><<<grid, 256, 0, stream>>>(reinterpret_cast<const bf16*>(x), sb, st, C, T, out);
+    } else if (dtype == GLF_DTYPE_F16) {
+      if (vec) spatial_sums_cl_kernel<f16, 8><<<grid, 256, 0, stream>>>(reinterpret_cast<const f16*>(x), sb, st, C, T, out);
+      else spatial_sums_cl_kernel<f16, 1><<<grid, 256, 0, stream>>>(reinterpret_cast<const f16*>(x), sb, st, C, T, out);
     } else {
       if (vec) spatial_sums_cl_kernel<float, 4><<<grid, 256, 0, stream>>>(reinterpret_cast<const float*>(x), sb, st, C, T, out);
       else spatial_sums_cl_kernel<float, 1><<<grid, 256, 0, stream>>>(reinterpret_cast<const float*>(x), sb, st, C, T, out);
@@ -351,6 +362,8 @@ int spatial_sums(const void* x, int dtype, int B, int C, int T, long long sb, lo
     const int grid = static_cast<int>((rows + 7) / 8);
     if (dtype == GLF_DTYPE_BF16)
       spatial_sums_any_kernel<bf16><<<grid, 256, 0, stream>>>(reinterpret_cast<const bf16*>(x), sb, sc, st, C, T, rows, out);
+    else if (dtype == GLF_DTYPE_F16)
+      spatial_sums_any_kernel<f16><<<grid, 256, 0, stream>>>(reinterpret_cast<const f16*>(x), sb, sc, st, C, T, rows, out);
     else
       spatial_sums_any_kernel<float><<<grid, 256, 0, stream>>>(reinterpret_cast<const float*>(x), sb, sc, st, C, T, rows, out);
   }

@@ -26,6 +26,16 @@ __device__ __forceinline__ void load8(const bf16* p, float (&f)[8]) {
     f[2 * i + 1] = t.y;
   }
 }
+__device__ __forceinline__ void load8(const f16* p, float (&f)[8]) {
+  const uint4 v = *reinterpret_cast<const uint4*>(p);
+  const uint32_t* u = reinterpret_cast<const uint32_t*>(&v);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 t = unpack2<f16>(u[i]);
+    f[2 * i] = t.x;
+    f[2 * i + 1] = t.y;
+  }
+}
 __device__ __forceinline__ void load8(const float* p, float (&f)[8]) {
   const float4 a = *reinterpret_cast<const float4*>(p);
   const float4 b = *reinterpret_cast<const float4*>(p + 4);
@@ -34,6 +44,10 @@ __device__ __forceinline__ void load8(const float* p, float (&f)[8]) {
 }
 __device__ __forceinline__ void store8(bf16* p, const float (&f)[8]) {
   uint4 v = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+  *reinterpret_cast<uint4*>(p) = v;
+}
+__device__ __forceinline__ void store8(f16* p, const float (&f)[8]) {
+  uint4 v = make_uint4(pack2<f16>(f[0], f[1]), pack2<f16>(f[2], f[3]), pack2<f16>(f[4], f[5]), pack2<f16>(f[6], f[7]));
   *reinterpret_cast<uint4*>(p) = v;
 }
 __device__ __forceinline__ void store8(float* p, const float (&f)[8]) {
@@ -249,9 +263,15 @@ __global__ void __launch_bounds__(32 * RED_Y)
 // the bytes in flight per warp (the kernels are latency-bound on HBM otherwise: ~45 % of peak measured without it).
 template <typename T> struct Raw8;
 template <> struct Raw8<bf16> { uint4 v; };
+template <> struct Raw8<f16> { uint4 v; };
 template <> struct Raw8<float> { float4 a, b; };
 __device__ __forceinline__ Raw8<bf16> ldraw(const bf16* p) {
   Raw8<bf16> r;
+  r.v = *reinterpret_cast<const uint4*>(p);
+  return r;
+}
+__device__ __forceinline__ Raw8<f16> ldraw(const f16* p) {
+  Raw8<f16> r;
   r.v = *reinterpret_cast<const uint4*>(p);
   return r;
 }
@@ -266,6 +286,15 @@ __device__ __forceinline__ void cvt8(const Raw8<bf16>& r, float (&f)[8]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const float2 t = unpack_bf16(u[i]);
+    f[2 * i] = t.x;
+    f[2 * i + 1] = t.y;
+  }
+}
+__device__ __forceinline__ void cvt8(const Raw8<f16>& r, float (&f)[8]) {
+  const uint32_t* u = reinterpret_cast<const uint32_t*>(&r.v);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 t = unpack2<f16>(u[i]);
     f[2 * i] = t.x;
     f[2 * i + 1] = t.y;
   }
@@ -515,11 +544,12 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// ring layout: [LN_DEPTH][nops][ROW_THREADS] uint4
+// ring layout: [LN_DEPTH][nops][ROW_THREADS] uint4.  TZ: bf16 or fp16 Z (same bytes per row).
+template <typename TZ>
 __global__ void __launch_bounds__(ROW_THREADS)
     bn_res_ln_fwd_ring_kernel(const bf16* __restrict__ U, const bf16* __restrict__ X, const float* __restrict__ bn_a,
                               const float* __restrict__ bn_b, const float* __restrict__ lw, const float* __restrict__ lb,
-                              bf16* __restrict__ Z, float* __restrict__ mu_o, float* __restrict__ r_o, long long rows, int C,
+                              TZ* __restrict__ Z, float* __restrict__ mu_o, float* __restrict__ r_o, long long rows, int C,
                               int S, float eps, int accumulate) {
   extern __shared__ __align__(16) uint4 ln_ring[];
   __shared__ float red[2 * ROW_WARPS * 2];
@@ -591,7 +621,7 @@ __global__ void __launch_bounds__(ROW_THREADS)
 #pragma unroll
       for (int i = 0; i < 8; ++i) o[i] = fmaf((v[i] - mu) * r, w[i], bb[i]);
       if (accumulate) {
-        Raw8<bf16> zc;
+        Raw8<TZ> zc;
         zc.v = src[2 * ROW_THREADS];
         float z0[8];
         cvt8(zc, z0);
@@ -620,14 +650,14 @@ struct LnPairWide {
   const float* lb[2];
   float* mu[2];
   float* r[2];
-  bf16* Z;
-  bf16* Z0;
+  void* Z;         // [rows, C] of the kernel's TZ (bf16 or fp16), like Z0
+  void* Z0;
   long long rows;
   int C, S, accumulate;
   float eps;
 };
 
-template <bool PARTS>
+template <bool PARTS, typename TZ>
 __global__ void __launch_bounds__(ROW_THREADS, 2) ln_pair_fwd_ring_kernel(const LnPairWide p) {
   extern __shared__ __align__(16) uint4 ln_ring[];
   __shared__ float red[2 * ROW_WARPS * 2];
@@ -665,7 +695,7 @@ __global__ void __launch_bounds__(ROW_THREADS, 2) ln_pair_fwd_ring_kernel(const 
       cp_async16(dst + ROW_THREADS, p.U[0] + off);
       cp_async16(dst + 2 * ROW_THREADS, p.X[1] + off);
       cp_async16(dst + 3 * ROW_THREADS, p.U[1] + off);
-      if (p.accumulate) cp_async16(dst + 4 * ROW_THREADS, p.Z + off);
+      if (p.accumulate) cp_async16(dst + 4 * ROW_THREADS, reinterpret_cast<const TZ*>(p.Z) + off);
     }
     cp_async_commit();
   };
@@ -718,20 +748,20 @@ __global__ void __launch_bounds__(ROW_THREADS, 2) ln_pair_fwd_ring_kernel(const 
           o0[i] = fmaf((v0[i] - mu0) * r0, w0[i], lbs[i]);
           o[i] = o0[i] + fmaf((v1[i] - mu1) * r1, w1[i], lb1[i]);
         }
-        store8(p.Z0 + row * C + c0, o0);
+        store8(reinterpret_cast<TZ*>(p.Z0) + row * C + c0, o0);
       } else {
 #pragma unroll
         for (int i = 0; i < 8; ++i) o[i] = fmaf((v0[i] - mu0) * r0, w0[i], fmaf((v1[i] - mu1) * r1, w1[i], lbs[i]));
       }
       if (p.accumulate) {
-        Raw8<bf16> zc;
+        Raw8<TZ> zc;
         zc.v = src[4 * ROW_THREADS];
         float z0[8];
         cvt8(zc, z0);
 #pragma unroll
         for (int i = 0; i < 8; ++i) o[i] += z0[i];
       }
-      store8(p.Z + row * C + c0, o);
+      store8(reinterpret_cast<TZ*>(p.Z) + row * C + c0, o);
       if (slice == 0 && lane == 0) {
         if (p.mu[0] != nullptr) { p.mu[0][row] = mu0; p.r[0][row] = r0; }
         if (p.mu[1] != nullptr) { p.mu[1][row] = mu1; p.r[1][row] = r1; }
@@ -741,8 +771,9 @@ __global__ void __launch_bounds__(ROW_THREADS, 2) ln_pair_fwd_ring_kernel(const 
   cp_async_wait<0>();
 }
 
+template <typename TZ>
 __global__ void __launch_bounds__(ROW_THREADS, 2)
-    bn_res_ln_bwd_ring_kernel(const bf16* __restrict__ dZ, const bf16* __restrict__ U, const bf16* __restrict__ X,
+    bn_res_ln_bwd_ring_kernel(const TZ* __restrict__ dZ, const bf16* __restrict__ U, const bf16* __restrict__ X,
                               const float* __restrict__ bn_a, const float* __restrict__ bn_b,
                               const float* __restrict__ bn_mean, const float* __restrict__ bn_rstd,
                               const float* __restrict__ lw, const float* __restrict__ mu_i, const float* __restrict__ r_i,
@@ -802,7 +833,8 @@ __global__ void __launch_bounds__(ROW_THREADS, 2)
 #pragma unroll
     for (int i = 0; i < 8; ++i) xh[i] = dxh[i] = dz[i] = uh[i] = 0.f;
     if (act) {
-      Raw8<bf16> xc, zc;
+      Raw8<bf16> xc;
+      Raw8<TZ> zc;
       xc.v = src[0];
       zc.v = src[ROW_THREADS];
       float x[8];
@@ -1065,14 +1097,21 @@ int transpose_cast(const void* in, void* out, int batch, int R, int S, int in_dt
   if (batch <= 0 || R <= 0 || S <= 0) return set_error(GLF_ERR_INVALID, "transpose: empty");
   dim3 grid((S + 63) / 64, (R + 63) / 64, batch);
   if (grid.y > 65535 || grid.z > 65535) return set_error(GLF_ERR_INVALID, "transpose: grid too large");
-  if (in_dtype == GLF_DTYPE_F32 && out_dtype == GLF_DTYPE_BF16)
-    transpose_kernel<float, bf16><<<grid, 256, 0, stream>>>((const float*)in, (bf16*)out, R, S);
-  else if (in_dtype == GLF_DTYPE_BF16 && out_dtype == GLF_DTYPE_BF16)
-    transpose_kernel<bf16, bf16><<<grid, 256, 0, stream>>>((const bf16*)in, (bf16*)out, R, S);
-  else if (in_dtype == GLF_DTYPE_BF16 && out_dtype == GLF_DTYPE_F32)
-    transpose_kernel<bf16, float><<<grid, 256, 0, stream>>>((const bf16*)in, (float*)out, R, S);
-  else
-    transpose_kernel<float, float><<<grid, 256, 0, stream>>>((const float*)in, (float*)out, R, S);
+  auto valid = [](int t) { return t == GLF_DTYPE_BF16 || t == GLF_DTYPE_F32 || t == GLF_DTYPE_F16; };
+  if (!valid(in_dtype) || !valid(out_dtype)) return set_error(GLF_ERR_INVALID, "transpose: bad dtype");
+  auto launch = [&](auto tin) {
+    using TI = decltype(tin);
+    const TI* src = reinterpret_cast<const TI*>(in);
+    if (out_dtype == GLF_DTYPE_BF16)
+      transpose_kernel<TI, bf16><<<grid, 256, 0, stream>>>(src, reinterpret_cast<bf16*>(out), R, S);
+    else if (out_dtype == GLF_DTYPE_F16)
+      transpose_kernel<TI, f16><<<grid, 256, 0, stream>>>(src, reinterpret_cast<f16*>(out), R, S);
+    else
+      transpose_kernel<TI, float><<<grid, 256, 0, stream>>>(src, reinterpret_cast<float*>(out), R, S);
+  };
+  if (in_dtype == GLF_DTYPE_BF16) launch(bf16{});
+  else if (in_dtype == GLF_DTYPE_F16) launch(f16{});
+  else launch(float{});
   return check_cuda(cudaGetLastError(), "transpose launch");
 }
 
@@ -1120,26 +1159,36 @@ int bn_res_ln_fwd(const void* U_, const void* X_, int act_dtype, const float* a,
                   const float* lb, void* Z, int z_dtype, float* mu, float* r, long long rows, int C, float eps,
                   int accumulate, cudaStream_t stream) {
   if (C % 8 != 0 || C > 2048) return set_error(GLF_ERR_INVALID, "LayerNorm kernel needs C %% 8 == 0 and C <= 2048");
-  if (act_dtype == GLF_DTYPE_BF16 && z_dtype == GLF_DTYPE_BF16 && U_ != nullptr && ln_tma_supported(C) &&
+  if (z_dtype == GLF_DTYPE_F16 && act_dtype != GLF_DTYPE_BF16)
+    return set_error(GLF_ERR_INVALID, "LayerNorm kernel: an fp16 Z needs bf16 activations");
+  const bool z16 = z_dtype == GLF_DTYPE_BF16 || z_dtype == GLF_DTYPE_F16;    // bf16 or fp16 Z: the fast paths
+  if (act_dtype == GLF_DTYPE_BF16 && z16 && U_ != nullptr && ln_tma_supported(C) &&
       aligned16(U_, X_, Z, a, b, lw, lb) && !debug_reg_ln()) {
     const bf16* Ua[1] = {(const bf16*)U_};
     const bf16* Xa[1] = {(const bf16*)X_};
     const float *aa[1] = {a}, *ba[1] = {b}, *lwa[1] = {lw}, *lba[1] = {lb};
     float *mua[1] = {mu}, *ra[1] = {r};
-    return ln_fwd_tma(1, Ua, Xa, aa, ba, lwa, lba, mua, ra, (bf16*)Z, rows, C, eps, accumulate, stream);
+    return ln_fwd_tma(1, Ua, Xa, aa, ba, lwa, lba, mua, ra, Z, rows, C, eps, accumulate, stream, nullptr, z_dtype);
   }
   int S = (C + 255) / 256;
   while (ROW_WARPS % S != 0) ++S;
   const int grid = row_grid(rows, S);
   if (act_dtype == GLF_DTYPE_BF16) {
     const bf16* U = (const bf16*)U_; const bf16* X = (const bf16*)X_;
-    if (S > 1 && z_dtype == GLF_DTYPE_BF16 && aligned16(U_ != nullptr ? U_ : X_, X_, Z) && !debug_reg_ln()) {
+    if (S > 1 && z16 && aligned16(U_ != nullptr ? U_ : X_, X_, Z) && !debug_reg_ln()) {
       const size_t ring = LN_DEPTH * 3 * ROW_THREADS * sizeof(uint4);       // 48 KB
-      cudaError_t e = cudaFuncSetAttribute(bn_res_ln_fwd_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
+      const void* kern = z_dtype == GLF_DTYPE_F16 ? reinterpret_cast<const void*>(bn_res_ln_fwd_ring_kernel<f16>)
+                                                  : reinterpret_cast<const void*>(bn_res_ln_fwd_ring_kernel<bf16>);
+      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
       if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln fwd ring)");
-      bn_res_ln_fwd_ring_kernel<<<grid, ROW_THREADS, ring, stream>>>(U, X, a, b, lw, lb, (bf16*)Z, mu, r, rows, C, S, eps, accumulate);
+      if (z_dtype == GLF_DTYPE_F16)
+        bn_res_ln_fwd_ring_kernel<f16><<<grid, ROW_THREADS, ring, stream>>>(U, X, a, b, lw, lb, (f16*)Z, mu, r, rows, C, S, eps, accumulate);
+      else
+        bn_res_ln_fwd_ring_kernel<bf16><<<grid, ROW_THREADS, ring, stream>>>(U, X, a, b, lw, lb, (bf16*)Z, mu, r, rows, C, S, eps, accumulate);
     } else if (z_dtype == GLF_DTYPE_BF16)
       bn_res_ln_fwd_kernel<bf16, bf16><<<grid, ROW_THREADS, 0, stream>>>(U, X, a, b, lw, lb, (bf16*)Z, mu, r, rows, C, S, eps, accumulate);
+    else if (z_dtype == GLF_DTYPE_F16)
+      bn_res_ln_fwd_kernel<f16, bf16><<<grid, ROW_THREADS, 0, stream>>>(U, X, a, b, lw, lb, (f16*)Z, mu, r, rows, C, S, eps, accumulate);
     else
       bn_res_ln_fwd_kernel<float, bf16><<<grid, ROW_THREADS, 0, stream>>>(U, X, a, b, lw, lb, (float*)Z, mu, r, rows, C, S, eps, accumulate);
   } else {
@@ -1156,9 +1205,10 @@ int bn_res_ln_fwd(const void* U_, const void* X_, int act_dtype, const float* a,
 bool ln_pair_wide_supported(int C) { return C > 256 && C <= 2048 && C % 8 == 0; }
 
 int ln_pair_fwd_wide(const bf16* const* U, const bf16* const* X, const float* const* a, const float* const* b,
-                     const float* const* lw, const float* const* lb, float* const* mu, float* const* r, bf16* Z,
-                     long long rows, int C, float eps, int accumulate, cudaStream_t stream, bf16* Z0) {
+                     const float* const* lw, const float* const* lb, float* const* mu, float* const* r, void* Z,
+                     long long rows, int C, float eps, int accumulate, cudaStream_t stream, void* Z0, int z_dtype) {
   if (!ln_pair_wide_supported(C)) return set_error(GLF_ERR_UNSUPPORTED, "ln_pair_fwd_wide: 256 < C <= 2048 expected");
+  if (z_dtype != GLF_DTYPE_BF16 && z_dtype != GLF_DTYPE_F16) return set_error(GLF_ERR_INVALID, "ln_pair_fwd_wide: Z must be bf16 or fp16");
   if (Z0 != nullptr && accumulate) return set_error(GLF_ERR_INVALID, "ln_pair_fwd_wide: parts with accumulate");
   int S = (C + 255) / 256;
   while (ROW_WARPS % S != 0) ++S;
@@ -1172,15 +1222,13 @@ int ln_pair_fwd_wide(const bf16* const* U, const bf16* const* X, const float* co
   p.Z = Z; p.Z0 = Z0; p.rows = rows; p.C = C; p.S = S; p.accumulate = accumulate; p.eps = eps;
   const int grid = row_grid(rows, S);
   const size_t ring = LN_DEPTH * 5 * ROW_THREADS * sizeof(uint4);       // 80 KB
-  if (Z0 != nullptr) {
-    cudaError_t e = cudaFuncSetAttribute(ln_pair_fwd_ring_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
-    if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln pair wide)");
-    ln_pair_fwd_ring_kernel<true><<<grid, ROW_THREADS, ring, stream>>>(p);
-  } else {
-    cudaError_t e = cudaFuncSetAttribute(ln_pair_fwd_ring_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
-    if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln pair wide)");
-    ln_pair_fwd_ring_kernel<false><<<grid, ROW_THREADS, ring, stream>>>(p);
-  }
+  const bool h = z_dtype == GLF_DTYPE_F16;
+  void (*kern)(const LnPairWide) =
+      Z0 != nullptr ? (h ? ln_pair_fwd_ring_kernel<true, f16> : ln_pair_fwd_ring_kernel<true, bf16>)
+                    : (h ? ln_pair_fwd_ring_kernel<false, f16> : ln_pair_fwd_ring_kernel<false, bf16>);
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
+  if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln pair wide)");
+  kern<<<grid, ROW_THREADS, ring, stream>>>(p);
   return check_cuda(cudaGetLastError(), "ln_pair_fwd_wide launch");
 }
 
@@ -1195,7 +1243,10 @@ int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U_, const void* X_, 
                   const float* b, const float* mean, const float* rstd, const float* lw, const float* mu,
                   const float* r, void* dV_, float* part, long long rows, int C, int* nblocks, cudaStream_t stream) {
   if (C % 8 != 0 || C > 2048) return set_error(GLF_ERR_INVALID, "LayerNorm kernel needs C %% 8 == 0 and C <= 2048");
-  if (act_dtype == GLF_DTYPE_BF16 && dz_dtype == GLF_DTYPE_BF16 && U_ != nullptr && ln_tma_supported(C) &&
+  if (dz_dtype == GLF_DTYPE_F16 && act_dtype != GLF_DTYPE_BF16)
+    return set_error(GLF_ERR_INVALID, "LayerNorm backward: an fp16 dZ needs bf16 activations");
+  const bool dz16 = dz_dtype == GLF_DTYPE_BF16 || dz_dtype == GLF_DTYPE_F16;  // bf16 or fp16 dZ: the fast paths
+  if (act_dtype == GLF_DTYPE_BF16 && dz16 && U_ != nullptr && ln_tma_supported(C) &&
       aligned16(dZ, U_, X_, dV_, a, b, lw, mu, r) && !debug_reg_ln()) {
     const bf16* Ua[1] = {(const bf16*)U_};
     const bf16* Xa[1] = {(const bf16*)X_};
@@ -1203,7 +1254,8 @@ int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U_, const void* X_, 
                 *ra[1] = {r};
     bf16* dVa[1] = {(bf16*)dV_};
     float* pa[1] = {part};
-    return ln_bwd_tma(1, (const bf16*)dZ, Ua, Xa, aa, ba, lwa, mna, rsa, mua, ra, dVa, pa, rows, C, nblocks, stream);
+    return ln_bwd_tma(1, dZ, Ua, Xa, aa, ba, lwa, mna, rsa, mua, ra, dVa, pa, rows, C, nblocks, stream, 0, nullptr, nullptr,
+                      0, dz_dtype);
   }
   int S = (C + 255) / 256;
   while (ROW_WARPS % S != 0) ++S;
@@ -1211,13 +1263,20 @@ int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U_, const void* X_, 
   if (nblocks) *nblocks = grid;
   if (act_dtype == GLF_DTYPE_BF16) {
     const bf16* U = (const bf16*)U_; const bf16* X = (const bf16*)X_; bf16* dV = (bf16*)dV_;
-    if (S > 1 && dz_dtype == GLF_DTYPE_BF16 && aligned16(U_ != nullptr ? U_ : X_, X_, dZ, dV_) && !debug_reg_ln()) {
+    if (S > 1 && dz16 && aligned16(U_ != nullptr ? U_ : X_, X_, dZ, dV_) && !debug_reg_ln()) {
       const size_t ring = LN_DEPTH * 3 * ROW_THREADS * sizeof(uint4);
-      cudaError_t e = cudaFuncSetAttribute(bn_res_ln_bwd_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
+      const void* kern = dz_dtype == GLF_DTYPE_F16 ? reinterpret_cast<const void*>(bn_res_ln_bwd_ring_kernel<f16>)
+                                                   : reinterpret_cast<const void*>(bn_res_ln_bwd_ring_kernel<bf16>);
+      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ring));
       if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln bwd ring)");
-      bn_res_ln_bwd_ring_kernel<<<grid, ROW_THREADS, ring, stream>>>((const bf16*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
+      if (dz_dtype == GLF_DTYPE_F16)
+        bn_res_ln_bwd_ring_kernel<f16><<<grid, ROW_THREADS, ring, stream>>>((const f16*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
+      else
+        bn_res_ln_bwd_ring_kernel<bf16><<<grid, ROW_THREADS, ring, stream>>>((const bf16*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
     } else if (dz_dtype == GLF_DTYPE_BF16)
       bn_res_ln_bwd_kernel<bf16, bf16><<<grid, ROW_THREADS, 0, stream>>>((const bf16*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
+    else if (dz_dtype == GLF_DTYPE_F16)
+      bn_res_ln_bwd_kernel<f16, bf16><<<grid, ROW_THREADS, 0, stream>>>((const f16*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
     else
       bn_res_ln_bwd_kernel<float, bf16><<<grid, ROW_THREADS, 0, stream>>>((const float*)dZ, U, X, a, b, mean, rstd, lw, mu, r, dV, part, rows, C, S);
   } else {

@@ -5,7 +5,10 @@
 // transposes it through shared memory and writes both token-major [B, V*h*w, C] operands with 128-bit stores.
 // The backward is the mirror pass: df4 = dXg + a * dXl (back to NCHW) plus the gate gradient da = sum_c f4 * dXl
 // chained through the two sigmoids / the class max to the logits.
+// f4 / df4 may be bf16, fp16 or fp32; the token-major operands are bf16 (fp32 for the F32X3 arm).  fp16 f4 is converted
+// where it is read and df4 rounded to fp16 where it is written: the fp16 forms move the same bytes as the bf16 ones.
 #include <cstdlib>
+#include <type_traits>
 
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
@@ -33,16 +36,25 @@ __device__ __forceinline__ void ld2(const bf16* p, float& a, float& b) {
   const float2 t = unpack_bf16(*reinterpret_cast<const uint32_t*>(p));
   a = t.x; b = t.y;
 }
+__device__ __forceinline__ void ld2(const f16* p, float& a, float& b) {
+  const float2 t = unpack2<f16>(*reinterpret_cast<const uint32_t*>(p));
+  a = t.x; b = t.y;
+}
 __device__ __forceinline__ void ld2(const float* p, float& a, float& b) {
   const float2 t = *reinterpret_cast<const float2*>(p);
   a = t.x; b = t.y;
 }
 __device__ __forceinline__ void st2(bf16* p, float a, float b) { *reinterpret_cast<uint32_t*>(p) = pack_bf16(a, b); }
+__device__ __forceinline__ void st2(f16* p, float a, float b) { *reinterpret_cast<uint32_t*>(p) = pack2<f16>(a, b); }
 __device__ __forceinline__ void st2(float* p, float a, float b) { *reinterpret_cast<float2*>(p) = make_float2(a, b); }
 // eight consecutive channels of one token (token-major side)
 __device__ __forceinline__ void st8(bf16* p, const float (&f)[8]) {
   *reinterpret_cast<uint4*>(p) =
       make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+}
+__device__ __forceinline__ void st8(f16* p, const float (&f)[8]) {
+  *reinterpret_cast<uint4*>(p) =
+      make_uint4(pack2<f16>(f[0], f[1]), pack2<f16>(f[2], f[3]), pack2<f16>(f[4], f[5]), pack2<f16>(f[6], f[7]));
 }
 __device__ __forceinline__ void st8(float* p, const float (&f)[8]) {
   *reinterpret_cast<float4*>(p) = make_float4(f[0], f[1], f[2], f[3]);
@@ -283,7 +295,8 @@ __device__ __forceinline__ void bulk_g2s_gate(uint32_t dst, const void* src, uin
                : "memory");
 }
 
-// grid: (ceil(hw/64), B*V); block 256 (8 warps: warp w owns positions 8w..8w+7 of the block)
+// grid: (ceil(hw/64), B*V); block 256 (8 warps: warp w owns positions 8w..8w+7 of the block).  TIO: bf16 or fp16 f4.
+template <typename TIO>
 __global__ void __launch_bounds__(256)
     gate_concat_fwd_tma_kernel(const __grid_constant__ ViewMaps maps, const ViewPtrs vp, bf16* __restrict__ xg,
                                bf16* __restrict__ xl, float* __restrict__ gate, int C, int Cs, int V, int hw, int ncls,
@@ -342,13 +355,15 @@ __global__ void __launch_bounds__(256)
     uint32_t r[4];
     ldmatrix_x4_trans(addr, r);
     if (p < hw) {
-      *reinterpret_cast<uint4*>(xg + tok + cg * 32) = make_uint4(r[0], r[1], r[2], r[3]);
-      uint32_t g[4];
+      uint32_t f[4], g[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        const float2 y = mul2(unpack_bf16(r[i]), a2);
+        const float2 x = unpack2<TIO>(r[i]);
+        const float2 y = mul2(x, a2);
+        f[i] = std::is_same<TIO, bf16>::value ? r[i] : pack_bf16(x.x, x.y);   // bf16 -> bf16 is the word as it is
         g[i] = pack_bf16(y.x, y.y);
       }
+      *reinterpret_cast<uint4*>(xg + tok + cg * 32) = make_uint4(f[0], f[1], f[2], f[3]);
       *reinterpret_cast<uint4*>(xl + tok + cg * 32) = make_uint4(g[0], g[1], g[2], g[3]);
     }
   }
@@ -356,6 +371,8 @@ __global__ void __launch_bounds__(256)
 
 // grid: (ceil(hw/64), B*V); block 256.  df4 = dXg + a * dXl back to NCHW and the complete gate gradient
 // da[p] = sum_c f4[c,p] * dXl[p,c] (the CTA sees every channel, so no partial table: da_part has one slice).
+// TIO: bf16 or fp16 f4 / df4 (the combined gradient is rounded to TIO once, in phase A; phase B moves 16-bit words).
+template <typename TIO>
 __global__ void __launch_bounds__(256)
     gate_concat_bwd_tma_kernel(const __grid_constant__ ViewMaps maps, const ViewPtrs vp, const float* __restrict__ gate,
                                const bf16* __restrict__ dxg, const bf16* __restrict__ dxl, float* __restrict__ da_part,
@@ -437,9 +454,9 @@ __global__ void __launch_bounds__(256)
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
           const float2 dl = unpack_bf16(l32[i]);
-          acc = fma2(unpack_bf16(f[i]), dl, acc);
+          acc = fma2(unpack2<TIO>(f[i]), dl, acc);
           const float2 t = fma2(a2, dl, unpack_bf16(g32[i]));
-          g32[i] = pack_bf16(t.x, t.y);
+          g32[i] = pack2<TIO>(t.x, t.y);
         }
       }
       __syncwarp();
@@ -460,7 +477,7 @@ __global__ void __launch_bounds__(256)
   {
     // phase B: [position][channel] -> NCHW.  ldmatrix rows = positions; thread T receives positions 8 (T%4) .. +7 of
     // channel 8 c8 + T/4
-    bf16* df4 = reinterpret_cast<bf16*>(vp.df4[v]) + (static_cast<long long>(b) * Ctot + c_base) * hw;
+    TIO* df4 = reinterpret_cast<TIO*>(vp.df4[v]) + (static_cast<long long>(b) * Ctot + c_base) * hw;
     const int nunits = 2 * (C / 8);               // (32-position group, 8-channel chunk)
     for (int u = warp; u < nunits; u += 8) {
       const int pg = u & 1, c8 = u >> 1;
@@ -474,8 +491,13 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+int check_io_dtype(int dt) {
+  if (dt == GLF_DTYPE_BF16 || dt == GLF_DTYPE_F16 || dt == GLF_DTYPE_F32) return 0;
+  return set_error(GLF_ERR_INVALID, "gate_concat: io_dtype must be GLF_DTYPE_BF16, GLF_DTYPE_F16 or GLF_DTYPE_F32");
+}
+
 bool gate_tma_ok(int C, int hw, int io_dtype, int x_dtype, const void* const* f4, int V) {
-  if (io_dtype != GLF_DTYPE_BF16 || x_dtype != GLF_DTYPE_BF16) return false;
+  if ((io_dtype != GLF_DTYPE_BF16 && io_dtype != GLF_DTYPE_F16) || x_dtype != GLF_DTYPE_BF16) return false;
   if (C % 64 != 0 || hw % 8 != 0) return false;
   if (C > 512 && C % 512 != 0) return false;      // wider rows are cut into 512- (forward) / 256-channel (backward) slabs
   for (int v = 0; v < V; ++v)
@@ -490,6 +512,9 @@ int launch_gate_fwd(dim3 grid, bool vec2, int io_dtype, const ViewPtrs& vp, void
   if (io_dtype == GLF_DTYPE_BF16) {
     if (vec2) gate_concat_fwd_kernel<bf16, 2, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
     else gate_concat_fwd_kernel<bf16, 1, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
+  } else if (io_dtype == GLF_DTYPE_F16) {
+    if (vec2) gate_concat_fwd_kernel<f16, 2, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
+    else gate_concat_fwd_kernel<f16, 1, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
   } else {
     if (vec2) gate_concat_fwd_kernel<float, 2, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
     else gate_concat_fwd_kernel<float, 1, TX><<<grid, 256, 0, stream>>>(vp, (TX*)xg, (TX*)xl, gate, C, V, hw, ncls, weight);
@@ -502,6 +527,9 @@ int launch_gate_bwd(dim3 grid, bool vec2, int io_dtype, const ViewPtrs& vp, cons
   if (io_dtype == GLF_DTYPE_BF16) {
     if (vec2) gate_concat_bwd_kernel<bf16, 2, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
     else gate_concat_bwd_kernel<bf16, 1, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
+  } else if (io_dtype == GLF_DTYPE_F16) {
+    if (vec2) gate_concat_bwd_kernel<f16, 2, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
+    else gate_concat_bwd_kernel<f16, 1, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
   } else {
     if (vec2) gate_concat_bwd_kernel<float, 2, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
     else gate_concat_bwd_kernel<float, 1, TX><<<grid, 256, 0, stream>>>(vp, gate, (const TX*)dxg, (const TX*)dxl, da_part, C, V, hw);
@@ -526,8 +554,10 @@ struct ClViews {
 // form keeps CL_TOK tokens x 3 operands within ~50 registers (the converted form needed 156: one CTA per SM)
 template <typename T> struct RawCl;
 template <> struct RawCl<bf16> { uint4 v; };
+template <> struct RawCl<f16> { uint4 v; };
 template <> struct RawCl<float> { float4 a, b; };
 __device__ __forceinline__ void ldr(const bf16* p, RawCl<bf16>& r) { r.v = __ldg(reinterpret_cast<const uint4*>(p)); }
+__device__ __forceinline__ void ldr(const f16* p, RawCl<f16>& r) { r.v = __ldg(reinterpret_cast<const uint4*>(p)); }
 __device__ __forceinline__ void ldr(const float* p, RawCl<float>& r) {
   r.a = __ldg(reinterpret_cast<const float4*>(p));
   r.b = __ldg(reinterpret_cast<const float4*>(p) + 1);
@@ -537,6 +567,15 @@ __device__ __forceinline__ void cvr(const RawCl<bf16>& r, float (&f)[8]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const float2 t = unpack_bf16(u[i]);
+    f[2 * i] = t.x;
+    f[2 * i + 1] = t.y;
+  }
+}
+__device__ __forceinline__ void cvr(const RawCl<f16>& r, float (&f)[8]) {
+  const uint32_t* u = reinterpret_cast<const uint32_t*>(&r.v);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 t = unpack2<f16>(u[i]);
     f[2 * i] = t.x;
     f[2 * i + 1] = t.y;
   }
@@ -664,6 +703,7 @@ template <typename TIn>
 __device__ __forceinline__ float ld_as_float(const TIn* p);
 template <> __device__ __forceinline__ float ld_as_float<float>(const float* p) { return __ldg(p); }
 template <> __device__ __forceinline__ float ld_as_float<bf16>(const bf16* p) { return __bfloat162float(*p); }
+template <> __device__ __forceinline__ float ld_as_float<f16>(const f16* p) { return __half2float(*p); }
 
 template <typename TIn>
 __global__ void __launch_bounds__(256) views_to_tokens_kernel(ViewsToTokens P, bf16* __restrict__ out, int V, int C,
@@ -698,7 +738,7 @@ __global__ void __launch_bounds__(256) views_to_tokens_kernel(ViewsToTokens P, b
     for (int i = 0; i < 4; ++i) {
       if (tt[i] < T) {
         bf16* dst = o + static_cast<long long>(tt[i]) * C + c0 + 8 * ((threadIdx.x + 256 * i) & 7);
-        if constexpr (sizeof(TIn) == 2) {
+        if constexpr (std::is_same<TIn, bf16>::value) {
           *reinterpret_cast<uint4*>(dst) = raw[i].v;          // bf16 -> bf16: the packed vector as it is
         } else {
           float f[8];
@@ -761,7 +801,7 @@ int views_to_tokens(int B, int C, int V, int T, int src_dtype, const void* const
     P.src[v] = on ? src[v] : nullptr;
     P.sb[v] = on ? sb[v] : 0; P.sc[v] = on ? sc[v] : 0; P.st[v] = on ? st[v] : 0;
     P.present[v] = on ? 1 : 0;
-    const long long per16 = src_dtype == GLF_DTYPE_BF16 ? 8 : 4;
+    const long long per16 = src_dtype == GLF_DTYPE_F32 ? 4 : 8;
     P.vec[v] = on && sc[v] == 1 && reinterpret_cast<uintptr_t>(src[v]) % 16 == 0 && sb[v] % per16 == 0 && st[v] % per16 == 0;
     if (on && sc[v] != 1 && st[v] != 1)
       return set_error(GLF_ERR_UNSUPPORTED, "views_to_tokens: a view needs unit channel or unit token stride");
@@ -769,6 +809,8 @@ int views_to_tokens(int B, int C, int V, int T, int src_dtype, const void* const
   const dim3 grid(((T + 127) / 128) * (C / 64), V, B);
   if (src_dtype == GLF_DTYPE_BF16)
     views_to_tokens_kernel<bf16><<<grid, 256, 0, stream>>>(P, reinterpret_cast<bf16*>(out), V, C, T);
+  else if (src_dtype == GLF_DTYPE_F16)
+    views_to_tokens_kernel<f16><<<grid, 256, 0, stream>>>(P, reinterpret_cast<bf16*>(out), V, C, T);
   else if (src_dtype == GLF_DTYPE_F32)
     views_to_tokens_kernel<float><<<grid, 256, 0, stream>>>(P, reinterpret_cast<bf16*>(out), V, C, T);
   else
@@ -781,21 +823,23 @@ int gate_concat_fwd(int B, int C, int V, int h, int w, int ncls, float weight, i
                     float* gate, cudaStream_t stream) {
   if (V < 1 || V > MAXV) return set_error(GLF_ERR_INVALID, "gate_concat: 1 <= V <= %d", MAXV);
   if (C % 8 != 0) return set_error(GLF_ERR_INVALID, "gate_concat: C %% 8 != 0");
+  if (int rc = check_io_dtype(io_dtype)) return rc;
   ViewPtrs vp{};
   for (int v = 0; v < V; ++v) { vp.f4[v] = f4[v]; vp.cls[v] = cls[v]; vp.ctr[v] = ctr[v]; }
   const int hw = h * w;
   if (gate_tma_ok(C, hw, io_dtype, x_dtype, f4, V) && B * V <= 65535) {
     ViewMaps maps;
     for (int v = 0; v < V; ++v) {
-      int rc = make_tmap_bf16(&maps.tm[v], f4[v], hw, C, B, hw, static_cast<long long>(C) * hw, 64);
+      int rc = make_tmap_bf16(&maps.tm[v], f4[v], hw, C, B, hw, static_cast<long long>(C) * hw, 64, io_dtype);
       if (rc) return rc;
     }
     for (int v = V; v < MAXV; ++v) maps.tm[v] = maps.tm[0];
     const int Cs = C <= 512 ? C : 512;
     const uint32_t smem = static_cast<uint32_t>(Cs / 64) * 8192u + 1024u;
-    cudaError_t e = cudaFuncSetAttribute(gate_concat_fwd_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    auto kern = io_dtype == GLF_DTYPE_F16 ? gate_concat_fwd_tma_kernel<f16> : gate_concat_fwd_tma_kernel<bf16>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gate_fwd_tma)");
-    gate_concat_fwd_tma_kernel<<<dim3((hw + 63) / 64, B * V, C / Cs), 256, smem, stream>>>(
+    kern<<<dim3((hw + 63) / 64, B * V, C / Cs), 256, smem, stream>>>(
         maps, vp, reinterpret_cast<bf16*>(xg), reinterpret_cast<bf16*>(xl), gate, C, Cs, V, hw, ncls, weight);
     return check_cuda(cudaGetLastError(), "gate_concat_fwd_tma launch");
   }
@@ -817,6 +861,7 @@ int gate_concat_bwd(int B, int C, int V, int h, int w, int ncls, float weight, i
   if (V < 1 || V > MAXV) return set_error(GLF_ERR_INVALID, "gate_concat: 1 <= V <= %d", MAXV);
   if (C % 8 != 0) return set_error(GLF_ERR_INVALID, "gate_concat: C %% 8 != 0");
   if (da_part == nullptr) return set_error(GLF_ERR_WORKSPACE, "gate_concat_bwd: scratch is NULL");
+  if (int rc = check_io_dtype(io_dtype)) return rc;
   ViewPtrs vp{};
   for (int v = 0; v < V; ++v) {
     vp.f4[v] = f4[v]; vp.cls[v] = cls[v]; vp.ctr[v] = ctr[v];
@@ -830,15 +875,16 @@ int gate_concat_bwd(int B, int C, int V, int h, int w, int ncls, float weight, i
   if (tma_ok) {
     ViewMaps maps;
     for (int v = 0; v < V; ++v) {
-      int rc = make_tmap_bf16(&maps.tm[v], f4[v], hw, C, B, hw, static_cast<long long>(C) * hw, 64);
+      int rc = make_tmap_bf16(&maps.tm[v], f4[v], hw, C, B, hw, static_cast<long long>(C) * hw, 64, io_dtype);
       if (rc) return rc;
     }
     for (int v = V; v < MAXV; ++v) maps.tm[v] = maps.tm[0];
     const int Cs = C <= 512 ? C : 256;
     const uint32_t smem = 3u * 64u * Cs * 2u + 1024u;
-    cudaError_t e = cudaFuncSetAttribute(gate_concat_bwd_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    auto kern = io_dtype == GLF_DTYPE_F16 ? gate_concat_bwd_tma_kernel<f16> : gate_concat_bwd_tma_kernel<bf16>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gate_bwd_tma)");
-    gate_concat_bwd_tma_kernel<<<dim3((hw + 63) / 64, B * V, C / Cs), 256, smem, stream>>>(
+    kern<<<dim3((hw + 63) / 64, B * V, C / Cs), 256, smem, stream>>>(
         maps, vp, gate, reinterpret_cast<const bf16*>(dxg), reinterpret_cast<const bf16*>(dxl), da_part, C, Cs, V, hw);
     int rc = check_cuda(cudaGetLastError(), "gate_concat_bwd_tma launch");
     if (rc) return rc;
@@ -867,9 +913,9 @@ namespace {
 int cl_check(int B, int C, int V, int hw, int io_dtype, const void* const* f4, const long long* sb, const long long* st) {
   if (V < 1 || V > MAXV) return set_error(GLF_ERR_INVALID, "gate_concat: 1 <= V <= %d", MAXV);
   if (C % 8 != 0) return set_error(GLF_ERR_INVALID, "gate_concat: C %% 8 != 0");
-  if (io_dtype != GLF_DTYPE_BF16 && io_dtype != GLF_DTYPE_F32) return set_error(GLF_ERR_INVALID, "gate_concat: bad dtype");
+  if (int rc = check_io_dtype(io_dtype)) return rc;
   if (static_cast<long long>(B) * V > 65535) return set_error(GLF_ERR_UNSUPPORTED, "gate_concat: B * V > 65535");
-  const long long per16 = io_dtype == GLF_DTYPE_BF16 ? 8 : 4;
+  const long long per16 = io_dtype == GLF_DTYPE_F32 ? 4 : 8;
   for (int v = 0; v < V; ++v)
     if (f4[v] == nullptr || (reinterpret_cast<uintptr_t>(f4[v]) & 15) != 0 || sb[v] % per16 != 0 || st[v] % per16 != 0 ||
         st[v] < C || (B > 1 && sb[v] < 1))
@@ -894,6 +940,8 @@ int gate_concat_cl_fwd(int B, int C, int V, int h, int w, int ncls, float weight
   const dim3 grid((hw + 8 * CL_TOK - 1) / (8 * CL_TOK), B * V);
   if (io_dtype == GLF_DTYPE_BF16)
     gate_cl_fwd_kernel<bf16><<<grid, 256, 0, stream>>>(cv, vp, reinterpret_cast<bf16*>(xg), reinterpret_cast<bf16*>(xl), gate, C, V, hw, ncls, weight);
+  else if (io_dtype == GLF_DTYPE_F16)
+    gate_cl_fwd_kernel<f16><<<grid, 256, 0, stream>>>(cv, vp, reinterpret_cast<bf16*>(xg), reinterpret_cast<bf16*>(xl), gate, C, V, hw, ncls, weight);
   else
     gate_cl_fwd_kernel<float><<<grid, 256, 0, stream>>>(cv, vp, reinterpret_cast<bf16*>(xg), reinterpret_cast<bf16*>(xl), gate, C, V, hw, ncls, weight);
   return check_cuda(cudaGetLastError(), "gate_cl_fwd launch");
@@ -921,6 +969,8 @@ int gate_concat_cl_bwd(int B, int C, int V, int h, int w, int ncls, float weight
   const dim3 grid((hw + 8 * CL_TOK - 1) / (8 * CL_TOK), B * V);
   if (io_dtype == GLF_DTYPE_BF16)
     gate_cl_bwd_kernel<bf16><<<grid, 256, 0, stream>>>(cv, gate, reinterpret_cast<const bf16*>(dxg), reinterpret_cast<const bf16*>(dxl), da, C, V, hw);
+  else if (io_dtype == GLF_DTYPE_F16)
+    gate_cl_bwd_kernel<f16><<<grid, 256, 0, stream>>>(cv, gate, reinterpret_cast<const bf16*>(dxg), reinterpret_cast<const bf16*>(dxl), da, C, V, hw);
   else
     gate_cl_bwd_kernel<float><<<grid, 256, 0, stream>>>(cv, gate, reinterpret_cast<const bf16*>(dxg), reinterpret_cast<const bf16*>(dxl), da, C, V, hw);
   rc = check_cuda(cudaGetLastError(), "gate_cl_bwd launch");

@@ -575,7 +575,8 @@ EncodeTiledFn get_encode_fn() {
 }
 
 // Tensor map over a bf16 operand: K-major -> dims {K, rows, batch, limb}; MN-major -> dims {rows, K, batch, limb}.
-int make_operand_map(CUtensorMap* tm, const GemmOperand& op, int rows, int K, int batch, int nlimbs, int box_rows) {
+int make_operand_map(CUtensorMap* tm, const GemmOperand& op, int rows, int K, int batch, int nlimbs, int box_rows,
+                     CUtensorMapDataType elem = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
   EncodeTiledFn enc = get_encode_fn();
   if (enc == nullptr) return set_error(GLF_ERR_DEVICE, "cuTensorMapEncodeTiled entry point unavailable");
   if ((reinterpret_cast<uintptr_t>(op.ptr) & 15) != 0) return set_error(GLF_ERR_INVALID, "GEMM operand not 16-byte aligned");
@@ -592,7 +593,7 @@ int make_operand_map(CUtensorMap* tm, const GemmOperand& op, int rows, int K, in
                            nlimbs > 1 ? static_cast<cuuint64_t>(op.limb_stride) * 2 : span * static_cast<cuuint64_t>(nb)};
   cuuint32_t box[4] = {64u, static_cast<cuuint32_t>(op.mn_major ? 64 : box_rows), 1u, 1u};
   cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(op.ptr), dims, strides, box, estr,
+  CUresult r = enc(tm, elem, 4, const_cast<void*>(op.ptr), dims, strides, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS)
@@ -627,15 +628,17 @@ int make_output_tmap(CUtensorMap* tm, void* D, int M, int N, int batch, long lon
   return make_output_map(tm, D, M, N, batch, ldd, strideD);
 }
 
-// bf16 tensor map over [batch][outer][inner] with row pitch `ld` elements, SWIZZLE_128B, box {64, box_outer, 1, 1}
+// 16-bit tensor map over [batch][outer][inner] with row pitch `ld` elements, SWIZZLE_128B, box {64, box_outer, 1, 1};
+// dtype GLF_DTYPE_BF16 or GLF_DTYPE_F16
 int make_tmap_bf16(CUtensorMap* tm, const void* ptr, long long inner, long long outer, long long batch, long long ld,
-                   long long batch_stride, int box_outer) {
+                   long long batch_stride, int box_outer, int dtype) {
   GemmOperand op;
   op.ptr = ptr;
   op.mn_major = 0;      // {K = inner, rows = outer}
   op.ld = ld;
   op.batch_stride = batch > 1 ? batch_stride : 0;
-  return make_operand_map(tm, op, static_cast<int>(outer), static_cast<int>(inner), static_cast<int>(batch), 1, box_outer);
+  return make_operand_map(tm, op, static_cast<int>(outer), static_cast<int>(inner), static_cast<int>(batch), 1, box_outer,
+                          dtype == GLF_DTYPE_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
 }
 
 namespace {

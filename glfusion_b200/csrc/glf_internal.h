@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -14,6 +15,7 @@ int check_cuda(cudaError_t e, const char* what); // 0 or GLF_ERR_DEVICE
 int check_device_sm100();                        // 0 or GLF_ERR_DEVICE
 
 using bf16 = __nv_bfloat16;
+using f16 = __half;        // I/O-only element type (GLF_DTYPE_F16): converted to bf16 / fp32 where it is read
 
 // ------------------------------------------------------------------------------------------------ GEMM
 struct GemmOperand {
@@ -59,8 +61,9 @@ int gemm_pair(const GemmArgs& a, int num_sms, cudaStream_t stream);
 // sequence): B resident in shared memory, only A streams
 bool gemm_bres_applicable(const GemmArgs& a, int num_sms);
 int gemm_bres(const GemmArgs& a, int num_sms, cudaStream_t stream);
+// (16-bit elements; dtype GLF_DTYPE_BF16 or GLF_DTYPE_F16 names the tensor map's element type)
 int make_tmap_bf16(CUtensorMap* tm, const void* ptr, long long inner, long long outer, long long batch, long long ld,
-                   long long batch_stride, int box_outer);
+                   long long batch_stride, int box_outer, int dtype = GLF_DTYPE_BF16);
 
 // ------------------------------------------------------------------------------------------------ element-wise
 int transpose_cast(const void* in, void* out, int batch, int R, int S, int in_dtype, int out_dtype,
@@ -79,23 +82,27 @@ int bn_res_ln_bwd_blocks(long long rows, int C);
 int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U, const void* X, int act_dtype, const float* a,
                   const float* b, const float* mean, const float* rstd, const float* lw, const float* mu,
                   const float* r, void* dV, float* part, long long rows, int C, int* nblocks, cudaStream_t stream);
-// bulk-copy staged forms (glf_ln.cu): bf16 activations, C <= 256; nmod = 2 fuses the MGFM and MLFM LayerNorms
+// bulk-copy staged forms (glf_ln.cu): bf16 activations, C <= 256; nmod = 2 fuses the MGFM and MLFM LayerNorms.
+// Z / Z0 (forward) and dZ / the per-view dz (backward) are of z_dtype: GLF_DTYPE_BF16 or GLF_DTYPE_F16.
 bool ln_tma_supported(int C);
 int ln_bwd_tma_blocks(long long rows);
 int ln_fwd_tma(int nmod, const bf16* const* U, const bf16* const* X, const float* const* a, const float* const* b,
-               const float* const* lw, const float* const* lb, float* const* mu, float* const* r, bf16* Z,
-               long long rows, int C, float eps, int accumulate, cudaStream_t stream, bf16* Z0 = nullptr);
-int ln_bwd_tma(int nmod, const bf16* dZ, const bf16* const* U, const bf16* const* X, const float* const* a,
+               const float* const* lw, const float* const* lb, float* const* mu, float* const* r, void* Z,
+               long long rows, int C, float eps, int accumulate, cudaStream_t stream, void* Z0 = nullptr,
+               int z_dtype = GLF_DTYPE_BF16);
+int ln_bwd_tma(int nmod, const void* dZ, const bf16* const* U, const bf16* const* X, const float* const* a,
                const float* const* b, const float* const* lw, const float* const* bn_mean,
                const float* const* bn_rstd, const float* const* mu, const float* const* r, bf16* const* dV,
                float* const* part, long long rows, int C, int* nblocks, cudaStream_t stream, int dz_nv = 0,
-               const void* const* dz_views = nullptr, const long long* dz_sb = nullptr, int dz_hw = 0);
+               const void* const* dz_views = nullptr, const long long* dz_sb = nullptr, int dz_hw = 0,
+               int dz_dtype = GLF_DTYPE_BF16);
 int ln_bwd_tma_tile_rows();
 // (glf_eltwise.cu) the fused MGFM + MLFM LayerNorm forward for wide rows, 256 < C <= 2048 (sliced rows, cp.async ring)
 bool ln_pair_wide_supported(int C);
 int ln_pair_fwd_wide(const bf16* const* U, const bf16* const* X, const float* const* a, const float* const* b,
-                     const float* const* lw, const float* const* lb, float* const* mu, float* const* r, bf16* Z,
-                     long long rows, int C, float eps, int accumulate, cudaStream_t stream, bf16* Z0);
+                     const float* const* lw, const float* const* lb, float* const* mu, float* const* r, void* Z,
+                     long long rows, int C, float eps, int accumulate, cudaStream_t stream, void* Z0,
+                     int z_dtype = GLF_DTYPE_BF16);
 int bn_bwd_finalize(const float* part, int np, int C, double count, const glf_desc* d, const glf_weights* w,
                     const float* mean, const float* rstd, const glf_grads* g, float* k1, float* k2, float* k3,
                     cudaStream_t stream);

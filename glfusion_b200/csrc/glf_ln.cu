@@ -1,7 +1,8 @@
 // glf_ln.cu — bulk-copy (TMA engine) staged versions of the two HBM-bound row kernels of the fusion path,
 //   forward : Z = sum_m LayerNorm_C(a_m * U_m + b_m + X_m) * lw_m + lb_m        (ours.py:908-915; m = MGFM, MLFM)
 //   backward: dV_m = d(pre-LayerNorm sum) and per-CTA partials of the four per-channel reductions
-// for bf16 activations with C <= 256 (one warp owns a row, one lane 8 channels).
+// for bf16 activations with C <= 256 (one warp owns a row, one lane 8 channels).  Z / dZ, the tensors the caller hands
+// over or receives, are bf16 or fp16 (TZ): the same bytes per row, converted where they are read or written.
 //
 // Why: the register-prefetch kernels of glf_eltwise.cu keep ~24 KB per SM in flight, B200 needs roughly twice that to
 // saturate HBM3e (measured 60-75 % of the copy bandwidth).  Here one producer warp streams contiguous row tiles
@@ -23,12 +24,13 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                : "memory");
 }
 
-// 8 bf16 from shared memory as four float2 (element pairs)
+// 8 16-bit elements (bf16 or fp16) from shared memory as four float2 (element pairs)
+template <typename T = bf16>
 __device__ __forceinline__ void lds8p(const uint8_t* p, float2 (&f)[4]) {
   const uint4 v = *reinterpret_cast<const uint4*>(p);
   const uint32_t* u = reinterpret_cast<const uint32_t*>(&v);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) f[i] = unpack_bf16(u[i]);
+  for (int i = 0; i < 4; ++i) f[i] = unpack2<T>(u[i]);
 }
 __device__ __forceinline__ void ldg8p(const float* p, float2 (&f)[4]) {
   const float4 a = *reinterpret_cast<const float4*>(p);
@@ -36,9 +38,10 @@ __device__ __forceinline__ void ldg8p(const float* p, float2 (&f)[4]) {
   f[0] = make_float2(a.x, a.y); f[1] = make_float2(a.z, a.w);
   f[2] = make_float2(b.x, b.y); f[3] = make_float2(b.z, b.w);
 }
-__device__ __forceinline__ void stg8p(bf16* p, const float2 (&f)[4]) {
-  *reinterpret_cast<uint4*>(p) = make_uint4(pack_bf16(f[0].x, f[0].y), pack_bf16(f[1].x, f[1].y),
-                                            pack_bf16(f[2].x, f[2].y), pack_bf16(f[3].x, f[3].y));
+template <typename T>
+__device__ __forceinline__ void stg8p(T* p, const float2 (&f)[4]) {
+  *reinterpret_cast<uint4*>(p) = make_uint4(pack2<T>(f[0].x, f[0].y), pack2<T>(f[1].x, f[1].y),
+                                            pack2<T>(f[2].x, f[2].y), pack2<T>(f[3].x, f[3].y));
 }
 __device__ __forceinline__ float hsum4(const float2 (&f)[4]) {
   const float2 t = add2(add2(f[0], f[1]), add2(f[2], f[3]));
@@ -64,8 +67,8 @@ struct LnFwdParams {
   const float* lb[2];
   float* mu[2];
   float* r[2];
-  bf16* Z;
-  bf16* Z0;        // PARTS only: the first module's own output (MGFM's f4_global_fusion, ours.py:1823), bf16 [rows, C]
+  void* Z;         // [rows, C] of the kernel's TZ
+  void* Z0;        // PARTS only: the first module's own output (MGFM's f4_global_fusion, ours.py:1823), TZ [rows, C]
   long long rows;
   int C, ntiles, stages, accumulate;
   uint32_t arr_bytes, stage_bytes;
@@ -74,7 +77,7 @@ struct LnFwdParams {
 
 // FULLC: C == 256, every lane owns 8 live channels.  PARTS: also store module 0's LayerNorm output on its own (the
 // cycle-consistency pass of the trainer, R/main.py:211-235, consumes f4_global_fusion beside the fused sum).
-template <int NMOD, bool FULLC, bool PARTS = false>
+template <int NMOD, bool FULLC, bool PARTS, typename TZ>
 __global__ void __launch_bounds__(F_THREADS, 1) ln_fwd_tma_kernel(const LnFwdParams p) {
   extern __shared__ uint8_t lsm_raw[];
   __shared__ uint64_t full_bar[MAX_STAGES], empty_bar[MAX_STAGES];
@@ -113,7 +116,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) ln_fwd_tma_kernel(const LnFwdPar
           bulk_g2s(dst + (2 * m) * p.arr_bytes, p.U[m] + off, bytes, fb);
           bulk_g2s(dst + (2 * m + 1) * p.arr_bytes, p.X[m] + off, bytes, fb);
         }
-        if (p.accumulate) bulk_g2s(dst + 2 * NMOD * p.arr_bytes, p.Z + off, bytes, fb);
+        if (p.accumulate) bulk_g2s(dst + 2 * NMOD * p.arr_bytes, reinterpret_cast<const TZ*>(p.Z) + off, bytes, fb);
       }
     }
     return;
@@ -165,7 +168,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) ln_fwd_tma_kernel(const LnFwdPar
         for (int i = 0; i < 4; ++i) o[i] = plsum[i];
         if (cact && p.accumulate) {
           float2 z0[4];
-          lds8p(st + 2 * NMOD * p.arr_bytes + roff, z0);
+          lds8p<TZ>(st + 2 * NMOD * p.arr_bytes + roff, z0);
 #pragma unroll
           for (int i = 0; i < 4; ++i) o[i] = add2(o[i], z0[i]);
         }
@@ -219,14 +222,14 @@ __global__ void __launch_bounds__(F_THREADS, 1) ln_fwd_tma_kernel(const LnFwdPar
             float2 o0[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i) o0[i] = fma2(v[0][i], mul2(pw[0][i], r2), plb0[i]);
-            stg8p(p.Z0 + row * p.C + c0, o0);
+            stg8p(reinterpret_cast<TZ*>(p.Z0) + row * p.C + c0, o0);
           }
           if (lane == 0 && p.mu[m] != nullptr) {
             p.mu[m][row] = mu[m];
             p.r[m][row] = r;
           }
         }
-        if (cact) stg8p(p.Z + row * p.C + c0, o);
+        if (cact) stg8p(reinterpret_cast<TZ*>(p.Z) + row * p.C + c0, o);
       }
     }
     __syncwarp();
@@ -241,7 +244,7 @@ constexpr int B_THREADS = (B_CW + 1) * 32;
 constexpr int B_ACC_PITCH = 256 + 8;
 
 struct LnBwdParams {
-  const bf16* dZ;
+  const void* dZ;            // [rows, C] of the kernel's TZ
   const bf16* U[2];
   const bf16* X[2];
   const float* a[2];
@@ -259,12 +262,12 @@ struct LnBwdParams {
   // dZ given per view (the dict-keyed call site: one gradient per view, rows of C channels): row (b, v, t) of the stack
   // lives at dzv[v] + b * dz_sb[v] + t * C.  dz_nv = 0: dZ is the token-major stack itself.  Needs hw % B_TR == 0 so
   // that a tile never straddles two views.
-  const bf16* dzv[8];
+  const void* dzv[8];
   long long dz_sb[8];
   int dz_nv, dz_hw;
 };
 
-template <int NMOD, bool FULLC>
+template <int NMOD, bool FULLC, typename TZ>
 __global__ void __launch_bounds__(B_THREADS, 1) ln_bwd_tma_kernel(const LnBwdParams p) {
   extern __shared__ uint8_t lsm_raw[];
   __shared__ uint64_t full_bar[MAX_STAGES], empty_bar[MAX_STAGES];
@@ -299,11 +302,11 @@ __global__ void __launch_bounds__(B_THREADS, 1) ln_bwd_tma_kernel(const LnBwdPar
         mbar_expect_tx(fb, bytes * (1 + 2 * NMOD) + (full_tile ? 2u * NMOD * B_TR * 4u : 0u));
         const uint32_t dst = ring_u32 + s * p.stage_bytes;
         const long long off = row0 * p.C;
-        const bf16* dzsrc = p.dZ + off;
+        const TZ* dzsrc = reinterpret_cast<const TZ*>(p.dZ) + off;
         if (p.dz_nv > 0) {
           const long long bv = row0 / p.dz_hw;
           const int v = static_cast<int>(bv % p.dz_nv);
-          dzsrc = p.dzv[v] + (bv / p.dz_nv) * p.dz_sb[v] + (row0 - bv * p.dz_hw) * p.C;
+          dzsrc = reinterpret_cast<const TZ*>(p.dzv[v]) + (bv / p.dz_nv) * p.dz_sb[v] + (row0 - bv * p.dz_hw) * p.C;
         }
         bulk_g2s(dst, dzsrc, bytes, fb);
 #pragma unroll
@@ -364,7 +367,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) ln_bwd_tma_kernel(const LnBwdPar
           for (int i = 0; i < 4; ++i) xh[i] = dxh[i] = dz[i] = u[i] = splat(0.f);
           if (cact) {
             float2 x[4];
-            lds8p(st + roff, dz);
+            lds8p<TZ>(st + roff, dz);
             lds8p(st + u_off + roff, u);
             lds8p(st + x_off + roff, x);
             const float2 r2 = splat(r), nmur = splat(-mu * r);
@@ -447,11 +450,12 @@ int ln_bwd_tma_blocks(long long rows) {
   return static_cast<int>(nt < sms ? nt : sms);
 }
 
-// Z (+)= sum over the nmod modules of LayerNorm(a U + b + X) lw + lb.  All activations bf16 [rows, C].
+// Z (+)= sum over the nmod modules of LayerNorm(a U + b + X) lw + lb.  U, X bf16 [rows, C]; Z (and Z0) of z_dtype.
 int ln_fwd_tma(int nmod, const bf16* const* U, const bf16* const* X, const float* const* a, const float* const* b,
-               const float* const* lw, const float* const* lb, float* const* mu, float* const* r, bf16* Z,
-               long long rows, int C, float eps, int accumulate, cudaStream_t stream, bf16* Z0) {
+               const float* const* lw, const float* const* lb, float* const* mu, float* const* r, void* Z,
+               long long rows, int C, float eps, int accumulate, cudaStream_t stream, void* Z0, int z_dtype) {
   if (!ln_tma_supported(C) || nmod < 1 || nmod > 2) return set_error(GLF_ERR_INVALID, "ln_fwd_tma: unsupported shape");
+  if (z_dtype != GLF_DTYPE_BF16 && z_dtype != GLF_DTYPE_F16) return set_error(GLF_ERR_INVALID, "ln_fwd_tma: Z must be bf16 or fp16");
   if (Z0 != nullptr && nmod != 2) return set_error(GLF_ERR_INVALID, "ln_fwd_tma: the parts output needs both modules");
   LnFwdParams p;
   p.Z0 = Z0;
@@ -471,10 +475,17 @@ int ln_fwd_tma(int nmod, const bf16* const* U, const bf16* const* X, const float
   const uint32_t smem = p.stages * p.stage_bytes + 128;
   const int sms = num_sms();
   const int grid = p.ntiles < sms ? p.ntiles : sms;
-  void (*kern)(const LnFwdParams) =
-      nmod == 2 ? (C == 256 ? ln_fwd_tma_kernel<2, true> : ln_fwd_tma_kernel<2, false>)
-                : (C == 256 ? ln_fwd_tma_kernel<1, true> : ln_fwd_tma_kernel<1, false>);
-  if (Z0 != nullptr) kern = C == 256 ? ln_fwd_tma_kernel<2, true, true> : ln_fwd_tma_kernel<2, false, true>;
+  const bool h = z_dtype == GLF_DTYPE_F16;
+  void (*kern)(const LnFwdParams);
+  if (Z0 != nullptr)
+    kern = C == 256 ? (h ? ln_fwd_tma_kernel<2, true, true, f16> : ln_fwd_tma_kernel<2, true, true, bf16>)
+                    : (h ? ln_fwd_tma_kernel<2, false, true, f16> : ln_fwd_tma_kernel<2, false, true, bf16>);
+  else if (nmod == 2)
+    kern = C == 256 ? (h ? ln_fwd_tma_kernel<2, true, false, f16> : ln_fwd_tma_kernel<2, true, false, bf16>)
+                    : (h ? ln_fwd_tma_kernel<2, false, false, f16> : ln_fwd_tma_kernel<2, false, false, bf16>);
+  else
+    kern = C == 256 ? (h ? ln_fwd_tma_kernel<1, true, false, f16> : ln_fwd_tma_kernel<1, true, false, bf16>)
+                    : (h ? ln_fwd_tma_kernel<1, false, false, f16> : ln_fwd_tma_kernel<1, false, false, bf16>);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln_fwd_tma)");
   kern<<<grid, F_THREADS, smem, stream>>>(p);
@@ -483,13 +494,15 @@ int ln_fwd_tma(int nmod, const bf16* const* U, const bf16* const* X, const float
 
 int ln_bwd_tma_tile_rows() { return B_TR; }
 
-// dV_m and per-CTA partials [blocks][4][C] per module; returns the number of partial rows through *nblocks.
-int ln_bwd_tma(int nmod, const bf16* dZ, const bf16* const* U, const bf16* const* X, const float* const* a,
+// dV_m and per-CTA partials [blocks][4][C] per module; returns the number of partial rows through *nblocks.  dZ (or the
+// per-view dz) of dz_dtype.
+int ln_bwd_tma(int nmod, const void* dZ, const bf16* const* U, const bf16* const* X, const float* const* a,
                const float* const* b, const float* const* lw, const float* const* bn_mean,
                const float* const* bn_rstd, const float* const* mu, const float* const* r, bf16* const* dV,
                float* const* part, long long rows, int C, int* nblocks, cudaStream_t stream, int dz_nv,
-               const void* const* dz_views, const long long* dz_sb, int dz_hw) {
+               const void* const* dz_views, const long long* dz_sb, int dz_hw, int dz_dtype) {
   if (!ln_tma_supported(C) || nmod < 1 || nmod > 2) return set_error(GLF_ERR_INVALID, "ln_bwd_tma: unsupported shape");
+  if (dz_dtype != GLF_DTYPE_BF16 && dz_dtype != GLF_DTYPE_F16) return set_error(GLF_ERR_INVALID, "ln_bwd_tma: dZ must be bf16 or fp16");
   LnBwdParams p;
   p.dZ = dZ;
   p.dz_nv = 0; p.dz_hw = 1;
@@ -501,7 +514,7 @@ int ln_bwd_tma(int nmod, const bf16* dZ, const bf16* const* U, const bf16* const
     for (int v = 0; v < dz_nv; ++v) {
       if (dz_views[v] == nullptr || (reinterpret_cast<uintptr_t>(dz_views[v]) & 15) != 0 || dz_sb[v] % 8 != 0)
         return set_error(GLF_ERR_INVALID, "ln_bwd_tma: per-view dz must be 16-byte aligned");
-      p.dzv[v] = reinterpret_cast<const bf16*>(dz_views[v]);
+      p.dzv[v] = dz_views[v];
       p.dz_sb[v] = dz_sb[v];
     }
     p.dz_nv = dz_nv; p.dz_hw = dz_hw;
@@ -526,9 +539,12 @@ int ln_bwd_tma(int nmod, const bf16* dZ, const bf16* const* U, const bf16* const
   const uint32_t smem = ring_bytes + 128;
   const int grid = ln_bwd_tma_blocks(rows);
   if (nblocks) *nblocks = grid;
+  const bool h = dz_dtype == GLF_DTYPE_F16;
   void (*kern)(const LnBwdParams) =
-      nmod == 2 ? (C == 256 ? ln_bwd_tma_kernel<2, true> : ln_bwd_tma_kernel<2, false>)
-                : (C == 256 ? ln_bwd_tma_kernel<1, true> : ln_bwd_tma_kernel<1, false>);
+      nmod == 2 ? (C == 256 ? (h ? ln_bwd_tma_kernel<2, true, f16> : ln_bwd_tma_kernel<2, true, bf16>)
+                            : (h ? ln_bwd_tma_kernel<2, false, f16> : ln_bwd_tma_kernel<2, false, bf16>))
+                : (C == 256 ? (h ? ln_bwd_tma_kernel<1, true, f16> : ln_bwd_tma_kernel<1, true, bf16>)
+                            : (h ? ln_bwd_tma_kernel<1, false, f16> : ln_bwd_tma_kernel<1, false, bf16>));
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(ln_bwd_tma)");
   kern<<<grid, B_THREADS, smem, stream>>>(p);

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -268,6 +269,20 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 __device__ __forceinline__ float2 unpack_bf16(uint32_t u) {
   __nv_bfloat162 v = *reinterpret_cast<__nv_bfloat162*>(&u);
   return __bfloat1622float2(v);
+}
+// The two 16-bit I/O element types as pairs in one 32-bit word: bf16, or fp16 (GLF_DTYPE_F16).  The fp16 pack rounds
+// to nearest, so a value beyond the fp16 range becomes +-inf (never clamped to 65504).
+template <typename T> __device__ __forceinline__ float2 unpack2(uint32_t u);
+template <> __device__ __forceinline__ float2 unpack2<__nv_bfloat16>(uint32_t u) { return unpack_bf16(u); }
+template <> __device__ __forceinline__ float2 unpack2<__half>(uint32_t u) {
+  __half2 v = *reinterpret_cast<__half2*>(&u);
+  return __half22float2(v);
+}
+template <typename T> __device__ __forceinline__ uint32_t pack2(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float lo, float hi) { return pack_bf16(lo, hi); }
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float lo, float hi) {
+  __half2 v = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<uint32_t*>(&v);
 }
 // Packed fp32 pairs (Blackwell FFMA2 / FADD2 / FMUL2): one instruction per two lanes of math.  The instruction-issue
 // bound row kernels (LayerNorm forward / backward) are written on float2.

@@ -21,8 +21,10 @@ from torch import nn
 from . import _lib as L
 import threading
 
-from .tpavi import (TPAVIModule, TPAVIState, _blob, _io_dtype, _stream_ptr, _weights_struct, claim_grad_out,
-                    tpavi_backward_raw, tpavi_forward_raw)
+from .tpavi import (_IO_DTYPES, TPAVIModule, TPAVIState, _blob, _check_precision_dtype, _io_dtype, _stream_ptr,
+                    _weights_struct, claim_grad_out, tpavi_backward_raw, tpavi_forward_raw)
+
+_HALF = (torch.bfloat16, torch.float16)     # the 2-byte activation dtypes: 8 elements per 16 bytes
 
 
 _SIDE_STREAMS = {}
@@ -56,9 +58,9 @@ def _channels_last_rows(views: Sequence[torch.Tensor], x_dtype) -> Optional[tupl
     if x_dtype != torch.bfloat16 or len(views) > 8:
         return None
     dt = views[0].dtype
-    if dt not in (torch.bfloat16, torch.float32):
+    if dt not in (torch.bfloat16, torch.float16, torch.float32):
         return None
-    per16 = 8 if dt == torch.bfloat16 else 4
+    per16 = 8 if dt in _HALF else 4
     B, C_, h, w = views[0].shape
     if C_ % 8 or B * len(views) > 65535:
         return None
@@ -80,6 +82,9 @@ def gate_concat_forward(f4: Sequence[torch.Tensor], cls: Sequence[torch.Tensor],
     dev = f4[0].device
     if not all(t.is_cuda for t in list(f4) + list(cls) + list(ctr)):
         raise L.GlfError("glfusion_b200 runs on CUDA (sm_100) tensors only; there is no CPU path")
+    if any(t.dtype != f4[0].dtype for t in f4):
+        # the kernels read every view with one element type: a mix would be misread, not converted
+        raise TypeError(f"the f4 views must share one dtype, got {sorted({str(t.dtype) for t in f4})}")
     cls = [t.float().contiguous() for t in cls]
     ctr = [t.float().contiguous() for t in ctr]
     ncls = cls[0].shape[1]
@@ -105,11 +110,15 @@ def gate_concat_forward(f4: Sequence[torch.Tensor], cls: Sequence[torch.Tensor],
     return xg, xl, gate, f4, cls, ctr
 
 
-def views_to_tokens(views: Sequence[Optional[torch.Tensor]], out: torch.Tensor) -> bool:
-    """Gather per-view [B,C,h,w] tensors (NCHW or channels-last strides, bf16 or fp32; None = zeros) into the
+_GATHER_DTYPES = (torch.bfloat16, torch.float32)
+
+
+def views_to_tokens(views: Sequence[Optional[torch.Tensor]], out: torch.Tensor, dtypes=_GATHER_DTYPES) -> bool:
+    """Gather per-view [B,C,h,w] tensors (NCHW or channels-last strides, of one of `dtypes`; None = zeros) into the
     token-major bf16 buffer `out` [B,V,h,w,C] with one kernel (glf_views_to_tokens) — the inverse of handing the
     dict-keyed caller one [B,C,h,w] view per key.  Returns False, having done nothing, when the kernel does not cover
-    the case (other dtypes / strides); the caller then copies view by view."""
+    the case (other dtypes / strides); the caller then copies view by view.  The kernel also reads float16; the fused
+    backward asks for it with dtypes=(torch.bfloat16, torch.float16, torch.float32)."""
     if out.dtype != torch.bfloat16 or not out.is_contiguous():
         return False
     B, V, h, w, Cn = out.shape
@@ -117,7 +126,7 @@ def views_to_tokens(views: Sequence[Optional[torch.Tensor]], out: torch.Tensor) 
     if not live or Cn % 64 or V > 8 or B > 65535:
         return False
     dt = live[0].dtype
-    if dt not in (torch.bfloat16, torch.float32):
+    if dt not in dtypes:
         return False
     sb, sc, st = [], [], []
     for g in views:
@@ -140,17 +149,17 @@ def views_to_tokens(views: Sequence[Optional[torch.Tensor]], out: torch.Tensor) 
 
 def _views_as_rows(grads, xg: torch.Tensor, st) -> Optional[tuple]:
     """The V per-view gradients as (tensors, batch strides) when the fused LayerNorm backward can read them in place
-    (glf_fusion_ln_bwd_views): all present, bf16, rows of C contiguous channels with contiguous tokens (channels_last or
-    views of a token-major stack), 16-byte aligned, h*w a multiple of the pass's row tile.  None otherwise: the caller
-    gathers them into one token-major buffer first."""
+    (glf_fusion_ln_bwd_views): all present, one 2-byte dtype (bf16 or fp16), rows of C contiguous channels with
+    contiguous tokens (channels_last or views of a token-major stack), 16-byte aligned, h*w a multiple of the pass's row
+    tile.  None otherwise: the caller gathers them into one token-major buffer first."""
     B, V, h, w, Cn = xg.shape
-    if any(g is None for g in grads) or xg.dtype != torch.bfloat16:
+    if any(g is None for g in grads) or xg.dtype != torch.bfloat16 or grads[0].dtype not in _HALF:
         return None
     if not L.load().glf_fusion_ln_bwd_views_supported(C.byref(st.desc)):
         return None
     sb = []
     for g in grads:
-        if g.dtype != torch.bfloat16 or tuple(g.shape) != (B, Cn, h, w) or g.device != xg.device:
+        if g.dtype != grads[0].dtype or tuple(g.shape) != (B, Cn, h, w) or g.device != xg.device:
             return None
         b_, c_, h_, w_ = g.stride()
         if c_ != 1 or w_ != Cn or h_ != w * Cn or b_ % 8 or g.data_ptr() % 16 or (B > 1 and b_ < h * w * Cn):
@@ -209,6 +218,7 @@ class _FusionFunction(torch.autograd.Function):
         prec = mg._precision_id()
         if ml._precision_id() != prec:
             raise ValueError("global_attn and local_attn must use the same compute_precision")
+        _check_precision_dtype(prec, f4[0].dtype)
         xdt = torch.float32 if prec == L.PRECISION_F32X3 else torch.bfloat16
         xg, xl, gate, f4c, clsc, ctrc = gate_concat_forward(f4, cls, ctr, fusion.center_aware_weight, xdt)
         B, V_, h, w, C_ = xg.shape
@@ -216,9 +226,11 @@ class _FusionFunction(torch.autograd.Function):
         tg, tl = mg._param_table(pg), ml._param_table(pl)
         shape = (B, V_, h, w, C_)
         pair = _pair_ln_ok(mg, ml, shape, xg, prec)
-        zsum = torch.empty(shape, dtype=xg.dtype, device=xg.device)
+        # fp16 f4: the fused LayerNorm pass writes the fp16 outputs itself (its z dtype, desc.reserved[2]); no cast pass
+        zdt = torch.float16 if pair and f4[0].dtype == torch.float16 else xg.dtype
+        zsum = torch.empty(shape, dtype=zdt, device=xg.device)
         parts = bool(parts) and pair
-        zglob = torch.empty(shape, dtype=xg.dtype, device=xg.device) if parts else None
+        zglob = torch.empty(shape, dtype=zdt, device=xg.device) if parts else None
         # MGFM and MLFM are independent up to the fused LayerNorm: the local block runs on a side stream (a parallel
         # branch when the step is captured in a CUDA graph), so one block's short latency-bound kernels (BN statistics,
         # the per-sequence W' products) overlap the other's streaming GEMMs
@@ -245,6 +257,7 @@ class _FusionFunction(torch.autograd.Function):
         if pair:
             # both blocks' BN + residual + LayerNorm and the `global + local` sum (ours.py:1834) in one HBM pass
             wg, wl = _weights_struct(tg, mg._buffer_table()), _weights_struct(tl, ml._buffer_table())
+            stg.desc.reserved[2] = _io_dtype(zsum)
             with torch.cuda.device(xg.device):
                 L.check(L.load().glf_fusion_ln_fwd_parts(C.byref(stg.desc), L.ptr(xg), L.ptr(xl), C.byref(wg),
                                                          C.byref(wl), L.ptr(zsum), L.ptr(zglob), L.ptr(svg), L.ptr(svl),
@@ -284,19 +297,19 @@ class _FusionFunction(torch.autograd.Function):
         stg, svg, stl, svl = ctx.states
         if svg is None:
             raise L.GlfError("backward called on a forward that ran without grad")
-        def token(t):                               # [B,C,V,h,w] gradient -> token-major [B,V,h,w,C] in the x dtype
+        def token(t, ln_pair=False):                # [B,C,V,h,w] gradient -> token-major [B,V,h,w,C] in the x dtype
             if ctx.per_view:
                 return t                            # assembled token-major below
             t = t.permute(0, 2, 3, 4, 1)
-            if t.dtype != xg.dtype:
-                t = t.to(xg.dtype)
+            if t.dtype != xg.dtype and not (ln_pair and t.dtype == torch.float16):
+                t = t.to(xg.dtype)                  # (the fused LayerNorm backward reads an fp16 dz itself)
             return t.contiguous()
 
         def assemble(gs):                           # per-view [B,C,h,w] gradients -> one token-major [B,V,h,w,C] buffer
             if all(g is None for g in gs):
                 return None
             buf = torch.empty(xg.shape, dtype=xg.dtype, device=xg.device)
-            if views_to_tokens(gs, buf):
+            if views_to_tokens(gs, buf, dtypes=tuple(_IO_DTYPES)):
                 return buf
             for v, g in enumerate(gs):
                 if g is None:
@@ -321,12 +334,13 @@ class _FusionFunction(torch.autograd.Function):
         if dglob is None:
             # both blocks see the same dz (ours.py:1834); with dz_rows it stays where autograd delivered it, one tensor
             # per view, and `dz` is only a placeholder (the blocks' backward continues from dV, it never reads dz)
-            dz = xg if dz_rows is not None else token(dout)
+            dz = xg if dz_rows is not None else token(dout, ln_pair=ctx.pair)
             wsg = wsl = None
             if ctx.pair:
                 # LayerNorm backward of both blocks in one pass (dz is read once); fills dV / partials inside each ws blob
                 stg.desc.dz_layout = stl.desc.dz_layout = L.LAYOUT_TOKEN
                 stg.desc.reserved[0] = stl.desc.reserved[0] = 1
+                stg.desc.reserved[2] = _io_dtype(dz_rows[0][0] if dz_rows is not None else dz)
                 wsg, wsl = _blob(stg.sizes.ws_bwd_bytes, xg.device), _blob(stl.sizes.ws_bwd_bytes, xg.device)
                 wg, wl = _weights_struct(tg, mg._buffer_table()), _weights_struct(tl, ml._buffer_table())
                 with torch.cuda.device(xg.device):

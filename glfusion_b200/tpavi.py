@@ -38,12 +38,23 @@ def set_default_precision(name: str) -> None:
 _PARAM_ORDER = ("theta_w", "theta_b", "phi_w", "phi_b", "g_w", "g_b", "wz_w", "wz_b", "bn_w", "bn_b", "ln_w", "ln_b")
 
 
+_IO_DTYPES = {torch.bfloat16: L.DTYPE_BF16, torch.float32: L.DTYPE_F32, torch.float16: L.DTYPE_F16}
+
+
 def _io_dtype(t: torch.Tensor) -> int:
-    if t.dtype == torch.bfloat16:
-        return L.DTYPE_BF16
-    if t.dtype == torch.float32:
-        return L.DTYPE_F32
-    raise TypeError(f"glfusion_b200 supports float32 and bfloat16 activations, got {t.dtype}")
+    """GLF_DTYPE_* of an activation.  float16 (torch.autocast's default) is an I/O dtype only: the kernels convert it to
+    bf16 where they read it and round to fp16 where they write; the products and statistics in between are unchanged."""
+    try:
+        return _IO_DTYPES[t.dtype]
+    except KeyError:
+        raise TypeError(f"glfusion_b200 supports float32, bfloat16 and float16 activations, got {t.dtype}") from None
+
+
+def _check_precision_dtype(precision: int, dtype: torch.dtype) -> None:
+    """The fp32-exact arm is an fp32 contract: float16 inputs would defeat it (the library rejects the pair too)."""
+    if precision == L.PRECISION_F32X3 and dtype == torch.float16:
+        raise TypeError("compute_precision='fp32' takes float32 or bfloat16 activations, not float16; keep the default "
+                        "compute_precision='bf16' for float16 (autocast) inputs")
 
 
 def _is_token_major(t: torch.Tensor) -> bool:
@@ -109,6 +120,7 @@ def tpavi_forward_raw(x: torch.Tensor, params: dict, buffers, *, mode: int, trai
     lib = L.load()
     if not x.is_cuda:
         raise L.GlfError("glfusion_b200 runs on CUDA (sm_100) tensors only; there is no CPU path")
+    _check_precision_dtype(precision, x.dtype)
     if token_shape is not None:
         B, T, H, W, C_ = token_shape
         layout = L.LAYOUT_TOKEN

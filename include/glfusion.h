@@ -38,7 +38,11 @@ extern "C" {
 typedef void* glf_stream_t; /* cudaStream_t */
 
 enum { GLF_MODE_DOT = 0, GLF_MODE_EMBEDDED = 1 };         /* TPAVIModule(mode=...)  ours.py:896-900 */
-enum { GLF_DTYPE_BF16 = 0, GLF_DTYPE_F32 = 1 };
+/* I/O dtypes of the activations a caller hands over.  GLF_DTYPE_F16 is an I/O type only (torch.autocast's default):
+ * the boundary kernels convert it to bf16 where they read it and round to fp16 where they write; everything between
+ * (tensor-core operands, statistics) is bf16 / fp32 as for bf16 input.  fp16 stores round to nearest, so a value
+ * beyond the fp16 range becomes +-inf (what torch.amp.GradScaler looks for), never a clamped 65504. */
+enum { GLF_DTYPE_BF16 = 0, GLF_DTYPE_F32 = 1, GLF_DTYPE_F16 = 2 };
 enum { GLF_LAYOUT_NCTHW = 0, GLF_LAYOUT_TOKEN = 1 };      /* [B,C,T,H,W] contiguous  |  [B,T,H,W,C] contiguous */
 enum { GLF_PRECISION_BF16 = 0, GLF_PRECISION_F32X3 = 1 }; /* tensor-core operand precision */
 
@@ -58,7 +62,7 @@ typedef struct glf_desc {
   int32_t x_layout;   /* physical layout of x and dx                   GLF_LAYOUT_* */
   int32_t dz_layout;  /* physical layout of dz (z itself is always GLF_LAYOUT_TOKEN, like the reference's
                          permuted LayerNorm output, ours.py:913-915) */
-  int32_t precision;  /* GLF_PRECISION_* */
+  int32_t precision;  /* GLF_PRECISION_* (GLF_PRECISION_F32X3 takes fp32 or bf16 io_dtype, not fp16) */
   int32_t training;   /* BatchNorm3d uses batch statistics and updates running stats (ours.py:822-825) */
   int32_t bn_layer;   /* 1: W_z = conv + BN ; 0: W_z = conv only (ours.py:829-833) */
   int32_t accumulate; /* fwd: z += result instead of z = result (fuses f4_global + f4_local, ours.py:1834) */
@@ -130,12 +134,13 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
  *   3. backward: glf_fusion_ln_bwd fills dV / the per-channel partials inside ws_g and ws_l (each sized
  *      ws_bwd_bytes), then glf_tpavi_bwd(d, dz, x_g, ..., ws_g) and glf_tpavi_bwd(d, dz, x_l, ..., ws_l) with
  *      d->reserved[0] = 1 continue from there.
- * Requirements (glf_fusion_ln_supported returns 1): bf16 token-major x / dz, GLF_PRECISION_BF16, C <= 2048 (C <= 256: one
- * bulk-copy pass each way; wider rows: one sliced-row pass forward, the two blocks' backward passes back to back). */
+ * Requirements (glf_fusion_ln_supported returns 1): bf16 token-major x, dz token-major, GLF_PRECISION_BF16, C <= 2048
+ * (C <= 256: one bulk-copy pass each way; wider rows: one sliced-row pass forward, the two blocks' backward passes back
+ * to back).  z, z_global and dz are bf16, or fp16 with d->reserved[2] = GLF_DTYPE_F16. */
 GLF_API int glf_fusion_ln_supported(const glf_desc* d);
 GLF_API int glf_fusion_ln_fwd(const glf_desc* d, const void* xg, const void* xl, const glf_weights* wg,
                       const glf_weights* wl, void* z, void* saved_g, void* saved_l, glf_stream_t stream);
-/* Same pass, also storing the MGFM part on its own: z_global = LN_g(BN_g(U_g) + x_g) (bf16 token-major, like z) —
+/* Same pass, also storing the MGFM part on its own: z_global = LN_g(BN_g(U_g) + x_g) (token-major, dtype of z) —
  * f4_global_fusion of R/models/ours.py:1823, which the trainer's cycle-consistency pass consumes (R/main.py:211-235);
  * the MLFM part is z - z_global.  z_global == NULL is glf_fusion_ln_fwd. */
 GLF_API int glf_fusion_ln_fwd_parts(const glf_desc* d, const void* xg, const void* xl, const glf_weights* wg,
@@ -156,7 +161,7 @@ GLF_API int glf_fusion_ln_bwd_views(const glf_desc* d, const void* dz, const voi
                             glf_stream_t stream);
 
 /* Gate + view concat (ours.py:1802-1820,1826-1827).
- *   f4[v]  : [B, C, h, w]  io_dtype, NCHW contiguous, v < V (host array of V device pointers, V <= 8)
+ *   f4[v]  : [B, C, h, w]  io_dtype (bf16, fp16 or fp32), NCHW contiguous, v < V (host array of V device pointers, V <= 8)
  *   cls[v] : [B, ncls, h, w] fp32 logits of classifier[view];  ctr[v] : [B, 1, h, w] fp32 logits of centerness[view]
  *   xg, xl : [B, V*h*w, C] token-major (view-major token order, i.e. T = V), x_dtype (bf16, or fp32 for the
  *            GLF_PRECISION_F32X3 arm)                                                 — MGFM / MLFM inputs
@@ -192,7 +197,8 @@ GLF_API int glf_gate_concat_cl_bwd(int B, int C, int V, int h, int w, int ncls, 
 
 /* The dict-keyed call site's backward: V per-view gradients ([B, C, h, w]; element strides of batch / channel / the
  * collapsed h*w axis given per view, one of the last two must be 1: NCHW or channels-last) gathered into ONE
- * token-major [B, V, T, C] bf16 buffer, the transposition ours.py:1819-1820 performs forward (permute + cat).  A NULL
+ * token-major [B, V, T, C] bf16 buffer, the transposition ours.py:1819-1820 performs forward (permute + cat); src_dtype
+ * bf16, fp16 or fp32 (converted on the way).  A stride of 0 is allowed (a broadcast gradient).  A NULL
  * entry of `src` (a view whose output received no gradient) is written as zeros.  C % 64 == 0, V <= 8. */
 GLF_API int glf_views_to_tokens(int B, int C, int V, int T, int src_dtype, const void* const* src,
                         const int64_t* stride_b, const int64_t* stride_c, const int64_t* stride_t, void* out,
@@ -246,8 +252,8 @@ GLF_API int glf_gram_contraction(const void* A, const void* X, void* D, float* c
 
 /* The two HBM-bound fused epilogues as standalone entry points (unit tests, roofline probes).
  *   fwd: Z = LayerNorm_C(bn_a * U + bn_b + X) * ln_w + ln_b   (ours.py:908-915 after the W_z GEMM); U, X bf16 [rows, C];
- *        Z [rows, C] of z_dtype; mu, r: per-row LayerNorm mean / rstd (kept for backward).
- *   bwd: dV = d(pre-LayerNorm sum) [rows, C] bf16, and per-CTA partials [nblocks][4][C] of
+ *        Z [rows, C] of z_dtype (bf16, fp16 or fp32); mu, r: per-row LayerNorm mean / rstd (kept for backward).
+ *   bwd: dV = d(pre-LayerNorm sum) [rows, C] bf16 from dZ of dz_dtype, and per-CTA partials [nblocks][4][C] of
  *        (d ln_w, d ln_b, d bn_gamma, d bn_beta); *nblocks_out receives the number of partial rows written.
  *        `part` must hold glf_bn_res_ln_bwd_max_blocks() * 4 * C floats. */
 GLF_API int glf_bn_res_ln_fwd(int64_t rows, int C, const void* U, const void* X, const float* bn_a, const float* bn_b,
@@ -276,7 +282,7 @@ GLF_API int glf_bn_res_ln_pair_bwd(int64_t rows, int C, const void* dZ, const vo
 /* ---- the cycle-consistency step that consumes the MGFM output (R/main.py:229-235) ---------------------------------
  * glf_spatial_sums: out[b, c] = sum_t x[b, c, t] (fp32) for one view [B, C, h*w] given by element strides — replaces
  *   cyc_feat_out[view].sum(dim=(2, 3)) (R/main.py:229); channels-last views (stride_c == 1, what the fusion path
- *   returns) are read coalesced along C.
+ *   returns) are read coalesced along C.  dtype: GLF_DTYPE_BF16, GLF_DTYPE_F16 or GLF_DTYPE_F32.
  * glf_cycle_loss: Trainer.seg_cycle (R/main.py:650-717: n_starts = 1, start = the np.random.choice draw, scale = 1)
  *   and Trainer.dense_seg_cycle (R/main.py:719-798: start = 0, step = 1 or chunk_size, n_starts positions, scale =
  *   1 / (target_region - chunk_size - cyc_off + 1), soft_label as there) on the [T, C] fp32 per-frame features.
@@ -289,7 +295,8 @@ GLF_API int glf_cycle_loss(const float* feat, int T, int C, int target_region, i
                    float temperature, int start, int step, int n_starts, int soft_label, float scale, float* loss,
                    float* dfeat, void* scratch, glf_stream_t stream);
 
-/* out[b, s, r] = in[b, r, s] with dtype conversion (NCTHW <-> token-major packing). dtypes: GLF_DTYPE_*. */
+/* out[b, s, r] = in[b, r, s] with dtype conversion (NCTHW <-> token-major packing). dtypes: GLF_DTYPE_* (fp16 <-> bf16
+ * and fp16 <-> fp32 included). */
 GLF_API int glf_transpose(const void* in, void* out, int batch, int R, int S, int in_dtype, int out_dtype,
                   glf_stream_t stream);
 
