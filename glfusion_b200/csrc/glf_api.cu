@@ -14,7 +14,6 @@
 // (tpavi_fwd_gram / tpavi_bwd_gram below; oracle/tpavi_oracle.py: tpavi_dot_gram_form): theta / phi / g and dU are never
 // materialised, the only token-sized products are S = X^T X, U = X Q^T, R = dV^T X and dX = [dV | X] [E ; F].
 #include <cstdarg>
-#include <cstdlib>
 #include <cstdio>
 #include <cstring>
 
@@ -334,19 +333,9 @@ int check_ptr(const void* p, const char* name) {
 
 
 // ------------------------------------------------------------------------------------------------ Gram form of 'dot'
-// Tuning aids (GLF_GRAM_WIDE / GLF_GRAM_BIG = 128 | 256): N tile of the Ca-wide small products / of U and dX.
-// Measured on B200 at cfg2 (profiles/README.md): 128 / 128 is fastest (the 256-wide tile has only three ring stages
-// for four k-blocks per tile), so that is the default.
-int gram_wide_tile() {
-  const char* e = getenv("GLF_GRAM_WIDE");
-  const int v = e ? atoi(e) : 0;
-  return (v == 128 || v == 256) ? v : 128;
-}
-int gram_big_tile() {
-  const char* e = getenv("GLF_GRAM_BIG");
-  const int v = e ? atoi(e) : 0;
-  return (v == 128 || v == 256) ? v : 128;
-}
+// The Ca-wide small products and U / dX run on 128-wide N tiles (bn_hint = 128). Measured on B200 at cfg2
+// (profiles/README.md): 128 is faster than the 256-wide tile, which has only three ring stages for four k-blocks per
+// tile and which gemm()'s heuristic would pick for U and dX at C >= 512.
 
 // Token contraction of a sequence, S = A^T X (A = X or dV): both operands MN-major views of token-major
 // activations, the column sums of A as the GEMM's row-sum side product; result = the augmented bf16 matrix
@@ -356,8 +345,7 @@ int gram_token_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* s
                            const float* rowscale, float corner, int B, int N, int C, int Ca, cudaStream_t stream,
                            const GramPrep* prep = nullptr, bool* prep_done = nullptr) {
   if (prep_done != nullptr) *prep_done = false;
-  const char* ek = getenv("GLF_GRAM_KERNEL");   // tuning aid: 0 = always the generic tile GEMM
-  if (gram_contraction_supported(C) && !(ek && ek[0] == '0')) {
+  if (gram_contraction_supported(C)) {
     // one CTA per sequence; few long sequences are split along the tokens to fill two rounds of the SMs
     int ks = 1;
     if (B < 96) {
@@ -426,7 +414,6 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
   const long long CaCa = static_cast<long long>(Ca) * Ca, CiCa = static_cast<long long>(Ci) * Ca;
   const long long CCa = static_cast<long long>(C) * Ca, CiCi = static_cast<long long>(Ci) * Ci;
   const long long CCi = static_cast<long long>(C) * Ci;
-  const int wide = gram_wide_tile();
   const bf16* X = reinterpret_cast<const bf16*>(x);
   if (m.pack_x) {
     if (d->x_layout == GLF_LAYOUT_NCTHW)
@@ -455,7 +442,7 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
       g.B = opnd(s.Sa, 0, Ca, CaCa);
       g.B.rows = C1;
       g.M = Ci; g.N = Ca; g.K = C1; g.batch = B;
-      g.bn_hint = wide;
+      g.bn_hint = 128;
       g.D = s.T; g.ldd = Ca; g.strideD = CiCa;
       GLF_TRY(gemm(g, stream));
     }
@@ -482,7 +469,7 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
       g.B = opnd(s.waug, 1, Ca, 0);
       g.B.rows = C1;
       g.M = C; g.N = Ca; g.K = Ci; g.batch = B;
-      g.bn_hint = wide;
+      g.bn_hint = 128;
       g.D = s.Qb; g.ldd = Ca; g.strideD = CCa;
       GLF_TRY(gemm(g, stream));
     }
@@ -494,7 +481,7 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
     g.A = opnd(X, 0, C, static_cast<long long>(N) * C);
     g.B = opnd(s.Qb, 0, Ca, CCa);
     g.M = N; g.N = C; g.K = C; g.batch = B;
-    if (C % 256 == 0) g.bn_hint = gram_big_tile();
+    if (C % 256 == 0) g.bn_hint = 128;
     g.bias = s.cvec; g.bias_stride = C;
     g.D = s.U; g.ldd = C; g.strideD = static_cast<long long>(N) * C;
     g.colstats = (d->training && d->bn_layer) ? wf.colstats : nullptr;
@@ -525,7 +512,6 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
   const long long CCa = static_cast<long long>(C) * Ca, CiCi = static_cast<long long>(Ci) * Ci;
   const long long CCi = static_cast<long long>(C) * Ci, CC = static_cast<long long>(C) * C;
   const float invN = 1.f / static_cast<float>(N);
-  const int wide = gram_wide_tile();   // N tile of the products whose output is Ca (= C + 8) columns wide
   const bool bn_train = d->bn_layer && d->training;   // k2, k3 != 0 only then
   // k1 * [R_b | rv_b]  with R_b = dV_b^T X_b, rv_b = dV_b^T 1: the BatchNorm-backward scale k1 (per channel of dV =
   // row of R) is applied in fp32 by the contraction's epilogue
@@ -548,7 +534,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(s.Sa, 0, Ca, CaCa);
     g.B.rows = C1;
     g.M = C; g.N = Ca; g.K = C1; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.addend = wb.Rb; g.ld_add = Ca; g.stride_add = CaCa;
     g.D = wb.dQa; g.ldd = Ca; g.strideD = CCa;
     GLF_TRY(gemm(g, stream));
@@ -568,7 +554,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(wb.dQa, 1, Ca, CCa);
     g.B.rows = C1;
     g.M = Ci; g.N = Ca; g.K = C; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.out_kind = 2;
     g.D = wb.dwaug; g.ldd = Ca; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
@@ -597,7 +583,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(s.T, 1, Ca, CiCa);
     g.B.rows = C1;
     g.M = Ci; g.N = Ca; g.K = Ci; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.alpha = invN;
     g.out_kind = 2;
     g.D = wb.dwaug + 2 * CiCa; g.ldd = Ca; g.strideD = 0;
@@ -609,7 +595,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(s.waug + 2 * CiCa, 1, Ca, 0);
     g.B.rows = C1;
     g.M = Ci; g.N = Ca; g.K = Ci; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.alpha = invN;
     g.D = wb.dT; g.ldd = Ca; g.strideD = CiCa;
     GLF_TRY(gemm(g, stream));
@@ -620,7 +606,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(s.Sa, 0, Ca, CaCa);
     g.B.rows = C1;
     g.M = Ci; g.N = Ca; g.K = C1; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.out_kind = 2;
     g.D = wb.dwaug + CiCa; g.ldd = Ca; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
@@ -631,7 +617,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(wb.dT, 1, Ca, CiCa);
     g.B.rows = C1;
     g.M = C; g.N = Ca; g.K = Ci; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.D = wb.G0; g.ldd = Ca; g.strideD = CCa;
     GLF_TRY(gemm(g, stream));
   }
@@ -641,7 +627,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(wb.AK, 1, Ca, CCa);
     g.B.rows = C1;
     g.M = C; g.N = Ca; g.K = C; g.batch = B;
-    g.bn_hint = wide;
+    g.bn_hint = 128;
     g.D = wb.Hf; g.ldd = Ca; g.strideD = CCa;
     GLF_TRY(gemm(g, stream));
   }
@@ -652,9 +638,10 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.A = opnd(nullptr, 0, C, static_cast<long long>(N) * C);
     g.B = opnd(nullptr, 1, C, 2 * CC);
     g.M = N; g.N = C; g.K = C; g.batch = B;
-    if (C % 256 == 0) g.bn_hint = gram_big_tile();
+    if (C % 256 == 0) g.bn_hint = 128;
     g.bias = wb.evec; g.bias_stride = C;
-    if (!(chain && gram_residual_in_E())) { g.addend = wb.dV; g.ld_add = C; g.stride_add = static_cast<long long>(N) * C; }
+    // (the chain folds the residual dV into its E' = E + I)
+    if (!chain) { g.addend = wb.dV; g.ld_add = C; g.stride_add = static_cast<long long>(N) * C; }
     g.D = m.pack_x ? static_cast<void*>(wb.dxtok) : dx; g.ldd = C; g.strideD = static_cast<long long>(N) * C;
     GLF_TRY(gemm_pair2(g, wb.dV, X, wb.EF, wb.EF + CC, stream));
   }

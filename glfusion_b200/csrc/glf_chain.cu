@@ -408,7 +408,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1)
 }
 
 struct ChainBwdParams {
-  int N, has_k2, trace, e_plus_i;
+  int N, has_k2, trace;
   const float *sfv, *cvec, *rv, *k1, *k2, *k3;   // s, c, rv [B][C]; BatchNorm-backward coefficients [C]
   const float *bth, *bphi, *bg;                  // biases [C'] fp32
   const bf16* Rb;                                // [B][Ca][Ca]: rows < C hold k1 [R | rv]
@@ -604,7 +604,10 @@ __global__ void __launch_bounds__(CH_THREADS, 1)
       const float qs = row_dot256(sgen + Z0, 256, tid, v_s);
       v_dc[tid] = fmaf(v_k1[tid], p.rv[bC + tid], fmaf(v_k2[tid], fmaf(fN, my_c, qs), fN * p.k3[tid]));
       p.dcv[bC + tid] = v_dc[tid];
-      // E = k1 Q -> EF[b][0]   (a warp moves one 512-byte row per iteration)
+      // E' = k1 Q + I -> EF[b][0]   (a warp moves one 512-byte row per iteration).  The residual dV of
+      // dX = dV E + X F + 1 e^T + dV is folded into the first operand (one more bf16 rounding of the 256 diagonal entries:
+      // <= 2^-9 |dV_j| on dX_j, an order below the bf16 rounding of dX itself), so the dX GEMM needs no addend pass over
+      // dV in its epilogue and its tiles leave through bulk tensor stores.
       bf16* E = p.EF + static_cast<long long>(b) * 2 * CC * CC;
 #pragma unroll 2
       for (int it = 0; it < 32; ++it) {
@@ -617,8 +620,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1)
         for (int t = 0; t < 4; ++t) {
           const float2 x = unpack_bf16(q32[t]);
           const int col = lane * 8 + 2 * t;
-          o[t] = pack_bf16(a1 * x.x + ((p.e_plus_i && col == row) ? 1.f : 0.f),
-                           a1 * x.y + ((p.e_plus_i && col + 1 == row) ? 1.f : 0.f));
+          o[t] = pack_bf16(a1 * x.x + (col == row ? 1.f : 0.f), a1 * x.y + (col + 1 == row ? 1.f : 0.f));
         }
         *reinterpret_cast<uint4*>(E + static_cast<long long>(row) * CC + lane * 8) = make_uint4(o[0], o[1], o[2], o[3]);
       }
@@ -846,15 +848,6 @@ __global__ void __launch_bounds__(CH_THREADS, 1)
 
 }  // namespace
 
-// dX = dV E + X F + 1 e^T + dV: the residual term dV is folded into the first operand, E' = E + I (one more bf16 rounding
-// of the 256 diagonal entries: <= 2^-9 |dV_j| on dX_j, an order below the bf16 rounding of dX itself), so the dX GEMM
-// needs no addend pass over dV in its epilogue and its tiles leave through bulk tensor stores.  GLF_GRAM_RESIDUAL_IN_E=0
-// restores the separate addend.
-bool gram_residual_in_E() {
-  const char* e = getenv("GLF_GRAM_RESIDUAL_IN_E");
-  return !(e && e[0] == '0');
-}
-
 bool gram_chain_supported(int C, int Ci) {
   if (const char* e = getenv("GLF_GRAM_CHAIN")) {   // tuning aid: GLF_GRAM_CHAIN=0 keeps the batched tile GEMMs
     if (e[0] == '0') return false;
@@ -903,7 +896,6 @@ int gram_chain_bwd(const bf16* Sa, const bf16* Qb, const bf16* waug, const bf16*
   p.N = N; p.has_k2 = has_k2;
   const char* tr = getenv("GLF_CHAIN_TRACE");
   p.trace = (tr && tr[0] == '1') ? 1 : 0;
-  p.e_plus_i = gram_residual_in_E() ? 1 : 0;
   p.sfv = sfv; p.cvec = cvec; p.rv = rv; p.k1 = k1; p.k2 = k2; p.k3 = k3;
   p.bth = bth; p.bphi = bphi; p.bg = bg;
   p.Rb = Rb;

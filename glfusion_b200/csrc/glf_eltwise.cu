@@ -4,7 +4,6 @@
 // All row kernels use 128-bit loads/stores, one warp per (row, 256-channel slice), warp-shuffle reductions, and
 // per-CTA partials + fixed-order finalisation for every cross-row (per-channel) statistic, so results are
 // deterministic (SURVEY.md §7 "hard parts").
-#include <cstdlib>
 
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
@@ -1076,12 +1075,6 @@ template <typename... P>
 bool aligned16(const P*... ptrs) {
   return (((reinterpret_cast<uintptr_t>(ptrs)) | ...) & 15) == 0;
 }
-// GLF_DEBUG_LN_REG=1 forces the register-prefetch LayerNorm kernels (A/B against the bulk-copy staged ones)
-bool debug_reg_ln() {
-  const char* e = getenv("GLF_DEBUG_LN_REG");
-  return e != nullptr && e[0] == '1';
-}
-
 int row_grid(long long rows, int S) {
   const int RPB = ROW_WARPS / S;
   long long blocks = (rows + RPB - 1) / RPB;
@@ -1163,7 +1156,7 @@ int bn_res_ln_fwd(const void* U_, const void* X_, int act_dtype, const float* a,
     return set_error(GLF_ERR_INVALID, "LayerNorm kernel: an fp16 Z needs bf16 activations");
   const bool z16 = z_dtype == GLF_DTYPE_BF16 || z_dtype == GLF_DTYPE_F16;    // bf16 or fp16 Z: the fast paths
   if (act_dtype == GLF_DTYPE_BF16 && z16 && U_ != nullptr && ln_tma_supported(C) &&
-      aligned16(U_, X_, Z, a, b, lw, lb) && !debug_reg_ln()) {
+      aligned16(U_, X_, Z, a, b, lw, lb)) {
     const bf16* Ua[1] = {(const bf16*)U_};
     const bf16* Xa[1] = {(const bf16*)X_};
     const float *aa[1] = {a}, *ba[1] = {b}, *lwa[1] = {lw}, *lba[1] = {lb};
@@ -1175,7 +1168,7 @@ int bn_res_ln_fwd(const void* U_, const void* X_, int act_dtype, const float* a,
   const int grid = row_grid(rows, S);
   if (act_dtype == GLF_DTYPE_BF16) {
     const bf16* U = (const bf16*)U_; const bf16* X = (const bf16*)X_;
-    if (S > 1 && z16 && aligned16(U_ != nullptr ? U_ : X_, X_, Z) && !debug_reg_ln()) {
+    if (S > 1 && z16 && aligned16(U_ != nullptr ? U_ : X_, X_, Z)) {
       const size_t ring = LN_DEPTH * 3 * ROW_THREADS * sizeof(uint4);       // 48 KB
       const void* kern = z_dtype == GLF_DTYPE_F16 ? reinterpret_cast<const void*>(bn_res_ln_fwd_ring_kernel<f16>)
                                                   : reinterpret_cast<const void*>(bn_res_ln_fwd_ring_kernel<bf16>);
@@ -1247,7 +1240,7 @@ int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U_, const void* X_, 
     return set_error(GLF_ERR_INVALID, "LayerNorm backward: an fp16 dZ needs bf16 activations");
   const bool dz16 = dz_dtype == GLF_DTYPE_BF16 || dz_dtype == GLF_DTYPE_F16;  // bf16 or fp16 dZ: the fast paths
   if (act_dtype == GLF_DTYPE_BF16 && dz16 && U_ != nullptr && ln_tma_supported(C) &&
-      aligned16(dZ, U_, X_, dV_, a, b, lw, mu, r) && !debug_reg_ln()) {
+      aligned16(dZ, U_, X_, dV_, a, b, lw, mu, r)) {
     const bf16* Ua[1] = {(const bf16*)U_};
     const bf16* Xa[1] = {(const bf16*)X_};
     const float *aa[1] = {a}, *ba[1] = {b}, *lwa[1] = {lw}, *mna[1] = {mean}, *rsa[1] = {rstd}, *mua[1] = {mu},
@@ -1263,7 +1256,7 @@ int bn_res_ln_bwd(const void* dZ, int dz_dtype, const void* U_, const void* X_, 
   if (nblocks) *nblocks = grid;
   if (act_dtype == GLF_DTYPE_BF16) {
     const bf16* U = (const bf16*)U_; const bf16* X = (const bf16*)X_; bf16* dV = (bf16*)dV_;
-    if (S > 1 && dz16 && aligned16(U_ != nullptr ? U_ : X_, X_, dZ, dV_) && !debug_reg_ln()) {
+    if (S > 1 && dz16 && aligned16(U_ != nullptr ? U_ : X_, X_, dZ, dV_)) {
       const size_t ring = LN_DEPTH * 3 * ROW_THREADS * sizeof(uint4);
       const void* kern = dz_dtype == GLF_DTYPE_F16 ? reinterpret_cast<const void*>(bn_res_ln_bwd_ring_kernel<f16>)
                                                    : reinterpret_cast<const void*>(bn_res_ln_bwd_ring_kernel<bf16>);

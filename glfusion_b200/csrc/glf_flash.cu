@@ -1,14 +1,13 @@
 // glf_flash.cu — mode='embedded' (softmax) attention of TPAVIModule (R/models/ours.py:878-902 with
 // f_div_C = softmax(f, dim=-1)):   Y_b = softmax(Theta_b Phi_b^T) G_b      (no 1/sqrt(d) scale in the reference).
 //
-// Debug / odd-width path (this header): exact attention with the N x N score matrix materialised for a bounded CHUNK of sequences
+// Odd-width path (this header): exact attention with the N x N score matrix materialised for a bounded CHUNK of sequences
 // at a time (scratch sized by attn_chunk()), every product on the tcgen05 GEMM of glf_gemm.cu:
 //   fwd : S = Theta Phi^T (fp32) -> row softmax (P bf16, lse fp32) -> Y = P G
 //   bwd : recompute S ; dPm = dY G^T ; P = exp(S - lse) ; dS = P o (dPm - delta) ; delta = rowsum(dY o Y)
 //         dTheta = dS Phi ; dPhi = dS^T Theta ; dG = P^T dY        (transposes are MN-major operand reads, no copies)
 // Memory is O(chunk * N^2), independent of the batch size; HBM traffic is O(N^2) per sequence, which is what a
 // single-kernel flash version (scores kept in TMEM, online softmax in registers) removes — same entry points.
-#include <cstdlib>
 
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
@@ -874,9 +873,6 @@ static int attn_fwd_materialized(const bf16* P3, bf16* Y, float* lse, int B, int
 }
 
 int flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* scratch, cudaStream_t stream) {
-  if (const char* e = getenv("GLF_DEBUG_ATTN_MATERIALIZED")) {
-    if (e[0] == '1') return attn_fwd_materialized(P3, Y, lse, B, N, Ci, scratch, stream);
-  }
   if (Ci == 128) return launch_flash_fwd<128>(P3, Y, lse, B, N, stream);
   if (Ci == 64) return launch_flash_fwd<64>(P3, Y, lse, B, N, stream);
   return attn_fwd_materialized(P3, Y, lse, B, N, Ci, scratch, stream);   // other head widths: exact chunked path
@@ -991,9 +987,7 @@ int flash_bwd_colsum_blocks(long long rows) {
 int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3, float* delta, float* cs_t,
               float* cs_p, float* cs_g, int cs_cap_rows, int* cs_rows_out, int B, int N, int Ci, void* scratch,
               cudaStream_t stream) {
-  bool materialized = !(Ci == 128 || Ci == 64);
-  if (const char* e = getenv("GLF_DEBUG_ATTN_MATERIALIZED")) materialized = materialized || e[0] == '1';
-  if (materialized)
+  if (Ci != 128 && Ci != 64)   // other head widths: exact chunked path
     return attn_bwd_materialized(P3, Y, dY, lse, dP3, delta, cs_t, cs_p, cs_g, cs_rows_out, B, N, Ci, scratch, stream);
   const long long rows = static_cast<long long>(B) * N;
   {

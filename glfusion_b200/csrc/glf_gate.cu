@@ -7,7 +7,6 @@
 // chained through the two sigmoids / the class max to the logits.
 // f4 / df4 may be bf16, fp16 or fp32; the token-major operands are bf16 (fp32 for the F32X3 arm).  fp16 f4 is converted
 // where it is read and df4 rounded to fp16 where it is written: the fp16 forms move the same bytes as the bf16 ones.
-#include <cstdlib>
 #include <type_traits>
 
 #include "glf_internal.h"
@@ -502,7 +501,6 @@ bool gate_tma_ok(int C, int hw, int io_dtype, int x_dtype, const void* const* f4
   if (C > 512 && C % 512 != 0) return false;      // wider rows are cut into 512- (forward) / 256-channel (backward) slabs
   for (int v = 0; v < V; ++v)
     if ((reinterpret_cast<uintptr_t>(f4[v]) & 15) != 0) return false;
-  if (const char* e = getenv("GLF_DEBUG_GATE_SIMT")) return e[0] != '1';
   return true;
 }
 

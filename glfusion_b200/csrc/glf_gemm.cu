@@ -15,7 +15,6 @@
 //                               squares) for the BatchNorm that follows W_z (ours.py:908).
 // Operands may be K-major ([rows, K]) or MN-major ([K, rows]); the latter is how the token-contraction products
 // (Phi^T G, dU^T Theta, dP^T X) read token-major activations without any transposed copy.
-#include <cstdlib>
 #include <mutex>
 
 #include "glf_internal.h"
@@ -53,8 +52,6 @@ struct GemmKParams {
   long long bias_stride;         // elements between the bias vectors of consecutive batch entries (0 = shared)
   float* rowsum;                 // optional [batch][M] fp32: sum over K of the A operand's row (BN <= 128, npairs == 1)
   long long rowsum_stride;
-  int dbg;                       // tuning aid (GLF_GEMM_DBG): 1 skip the MMAs of the second M sub-tile, 2 skip the epilogue's
-                                 // staging and stores, 4 skip the loads of the second A sub-tile (results are then WRONG)
 };
 
 // MT = 128-row accumulators per CTA tile: MT = 2 computes a 256 x BN super-tile, so each k-block of the B operand is
@@ -65,7 +62,7 @@ struct GemmCfg {
   // persistent kernel, one CTA per SM: ring + separate epilogue staging must fit in 227 KB
   // MT = 2: every spare byte goes to the ring (the big K-major products are bound by bytes in flight per SM: with
   // three 48 KB stages the ring turns over once per HBM round trip, ~76 GB/s per SM; profiles/r02_gemm_bound_probe.txt)
-  static constexpr int STAGES = (MT == 2) ? ((BN == 256) ? 3 : 4) : ((BN == 256) ? 3 : ((BN == 128) ? 5 : 6));
+  static constexpr int STAGES = (MT == 2) ? 4 : ((BN == 256) ? 3 : ((BN == 128) ? 5 : 6));
   static constexpr uint32_t A_TILE = BM * BK * 2;
   static constexpr uint32_t A_BYTES = MT * A_TILE;
   static constexpr uint32_t B_BYTES = BN * BK * 2;
@@ -73,23 +70,21 @@ struct GemmCfg {
   static constexpr uint32_t RING_BYTES = STAGES * STAGE_BYTES;
   static constexpr uint32_t WARP_STG = 32 * 64;     // warp-private 32 rows x 32 bf16, XOR-swizzled 16-byte chunks
   static constexpr uint32_t WARP_BIAS = 32 * 4;     // warp-private bias slice of the current 32-column chunk
-  // 256 x 256 CTA tiles (MT = 2, BN = 256): every byte of shared memory goes to the ring; no CTA-wide bias copy, no
-  // ones tile, a single accumulator stage (all 512 TMEM columns)
-  static constexpr bool WIDE2 = (MT == 2);          // (both MT = 2 shapes run without the CTA-wide bias copy / ones tile)
-  static constexpr uint32_t BIAS_ALL = WIDE2 ? 0 : 4096 * 4;   // the whole bias vector (N <= 4096) is staged once per CTA
+  // MT = 2 runs without the CTA-wide bias copy and the ones tile: those bytes go to the ring
+  static constexpr uint32_t BIAS_ALL = (MT == 2) ? 0 : 4096 * 4;   // the whole bias vector (N <= 4096) is staged once per CTA
   static constexpr uint32_t EPI_BYTES = EPI_WARPS * (WARP_STG + WARP_BIAS) + BIAS_ALL;
   // all-ones K-major B tile [16 rows][64 k] for the row-sum side product (RING_BYTES and EPI_BYTES are multiples of
   // 1024, so it sits on a swizzle-atom boundary)
-  static constexpr uint32_t ONES_BYTES = WIDE2 ? 0 : 2048;
+  static constexpr uint32_t ONES_BYTES = (MT == 2) ? 0 : 2048;
   static constexpr uint32_t BAR_BYTES = 256;        // mbarriers + TMEM address, after the ones tile
-  static constexpr uint32_t SLACK = WIDE2 ? 512 : 1024;   // alignment slack of the dynamic shared-memory base
+  static constexpr uint32_t SLACK = (MT == 2) ? 512 : 1024;   // alignment slack of the dynamic shared-memory base
   static constexpr uint32_t SMEM_BYTES = RING_BYTES + EPI_BYTES + ONES_BYTES + BAR_BYTES + SLACK;
   // two accumulator stages (+ two 16-column row-sum accumulators at column 2 BN when BN <= 128)
   static constexpr uint32_t TMEM_COLS = (BN == 64) ? 256 : 512;
   static constexpr uint32_t ACC_COLS = MT * BN;     // TMEM columns of one accumulator stage
   static constexpr int NACC = (2 * ACC_COLS <= TMEM_COLS) ? 2 : 1;   // accumulator stages
   static constexpr uint32_t RS_COL = 2 * BN;        // (MT == 1 only)
-  static_assert(MT == 1 || (MT == 2 && BN >= 128), "MT = 2 is instantiated for BN = 128 / 256");
+  static_assert(MT == 1 || (MT == 2 && BN == 128), "MT = 2 is instantiated for BN = 128");
   static_assert(NACC * ACC_COLS <= TMEM_COLS, "TMEM budget of the accumulator stages");
   static_assert(EPI_BYTES % 1024 == 0 && RING_BYTES % 1024 == 0, "ones tile alignment");
   static_assert(SMEM_BYTES <= 232448, "shared memory budget");
@@ -111,18 +106,12 @@ __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, 
 
 // Persistent: CTA c processes tiles c, c + gridDim.x, ... ; tile index runs n-tile fastest, then m-tile, then
 // (batch, k-split), so the CTAs that are resident together share A slabs through L2.
-// CL2: launched as clusters of two CTAs that work on the two n-tiles of the same 256-row super-tile (the tile index
-// runs n-tile fastest and the grid is even): each CTA fetches ONE of the two 128-row A sub-tiles and multicasts it into
-// both CTAs' rings, so the A operand crosses the L2 -> SM fabric once instead of twice (the big K-major products are
-// bound by that fabric: profiles/r02_gemm_bound_probe.txt).
-template <bool A_MN, bool B_MN, int BN, int MT = 1, bool CL2 = false>
+template <bool A_MN, bool B_MN, int BN, int MT = 1>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
     gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                 const __grid_constant__ CUtensorMap tmD, const GemmKParams p) {
   using Cfg = GemmCfg<BN, MT>;
   static_assert(MT == 1 || !A_MN, "MT = 2 takes a K-major A operand");
-  static_assert(!CL2 || MT == 2, "the cluster variant shares the two A sub-tiles of a 256-row super-tile");
-  const uint32_t crank = CL2 ? cluster_ctarank() : 0u;
   constexpr int BMT = BM * MT;                 // output rows of one CTA tile
   constexpr int STAGES = Cfg::STAGES;
   constexpr int NACC = Cfg::NACC;
@@ -150,7 +139,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 #pragma unroll
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(smem_u32(&full_bar[s]), 1);
-      mbar_init(smem_u32(&empty_bar[s]), CL2 ? 2 : 1);   // CL2: both CTAs' MMAs must have consumed the slot
+      mbar_init(smem_u32(&empty_bar[s]), 1);
     }
 #pragma unroll
     for (int s = 0; s < 2; ++s) {
@@ -169,7 +158,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
   }
   tc_fence_before();
   __syncthreads();
-  if (CL2) cluster_sync_all();     // the peer's barriers are initialised before anything is multicast to them
   tc_fence_after();
   const uint32_t tmem_base = tmem_holder;
 
@@ -195,13 +183,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
           mbar_expect_tx(fb, Cfg::STAGE_BYTES);
           const uint32_t sa = smem_base + stage * Cfg::STAGE_BYTES;
           const uint32_t sb = sa + Cfg::A_BYTES;
-          if (CL2) {
-            // this CTA's half of the A stage goes to both CTAs; the peer delivers the other half
-            tma_load_4d_mcast(&tmA, fb, sa + crank * Cfg::A_TILE, k0, m0 + static_cast<int>(crank) * BM, ab,
-                              p.pairA[pair], static_cast<uint16_t>(3));
-          } else if (!A_MN) {
+          if (!A_MN) {
 #pragma unroll
-            for (int j = 0; j < MT; ++j) tma_load_4d(&tmA, fb, sa + j * Cfg::A_TILE, k0, ((p.dbg & 4) ? m0 : m0 + j * BM), ab, p.pairA[pair]);
+            for (int j = 0; j < MT; ++j) tma_load_4d(&tmA, fb, sa + j * Cfg::A_TILE, k0, m0 + j * BM, ab, p.pairA[pair]);
           } else {
             tma_load_4d(&tmA, fb, sa, m0, k0, ab, p.pairA[pair]);
             tma_load_4d(&tmA, fb, sa + 8192, m0 + 64, k0, ab, p.pairA[pair]);
@@ -250,7 +234,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
           for (int k = 0; k < BK / 16; ++k) {
             const uint64_t bd = B_MN ? make_sdesc(sb + k * 2048, 8192, 1024) : make_sdesc(sb + k * 32, 16, 1024);
 #pragma unroll
-            for (int j = 0; j < ((p.dbg & 1) ? 1 : MT); ++j) {
+            for (int j = 0; j < MT; ++j) {
               const uint64_t ad = A_MN ? make_sdesc(sa + k * 2048, 8192, 1024)
                                        : make_sdesc(sa + j * Cfg::A_TILE + k * 32, 16, 1024);
               umma_f16(tacc + j * BN, ad, bd, idesc, (it | k) != 0 ? 1u : 0u);
@@ -265,8 +249,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                        (it | k) != 0 ? 1u : 0u);
             }
           }
-          if (CL2) umma_commit_mcast(smem_u32(&empty_bar[stage]), static_cast<uint16_t>(3));
-          else umma_commit(smem_u32(&empty_bar[stage]));  // slot reusable once these MMAs have read it
+          umma_commit(smem_u32(&empty_bar[stage]));  // slot reusable once these MMAs have read it
           if (++stage == STAGES) {
             stage = 0;
             phase ^= 1u;
@@ -357,7 +340,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
         __syncwarp();
         if (sub == MT - 1 && c + 4 >= NCHUNK && lane == 0)   // last TMEM read of this warp for the tile: release it
           mbar_arrive(smem_u32(&tmem_empty_bar[acc]));
-        if (p.dbg & 2) continue;
         float2 f[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) f[j] = make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
@@ -551,7 +533,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
   }
   tc_fence_before();
   __syncthreads();
-  if (CL2) cluster_sync_all();     // no CTA leaves while its peer may still multicast into it / signal its barriers
   if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
@@ -643,11 +624,11 @@ int make_tmap_bf16(CUtensorMap* tm, const void* ptr, long long inner, long long 
 
 namespace {
 
-template <bool A_MN, bool B_MN, int BN, int MT = 1, bool CL2 = false>
+template <bool A_MN, bool B_MN, int BN, int MT = 1>
 int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmD, GemmKParams p, int num_sms,
            int* cs_rows, cudaStream_t stream) {
   using Cfg = GemmCfg<BN, MT>;
-  auto kern = gemm_kernel<A_MN, B_MN, BN, MT, CL2>;
+  auto kern = gemm_kernel<A_MN, B_MN, BN, MT>;
   p.tiles_m = (p.M + BM * MT - 1) / (BM * MT);
   // per launch: the attribute is per device, and callers may drive several GPUs from one process (nn.DataParallel)
   cudaError_t attr_err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
@@ -669,22 +650,6 @@ int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tm
   p.step_n = grid % p.tiles_n;
   p.step_m = (grid / p.tiles_n) % p.tiles_m;
   p.step_z = grid / (p.tiles_m * p.tiles_n);
-  if (CL2) {
-    if (grid % 2 != 0 || total % 2 != 0 || p.tiles_n != 2) return set_error(GLF_ERR_INVALID, "gemm: cluster variant needs an even grid and two n-tiles");
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(GEMM_THREADS);
-    cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return check_cuda(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmD, p), "gemm launch (cluster)");
-  }
   kern<<<grid, GEMM_THREADS, Cfg::SMEM_BYTES, stream>>>(tmA, tmB, tmD, p);
   return check_cuda(cudaGetLastError(), "gemm launch");
 }
@@ -716,10 +681,6 @@ int gemm(const GemmArgs& a, cudaStream_t stream) {
   // loads.  Large-K (tensor-bound, e.g. C=2048) products take the 128x256 tile.
   int BN = (a.N <= 64) ? 64 : ((a.K >= 512 && a.N % 256 == 0) ? 256 : 128);
   if (a.bn_hint == 64 || a.bn_hint == 128 || a.bn_hint == 256) BN = a.bn_hint;
-  if (const char* e = getenv("GLF_DEBUG_BN")) {  // tuning aid: force the N tile of K-major x K-major products
-    const int v = atoi(e);
-    if ((v == 128 || v == 256) && a.N > 64 && !a.A.mn_major) BN = v;
-  }
   if (a.rowsum != nullptr && BN > 128) BN = 128;   // the side accumulator needs TMEM columns beyond the two stages
   int dev = 0, num_sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess ||
@@ -729,20 +690,6 @@ int gemm(const GemmArgs& a, cudaStream_t stream) {
   // the big K-major products with N = 256 (U, dX of the Gram form) run on CTA pairs (glf_gemm2.cu)
   if (gemm_bres_applicable(a, num_sms)) return gemm_bres(a, num_sms, stream);
   if (gemm_pair_applicable(a, num_sms)) return gemm_pair(a, num_sms, stream);
-  // GLF_GEMM_WIDE2=1 (or bn_hint = 512): 256 x 256 CTA tiles for N == 256 (one n-tile: the A operand crosses the
-  // L2 -> SM fabric once, the B operand once per 256 rows)
-  bool wide2 = !amn && a.N == 256 && a.rowsum == nullptr && a.M >= 1024 && a.split_k <= 1;
-  {
-    const char* e = getenv("GLF_GEMM_WIDE2");
-    wide2 = wide2 && (a.bn_hint == 512 || (e && e[0] == '1'));
-    if (e && e[0] == '0') wide2 = false;
-    if (wide2 && a.colstats != nullptr) {   // the per-CTA running column statistics need grid <= batch * m-tiles
-      const long long tm2 = (a.M + 2 * BM - 1) / (2 * BM);
-      const long long total = tm2 * a.batch;
-      wide2 = (total < num_sms ? total : num_sms) <= static_cast<long long>(a.batch) * tm2;
-    }
-  }
-  if (wide2) BN = 256;
   int nlimbsA = 1, nlimbsB = 1;
   for (int i = 0; i < a.npairs; ++i) {
     nlimbsA = a.pairA[i] + 1 > nlimbsA ? a.pairA[i] + 1 : nlimbsA;
@@ -754,10 +701,9 @@ int gemm(const GemmArgs& a, cudaStream_t stream) {
   rc = make_operand_map(&tmB, a.B, a.B.rows > 0 ? a.B.rows : a.N, a.K, a.batch, nlimbsB, BN);
   if (rc) return rc;
 
-  // bf16 outputs without a residual addend leave through bulk tensor stores (GLF_DEBUG_NO_TMA_STORE=1: per-lane stores)
+  // bf16 outputs without a residual addend leave through bulk tensor stores
   CUtensorMap tmD = tmA;
-  bool tma_store = a.out_kind == 0 && a.addend == nullptr && a.M >= 32 && a.N >= 32 && a.strideD % 8 == 0;
-  if (const char* e = getenv("GLF_DEBUG_NO_TMA_STORE")) tma_store = tma_store && e[0] != '1';
+  const bool tma_store = a.out_kind == 0 && a.addend == nullptr && a.M >= 32 && a.N >= 32 && a.strideD % 8 == 0;
   if (tma_store) {
     rc = make_output_map(&tmD, a.D, a.M, a.N, a.batch, a.ldd, a.strideD);
     if (rc) return rc;
@@ -785,42 +731,20 @@ int gemm(const GemmArgs& a, cudaStream_t stream) {
   p.rowsum = a.rowsum;
   p.rowsum_stride = a.rowsum_stride;
   p.cs_accum = 0;
-  {
-    const char* e = getenv("GLF_GEMM_DBG");
-    p.dbg = e ? atoi(e) : 0;
-  }
   p.tiles_m = gemm_tiles_m(a.M);
   p.tiles_n = 0;  // set per tile shape in launch()
   // 256-row super-tiles (MT = 2) for the big K-major products: halves the B-operand traffic per output row.  The
   // column statistics need the per-CTA running-sum mode there (one partial row per CTA).
-  bool mt2 = !amn && (BN == 128 || wide2) && a.rowsum == nullptr && a.M >= 1024;
-  if (const char* e = getenv("GLF_GEMM_MT")) mt2 = mt2 && e[0] != '1';   // tuning aid: GLF_GEMM_MT=1 disables it
+  bool mt2 = !amn && BN == 128 && a.rowsum == nullptr && a.M >= 1024;
   if (mt2 && a.colstats != nullptr) {
     const long long tm2 = (a.M + 2 * BM - 1) / (2 * BM), tn = (a.N + BN - 1) / BN;
     const long long total = tm2 * tn * a.batch * p.split_k;
     const long long grid = total < num_sms ? total : num_sms;
     mt2 = tn * ((BN / 32 + 3) / 4) <= 4 && grid <= static_cast<long long>(a.batch) * tm2;
   }
-  if (mt2 && wide2)
-    return bmn ? launch<false, true, 256, 2>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream)
-               : launch<false, false, 256, 2>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream);
-
-  if (mt2) {
-    // two n-tiles, an even number of CTAs and of tiles: CTA pairs share the A operand through TMA multicast
-    bool cl2 = a.N > 128 && a.N <= 256 && num_sms % 2 == 0 &&
-               (static_cast<long long>((a.M + 2 * BM - 1) / (2 * BM)) * 2 * a.batch * p.split_k) >= num_sms;
-    // measured (profiles/r02_gemm_bound_probe.txt): no gain on B200 — multicast to a 2-CTA cluster does not reduce the
-    // L2 output traffic — so it stays off unless GLF_GEMM_CL2=1
-    {
-      const char* e = getenv("GLF_GEMM_CL2");
-      cl2 = cl2 && e != nullptr && e[0] == '1';
-    }
-    if (cl2)
-      return bmn ? launch<false, true, 128, 2, true>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream)
-                 : launch<false, false, 128, 2, true>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream);
+  if (mt2)
     return bmn ? launch<false, true, 128, 2>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream)
                : launch<false, false, 128, 2>(tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream);
-  }
   switch (BN) {
     case 64: return launch_major<64>(amn, bmn, tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream);
     case 128: return launch_major<128>(amn, bmn, tmA, tmB, tmD, p, num_sms, a.colstats_rows, stream);

@@ -12,10 +12,8 @@
 //               counted on the LEADER's full barrier (cp.async.bulk.tensor ... .cta_group::2)
 //   warp 1      MMA issuer (leader only); tcgen05.commit multicasts to both CTAs' empty / accumulator-full barriers
 //   warps 2-17  epilogue (both CTAs): tcgen05.ld -> bias -> bf16 staging -> bulk tensor stores (+ BatchNorm column
-//               statistics as per-CTA running sums); the last read of an accumulator stage arrives on the LEADER's
-//               accumulator-empty barrier (count = both CTAs' epilogue warps)
-#include <cstdlib>
-
+//               statistics, one partial row per 32-row sub-block); the last read of an accumulator stage arrives on the
+//               LEADER's accumulator-empty barrier (count = both CTAs' epilogue warps)
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
 
@@ -47,16 +45,14 @@ struct Gemm2Params {
   int total;               // pair tiles
   const float* bias;
   long long bias_stride;
-  float* colstats;         // [gridDim.x][2][N] per-CTA running sums (or null)
-  int cs_blocks;           // 1: N spans several column tiles -> one partial row per 32-row sub-block instead,
-  int tiles_m128;          //    [batch * tiles_m128 * 4][2][N] (the single-CTA kernel's table layout)
+  float* colstats;         // [batch * tiles_m128 * 4][2][N]: one partial row per 32-row sub-block (or null),
+  int tiles_m128;          //    the single-CTA kernel's table layout
   float alpha;
   const bf16* addend;      // optional bf16 [M, N] added before the store
   long long ld_add, stride_add;
   int split_k, kb_per_split;   // K slices per tile (fp32 atomic output only)
   float* Df;               // out_kind 2: fp32 output, red.global.add (split-K slices / batch-reduced products)
   long long ldd, strideD;
-  int dbg;                 // tuning aid (GLF_GEMM_DBG & 2): skip the epilogue's staging and stores (results WRONG)
 };
 
 __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
@@ -183,8 +179,6 @@ __global__ void __launch_bounds__(G2_THREADS, 1)
     int nchunk = 0;
     const int sw_w = (lane >> 1) & 3;
     const int hl = lane & 15, half = lane >> 4;
-    float2 cs1[2], cs2[2];
-    cs1[0] = cs1[1] = cs2[0] = cs2[1] = make_float2(0.f, 0.f);
     const uint32_t leader_empty0 = mapa_shared(smem_u32(&tmem_empty_bar[0]), 0);
     const uint32_t leader_empty1 = mapa_shared(smem_u32(&tmem_empty_bar[1]), 0);
     int local = 0;
@@ -218,7 +212,6 @@ __global__ void __launch_bounds__(G2_THREADS, 1)
         tc_fence_before();
         __syncwarp();
         if (ci == 1 && lane == 0) mbar_arrive_cluster(acc == 0 ? leader_empty0 : leader_empty1);
-        if (p.dbg & 2) continue;
         float2 f[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) f[j] = make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
@@ -295,14 +288,11 @@ __global__ void __launch_bounds__(G2_THREADS, 1)
           sa2.y += __shfl_xor_sync(0xffffffffu, sa2.y, 16);
           sq2.x += __shfl_xor_sync(0xffffffffu, sq2.x, 16);
           sq2.y += __shfl_xor_sync(0xffffffffu, sq2.y, 16);
-          if (p.cs_blocks) {
-            if (half == 0 && m0 < p.M) {                       // (a 128-row half entirely beyond M has no table rows)
-              float* cs = p.colstats + ((static_cast<long long>(b) * p.tiles_m128 + (m0 >> 7)) * 4 + q) * 2 * p.N;
-              *reinterpret_cast<float2*>(cs + gc0 + 2 * hl) = sa2;
-              *reinterpret_cast<float2*>(cs + p.N + gc0 + 2 * hl) = sq2;
-            }
-          } else if (ci == 0) { cs1[0] = add2(cs1[0], sa2); cs2[0] = add2(cs2[0], sq2); }
-          else { cs1[1] = add2(cs1[1], sa2); cs2[1] = add2(cs2[1], sq2); }
+          if (half == 0 && m0 < p.M) {                         // (a 128-row half entirely beyond M has no table rows)
+            float* cs = p.colstats + ((static_cast<long long>(b) * p.tiles_m128 + (m0 >> 7)) * 4 + q) * 2 * p.N;
+            *reinterpret_cast<float2*>(cs + gc0 + 2 * hl) = sa2;
+            *reinterpret_cast<float2*>(cs + p.N + gc0 + 2 * hl) = sq2;
+          }
         }
         fence_proxy_async_smem();
         __syncwarp();
@@ -313,37 +303,6 @@ __global__ void __launch_bounds__(G2_THREADS, 1)
       }
     }
     if (lane == 0) tma_store_wait_all<0>();
-    if (p.colstats != nullptr && !p.cs_blocks) {
-      // ONE partial row per CTA: the four warps that share a column chunk (one per 32-row quarter) combine their
-      // running sums through the idle staging tiles, in a fixed order
-      __syncwarp();
-      uint8_t* wstg = wstg0;
-      float2* xs = reinterpret_cast<float2*>(wstg);            // [slot][sum | sum of squares][16 column pairs]
-      if (half == 0) {
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-          xs[(2 * i) * 16 + hl] = cs1[i];
-          xs[(2 * i + 1) * 16 + hl] = cs2[i];
-        }
-      }
-      named_bar_sync(1, EPI_THREADS);
-      if ((ew & 3) == 0 && half == 0) {
-        float* cs = p.colstats + static_cast<long long>(blockIdx.x) * 2 * p.N;
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-          const int col = (cc0 + 4 * i) * 32 + 2 * hl;
-          float2 t1 = make_float2(0.f, 0.f), t2 = make_float2(0.f, 0.f);
-#pragma unroll
-          for (int w4 = 0; w4 < 4; ++w4) {
-            const float2* o = reinterpret_cast<const float2*>(wstg + w4 * 2 * WARP_STG);
-            t1 = add2(t1, o[(2 * i) * 16 + hl]);
-            t2 = add2(t2, o[(2 * i + 1) * 16 + hl]);
-          }
-          *reinterpret_cast<float2*>(cs + col) = t1;
-          *reinterpret_cast<float2*>(cs + p.N + col) = t2;
-        }
-      }
-    }
   }
   tc_fence_before();
   __syncthreads();
@@ -375,8 +334,6 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
 }  // namespace
 
 bool gemm_pair_applicable(const GemmArgs& a, int num_sms) {
-  const char* e = getenv("GLF_GEMM_PAIR");       // tuning aid: GLF_GEMM_PAIR=0 keeps the single-CTA tiles
-  if (e && e[0] == '0') return false;
   if (a.N % BN2 != 0 || a.M < 1024 || a.out_kind == 1 || a.rowsum != nullptr) return false;
   if (a.npairs > 6 || num_sms < 2) return false;
   if (a.out_kind == 0 && (a.split_k > 1 || a.strideD % 8 != 0)) return false;
@@ -388,16 +345,13 @@ bool gemm_pair_applicable(const GemmArgs& a, int num_sms) {
   if (a.K % BK != 0 && !(a.A.mn_major && a.B.mn_major)) return false;   // (a K tail is zero-filled by TMA for MN-major operands)
   if (a.addend != nullptr && (a.ld_add % 8 != 0 || a.stride_add % 8 != 0 || (reinterpret_cast<uintptr_t>(a.addend) & 15) != 0))
     return false;
-  if (a.colstats != nullptr && a.N == BN2) {   // measured at K = 256: with the column statistics in the epilogue the
-    const char* ec = getenv("GLF_GEMM_PAIR_STATS");   // single-CTA tile is faster (HBM-bound shape)
-    if (!(ec && ec[0] == '1')) return false;
-  }
+  // measured at K = 256: with the column statistics in the epilogue the single-CTA tile is faster (HBM-bound shape)
+  if (a.colstats != nullptr && a.N == BN2) return false;
   // several column tiles (the C = 2048 products): per-sub-block partial rows; worth it once the product is tensor-bound
-  if (a.colstats != nullptr && a.N != BN2 && a.K < 1024) return false;
+  if (a.colstats != nullptr && a.K < 1024) return false;
   const long long tiles = static_cast<long long>((a.M + 255) / 256) * a.batch * (a.N / BN2) * (a.split_k > 1 ? a.split_k : 1);
   const int grid = (num_sms / 2) * 2;
   if (tiles < grid / 2) return false;            // not enough pair tiles to fill the machine
-  if (a.colstats != nullptr && a.N == BN2 && grid > static_cast<long long>(a.batch) * ((a.M + 127) / 128) * 4) return false;
   return true;
 }
 
@@ -439,19 +393,13 @@ int gemm_pair(const GemmArgs& a, int num_sms, cudaStream_t stream) {
   p.bias = a.bias;
   p.bias_stride = a.bias != nullptr ? a.bias_stride : 0;
   p.colstats = a.colstats;
-  p.cs_blocks = a.colstats != nullptr && a.N != BN2;
   p.tiles_m128 = gemm_tiles_m(a.M);
   p.alpha = a.alpha;
   p.addend = a.addend;
   p.ld_add = a.ld_add;
   p.stride_add = a.stride_add;
-  {
-    const char* e = getenv("GLF_GEMM_DBG");
-    p.dbg = e ? atoi(e) : 0;
-  }
   const int grid = (num_sms / 2) * 2;
-  if (a.colstats_rows != nullptr)
-    *a.colstats_rows = a.colstats == nullptr ? 0 : (p.cs_blocks ? a.batch * p.tiles_m128 * 4 : grid);
+  if (a.colstats_rows != nullptr) *a.colstats_rows = a.colstats == nullptr ? 0 : a.batch * p.tiles_m128 * 4;
   if (a.A.mn_major)
     return a.B.mn_major ? launch_pair<true, true>(tmA, tmB, tmD, p, grid, stream)
                         : launch_pair<true, false>(tmA, tmB, tmD, p, grid, stream);

@@ -12,8 +12,6 @@
 //   warp 1      MMA issuer: M = 128, N = 256, K = 16 tcgen05.mma, two TMEM accumulator stages of 256 columns
 //   warps 2-17  epilogue: tcgen05.ld -> per-sequence bias -> bf16 staging -> bulk tensor store (+ BatchNorm column
 //               statistics of the stored values as per-CTA running sums, one partial row per CTA, fixed order)
-#include <cstdlib>
-
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
 
@@ -45,7 +43,6 @@ struct Gemm3Params {
   long long bias_stride;
   float* colstats;         // [gridDim.x][2][N] per-CTA running sums (or null)
   float alpha;
-  int dbg;                 // tuning aid (GLF_GEMM_DBG & 2): skip the epilogue's staging and stores (results WRONG)
 };
 
 __global__ void __launch_bounds__(G3_THREADS, 1)
@@ -199,7 +196,6 @@ __global__ void __launch_bounds__(G3_THREADS, 1)
         tc_fence_before();
         __syncwarp();
         if (ci == 1 && lane == 0) mbar_arrive(smem_u32(&tmem_empty_bar[acc]));
-        if (p.dbg & 2) continue;
         float2 f[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) f[j] = make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
@@ -294,8 +290,6 @@ __global__ void __launch_bounds__(G3_THREADS, 1)
 }  // namespace
 
 bool gemm_bres_applicable(const GemmArgs& a, int num_sms) {
-  const char* e = getenv("GLF_GEMM_BRES");       // tuning aid: GLF_GEMM_BRES=0 keeps the tile GEMMs
-  if (e && e[0] == '0') return false;
   if (a.A.mn_major || a.B.mn_major || a.N != BN3 || a.K % BK != 0 || a.K > G3_KB_MAX * BK) return false;
   if (a.out_kind != 0 || a.addend != nullptr || a.rowsum != nullptr || a.split_k > 1 || a.npairs != 1) return false;
   if (a.A.limb_stride != 0 || a.B.limb_stride != 0 || a.strideD % 8 != 0) return false;
@@ -325,10 +319,6 @@ int gemm_bres(const GemmArgs& a, int num_sms, cudaStream_t stream) {
   p.bias_stride = a.bias != nullptr ? a.bias_stride : 0;
   p.colstats = a.colstats;
   p.alpha = a.alpha;
-  {
-    const char* e = getenv("GLF_GEMM_DBG");
-    p.dbg = e ? atoi(e) : 0;
-  }
   const int grid = num_sms < p.total ? num_sms : p.total;
   if (a.colstats_rows != nullptr) *a.colstats_rows = a.colstats != nullptr ? grid : 0;
   cudaError_t e = cudaFuncSetAttribute(gemm_bres_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G3_SMEM);

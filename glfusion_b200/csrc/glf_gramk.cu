@@ -351,10 +351,7 @@ int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch
   p.kb_per_split = (p.kb_total + ks - 1) / ks;
   p.ksplit = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
   p.same = (A == X) ? 1 : 0;
-  {
-    const char* e = getenv("GLF_GRAM_SYM");      // tuning aid: GLF_GRAM_SYM=0 computes all four blocks of S
-    p.sym = (p.same && C == 256 && p.ksplit == 1 && rowscale == nullptr && out_aug != nullptr && !(e && e[0] == '0')) ? 1 : 0;
-  }
+  p.sym = (p.same && C == 256 && p.ksplit == 1 && rowscale == nullptr && out_aug != nullptr) ? 1 : 0;
   p.out = out_aug; p.outf = scratch; p.rowsum = rowsum; p.rowscale = rowscale;
   p.rowv = rowv; p.corner = corner;
   p.border = (border && Ca > C) ? 1 : 0;

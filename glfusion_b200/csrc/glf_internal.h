@@ -149,7 +149,6 @@ int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch
 int gram_unpack_grads(const float* dwaug, const glf_grads* g, int C, int Ci, int Ca, cudaStream_t stream);
 // One CTA per sequence runs the whole [C x C] chain between the token-sized products (glf_chain.cu), C = 256, C' = 128
 bool gram_chain_supported(int C, int Ci);
-bool gram_residual_in_E();   // chain path: E' = E + I carries the residual dV of dX (no addend in the dX GEMM)
 int gram_chain_fwd(const bf16* Sa, const float* sfv, const bf16* waug, const bf16* wz, const float* bphi,
                    const float* bg, const float* bth, bf16* T, bf16* Mb, bf16* Wp, bf16* Qb, float* cvec, float* tv, int B,
                    int N, cudaStream_t stream);

@@ -91,15 +91,6 @@ __device__ __forceinline__ void tma_load_4d(const CUtensorMap* m, uint32_t bar, 
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
-// Same load, delivered to the same CTA-relative shared-memory offset (and mbarrier) of every CTA in cta_mask.
-__device__ __forceinline__ void tma_load_4d_mcast(const CUtensorMap* m, uint32_t bar, uint32_t dst, int c0, int c1,
-                                                  int c2, int c3, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(cta_mask)
-      : "memory");
-}
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2, int c3) {
   asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
                    reinterpret_cast<uint64_t>(m)),
@@ -152,13 +143,6 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, ui
 // Arrive on an mbarrier when every previously issued tcgen05.mma of this thread has completed.
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// Same, arriving on the barrier at this CTA-relative offset in every CTA of cta_mask (cluster launch).
-__device__ __forceinline__ void umma_commit_mcast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-      "h"(cta_mask)
-      : "memory");
 }
 // ---- cta_group::2: a CTA pair (cluster of two) sharing one MMA: M = 256 over both CTAs' 128 TMEM lanes, each CTA
 //      supplies its own 128 A rows and HALF of the B rows from its own shared memory; issued by the leader CTA only.
