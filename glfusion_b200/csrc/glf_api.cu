@@ -70,6 +70,8 @@ struct Dims {
   bool dot;
   bool gram;       // mode='dot' in its Gram form (channel-space products only)
   int Ca;          // augmented width of the per-sequence matrices (gram)
+  int pdt;         // GLF_DTYPE_* of the glf_weights / glf_grads tensors (glf_desc.reserved[3])
+  bool half_params;   // bf16 / fp16 parameters: an fp32 shadow in `saved`, fp32 gradient staging in ws_bwd
 };
 
 int make_dims(const glf_desc* d, Dims* o) {
@@ -91,6 +93,13 @@ int make_dims(const glf_desc* d, Dims* o) {
     return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 takes fp32 or bf16 activations, not fp16 (GLF_DTYPE_F16)");
   if (d->reserved[2] != GLF_DTYPE_BF16 && d->reserved[2] != GLF_DTYPE_F16)
     return set_error(GLF_ERR_INVALID, "reserved[2] (dtype of the fused LayerNorm's z / dz) must be GLF_DTYPE_BF16 or GLF_DTYPE_F16");
+  if (d->reserved[3] != GLF_PARAMS_F32 && d->reserved[3] != GLF_PARAMS_BF16 && d->reserved[3] != GLF_PARAMS_F16)
+    return set_error(GLF_ERR_INVALID, "reserved[3] (parameter dtype) must be GLF_PARAMS_F32, GLF_PARAMS_BF16 or GLF_PARAMS_F16");
+  // the exact arm is an fp32 contract for the parameters too
+  if (d->precision == GLF_PRECISION_F32X3 && d->reserved[3] != GLF_PARAMS_F32)
+    return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 takes fp32 parameters, not bf16 / fp16 (reserved[3])");
+  o->pdt = param_dtype(d);
+  o->half_params = o->pdt != GLF_DTYPE_F32;
   o->B = d->B;
   o->N = static_cast<long long>(d->T) * d->H * d->W;
   o->rows = o->B * o->N;
@@ -122,7 +131,63 @@ int make_dims(const glf_desc* d, Dims* o) {
   return 0;
 }
 
+// Element counts of the twelve parameter tensors, glf_grads order.
+void param_counts(const Dims& m, long long n[NPARAMS]) {
+  const long long CCi = static_cast<long long>(m.C) * m.Ci;
+  const long long v[NPARAMS] = {CCi, m.Ci, CCi, m.Ci, CCi, m.Ci, CCi, m.C, m.C, m.C, m.C, m.C};
+  for (int k = 0; k < NPARAMS; ++k) n[k] = v[k];
+}
+// fp32 copies of the twelve parameter tensors (half parameters only; NULL otherwise)
+void carve_params(Carver& c, const Dims& m, float* out[NPARAMS]) {
+  long long n[NPARAMS];
+  param_counts(m, n);
+  for (int k = 0; k < NPARAMS; ++k) out[k] = m.half_params ? c.take<float>(n[k]) : nullptr;
+}
+void weight_list(const glf_weights* w, const void* p[NPARAMS]) {
+  const void* v[NPARAMS] = {w->theta_w, w->theta_b, w->phi_w, w->phi_b, w->g_w, w->g_b,
+                            w->wz_w,    w->wz_b,    w->bn_w,  w->bn_b,  w->ln_w, w->ln_b};
+  for (int k = 0; k < NPARAMS; ++k) p[k] = v[k];
+}
+// `w` with its parameter tensors replaced by the fp32 shadow (running statistics untouched: bn_finalize reads and
+// updates them in their own dtype); an absent tensor (bn_layer = 0) stays absent
+glf_weights shadow_weights(const glf_weights* w, float* const sh[NPARAMS]) {
+  glf_weights o = *w;
+  const float** f[NPARAMS] = {&o.theta_w, &o.theta_b, &o.phi_w, &o.phi_b, &o.g_w, &o.g_b,
+                              &o.wz_w,    &o.wz_b,    &o.bn_w,  &o.bn_b,  &o.ln_w, &o.ln_b};
+  for (int k = 0; k < NPARAMS; ++k) *f[k] = *f[k] != nullptr ? sh[k] : nullptr;
+  return o;
+}
+glf_grads grads_table(float* const st[NPARAMS]) {
+  glf_grads g;
+  float** f[NPARAMS] = {&g.theta_w, &g.theta_b, &g.phi_w, &g.phi_b, &g.g_w, &g.g_b,
+                        &g.wz_w,    &g.wz_b,    &g.bn_w,  &g.bn_b,  &g.ln_w, &g.ln_b};
+  for (int k = 0; k < NPARAMS; ++k) *f[k] = st[k];
+  return g;
+}
+// forward: the 2-byte masters into the fp32 shadow that every consumer reads
+int stage_params(const Dims& m, const glf_weights* w, float* const sh[NPARAMS], cudaStream_t stream) {
+  ParamCopy p;
+  weight_list(w, p.src);
+  param_counts(m, p.n);
+  for (int k = 0; k < NPARAMS; ++k) p.dst[k] = sh[k];
+  return convert_params(p, m.pdt, GLF_DTYPE_F32, stream);
+}
+// backward: the fp32 gradients every writer left in the staging area, rounded into the caller's tensors
+int emit_grads(const Dims& m, float* const st[NPARAMS], const glf_grads* g, cudaStream_t stream) {
+  if (!m.half_params) return 0;
+  ParamCopy p;
+  void* v[NPARAMS] = {g->theta_w, g->theta_b, g->phi_w, g->phi_b, g->g_w, g->g_b,
+                      g->wz_w,    g->wz_b,    g->bn_w,  g->bn_b,  g->ln_w, g->ln_b};
+  param_counts(m, p.n);
+  for (int k = 0; k < NPARAMS; ++k) {
+    p.src[k] = st[k];
+    p.dst[k] = v[k];
+  }
+  return convert_params(p, GLF_DTYPE_F32, m.pdt, stream);
+}
+
 struct Saved {
+  float* pshadow[NPARAMS];    // fp32 copies of bf16 / fp16 parameters (the fused LayerNorm pass reads ln_w / ln_b here)
   bf16 *xtok, *P, *Y, *U, *Mb, *Wp, *wcat, *wcatT, *wz, *wzT;
   float *lse, *bcat, *bn_mean, *bn_rstd, *bn_a, *bn_b, *ln_mu, *ln_r;
   bf16 *Sa, *T, *Qb, *waug;   // Gram form: S~ [B][Ca][Ca], T = W~phi S~ [B][Ci][Ca], Q~ [B][C][Ca], W~ [3][Ci][Ca]
@@ -132,6 +197,7 @@ struct Saved {
 size_t carve_saved(const Dims& m, void* base, Saved* s) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
+  carve_params(c, m, s->pshadow);
   s->xtok = m.pack_x ? c.take<bf16>(rows * C) : nullptr;
   s->Sa = s->T = s->Qb = s->waug = nullptr;
   s->sfv = s->cvec = s->tv = nullptr;
@@ -203,6 +269,7 @@ size_t carve_ws_fwd(const Dims& m, void* base, WsFwd* w, size_t saved_bytes) {
 }
 
 struct WsBwd {
+  float* gstage[NPARAMS];     // fp32 gradients of bf16 / fp16 parameters, before emit_grads rounds them
   bf16 *dztok, *dV, *dU, *dP, *dY, *dxtok, *dM, *dWpb;
   float *dWpf, *part_ln, *k1, *k2, *k3, *cs_t, *cs_p, *cs_g, *red1, *dwcat, *delta;
   void* attn;
@@ -213,6 +280,7 @@ struct WsBwd {
 size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
+  carve_params(c, m, w->gstage);
   w->dztok = m.pack_dz ? c.take<bf16>(rows * C) : nullptr;
   w->dV = c.take<bf16>(rows * C);
   w->Rf = w->rv = w->evec = w->dwaug = w->dcv = w->dtv = w->wpart = nullptr;
@@ -694,6 +762,12 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
   const size_t saved_bytes = carve_saved(m, nullptr, &s);
   carve_ws_fwd(m, ws, &wf, saved_bytes);
   carve_saved(m, saved ? saved : wf.saved_fallback, &s);
+  glf_weights wh;
+  if (m.half_params) {
+    GLF_TRY(stage_params(m, w, s.pshadow, stream));
+    wh = shadow_weights(w, s.pshadow);
+    w = &wh;
+  }
   if (m.gram) return tpavi_fwd_gram(d, m, x, w, z, s, wf, stream);
   const int C = m.C, Ci = m.Ci;
   const int N = static_cast<int>(m.N), rows = static_cast<int>(m.rows), B = static_cast<int>(m.B);
@@ -803,6 +877,15 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
   Saved s; WsBwd wb;
   carve_saved(m, const_cast<void*>(saved), &s);
   carve_ws_bwd(d, m, ws, &wb);
+  const glf_grads* g_out = g_;
+  glf_weights wh;
+  glf_grads gh;
+  if (m.half_params) {   // every consumer reads the forward's fp32 shadow, every writer fills the fp32 staging
+    wh = shadow_weights(w, s.pshadow);
+    w = &wh;
+    gh = grads_table(wb.gstage);
+    g_ = &gh;
+  }
   const int C = m.C, Ci = m.Ci;
   const int N = static_cast<int>(m.N), rows = static_cast<int>(m.rows), B = static_cast<int>(m.B);
   const bf16* X = m.pack_x ? s.xtok : reinterpret_cast<const bf16*>(x);
@@ -825,7 +908,10 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
   }
   GLF_TRY(bn_bwd_finalize(wb.part_ln, nb, C, static_cast<double>(m.rows), d, w, s.bn_mean, s.bn_rstd, g_, wb.k1, wb.k2,
                           wb.k3, stream));
-  if (m.gram) return tpavi_bwd_gram(d, m, X, w, s, wb, dx, g_, stream);
+  if (m.gram) {
+    GLF_TRY(tpavi_bwd_gram(d, m, X, w, s, wb, dx, g_, stream));
+    return emit_grads(m, wb.gstage, g_out, stream);
+  }
   const bf16* dU = wb.dV;
   if (d->bn_layer) {
     GLF_TRY(bn_bwd_apply(wb.dV, s.U, GLF_DTYPE_BF16, wb.k1, wb.k2, wb.k3, wb.dU, m.rows, C, stream));
@@ -979,7 +1065,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     else
       GLF_TRY(transpose_cast(wb.dxtok, dx, 1, 1, static_cast<int>(m.rows * C), GLF_DTYPE_BF16, d->io_dtype, stream));
   }
-  return 0;
+  return emit_grads(m, wb.gstage, g_out, stream);
 }
 
 GLF_API int glf_fusion_ln_supported(const glf_desc* d) {
@@ -1014,6 +1100,13 @@ GLF_API int glf_fusion_ln_fwd_parts(const glf_desc* d, const void* xg, const voi
   Saved sg, sl;
   carve_saved(m, saved_g, &sg);
   carve_saved(m, saved_l, &sl);
+  glf_weights wgh, wlh;
+  if (m.half_params) {   // ln_w / ln_b from the fp32 shadows the blocks' forward left in their saved blobs
+    wgh = shadow_weights(wg, sg.pshadow);
+    wlh = shadow_weights(wl, sl.pshadow);
+    wg = &wgh;
+    wl = &wlh;
+  }
   const bf16* U[2] = {sg.U, sl.U};
   const bf16* X[2] = {reinterpret_cast<const bf16*>(xg), reinterpret_cast<const bf16*>(xl)};
   const float* a[2] = {sg.bn_a, sl.bn_a};
@@ -1066,6 +1159,13 @@ GLF_API int glf_fusion_ln_bwd_views(const glf_desc* d, const void* dz, const voi
   carve_saved(m, const_cast<void*>(saved_l), &sl);
   carve_ws_bwd(d, m, ws_g, &bg);
   carve_ws_bwd(d, m, ws_l, &bl);
+  glf_weights wgh, wlh;
+  if (m.half_params) {
+    wgh = shadow_weights(wg, sg.pshadow);
+    wlh = shadow_weights(wl, sl.pshadow);
+    wg = &wgh;
+    wl = &wlh;
+  }
   const bf16* U[2] = {sg.U, sl.U};
   const bf16* X[2] = {reinterpret_cast<const bf16*>(xg), reinterpret_cast<const bf16*>(xl)};
   const float* a[2] = {sg.bn_a, sl.bn_a};

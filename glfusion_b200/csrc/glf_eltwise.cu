@@ -5,6 +5,8 @@
 // per-CTA partials + fixed-order finalisation for every cross-row (per-channel) statistic, so results are
 // deterministic (SURVEY.md §7 "hard parts").
 
+#include <type_traits>
+
 #include "glf_internal.h"
 #include "glf_ptx.cuh"
 
@@ -215,12 +217,21 @@ __global__ void __launch_bounds__(32 * RED_Y)
   }
 }
 
+// running statistics in the parameters' element type, updated in fp64 and rounded once
+__device__ __forceinline__ double ld_stat(const float* p) { return *p; }
+__device__ __forceinline__ double ld_stat(const bf16* p) { return __bfloat162float(*p); }
+__device__ __forceinline__ double ld_stat(const f16* p) { return __half2float(*p); }
+__device__ __forceinline__ void st_stat(float* p, double v) { *p = static_cast<float>(v); }
+__device__ __forceinline__ void st_stat(bf16* p, double v) { *p = __double2bfloat16(v); }
+__device__ __forceinline__ void st_stat(f16* p, double v) { *p = __double2half(v); }
+
 // partials: [np][2][C] (sum, sum of squares) -> mean, rstd, affine a = gamma*rstd, b = beta - mean*a; running stats.
+template <typename TR>
 __global__ void __launch_bounds__(32 * RED_Y)
     bn_finalize_kernel(const float* __restrict__ part, int np, int C, double count, const float* __restrict__ gamma,
                        const float* __restrict__ beta, const float* __restrict__ bz, float eps, float momentum,
                        int training, int bn_layer,
-                       float* __restrict__ rm, float* __restrict__ rv, long long* __restrict__ nbt,
+                       TR* __restrict__ rm, TR* __restrict__ rv, long long* __restrict__ nbt,
                        float* __restrict__ mean_o, float* __restrict__ rstd_o, float* __restrict__ a_o,
                        float* __restrict__ b_o) {
   __shared__ double sm[2][RED_Y][33];
@@ -243,11 +254,11 @@ __global__ void __launch_bounds__(32 * RED_Y)
     var = st[1] / count - mean * mean;
     if (var < 0.0) var = 0.0;
     const double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-    rm[c] = static_cast<float>((1.0 - momentum) * rm[c] + momentum * (mean + shift));
-    rv[c] = static_cast<float>((1.0 - momentum) * rv[c] + momentum * unbiased);
+    st_stat(rm + c, (1.0 - momentum) * ld_stat(rm + c) + momentum * (mean + shift));
+    st_stat(rv + c, (1.0 - momentum) * ld_stat(rv + c) + momentum * unbiased);
   } else {
-    mean = rm[c] - shift;
-    var = rv[c];
+    mean = ld_stat(rm + c) - shift;
+    var = ld_stat(rv + c);
   }
   const double rstd = 1.0 / sqrt(var + static_cast<double>(eps));
   const double a = gamma[c] * rstd;
@@ -1082,9 +1093,48 @@ int row_grid(long long rows, int S) {
   return static_cast<int>(blocks < cap ? (blocks < 1 ? 1 : blocks) : cap);
 }
 
+// ------------------------------------------------------------------------------------------------ 2-byte parameters
+// blockIdx.y = tensor; 8-element vectors where both pointers are 16-byte aligned, elements otherwise.  The conversion is
+// exact towards fp32 and rounds to nearest away from it (static_cast / pack2), so an fp16 overflow becomes +-inf.
+template <typename TS, typename TD>
+__global__ void __launch_bounds__(256) convert_params_kernel(const ParamCopy p) {
+  const int k = blockIdx.y;
+  const TS* __restrict__ src = static_cast<const TS*>(p.src[k]);
+  TD* __restrict__ dst = static_cast<TD*>(p.dst[k]);
+  if (src == nullptr || dst == nullptr) return;
+  const long long n = p.n[k];
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  long long head = 0;
+  if (((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0) {
+    head = n / 8;
+    for (long long v = t; v < head; v += stride) {
+      float f[8];
+      load8(src + 8 * v, f);
+      store8(dst + 8 * v, f);
+    }
+    head *= 8;
+  }
+  for (long long i = head + t; i < n; i += stride) dst[i] = static_cast<TD>(static_cast<float>(src[i]));
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------ host launchers
+int convert_params(const ParamCopy& p, int src_dtype, int dst_dtype, cudaStream_t stream) {
+  long long nmax = 0;
+  for (int k = 0; k < NPARAMS; ++k) nmax = p.n[k] > nmax ? p.n[k] : nmax;
+  long long gx = (nmax + 8 * 256 - 1) / (8 * 256);
+  gx = gx < 1 ? 1 : (gx > 128 ? 128 : gx);
+  const dim3 grid(static_cast<unsigned>(gx), NPARAMS);
+  if (src_dtype == GLF_DTYPE_BF16 && dst_dtype == GLF_DTYPE_F32) convert_params_kernel<bf16, float><<<grid, 256, 0, stream>>>(p);
+  else if (src_dtype == GLF_DTYPE_F16 && dst_dtype == GLF_DTYPE_F32) convert_params_kernel<f16, float><<<grid, 256, 0, stream>>>(p);
+  else if (src_dtype == GLF_DTYPE_F32 && dst_dtype == GLF_DTYPE_BF16) convert_params_kernel<float, bf16><<<grid, 256, 0, stream>>>(p);
+  else if (src_dtype == GLF_DTYPE_F32 && dst_dtype == GLF_DTYPE_F16) convert_params_kernel<float, f16><<<grid, 256, 0, stream>>>(p);
+  else return set_error(GLF_ERR_INVALID, "convert_params: fp32 <-> bf16 / fp16 only");
+  return check_cuda(cudaGetLastError(), "convert_params launch");
+}
+
 int transpose_cast(const void* in, void* out, int batch, int R, int S, int in_dtype, int out_dtype,
                    cudaStream_t stream) {
   if (batch <= 0 || R <= 0 || S <= 0) return set_error(GLF_ERR_INVALID, "transpose: empty");
@@ -1140,11 +1190,17 @@ int reduce_stage1(const float* p0, const float* p1, const float* p2, int ntab, c
 
 int bn_finalize(const float* part, int np, int C, double count, const glf_desc* d, const glf_weights* w, const float* bz,
                 float* mean, float* rstd, float* a, float* b, cudaStream_t stream) {
-  bn_finalize_kernel<<<(C + 31) / 32, dim3(32, RED_Y), 0, stream>>>(part, np, C, count, w->bn_w, w->bn_b, bz, d->eps_bn, d->momentum,
-                                                          d->training, d->bn_layer, w->bn_running_mean,
-                                                          w->bn_running_var,
-                                                          reinterpret_cast<long long*>(w->bn_num_batches_tracked), mean,
-                                                          rstd, a, b);
+  auto launch = [&](auto* tag) {
+    using TR = std::remove_pointer_t<decltype(tag)>;
+    bn_finalize_kernel<TR><<<(C + 31) / 32, dim3(32, RED_Y), 0, stream>>>(
+        part, np, C, count, w->bn_w, w->bn_b, bz, d->eps_bn, d->momentum, d->training, d->bn_layer,
+        reinterpret_cast<TR*>(w->bn_running_mean), reinterpret_cast<TR*>(w->bn_running_var),
+        reinterpret_cast<long long*>(w->bn_num_batches_tracked), mean, rstd, a, b);
+  };
+  const int rdt = param_dtype(d);    // the running statistics are stored like the parameters
+  if (rdt == GLF_DTYPE_BF16) launch(static_cast<bf16*>(nullptr));
+  else if (rdt == GLF_DTYPE_F16) launch(static_cast<f16*>(nullptr));
+  else launch(static_cast<float*>(nullptr));
   return check_cuda(cudaGetLastError(), "bn_finalize launch");
 }
 

@@ -120,6 +120,19 @@ int reduce_partials(const float* part, int np, long long stride, int n, float al
 int reduce_partials3(const float* p0, const float* p1, const float* p2, int np, long long stride, int n, float* o0,
                      float* o1, float* o2, cudaStream_t stream);
 int cast_bf16(const float* in, bf16* out, long long n, cudaStream_t stream);
+// GLF_DTYPE_* element type of the glf_weights / glf_grads tensors (glf_desc.reserved[3], validated by make_dims)
+inline int param_dtype(const glf_desc* d) {
+  return d->reserved[3] == GLF_PARAMS_BF16 ? GLF_DTYPE_BF16 : d->reserved[3] == GLF_PARAMS_F16 ? GLF_DTYPE_F16 : GLF_DTYPE_F32;
+}
+// A block's twelve parameter tensors (glf_grads order) copied between two element types in one launch: 2-byte
+// masters -> fp32 (forward) or fp32 gradients -> 2-byte, rounded to nearest (backward).  A NULL src or dst is skipped.
+constexpr int NPARAMS = 12;
+struct ParamCopy {
+  const void* src[NPARAMS];
+  void* dst[NPARAMS];
+  long long n[NPARAMS];
+};
+int convert_params(const ParamCopy& p, int src_dtype, int dst_dtype, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------ Gram form (glf_gram.cu)
 // Augmented width of the per-sequence matrices: column C is the homogeneous coordinate, the rest zero padding.

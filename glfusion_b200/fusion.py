@@ -74,6 +74,11 @@ def _channels_last_rows(views: Sequence[torch.Tensor], x_dtype) -> Optional[tupl
     return sb, st
 
 
+def _f32(t: torch.Tensor) -> torch.Tensor:
+    """Contiguous fp32 logits, with no cast call when they already are (the fused node then makes no aten::to)."""
+    return t if t.dtype == torch.float32 and t.is_contiguous() else t.float().contiguous()
+
+
 def gate_concat_forward(f4: Sequence[torch.Tensor], cls: Sequence[torch.Tensor], ctr: Sequence[torch.Tensor],
                         weight: float, x_dtype=torch.bfloat16):
     lib = L.load()
@@ -85,8 +90,8 @@ def gate_concat_forward(f4: Sequence[torch.Tensor], cls: Sequence[torch.Tensor],
     if any(t.dtype != f4[0].dtype for t in f4):
         # the kernels read every view with one element type: a mix would be misread, not converted
         raise TypeError(f"the f4 views must share one dtype, got {sorted({str(t.dtype) for t in f4})}")
-    cls = [t.float().contiguous() for t in cls]
-    ctr = [t.float().contiguous() for t in ctr]
+    cls = [_f32(t) for t in cls]
+    ctr = [_f32(t) for t in ctr]
     ncls = cls[0].shape[1]
     xg = torch.empty((B, V, h, w, C_), dtype=x_dtype, device=dev)
     xl = torch.empty_like(xg)
@@ -218,12 +223,18 @@ class _FusionFunction(torch.autograd.Function):
         prec = mg._precision_id()
         if ml._precision_id() != prec:
             raise ValueError("global_attn and local_attn must use the same compute_precision")
-        _check_precision_dtype(prec, f4[0].dtype)
+        # one parameter dtype for both blocks (the fused LayerNorm pass reads both with one descriptor): 2-byte only when
+        # both blocks hold it throughout, fp32 copies otherwise
+        pdt = mg._storage_dtype(pg)
+        if ml._storage_dtype(pl) != pdt:
+            pdt = torch.float32
+        _check_precision_dtype(prec, f4[0].dtype, pdt)
+        tg, tl = mg._param_table(pg, pdt), ml._param_table(pl, pdt)
+        bg, bl = mg._buffer_table(pdt), ml._buffer_table(pdt)
         xdt = torch.float32 if prec == L.PRECISION_F32X3 else torch.bfloat16
         xg, xl, gate, f4c, clsc, ctrc = gate_concat_forward(f4, cls, ctr, fusion.center_aware_weight, xdt)
         B, V_, h, w, C_ = xg.shape
         need = any(ctx.needs_input_grad)
-        tg, tl = mg._param_table(pg), ml._param_table(pl)
         shape = (B, V_, h, w, C_)
         pair = _pair_ln_ok(mg, ml, shape, xg, prec)
         # fp16 f4: the fused LayerNorm pass writes the fp16 outputs itself (its z dtype, desc.reserved[2]); no cast pass
@@ -239,24 +250,24 @@ class _FusionFunction(torch.autograd.Function):
             cur = torch.cuda.current_stream(xg.device)
             side.wait_stream(cur)
             with torch.cuda.stream(side):
-                _, stl, svl, _ = tpavi_forward_raw(xl, tl, ml._buffer_table(), mode=ml._mode_id, **ml._norm_config(),
+                _, stl, svl, _ = tpavi_forward_raw(xl, tl, bl, mode=ml._mode_id, **ml._norm_config(),
                                                    bn_layer=ml._bn_layer, Ci=ml.inter_channels,
                                                    keep_for_backward=True, z_out=zsum, accumulate=False,
                                                    token_shape=shape, precision=prec, defer_ln=True)
-        _, stg, svg, _ = tpavi_forward_raw(xg, tg, mg._buffer_table(), mode=mg._mode_id, **mg._norm_config(),
+        _, stg, svg, _ = tpavi_forward_raw(xg, tg, bg, mode=mg._mode_id, **mg._norm_config(),
                                            bn_layer=mg._bn_layer, Ci=mg.inter_channels,
                                            keep_for_backward=need or pair, z_out=zsum, token_shape=shape,
                                            precision=prec, defer_ln=pair)
         if side is not None:
             cur.wait_stream(side)
         else:
-            _, stl, svl, _ = tpavi_forward_raw(xl, tl, ml._buffer_table(), mode=ml._mode_id, **ml._norm_config(),
+            _, stl, svl, _ = tpavi_forward_raw(xl, tl, bl, mode=ml._mode_id, **ml._norm_config(),
                                                bn_layer=ml._bn_layer, Ci=ml.inter_channels,
                                                keep_for_backward=need or pair, z_out=zsum, accumulate=not pair,
                                                token_shape=shape, precision=prec, defer_ln=pair)
         if pair:
             # both blocks' BN + residual + LayerNorm and the `global + local` sum (ours.py:1834) in one HBM pass
-            wg, wl = _weights_struct(tg, mg._buffer_table()), _weights_struct(tl, ml._buffer_table())
+            wg, wl = _weights_struct(tg, bg), _weights_struct(tl, bl)
             stg.desc.reserved[2] = _io_dtype(zsum)
             with torch.cuda.device(xg.device):
                 L.check(L.load().glf_fusion_ln_fwd_parts(C.byref(stg.desc), L.ptr(xg), L.ptr(xl), C.byref(wg),
@@ -265,6 +276,7 @@ class _FusionFunction(torch.autograd.Function):
             if not need:
                 svg = svl = None
         ctx.pair = pair
+        ctx.pdt = pdt
         ctx.fusion, ctx.V, ctx.ng = fusion, V, ng
         ctx.states = (stg, svg, stl, svl)
         ctx.io_dtype = f4[0].dtype
@@ -329,7 +341,8 @@ class _FusionFunction(torch.autograd.Function):
         n_in = 5 + 3 * V + 2 * ng
         if dout is None and dglob is None:
             return (None,) * n_in
-        tg, tl = mg._param_table(pg), ml._param_table(pl)
+        tg, tl = mg._param_table(pg, ctx.pdt), ml._param_table(pl, ctx.pdt)
+        bg, bl = mg._buffer_table(ctx.pdt), ml._buffer_table(ctx.pdt)
         gl = None
         if dglob is None:
             # both blocks see the same dz (ours.py:1834); with dz_rows it stays where autograd delivered it, one tensor
@@ -342,7 +355,7 @@ class _FusionFunction(torch.autograd.Function):
                 stg.desc.reserved[0] = stl.desc.reserved[0] = 1
                 stg.desc.reserved[2] = _io_dtype(dz_rows[0][0] if dz_rows is not None else dz)
                 wsg, wsl = _blob(stg.sizes.ws_bwd_bytes, xg.device), _blob(stl.sizes.ws_bwd_bytes, xg.device)
-                wg, wl = _weights_struct(tg, mg._buffer_table()), _weights_struct(tl, ml._buffer_table())
+                wg, wl = _weights_struct(tg, bg), _weights_struct(tl, bl)
                 with torch.cuda.device(xg.device):
                     if dz_rows is not None:
                         views, sb = dz_rows
@@ -360,14 +373,14 @@ class _FusionFunction(torch.autograd.Function):
                 cur = torch.cuda.current_stream(xg.device)
                 side.wait_stream(cur)
                 with torch.cuda.stream(side):
-                    dxl, gl = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xl, stl, svl, tl, ml._buffer_table(), ws=wsl,
+                    dxl, gl = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xl, stl, svl, tl, bl, ws=wsl,
                                                  grad_out=gout_l)
-            dxg, gg = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xg, stg, svg, tg, mg._buffer_table(), ws=wsg,
+            dxg, gg = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xg, stg, svg, tg, bg, ws=wsg,
                                          grad_out=gout_g)
             if side is not None:
                 cur.wait_stream(side)
             else:
-                dxl, gl = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xl, stl, svl, tl, ml._buffer_table(), ws=wsl,
+                dxl, gl = tpavi_backward_raw(dz, L.LAYOUT_TOKEN, xl, stl, svl, tl, bl, ws=wsl,
                                              grad_out=gout_l)
             hook = ctx.fusion.on_weight_grads_ready
             if hook is not None and gout_g is not None and gout_l is not None:
@@ -378,11 +391,11 @@ class _FusionFunction(torch.autograd.Function):
             # block is not on the path at all
             dzg = token(dglob) if dout is None else token(dout) + token(dglob)
             stg.desc.reserved[0] = 0
-            dxg, gg = tpavi_backward_raw(dzg, L.LAYOUT_TOKEN, xg, stg, svg, tg, mg._buffer_table(),
+            dxg, gg = tpavi_backward_raw(dzg, L.LAYOUT_TOKEN, xg, stg, svg, tg, bg,
                                          grad_out=claim_grad_out(mg))
             if dout is not None:
                 stl.desc.reserved[0] = 0
-                dxl, gl = tpavi_backward_raw(token(dout), L.LAYOUT_TOKEN, xl, stl, svl, tl, ml._buffer_table(),
+                dxl, gl = tpavi_backward_raw(token(dout), L.LAYOUT_TOKEN, xl, stl, svl, tl, bl,
                                              grad_out=claim_grad_out(ml))
             else:
                 dxl = torch.zeros_like(dxg)
@@ -394,7 +407,7 @@ class _FusionFunction(torch.autograd.Function):
                     out.append(None)
                     continue
                 t = gr[mod._grad_key(name)].reshape(p.shape)
-                out.append(t if p.dtype == torch.float32 else t.to(p.dtype))
+                out.append(t if t.dtype == p.dtype else t.to(p.dtype))
         return tuple(out)
 
 

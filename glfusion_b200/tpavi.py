@@ -50,11 +50,19 @@ def _io_dtype(t: torch.Tensor) -> int:
         raise TypeError(f"glfusion_b200 supports float32, bfloat16 and float16 activations, got {t.dtype}") from None
 
 
-def _check_precision_dtype(precision: int, dtype: torch.dtype) -> None:
-    """The fp32-exact arm is an fp32 contract: float16 inputs would defeat it (the library rejects the pair too)."""
+# Parameter dtypes the kernels read and write as they are (glf_desc.reserved[3]); anything else runs on fp32 copies.
+_PARAM_DTYPES = {torch.float32: L.PARAMS_F32, torch.bfloat16: L.PARAMS_BF16, torch.float16: L.PARAMS_F16}
+
+
+def _check_precision_dtype(precision: int, dtype: torch.dtype, param_dtype: torch.dtype = torch.float32) -> None:
+    """The fp32-exact arm is an fp32 contract: float16 inputs or 2-byte parameters would defeat it (the library rejects
+    both too)."""
     if precision == L.PRECISION_F32X3 and dtype == torch.float16:
         raise TypeError("compute_precision='fp32' takes float32 or bfloat16 activations, not float16; keep the default "
                         "compute_precision='bf16' for float16 (autocast) inputs")
+    if precision == L.PRECISION_F32X3 and param_dtype != torch.float32:
+        raise TypeError(f"compute_precision='fp32' takes float32 parameters, not {param_dtype}; keep the default "
+                        "compute_precision='bf16' for a .half() / .bfloat16() module")
 
 
 def _is_token_major(t: torch.Tensor) -> bool:
@@ -79,7 +87,8 @@ class TPAVIState:
     """Everything one forward/backward pair shares: descriptor, weights table, saved blob."""
 
     def __init__(self, B, C_, T, H, W, Ci, mode, io_dtype, x_layout, training, bn_layer, accumulate=False,
-                 eps_bn=1e-5, eps_ln=1e-5, momentum=0.1, precision=L.PRECISION_BF16, defer_ln=False):
+                 eps_bn=1e-5, eps_ln=1e-5, momentum=0.1, precision=L.PRECISION_BF16, defer_ln=False,
+                 param_dtype=L.PARAMS_F32):
         d = L.GlfDesc()
         d.B, d.T, d.H, d.W, d.C, d.Ci = B, T, H, W, C_, Ci
         d.mode = mode
@@ -93,6 +102,7 @@ class TPAVIState:
         d.eps_bn, d.eps_ln, d.momentum = eps_bn, eps_ln, momentum
         d.reserved[0] = 1 if defer_ln else 0     # LayerNorm stage run for MGFM + MLFM together (glf_fusion_ln_*)
         d.reserved[1] = DOT_ALGO                 # 0 = library chooses, 1 = token-space form, 2 = Gram form
+        d.reserved[3] = param_dtype              # dtype of the parameter tensors, gradients and running statistics
         self.desc = d
         sz = L.GlfSizes()
         L.check(L.load().glf_tpavi_sizes(C.byref(d), C.byref(sz)))
@@ -120,7 +130,8 @@ def tpavi_forward_raw(x: torch.Tensor, params: dict, buffers, *, mode: int, trai
     lib = L.load()
     if not x.is_cuda:
         raise L.GlfError("glfusion_b200 runs on CUDA (sm_100) tensors only; there is no CPU path")
-    _check_precision_dtype(precision, x.dtype)
+    pdt = params["ln_w"].dtype      # _param_table: one dtype for every tensor of the table
+    _check_precision_dtype(precision, x.dtype, pdt)
     if token_shape is not None:
         B, T, H, W, C_ = token_shape
         layout = L.LAYOUT_TOKEN
@@ -132,7 +143,8 @@ def tpavi_forward_raw(x: torch.Tensor, params: dict, buffers, *, mode: int, trai
             x = x.contiguous()
             layout = L.LAYOUT_NCTHW
     st = TPAVIState(B, C_, T, H, W, Ci, mode, _io_dtype(x), layout, training, bn_layer, accumulate,
-                    eps_bn=eps_bn, eps_ln=eps_ln, momentum=momentum, precision=precision, defer_ln=defer_ln)
+                    eps_bn=eps_bn, eps_ln=eps_ln, momentum=momentum, precision=precision, defer_ln=defer_ln,
+                    param_dtype=_PARAM_DTYPES[pdt])
     dev = x.device
     if z_out is None:
         z_out = torch.empty((B, T, H, W, C_), dtype=x.dtype, device=dev)
@@ -148,14 +160,15 @@ def tpavi_forward_raw(x: torch.Tensor, params: dict, buffers, *, mode: int, trai
 def tpavi_backward_raw(dz: torch.Tensor, dz_layout: int, x: torch.Tensor, st: TPAVIState, saved: torch.Tensor,
                        params: dict, buffers, dx_out: Optional[torch.Tensor] = None,
                        ws: Optional[torch.Tensor] = None, grad_out: Optional[dict] = None):
-    """Run glf_tpavi_bwd.  Returns (dx buffer in the layout of x, dict of fp32 parameter gradients).
-    `grad_out` (optional): name -> preallocated fp32 tensor the kernels write that gradient into (e.g. views of a
-    data-parallel all-reduce bucket, dp.GradBucket.bind): the returned gradient then aliases it."""
+    """Run glf_tpavi_bwd.  Returns (dx buffer in the layout of x, dict of parameter gradients in the dtype of `params`).
+    `grad_out` (optional): name -> preallocated tensor of that dtype the kernels write that gradient into (e.g. views of
+    a data-parallel all-reduce bucket, dp.GradBucket.bind): the returned gradient then aliases it."""
     lib = L.load()
     dev = x.device
     d = st.desc
     d.dz_layout = dz_layout
     grads = {}
+    gdt = params["ln_w"].dtype
     g = L.GlfGrads()
     for name in _PARAM_ORDER:
         ref = params.get(name)
@@ -163,10 +176,10 @@ def tpavi_backward_raw(dz: torch.Tensor, dz_layout: int, x: torch.Tensor, st: TP
             # bn_layer=False: no BN affine; the kernels still want a scratch target
             ref = params["ln_w"]
         dst = grad_out.get(name) if grad_out is not None and params.get(name) is not None else None
-        if dst is not None and dst.dtype == torch.float32 and dst.shape == ref.shape and dst.is_contiguous():
+        if dst is not None and dst.dtype == gdt and dst.shape == ref.shape and dst.is_contiguous():
             t = dst.detach()        # fresh alias: autograd may adopt it as .grad without a copy
         else:
-            t = torch.empty(ref.shape, dtype=torch.float32, device=dev)
+            t = torch.empty(ref.shape, dtype=gdt, device=dev)
         grads[name] = t
         setattr(g, name, t.data_ptr())
     if dx_out is None:
@@ -209,14 +222,16 @@ class _TPAVIFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, module, *plist):
         module._grad_out_claimed = False
-        params = module._param_table(plist)
-        buffers = module._buffer_table()
+        pdt = module._storage_dtype(plist)
+        params = module._param_table(plist, pdt)
+        buffers = module._buffer_table(pdt)
         need_grad = any(ctx.needs_input_grad)      # grad mode is off inside Function.forward
         z, st, saved, x_used = tpavi_forward_raw(x, params, buffers, mode=module._mode_id,
                                                  bn_layer=module._bn_layer,
                                                  Ci=module.inter_channels, keep_for_backward=need_grad,
                                                  precision=module._precision_id(), **module._norm_config())
         ctx.module = module
+        ctx.pdt = pdt
         ctx.st = st
         ctx.saved_blob = saved
         ctx.x_dtype = x.dtype
@@ -228,7 +243,7 @@ class _TPAVIFunction(torch.autograd.Function):
     def backward(ctx, dz):
         x_used, *plist = ctx.saved_tensors
         module = ctx.module
-        params = module._param_table(plist)
+        params = module._param_table(plist, ctx.pdt)
         if ctx.saved_blob is None:
             raise L.GlfError("backward called on a forward that ran without grad")
         if dz.dtype != x_used.dtype:
@@ -238,7 +253,7 @@ class _TPAVIFunction(torch.autograd.Function):
         else:
             dz = dz.contiguous()
             layout = L.LAYOUT_NCTHW
-        dx, grads = tpavi_backward_raw(dz, layout, x_used, ctx.st, ctx.saved_blob, params, module._buffer_table(),
+        dx, grads = tpavi_backward_raw(dz, layout, x_used, ctx.st, ctx.saved_blob, params, module._buffer_table(ctx.pdt),
                                        grad_out=claim_grad_out(module))
         if ctx.st.desc.x_layout == L.LAYOUT_TOKEN:
             dx = dx.permute(0, 4, 1, 2, 3)
@@ -246,7 +261,7 @@ class _TPAVIFunction(torch.autograd.Function):
         for name, p in zip(module._plist_names(), plist):
             gname = module._grad_key(name)
             gr = grads[gname].reshape(p.shape)
-            out.append(gr if p.dtype == torch.float32 else gr.to(p.dtype))
+            out.append(gr if gr.dtype == p.dtype else gr.to(p.dtype))
         return tuple(out)
 
 
@@ -339,11 +354,25 @@ class TPAVIModule(nn.Module):
         table = dict(self.named_parameters())
         return [table[n] for n in self._plist_names()]
 
-    def _param_table(self, plist):
+    def _storage_dtype(self, plist) -> torch.dtype:
+        """bfloat16 / float16 when every parameter of the block and both BatchNorm running statistics share that dtype
+        (``.half()``, ``.bfloat16()``): the kernels read them, and write gradients and running statistics, in it.
+        float32 otherwise, a mix such as bf16 convs beside fp32 norm layers included: that block runs on fp32 copies."""
+        ts = list(plist)
+        if self._bn_layer:
+            ts += [self.W_z[1].running_mean, self.W_z[1].running_var]
+        dts = {t.dtype for t in ts}
+        dt = dts.pop() if len(dts) == 1 else torch.float32
+        return dt if dt in (torch.bfloat16, torch.float16) else torch.float32
+
+    def _param_table(self, plist, dtype=None):
+        """Kernel-side name -> parameter tensor, all of `dtype` (default: _storage_dtype): fp32 copies where needed."""
+        if dtype is None:
+            dtype = self._storage_dtype(plist)
         out = {}
         for name, p in zip(self._plist_names(), plist):
             t = p.detach()
-            if t.dtype != torch.float32:
+            if t.dtype != dtype:
                 t = t.float()
             out[self._KEYMAP[name]] = t.contiguous()
         if not self._bn_layer:
@@ -351,12 +380,13 @@ class TPAVIModule(nn.Module):
             out["bn_b"] = None
         return out
 
-    def _buffer_table(self):
+    def _buffer_table(self, dtype=torch.float32):
         if not self._bn_layer:
             return (None, None, None)
         bn = self.W_z[1]
-        if bn.running_mean.dtype != torch.float32:
-            raise L.GlfError("BatchNorm running statistics must stay float32")
+        if bn.running_mean.dtype != dtype or bn.running_var.dtype != dtype:
+            raise L.GlfError("BatchNorm running statistics must stay float32 unless every parameter of the block "
+                             "shares their bfloat16 / float16 dtype")
         return (bn.running_mean, bn.running_var, bn.num_batches_tracked)
 
     # ---- forward ------------------------------------------------------------------------------------------------

@@ -45,6 +45,8 @@ enum { GLF_MODE_DOT = 0, GLF_MODE_EMBEDDED = 1 };         /* TPAVIModule(mode=..
 enum { GLF_DTYPE_BF16 = 0, GLF_DTYPE_F32 = 1, GLF_DTYPE_F16 = 2 };
 enum { GLF_LAYOUT_NCTHW = 0, GLF_LAYOUT_TOKEN = 1 };      /* [B,C,T,H,W] contiguous  |  [B,T,H,W,C] contiguous */
 enum { GLF_PRECISION_BF16 = 0, GLF_PRECISION_F32X3 = 1 }; /* tensor-core operand precision */
+/* Storage dtype of the glf_weights / glf_grads tensors (glf_desc.reserved[3]); 0 is fp32, the default. */
+enum { GLF_PARAMS_F32 = 0, GLF_PARAMS_BF16 = 1, GLF_PARAMS_F16 = 2 };
 
 enum {
   GLF_OK = 0,
@@ -73,10 +75,17 @@ typedef struct glf_desc {
                           reserved[1]: algorithm of mode='dot' (both are exact reassociations of ours.py:881-902):
                           0 = the library chooses (Gram form when N >= 5 C), 1 = token-space form (theta/phi/g formed
                           per token), 2 = Gram form (S = X~^T X~ per sequence, channel-space products only).
-                          Others: 0. */
+                          reserved[2]: dtype of z / z_global / dz of the fused LayerNorm pass (GLF_DTYPE_BF16 or F16).
+                          reserved[3]: GLF_PARAMS_* — element type of every glf_weights / glf_grads tensor, the running
+                          statistics included (bn_num_batches_tracked stays int64).  With GLF_PARAMS_BF16 / F16 the block
+                          computes exactly what fp32 parameters holding the same values compute: one launch per block
+                          converts them to an fp32 copy inside `saved` (inside ws when saved is NULL) forward, and one
+                          rounds the fp32 gradients to nearest into glf_grads backward (fp16 overflow: +-inf); the running
+                          statistics are updated in place, rounded once.  GLF_PRECISION_F32X3 needs GLF_PARAMS_F32. */
 } glf_desc;
 
-/* fp32 master parameters, same shapes as the reference state_dict (SURVEY.md §8b). */
+/* Master parameters, same shapes as the reference state_dict (SURVEY.md §8b): fp32, or the bf16 / fp16 element type
+ * glf_desc.reserved[3] names (the pointers are then read as that type). */
 typedef struct glf_weights {
   const float* theta_w; /* [Ci, C]   theta.weight[Ci,C,1,1,1] */
   const float* theta_b; /* [Ci] */
@@ -95,7 +104,7 @@ typedef struct glf_weights {
   const float* ln_b; /* [C]  norm_layer.bias */
 } glf_weights;
 
-/* fp32 gradients, written (not accumulated) by glf_tpavi_bwd. */
+/* Gradients in the parameters' element type (glf_desc.reserved[3]), written (not accumulated) by glf_tpavi_bwd. */
 typedef struct glf_grads {
   float* theta_w; float* theta_b;
   float* phi_w;   float* phi_b;
