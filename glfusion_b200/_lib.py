@@ -25,7 +25,8 @@ EXPORTS = ("glf_version", "glf_last_error", "glf_tpavi_sizes", "glf_tpavi_fwd", 
            "glf_bn_res_ln_pair_fwd",
            "glf_bn_res_ln_pair_bwd", "glf_gemm_bf16_ex", "glf_gram_contraction", "glf_p2p_signal_bytes", "glf_p2p_max_floats",
            "glf_p2p_export", "glf_p2p_open", "glf_p2p_close", "glf_p2p_allreduce", "glf_spatial_sums",
-           "glf_cycle_loss_scratch_bytes", "glf_cycle_loss")
+           "glf_cycle_loss_scratch_bytes", "glf_cycle_loss", "glf_attention_scratch_bytes", "glf_attention_fwd",
+           "glf_attention_bwd")
 
 
 class GlfDesc(C.Structure):
@@ -118,10 +119,14 @@ def load() -> C.CDLL:
         lib.glf_bn_res_ln_bwd.argtypes = [i64, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                           C.POINTER(C.c_int), vp]
         lib.glf_bn_res_ln_bwd_max_blocks.argtypes = []
+        lib.glf_attention_scratch_bytes.argtypes = [i32, i32, i32, i32]
+        lib.glf_attention_scratch_bytes.restype = C.c_size_t
+        lib.glf_attention_fwd.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
+        lib.glf_attention_bwd.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp]
         for name in EXPORTS:
             fn = getattr(lib, name)
             if name not in ("glf_last_error", "glf_gate_concat_bwd_scratch_bytes", "glf_p2p_signal_bytes",
-                            "glf_p2p_max_floats"):
+                            "glf_p2p_max_floats", "glf_attention_scratch_bytes"):
                 fn.restype = C.c_int
         _lib = lib
         return lib

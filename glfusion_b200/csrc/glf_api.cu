@@ -723,6 +723,62 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
   return 0;
 }
 
+// Bias gradients = column sums of dTheta / dPhi / dG, from the partial tables their producers wrote: the three GEMM
+// epilogues (np, np_p, np_g rows of [2][Ci] each; the row counts can differ, tile shape and grid differ per product),
+// or the flash backward (np < 0: one table of -np rows of [2][3Ci] in cs_t, the column sums of dP = [dTheta|dPhi|dG]).
+int reduce_bias_grads(const float* cs_t, const float* cs_p, const float* cs_g, int np, int np_p, int np_g, int Ci,
+                      float* red1, float* db_t, float* db_p, float* db_g, cudaStream_t stream) {
+  long long rs = 2LL * Ci;
+  const float *t0 = cs_t, *t1 = cs_p, *t2 = cs_g;
+  if (np < 0) {
+    np = np_p = np_g = -np;
+    rs = 2LL * 3 * Ci;
+    t1 = cs_t + Ci;
+    t2 = cs_t + 2 * Ci;
+  }
+  if (np == np_p && np == np_g && np <= 4 * REDUCE_STAGE1_ROWS)   // short tables (one row per CTA): one fixed-order pass
+    return reduce_partials3(t0, t1, t2, np, rs, Ci, db_t, db_p, db_g, stream);
+  const int np_in[3] = {np, np_p, np_g};
+  GLF_TRY(reduce_stage1(t0, t1, t2, 3, np_in, &np, &rs, 0, 1, Ci, red1, stream));
+  return reduce_partials3(red1, red1 + static_cast<long long>(REDUCE_STAGE1_ROWS) * Ci,
+                          red1 + 2LL * REDUCE_STAGE1_ROWS * Ci, np, rs, Ci, db_t, db_p, db_g, stream);
+}
+
+// Scratch of the standalone attention entry points: the same pieces, sized the same way, as ws_bwd / ws_fwd give the
+// module's attention (attention scratch, delta, the three column-statistic tables and the reduction buffer).
+struct WsAttn { void* attn; float *delta, *cs_t, *cs_p, *cs_g, *red1; int cs_cap_rows; };
+size_t carve_ws_attn(long long B, long long N, int Ci, bool backward, void* base, WsAttn* w) {
+  Carver c(base);
+  w->attn = c.take<uint8_t>(attn_scratch_bytes(B, N, backward));
+  w->delta = w->cs_t = w->cs_p = w->cs_g = w->red1 = nullptr;
+  w->cs_cap_rows = 4 * static_cast<int>(B) * gemm_tiles_m(static_cast<int>(N));   // one partial per (tile, 32-row quarter)
+  if (backward) {
+    const size_t np = static_cast<size_t>(w->cs_cap_rows);
+    w->delta = c.take<float>(static_cast<size_t>(B * N));
+    w->cs_t = c.take<float>(np * 2 * Ci);
+    w->cs_p = c.take<float>(np * 2 * Ci);
+    w->cs_g = c.take<float>(np * 2 * Ci);
+    w->red1 = c.take<float>(static_cast<size_t>(REDUCE_STAGE1_ROWS) * 3 * Ci);
+  }
+  return (c.off + 255) & ~static_cast<size_t>(255);
+}
+
+// the limits make_dims puts on a TPAVIModule's attention
+int check_attn_dims(int B, int N, int Ci) {
+  if (B <= 0 || N <= 0) return set_error(GLF_ERR_INVALID, "attention: empty input (B and N must be > 0, got %d, %d)", B, N);
+  if (Ci <= 0 || Ci % 8 != 0 || Ci > 2048)
+    return set_error(GLF_ERR_INVALID, "attention: Ci must be a positive multiple of 8, at most 2048 (got %d)", Ci);
+  if (static_cast<long long>(B) * N > 0x7fffff00LL || 4LL * B * gemm_tiles_m(N) > 0x7fffffffLL)
+    return set_error(GLF_ERR_INVALID, "attention: too many tokens");
+  return 0;
+}
+
+int check_scratch(const void* scratch) {
+  GLF_TRY(check_ptr(scratch, "scratch"));
+  if ((reinterpret_cast<uintptr_t>(scratch) & 255) != 0) return set_error(GLF_ERR_WORKSPACE, "scratch must be 256-byte aligned");
+  return 0;
+}
+
 }  // namespace
 }  // namespace glf
 
@@ -1010,9 +1066,12 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.split_k = pick_split_rounds(C, Ci, 1, rows);
       GLF_TRY(gemm(g, stream));
     }
-    GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, &np, B, N,
-                      Ci, wb.attn, stream));
-    np_p = np_g = np;
+    int cs_rows[3];
+    GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows, B,
+                      N, Ci, wb.attn, stream));
+    np = cs_rows[0];
+    np_p = cs_rows[1];
+    np_g = cs_rows[2];
   }
   GLF_TRY(check_cuda(cudaMemsetAsync(wb.dwcat, 0, sizeof(float) * 3 * Ci * C, stream), "memset dWcat"));
   {  // dWcat[r,c] = sum_n dP[n,r] X[n,c]
@@ -1038,27 +1097,8 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     g.D = m.pack_x ? static_cast<void*>(wb.dxtok) : dx; g.ldd = C;
     GLF_TRY(gemm(g, stream));
   }
-  {  // bias gradients = column sums of dTheta / dPhi / dG, from the per-sub-block partials of their GEMM epilogues
-    // the three tables can have different row counts (tile shape and grid differ per product): stage 1 always
-    long long rs = 2LL * Ci;
-    const float *t0 = wb.cs_t, *t1 = wb.cs_p, *t2 = wb.cs_g;
-    if (np < 0) {  // flash backward: one table of width 3Ci (column sums of dP = [dTheta | dPhi | dG])
-      np = np_p = np_g = -np;
-      rs = 2LL * 3 * Ci;
-      t1 = wb.cs_t + Ci;
-      t2 = wb.cs_t + 2 * Ci;
-    }
-    if (np == np_p && np == np_g && np <= 4 * REDUCE_STAGE1_ROWS) {
-      // short tables (one row per CTA): a single fixed-order reduction
-      GLF_TRY(reduce_partials3(t0, t1, t2, np, rs, Ci, g_->theta_b, g_->phi_b, g_->g_b, stream));
-    } else {
-      const int np_in[3] = {np, np_p, np_g};
-      GLF_TRY(reduce_stage1(t0, t1, t2, 3, np_in, &np, &rs, 0, 1, Ci, wb.red1, stream));
-      GLF_TRY(reduce_partials3(wb.red1, wb.red1 + static_cast<long long>(REDUCE_STAGE1_ROWS) * Ci,
-                               wb.red1 + 2LL * REDUCE_STAGE1_ROWS * Ci, np, rs, Ci, g_->theta_b, g_->phi_b, g_->g_b,
-                               stream));
-    }
-  }
+  GLF_TRY(reduce_bias_grads(wb.cs_t, wb.cs_p, wb.cs_g, np, np_p, np_g, Ci, wb.red1, g_->theta_b, g_->phi_b, g_->g_b,
+                            stream));
   if (m.pack_x) {
     if (d->x_layout == GLF_LAYOUT_NCTHW)
       GLF_TRY(transpose_cast(wb.dxtok, dx, B, N, C, GLF_DTYPE_BF16, d->io_dtype, stream));
@@ -1346,6 +1386,49 @@ GLF_API int glf_gram_contraction(const void* A, const void* X, void* D, float* c
   return gram_contraction(reinterpret_cast<const bf16*>(A), reinterpret_cast<const bf16*>(X), reinterpret_cast<bf16*>(D),
                           nullptr, colsum, nullptr, nullptr, 0.f, 0, B, N, C, ldd, 1,
                           reinterpret_cast<cudaStream_t>(stream));
+}
+
+GLF_API size_t glf_attention_scratch_bytes(int B, int N, int Ci, int backward) {
+  if (check_attn_dims(B, N, Ci) != 0) return 0;
+  WsAttn w;
+  return carve_ws_attn(B, N, Ci, backward != 0, nullptr, &w);
+}
+
+GLF_API int glf_attention_fwd(const void* P3, void* Y, float* lse, int B, int N, int Ci, void* scratch,
+                              glf_stream_t stream) {
+  GLF_TRY(check_attn_dims(B, N, Ci));
+  GLF_TRY(check_ptr(P3, "P3"));
+  GLF_TRY(check_ptr(Y, "Y"));
+  GLF_TRY(check_ptr(lse, "lse"));
+  GLF_TRY(check_scratch(scratch));
+  GLF_TRY(check_device_sm100());
+  WsAttn w;
+  carve_ws_attn(B, N, Ci, false, scratch, &w);
+  return flash_fwd(reinterpret_cast<const bf16*>(P3), reinterpret_cast<bf16*>(Y), lse, B, N, Ci, w.attn,
+                   reinterpret_cast<cudaStream_t>(stream));
+}
+
+GLF_API int glf_attention_bwd(const void* P3, const void* Y, const void* dY, const float* lse, void* dP3,
+                              float* bias_grad, int B, int N, int Ci, void* scratch, glf_stream_t stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  GLF_TRY(check_attn_dims(B, N, Ci));
+  GLF_TRY(check_ptr(P3, "P3"));
+  GLF_TRY(check_ptr(Y, "Y"));
+  GLF_TRY(check_ptr(dY, "dY"));
+  GLF_TRY(check_ptr(lse, "lse"));
+  GLF_TRY(check_ptr(dP3, "dP3"));
+  if (bias_grad != nullptr) GLF_TRY(check_ptr(bias_grad, "bias_grad"));
+  GLF_TRY(check_scratch(scratch));
+  GLF_TRY(check_device_sm100());
+  WsAttn w;
+  carve_ws_attn(B, N, Ci, true, scratch, &w);
+  int np[3];
+  GLF_TRY(flash_bwd(reinterpret_cast<const bf16*>(P3), reinterpret_cast<const bf16*>(Y), reinterpret_cast<const bf16*>(dY),
+                    lse, reinterpret_cast<bf16*>(dP3), w.delta, w.cs_t, w.cs_p, w.cs_g, w.cs_cap_rows, np, B, N, Ci,
+                    w.attn, stream));
+  if (bias_grad == nullptr) return 0;
+  return reduce_bias_grads(w.cs_t, w.cs_p, w.cs_g, np[0], np[1], np[2], Ci, w.red1, bias_grad, bias_grad + Ci,
+                           bias_grad + 2 * Ci, stream);
 }
 
 GLF_API int glf_bn_res_ln_fwd(int64_t rows, int C, const void* U, const void* X, const float* bn_a, const float* bn_b,

@@ -879,7 +879,7 @@ int flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* s
 }
 
 static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3,
-                                 float* delta, float* cs_t, float* cs_p, float* cs_g, int* cs_rows_out, int B, int N,
+                                 float* delta, float* cs_t, float* cs_p, float* cs_g, int cs_rows_out[3], int B, int N,
                                  int Ci, void* scratch, cudaStream_t stream) {
   const int ld = attn_ld(N);
   const int nb = attn_chunk(B, N);
@@ -890,7 +890,9 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
   bf16* dS = Pm + nb * per;
   const long long seqP = static_cast<long long>(N) * 3 * Ci;
   const long long rows = static_cast<long long>(B) * N;
-  int cs_rows_total = 0;   // rows of the three column-stat tables written so far (same for all three)
+  // rows of each column-stat table written so far: the three products can leave different row counts per chunk (the
+  // dTheta GEMM runs 256-row super-tiles for N >= 1024, the other two do not), so each table has its own offset
+  int cs_rows_total[3] = {0, 0, 0};
   {
     const long long threads = rows * 32;
     rowdot_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, stream>>>(dY, Y, delta, rows, Ci);
@@ -902,7 +904,6 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
     const bf16* Pb = P3 + b0 * seqP;
     const bf16* dYb = dY + static_cast<long long>(b0) * N * Ci;
     bf16* dPb = dP3 + b0 * seqP;
-    const long long cs_off = static_cast<long long>(cs_rows_total) * 2 * Ci;
     int r_t = 0, r_p = 0, r_g = 0;
     int rc;
     {  // S = Theta Phi^T (recompute)
@@ -948,7 +949,7 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
       g.B = op(Pb + Ci, 1, 3 * Ci, seqP);
       g.M = N; g.N = Ci; g.K = N; g.batch = cb;
       g.D = dPb; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_t + cs_off;
+      g.colstats = cs_t + static_cast<long long>(cs_rows_total[0]) * 2 * Ci;
       g.colstats_rows = &r_t;
       if ((rc = gemm(g, stream))) return rc;
     }
@@ -958,7 +959,7 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
       g.B = op(Pb, 1, 3 * Ci, seqP);
       g.M = N; g.N = Ci; g.K = N; g.batch = cb;
       g.D = dPb + Ci; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_p + cs_off;
+      g.colstats = cs_p + static_cast<long long>(cs_rows_total[1]) * 2 * Ci;
       g.colstats_rows = &r_p;
       if ((rc = gemm(g, stream))) return rc;
     }
@@ -968,14 +969,15 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
       g.B = op(dYb, 1, Ci, static_cast<long long>(N) * Ci);
       g.M = N; g.N = Ci; g.K = N; g.batch = cb;
       g.D = dPb + 2 * Ci; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_g + cs_off;
+      g.colstats = cs_g + static_cast<long long>(cs_rows_total[2]) * 2 * Ci;
       g.colstats_rows = &r_g;
       if ((rc = gemm(g, stream))) return rc;
     }
-    if (r_p != r_t || r_g != r_t) return set_error(GLF_ERR_INVALID, "internal: column-stat tables disagree");
-    cs_rows_total += r_t;
+    cs_rows_total[0] += r_t;
+    cs_rows_total[1] += r_p;
+    cs_rows_total[2] += r_g;
   }
-  *cs_rows_out = cs_rows_total;
+  for (int i = 0; i < 3; ++i) cs_rows_out[i] = cs_rows_total[i];
   return 0;
 }
 
@@ -985,7 +987,7 @@ int flash_bwd_colsum_blocks(long long rows) {
 }
 
 int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3, float* delta, float* cs_t,
-              float* cs_p, float* cs_g, int cs_cap_rows, int* cs_rows_out, int B, int N, int Ci, void* scratch,
+              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
               cudaStream_t stream) {
   if (Ci != 128 && Ci != 64)   // other head widths: exact chunked path
     return attn_bwd_materialized(P3, Y, dY, lse, dP3, delta, cs_t, cs_p, cs_g, cs_rows_out, B, N, Ci, scratch, stream);
@@ -1005,7 +1007,7 @@ int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, b
   if (grid > cs_cap_rows / 3) grid = cs_cap_rows / 3 > 0 ? cs_cap_rows / 3 : 1;   // cs_t holds cs_cap_rows x 2 x Ci floats
   colsum_bf16_kernel<<<grid, 256, 0, stream>>>(dP3, cs_t, rows, 3 * Ci);
   if ((rc = check_cuda(cudaGetLastError(), "colsum launch"))) return rc;
-  *cs_rows_out = -grid;   // negative: "single table of width 3Ci" (see glf_tpavi_bwd)
+  cs_rows_out[0] = cs_rows_out[1] = cs_rows_out[2] = -grid;   // negative: "single table of width 3Ci" (see glf_tpavi_bwd)
   return 0;
 }
 

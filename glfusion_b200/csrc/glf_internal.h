@@ -217,9 +217,10 @@ int attn_ld(int N);
 int attn_chunk(long long B, long long N);
 size_t attn_scratch_bytes(long long B, long long N, bool backward);
 int flash_fwd(const bf16* P, bf16* Y, float* lse, int B, int N, int Ci, void* scratch, cudaStream_t stream);
-// *cs_rows_out > 0: three tables [rows][2][Ci] (cs_t, cs_p, cs_g);  < 0: one table [-rows][2][3Ci] in cs_t
+// cs_rows_out[i] > 0: rows of the three tables [rows][2][Ci] (cs_t, cs_p, cs_g);  < 0 (all three): one table
+// [-rows][2][3Ci] in cs_t
 int flash_bwd(const bf16* P, const bf16* Y, const bf16* dY, const float* lse, bf16* dP, float* delta, float* cs_t,
-              float* cs_p, float* cs_g, int cs_cap_rows, int* cs_rows_out, int B, int N, int Ci, void* scratch,
+              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
               cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------ P2P all-reduce (glf_p2p.cu)

@@ -259,6 +259,19 @@ GLF_API int glf_gemm_bf16_ex(const void* A, const void* B, void* D, int M, int N
 GLF_API int glf_gram_contraction(const void* A, const void* X, void* D, float* colsum, int B, int N, int C, int ldd,
                          glf_stream_t stream);
 
+/* The softmax attention of mode='embedded' on its own (unit tests): the functions glf_tpavi_fwd / glf_tpavi_bwd run,
+ * with the same head-width dispatch (flash kernels for Ci = 64 and 128, the chunked exact path otherwise).
+ *   fwd: Y = softmax(Theta Phi^T) G per sequence, no 1/sqrt(Ci) scale;  lse = logsumexp of each score row (natural log).
+ *   bwd: dP3 = [dTheta | dPhi | dG] from dY and the forward's Y and lse;  bias_grad (optional, may be NULL): the 3 Ci
+ *        column sums of dP3 over all B * N rows, reduced as glf_tpavi_bwd reduces its bias gradients.
+ *   P3: [B, N, 3 Ci] bf16 = [Theta | Phi | G] per token;  Y, dY: [B, N, Ci] bf16;  lse: [B, N] fp32;  dP3 like P3.
+ *   B, N > 0;  Ci a positive multiple of 8, <= 2048;  16-byte aligned pointers.
+ *   scratch: glf_attention_scratch_bytes(B, N, Ci, backward) bytes, 256-byte aligned (0 = invalid arguments). */
+GLF_API size_t glf_attention_scratch_bytes(int B, int N, int Ci, int backward);
+GLF_API int glf_attention_fwd(const void* P3, void* Y, float* lse, int B, int N, int Ci, void* scratch, glf_stream_t s);
+GLF_API int glf_attention_bwd(const void* P3, const void* Y, const void* dY, const float* lse, void* dP3, float* bias_grad,
+                      int B, int N, int Ci, void* scratch, glf_stream_t s);
+
 /* The two HBM-bound fused epilogues as standalone entry points (unit tests, roofline probes).
  *   fwd: Z = LayerNorm_C(bn_a * U + bn_b + X) * ln_w + ln_b   (ours.py:908-915 after the W_z GEMM); U, X bf16 [rows, C];
  *        Z [rows, C] of z_dtype (bf16, fp16 or fp32); mu, r: per-row LayerNorm mean / rstd (kept for backward).
