@@ -9,7 +9,7 @@ import threading
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libglf_sm100a.so")
 
-MODE_DOT, MODE_EMBEDDED = 0, 1
+MODE_DOT, MODE_EMBEDDED, MODE_GAUSSIAN = 0, 1, 2
 DTYPE_BF16, DTYPE_F32, DTYPE_F16 = 0, 1, 2
 LAYOUT_NCTHW, LAYOUT_TOKEN = 0, 1
 PRECISION_BF16, PRECISION_F32X3 = 0, 1
@@ -26,7 +26,8 @@ EXPORTS = ("glf_version", "glf_last_error", "glf_tpavi_sizes", "glf_tpavi_fwd", 
            "glf_bn_res_ln_pair_bwd", "glf_gemm_bf16_ex", "glf_gram_contraction", "glf_p2p_signal_bytes", "glf_p2p_max_floats",
            "glf_p2p_export", "glf_p2p_open", "glf_p2p_close", "glf_p2p_allreduce", "glf_spatial_sums",
            "glf_cycle_loss_scratch_bytes", "glf_cycle_loss", "glf_attention_scratch_bytes", "glf_attention_fwd",
-           "glf_attention_bwd")
+           "glf_attention_bwd", "glf_attention_gaussian_scratch_bytes", "glf_attention_gaussian_fwd",
+           "glf_attention_gaussian_bwd")
 
 
 class GlfDesc(C.Structure):
@@ -123,10 +124,15 @@ def load() -> C.CDLL:
         lib.glf_attention_scratch_bytes.restype = C.c_size_t
         lib.glf_attention_fwd.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
         lib.glf_attention_bwd.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp]
+        lib.glf_attention_gaussian_scratch_bytes.argtypes = [i32, i32, i32, i32, i32]
+        lib.glf_attention_gaussian_scratch_bytes.restype = C.c_size_t
+        lib.glf_attention_gaussian_fwd.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp, vp]
+        lib.glf_attention_gaussian_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp]
         for name in EXPORTS:
             fn = getattr(lib, name)
             if name not in ("glf_last_error", "glf_gate_concat_bwd_scratch_bytes", "glf_p2p_signal_bytes",
-                            "glf_p2p_max_floats", "glf_attention_scratch_bytes"):
+                            "glf_p2p_max_floats", "glf_attention_scratch_bytes",
+                            "glf_attention_gaussian_scratch_bytes"):
                 fn.restype = C.c_int
         _lib = lib
         return lib

@@ -10,6 +10,8 @@
 //         BN finalise, then  Z = LN(BN(U) + X)    HBM-bound fused epilogue
 //   bwd:  LN/BN backward (two HBM-bound passes), then six tcgen05 GEMMs (dTheta, dW', dPhi, dG, dWcat, dX) and two
 //         small fp32 products (dW_z, dM).
+// mode='embedded' and mode='gaussian' run the softmax attention of glf_flash.cu between the projection and the W_z GEMM;
+// gaussian projects g alone (P = G) and its attention reads x itself as Q and K, so dX gets dS X + dS^T X as well.
 // When the sequences are long against the channel count (N >= 5 C) mode='dot' runs in its Gram form instead
 // (tpavi_fwd_gram / tpavi_bwd_gram below; oracle/tpavi_oracle.py: tpavi_dot_gram_form): theta / phi / g and dU are never
 // materialised, the only token-sized products are S = X^T X, U = X Q^T, R = dV^T X and dX = [dV | X] [E ; F].
@@ -68,6 +70,7 @@ struct Dims {
   bool pack_x;     // x must be repacked to token-major bf16
   bool pack_dz;
   bool dot;
+  bool gauss;      // mode='gaussian': Q = K = X, only the g projection runs
   bool gram;       // mode='dot' in its Gram form (channel-space products only)
   int Ca;          // augmented width of the per-sequence matrices (gram)
   int pdt;         // GLF_DTYPE_* of the glf_weights / glf_grads tensors (glf_desc.reserved[3])
@@ -80,8 +83,8 @@ int make_dims(const glf_desc* d, Dims* o) {
   if (d->C <= 0 || d->Ci <= 0 || d->C % 8 != 0 || d->Ci % 8 != 0)
     return set_error(GLF_ERR_INVALID, "C and inter_channels must be positive multiples of 8 (got %d, %d)", d->C, d->Ci);
   if (d->C > 2048) return set_error(GLF_ERR_INVALID, "C <= 2048 supported (got %d)", d->C);
-  if (d->mode != GLF_MODE_DOT && d->mode != GLF_MODE_EMBEDDED)
-    return set_error(GLF_ERR_UNSUPPORTED, "mode must be dot or embedded ('gaussian'/'concatenate' are not built by the reference network)");
+  if (d->mode != GLF_MODE_DOT && d->mode != GLF_MODE_EMBEDDED && d->mode != GLF_MODE_GAUSSIAN)
+    return set_error(GLF_ERR_UNSUPPORTED, "mode must be dot, embedded or gaussian ('concatenate' is not built by the reference network)");
   if (d->precision != GLF_PRECISION_BF16 && d->precision != GLF_PRECISION_F32X3)
     return set_error(GLF_ERR_INVALID, "bad precision (GLF_PRECISION_BF16 or GLF_PRECISION_F32X3)");
   if (d->precision == GLF_PRECISION_F32X3 && d->mode != GLF_MODE_DOT)
@@ -115,6 +118,7 @@ int make_dims(const glf_desc* d, Dims* o) {
     return set_error(GLF_ERR_INVALID, "token-major fp32 / fp16 input too large for the cast kernel");
   o->pack_dz = d->dz_layout != GLF_LAYOUT_TOKEN;
   o->dot = d->mode == GLF_MODE_DOT;
+  o->gauss = d->mode == GLF_MODE_GAUSSIAN;
   // reserved[1]: 0 = choose, 1 = token-space form (theta/phi/g per token), 2 = Gram form
   if (d->reserved[1] < 0 || d->reserved[1] > 2) return set_error(GLF_ERR_INVALID, "reserved[1] (dot algorithm) must be 0, 1 or 2");
   const bool gram_ok = o->dot && d->precision == GLF_PRECISION_BF16 && o->B <= 65535;
@@ -181,7 +185,7 @@ int emit_grads(const Dims& m, float* const st[NPARAMS], const glf_grads* g, cuda
   param_counts(m, p.n);
   for (int k = 0; k < NPARAMS; ++k) {
     p.src[k] = st[k];
-    p.dst[k] = v[k];
+    p.dst[k] = (m.gauss && k < 4) ? nullptr : v[k];   // gaussian: theta / phi take no part and receive no gradient
   }
   return convert_params(p, GLF_DTYPE_F32, m.pdt, stream);
 }
@@ -224,7 +228,7 @@ size_t carve_saved(const Dims& m, void* base, Saved* s) {
     s->ln_r = c.take<float>(rows);
     return (c.off + 255) & ~static_cast<size_t>(255);
   }
-  s->P = c.take<bf16>(rows * 3 * Ci);
+  s->P = c.take<bf16>(rows * (m.gauss ? Ci : 3 * Ci));   // [Theta | Phi | G], or G alone (gaussian)
   s->U = c.take<bf16>(rows * C);
   if (m.dot) {
     s->Y = nullptr; s->lse = nullptr;
@@ -235,9 +239,10 @@ size_t carve_saved(const Dims& m, void* base, Saved* s) {
     s->lse = c.take<float>(rows);
     s->Mb = nullptr; s->Wp = nullptr;
   }
-  s->wcat = c.take<bf16>(3 * Ci * C);
-  s->wcatT = c.take<bf16>(3 * Ci * C);
-  s->bcat = c.take<float>(3 * Ci);
+  // gaussian: wcat = W_g [Ci, C], bcat = b_g, wcatT = [I | I | W_g^T] [C, 2C + Ci] (prep_weights_gaussian)
+  s->wcat = c.take<bf16>((m.gauss ? 1 : 3) * Ci * C);
+  s->wcatT = c.take<bf16>(m.gauss ? C * (2 * C + Ci) : 3 * Ci * C);
+  s->bcat = c.take<float>((m.gauss ? 1 : 3) * Ci);
   s->wz = c.take<bf16>(C * Ci);
   s->wzT = c.take<bf16>(C * Ci);
   s->bn_mean = c.take<float>(C);
@@ -314,7 +319,7 @@ size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
     return (c.off + 255) & ~static_cast<size_t>(255);
   }
   w->dU = d->bn_layer ? c.take<bf16>(rows * C) : nullptr;
-  w->dP = c.take<bf16>(rows * 3 * Ci);
+  w->dP = c.take<bf16>(rows * (m.gauss ? 2 * C + Ci : 3 * Ci));   // [dTheta | dPhi | dG], or [dS X | dS^T X | dG]
   w->dxtok = m.pack_x ? c.take<bf16>(rows * C) : nullptr;
   if (m.dot) {
     w->dY = nullptr; w->delta = nullptr;
@@ -744,13 +749,24 @@ int reduce_bias_grads(const float* cs_t, const float* cs_p, const float* cs_g, i
                           red1 + 2LL * REDUCE_STAGE1_ROWS * Ci, np, rs, Ci, db_t, db_p, db_g, stream);
 }
 
+// The g bias gradient of mode='gaussian' from the one table of column sums of dG the attention backward left in cs
+int reduce_bias_grad1(const float* cs, int np, int Ci, float* red1, float* db, cudaStream_t stream) {
+  long long rs = 2LL * Ci;
+  if (np <= 4 * REDUCE_STAGE1_ROWS) return reduce_partials(cs, np, rs, Ci, 1.f, db, stream);
+  const int np_in[1] = {np};
+  GLF_TRY(reduce_stage1(cs, nullptr, nullptr, 1, np_in, &np, &rs, 0, 1, Ci, red1, stream));
+  return reduce_partials(red1, np, rs, Ci, 1.f, db, stream);
+}
+
 // Scratch of the standalone attention entry points: the same pieces, sized the same way, as ws_bwd / ws_fwd give the
 // module's attention (attention scratch, delta, the three column-statistic tables and the reduction buffer).
-struct WsAttn { void* attn; float *delta, *cs_t, *cs_p, *cs_g, *red1; int cs_cap_rows; };
-size_t carve_ws_attn(long long B, long long N, int Ci, bool backward, void* base, WsAttn* w) {
+// C > 0 (mode='gaussian'): also the [B * N, 2C] pair dS X | dS^T X that the backward sums into dX.
+struct WsAttn { void* attn; float *delta, *cs_t, *cs_p, *cs_g, *red1; bf16* dx2; int cs_cap_rows; };
+size_t carve_ws_attn(long long B, long long N, int Ci, bool backward, void* base, WsAttn* w, int C = 0) {
   Carver c(base);
   w->attn = c.take<uint8_t>(attn_scratch_bytes(B, N, backward));
   w->delta = w->cs_t = w->cs_p = w->cs_g = w->red1 = nullptr;
+  w->dx2 = (backward && C > 0) ? c.take<bf16>(static_cast<size_t>(B * N) * 2 * C) : nullptr;
   w->cs_cap_rows = 4 * static_cast<int>(B) * gemm_tiles_m(static_cast<int>(N));   // one partial per (tile, 32-row quarter)
   if (backward) {
     const size_t np = static_cast<size_t>(w->cs_cap_rows);
@@ -828,7 +844,10 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
   const int C = m.C, Ci = m.Ci;
   const int N = static_cast<int>(m.N), rows = static_cast<int>(m.rows), B = static_cast<int>(m.B);
 
-  GLF_TRY(prep_weights(w, C, Ci, s.wcat, s.wcatT, s.bcat, s.wz, s.wzT, stream));
+  if (m.gauss)
+    GLF_TRY(prep_weights_gaussian(w, C, Ci, s.wcat, s.wcatT, s.bcat, s.wz, s.wzT, stream));
+  else
+    GLF_TRY(prep_weights(w, C, Ci, s.wcat, s.wcatT, s.bcat, s.wz, s.wzT, stream));
   const bf16* X = reinterpret_cast<const bf16*>(x);
   if (m.pack_x) {
     if (d->x_layout == GLF_LAYOUT_NCTHW)
@@ -837,13 +856,14 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
       GLF_TRY(transpose_cast(x, s.xtok, 1, 1, static_cast<int>(m.rows * C), d->io_dtype, GLF_DTYPE_BF16, stream));  // cast only
     X = s.xtok;
   }
-  {  // P = X Wcat^T + bcat
+  const int Pw = m.gauss ? Ci : 3 * Ci;
+  {  // P = X Wcat^T + bcat   (gaussian: G = X Wg^T + bg)
     GemmArgs g;
     g.A = opnd(X, 0, C, 0);
     g.B = opnd(s.wcat, 0, C, 0);
-    g.M = rows; g.N = 3 * Ci; g.K = C;
+    g.M = rows; g.N = Pw; g.K = C;
     g.bias = s.bcat;
-    g.D = s.P; g.ldd = 3 * Ci;
+    g.D = s.P; g.ldd = Pw;
     GLF_TRY(gemm(g, stream));
   }
   int np = 0;
@@ -888,7 +908,11 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
       GLF_TRY(gemm(g, stream));
     }
   } else {
-    GLF_TRY(flash_fwd(s.P, s.Y, s.lse, B, N, Ci, wf.attn, stream));
+    if (m.gauss)   // Y = softmax(X X^T) G
+      GLF_TRY(attn_fwd(attn_args_gaussian(X, s.P, nullptr, nullptr, nullptr, 0, 0, C, Ci), s.Y, s.lse, B, N, wf.attn,
+                       stream));
+    else
+      GLF_TRY(flash_fwd(s.P, s.Y, s.lse, B, N, Ci, wf.attn, stream));
     {  // U = Y Wz^T   (bz folded into the BN affine)
       GemmArgs g;
       g.A = opnd(s.Y, 0, Ci, 0);
@@ -1067,38 +1091,57 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       GLF_TRY(gemm(g, stream));
     }
     int cs_rows[3];
-    GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows, B,
-                      N, Ci, wb.attn, stream));
+    if (m.gauss) {   // dP = [dS X | dS^T X | dG]: the two attention terms of dX side by side, summed by the dX product
+      const long long ldp = 2LL * C + Ci;
+      const AttnArgs a = attn_args_gaussian(X, s.P, wb.dP, wb.dP + C, wb.dP + 2 * C, ldp, ldp, C, Ci);
+      GLF_TRY(attn_bwd(a, s.Y, wb.dY, s.lse, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows, B, N,
+                       wb.attn, stream));
+    } else {
+      GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows,
+                        B, N, Ci, wb.attn, stream));
+    }
     np = cs_rows[0];
     np_p = cs_rows[1];
     np_g = cs_rows[2];
   }
-  GLF_TRY(check_cuda(cudaMemsetAsync(wb.dwcat, 0, sizeof(float) * 3 * Ci * C, stream), "memset dWcat"));
+  // dP columns [wrow, ldp) are the projection gradients (all three, or dG alone for gaussian)
+  const int ldp = m.gauss ? 2 * C + Ci : 3 * Ci;
+  const int wrow = m.gauss ? 2 * C : 0;
+  const int nproj = m.gauss ? Ci : 3 * Ci;
+  GLF_TRY(check_cuda(cudaMemsetAsync(wb.dwcat, 0, sizeof(float) * nproj * C, stream), "memset dWcat"));
   {  // dWcat[r,c] = sum_n dP[n,r] X[n,c]
     GemmArgs g;
-    g.A = opnd(wb.dP, 1, 3 * Ci, 0);
+    g.A = opnd(wb.dP + wrow, 1, ldp, 0);
     g.B = opnd(X, 1, C, 0);
-    g.M = 3 * Ci; g.N = C; g.K = rows;
+    g.M = nproj; g.N = C; g.K = rows;
     g.out_kind = 2;
     g.D = wb.dwcat; g.ldd = C;
-    g.split_k = pick_split_rounds(3 * Ci, C, 1, rows);
+    g.split_k = pick_split_rounds(nproj, C, 1, rows);
     GLF_TRY(gemm(g, stream));
   }
   const size_t wbytes = sizeof(float) * Ci * C;
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->theta_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dtheta"));
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->phi_w, wb.dwcat + static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dphi"));
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat + 2 * static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
-  {  // dX = dP Wcat + dV
+  if (m.gauss) {
+    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
+  } else {
+    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->theta_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dtheta"));
+    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->phi_w, wb.dwcat + static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dphi"));
+    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat + 2 * static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
+  }
+  {  // dX = dP Wcat + dV   (gaussian: [dS X | dS^T X | dG] [I | I | Wg^T]^T + dV, each attention term rounded to bf16
+     // once before this fp32 sum)
     GemmArgs g;
-    g.A = opnd(wb.dP, 0, 3 * Ci, 0);
-    g.B = opnd(s.wcatT, 0, 3 * Ci, 0);
-    g.M = rows; g.N = C; g.K = 3 * Ci;
+    g.A = opnd(wb.dP, 0, ldp, 0);
+    g.B = opnd(s.wcatT, 0, ldp, 0);
+    g.M = rows; g.N = C; g.K = ldp;
     g.addend = wb.dV; g.ld_add = C;
     g.D = m.pack_x ? static_cast<void*>(wb.dxtok) : dx; g.ldd = C;
     GLF_TRY(gemm(g, stream));
   }
-  GLF_TRY(reduce_bias_grads(wb.cs_t, wb.cs_p, wb.cs_g, np, np_p, np_g, Ci, wb.red1, g_->theta_b, g_->phi_b, g_->g_b,
-                            stream));
+  if (m.gauss)
+    GLF_TRY(reduce_bias_grad1(wb.cs_g, np_g, Ci, wb.red1, g_->g_b, stream));
+  else
+    GLF_TRY(reduce_bias_grads(wb.cs_t, wb.cs_p, wb.cs_g, np, np_p, np_g, Ci, wb.red1, g_->theta_b, g_->phi_b, g_->g_b,
+                              stream));
   if (m.pack_x) {
     if (d->x_layout == GLF_LAYOUT_NCTHW)
       GLF_TRY(transpose_cast(wb.dxtok, dx, B, N, C, GLF_DTYPE_BF16, d->io_dtype, stream));
@@ -1429,6 +1472,57 @@ GLF_API int glf_attention_bwd(const void* P3, const void* Y, const void* dY, con
   if (bias_grad == nullptr) return 0;
   return reduce_bias_grads(w.cs_t, w.cs_p, w.cs_g, np[0], np[1], np[2], Ci, w.red1, bias_grad, bias_grad + Ci,
                            bias_grad + 2 * Ci, stream);
+}
+
+GLF_API size_t glf_attention_gaussian_scratch_bytes(int B, int N, int C, int Ci, int backward) {
+  if (check_attn_dims(B, N, Ci) != 0 || check_attn_dims(B, N, C) != 0) return 0;
+  WsAttn w;
+  return carve_ws_attn(B, N, Ci, backward != 0, nullptr, &w, C);
+}
+
+GLF_API int glf_attention_gaussian_fwd(const void* X, const void* G, void* Y, float* lse, int B, int N, int C, int Ci,
+                                       void* scratch, glf_stream_t stream) {
+  GLF_TRY(check_attn_dims(B, N, Ci));
+  GLF_TRY(check_attn_dims(B, N, C));
+  GLF_TRY(check_ptr(X, "X"));
+  GLF_TRY(check_ptr(G, "G"));
+  GLF_TRY(check_ptr(Y, "Y"));
+  GLF_TRY(check_ptr(lse, "lse"));
+  GLF_TRY(check_scratch(scratch));
+  GLF_TRY(check_device_sm100());
+  WsAttn w;
+  carve_ws_attn(B, N, Ci, false, scratch, &w, C);
+  const AttnArgs a = attn_args_gaussian(reinterpret_cast<const bf16*>(X), reinterpret_cast<const bf16*>(G), nullptr,
+                                        nullptr, nullptr, 0, 0, C, Ci);
+  return attn_fwd(a, reinterpret_cast<bf16*>(Y), lse, B, N, w.attn, reinterpret_cast<cudaStream_t>(stream));
+}
+
+GLF_API int glf_attention_gaussian_bwd(const void* X, const void* G, const void* Y, const void* dY, const float* lse,
+                                       void* dX, void* dG, float* bias_grad, int B, int N, int C, int Ci, void* scratch,
+                                       glf_stream_t stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  GLF_TRY(check_attn_dims(B, N, Ci));
+  GLF_TRY(check_attn_dims(B, N, C));
+  GLF_TRY(check_ptr(X, "X"));
+  GLF_TRY(check_ptr(G, "G"));
+  GLF_TRY(check_ptr(Y, "Y"));
+  GLF_TRY(check_ptr(dY, "dY"));
+  GLF_TRY(check_ptr(lse, "lse"));
+  GLF_TRY(check_ptr(dX, "dX"));
+  GLF_TRY(check_ptr(dG, "dG"));
+  if (bias_grad != nullptr) GLF_TRY(check_ptr(bias_grad, "bias_grad"));
+  GLF_TRY(check_scratch(scratch));
+  GLF_TRY(check_device_sm100());
+  WsAttn w;
+  carve_ws_attn(B, N, Ci, true, scratch, &w, C);
+  const AttnArgs a = attn_args_gaussian(reinterpret_cast<const bf16*>(X), reinterpret_cast<const bf16*>(G), w.dx2,
+                                        w.dx2 + C, reinterpret_cast<bf16*>(dG), 2LL * C, Ci, C, Ci);
+  int np[3];
+  GLF_TRY(attn_bwd(a, reinterpret_cast<const bf16*>(Y), reinterpret_cast<const bf16*>(dY), lse, w.delta, w.cs_t, w.cs_p,
+                   w.cs_g, w.cs_cap_rows, np, B, N, w.attn, stream));
+  GLF_TRY(sum_halves(w.dx2, reinterpret_cast<bf16*>(dX), static_cast<long long>(B) * N, C, stream));
+  if (bias_grad == nullptr) return 0;
+  return reduce_bias_grad1(w.cs_g, np[2], Ci, w.red1, bias_grad, stream);
 }
 
 GLF_API int glf_bn_res_ln_fwd(int64_t rows, int C, const void* U, const void* X, const float* bn_a, const float* bn_b,

@@ -1166,6 +1166,53 @@ int prep_weights(const glf_weights* w, int C, int Ci, bf16* wcat, bf16* wcatT, f
   return check_cuda(cudaGetLastError(), "prep_weights launch");
 }
 
+namespace {
+// mode='gaussian': wg = bf16(g.weight) [Ci, C], bg [Ci], wgT [C, 2C + Ci] = [I | I | g.weight^T], and W_z as
+// prep_weights_kernel writes it.  One element per thread (grid-stride): the transposed reads of g.weight / W_z are
+// strided, which a per-call pass over C (2C + Ci) elements can afford.
+__global__ void __launch_bounds__(256) prep_weights_gaussian_kernel(const float* __restrict__ gw,
+                                                                     const float* __restrict__ gb,
+                                                                     const float* __restrict__ wz, bf16* __restrict__ wg,
+                                                                     bf16* __restrict__ wgT, float* __restrict__ bg,
+                                                                     bf16* __restrict__ wzb, bf16* __restrict__ wzT,
+                                                                     int C, int Ci) {
+  const long long W = 2LL * C + Ci;
+  const long long n_t = static_cast<long long>(C) * W, n_w = static_cast<long long>(Ci) * C;
+  const long long total = n_t + 2 * n_w + Ci;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    if (i < n_t) {
+      const long long c = i / W, k = i % W;
+      float v;
+      if (k < 2LL * C) v = (k % C) == c ? 1.f : 0.f;
+      else v = gw[(k - 2LL * C) * C + c];
+      wgT[i] = __float2bfloat16(v);
+    } else if (i < n_t + n_w) {
+      const long long j = i - n_t;                         // g.weight, row-major [Ci, C]
+      wg[j] = __float2bfloat16(gw[j]);
+    } else if (i < n_t + 2 * n_w) {
+      const long long j = i - n_t - n_w;                   // W_z [C, Ci] and its transpose [Ci, C]
+      const float v = wz[j];
+      wzb[j] = __float2bfloat16(v);
+      wzT[(j % Ci) * C + j / Ci] = __float2bfloat16(v);
+    } else {
+      const long long j = i - n_t - 2 * n_w;
+      bg[j] = gb[j];
+    }
+  }
+}
+}  // namespace
+
+int prep_weights_gaussian(const glf_weights* w, int C, int Ci, bf16* wg, bf16* wgT, float* bg, bf16* wz, bf16* wzT,
+                          cudaStream_t stream) {
+  const long long total = static_cast<long long>(C) * (2LL * C + Ci) + 2LL * Ci * C + Ci;
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  prep_weights_gaussian_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(w->g_w, w->g_b, w->wz_w, wg, wgT, bg,
+                                                                                  wz, wzT, C, Ci);
+  return check_cuda(cudaGetLastError(), "prep_weights_gaussian launch");
+}
+
 // stage-1 launcher: returns the reduced table (in `scratch`) and its row count through *np
 int reduce_stage1(const float* p0, const float* p1, const float* p2, int ntab, const int* np_in, int* np,
                   long long* row_stride, long long stat_stride, int NS, int C, float* scratch, cudaStream_t stream) {

@@ -123,30 +123,36 @@ constexpr float kLn2 = 0.6931471805599453f;
 // The two query tiles ping-pong: while warpgroup t does the softmax of S_t, the tensor pipe computes the other
 // tile's P V product and next scores.  MMA issue order per key tile j (t = 0, 1):
 //       wait P_t(j) ;  O_t += P_t(j) V_j ;  S_t(j+1) = Q_t K_{j+1}^T
-// TMEM (512 columns): S0/P0 [0,128), S1/P1 [128,256), O0 [256,256+D), O1 [384,384+D).
+// TMEM (512 columns): S0/P0 [0,128), S1/P1 [128,256), O0 [256,256+DV), O1 [384,384+DV).
 // Online softmax with a lazy reference maximum (log2 domain): the running maximum is only raised -- and O rescaled in
 // TMEM -- when a tile's maximum exceeds it by more than 8 (P <= 2^8 stays exact enough in bf16/fp32), so after the
 // first few tiles the rescale pass disappears.  lse = (m + log2 l) ln 2 is exact irrespective of the reference.
-template <int D>
+// DQK: width of Q and K (the score product's K extent); DV: width of V, O, dY and dV.  mode='embedded' runs DQK = DV =
+// Ci; mode='gaussian' reads Q = K = X (DQK = C) against V = G (DV = C').
+template <int DQK, int DV>
 struct FlashCfg {
-  static constexpr uint32_t TILE = 128 * D * 2;              // bytes of a 128 x D bf16 tile (D/64 swizzle atoms)
-  static constexpr uint32_t SUB = 64 * D * 2;                // bytes of a 64 x D bf16 tile
-  static constexpr uint32_t SMEM_FWD = TILE * 6 + 1024;      // 2 Q + 2 K + 2 V
-  static constexpr uint32_t SMEM_BWD = TILE * 2 + 4 * 2 * SUB + 1024;   // 2 resident tiles + 4-deep ring of sub-tile pairs
+  static constexpr uint32_t TILE_QK = 128 * DQK * 2;         // bytes of a 128 x DQK bf16 tile (DQK/64 swizzle atoms)
+  static constexpr uint32_t TILE_V = 128 * DV * 2;
+  static constexpr uint32_t SUB_QK = 64 * DQK * 2;           // bytes of a 64-row sub-tile
+  static constexpr uint32_t SUB_V = 64 * DV * 2;
+  static constexpr uint32_t SMEM_FWD = TILE_QK * 4 + TILE_V * 2 + 1024;   // 2 Q + 2 K + 2 V
+  // 2 resident tiles (Q | dY, or K | V) + 4-deep ring of sub-tile pairs (K | V, or Q | dY)
+  static constexpr uint32_t SMEM_BWD = TILE_QK + TILE_V + 4 * (SUB_QK + SUB_V) + 1024;
+  static_assert(DQK % 64 == 0 && DV % 64 == 0 && DQK <= 128 && DV <= 128, "TMEM / shared-memory layout of the kernels");
 };
 constexpr int FLASH_THREADS = 320;
 
-template <int D>
+template <int DQK, int DV>
 __global__ void __launch_bounds__(FLASH_THREADS, 1)
     flash_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                      const __grid_constant__ CUtensorMap tmV, bf16* __restrict__ Y, float* __restrict__ lse, int N,
                      int q_pairs) {
-  using Cfg = FlashCfg<D>;
+  using Cfg = FlashCfg<DQK, DV>;
   extern __shared__ uint8_t fsm_raw[];
   __shared__ uint64_t q_full, k_full[2], k_empty[2], v_full[2], v_empty[2], s_full[2], p_full[2], o_done[2];
   __shared__ uint32_t tmem_holder;
   const uint32_t base = (smem_u32(fsm_raw) + 1023u) & ~1023u;
-  const uint32_t sQ = base, sK = base + 2 * Cfg::TILE, sV = base + 4 * Cfg::TILE;
+  const uint32_t sQ = base, sK = base + 2 * Cfg::TILE_QK, sV = base + 4 * Cfg::TILE_QK;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x / q_pairs, qp = blockIdx.x % q_pairs;
   const int q0 = qp * 256;
@@ -177,36 +183,36 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
 
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(smem_u32(&q_full), ntile * Cfg::TILE);
+      mbar_expect_tx(smem_u32(&q_full), ntile * Cfg::TILE_QK);
       for (int t = 0; t < ntile; ++t) {
 #pragma unroll
-        for (int kb = 0; kb < D / 64; ++kb)
-          tma_load_4d(&tmQ, smem_u32(&q_full), sQ + t * Cfg::TILE + kb * 16384, kb * 64, q0 + t * 128, b, 0);
+        for (int kb = 0; kb < DQK / 64; ++kb)
+          tma_load_4d(&tmQ, smem_u32(&q_full), sQ + t * Cfg::TILE_QK + kb * 16384, kb * 64, q0 + t * 128, b, 0);
       }
       for (int j = 0; j < T; ++j) {
         const int st = j & 1;
         const uint32_t ph = static_cast<uint32_t>(j >> 1) & 1u;
         mbar_wait(smem_u32(&k_empty[st]), ph ^ 1u);
-        mbar_expect_tx(smem_u32(&k_full[st]), Cfg::TILE);
+        mbar_expect_tx(smem_u32(&k_full[st]), Cfg::TILE_QK);
 #pragma unroll
-        for (int kb = 0; kb < D / 64; ++kb)
-          tma_load_4d(&tmK, smem_u32(&k_full[st]), sK + st * Cfg::TILE + kb * 16384, kb * 64, j * 128, b, 0);
+        for (int kb = 0; kb < DQK / 64; ++kb)
+          tma_load_4d(&tmK, smem_u32(&k_full[st]), sK + st * Cfg::TILE_QK + kb * 16384, kb * 64, j * 128, b, 0);
         mbar_wait(smem_u32(&v_empty[st]), ph ^ 1u);
-        mbar_expect_tx(smem_u32(&v_full[st]), Cfg::TILE);
+        mbar_expect_tx(smem_u32(&v_full[st]), Cfg::TILE_V);
 #pragma unroll
-        for (int kb = 0; kb < D / 64; ++kb)
-          tma_load_4d(&tmV, smem_u32(&v_full[st]), sV + st * Cfg::TILE + kb * 16384, kb * 64, j * 128, b, 0);
+        for (int kb = 0; kb < DV / 64; ++kb)
+          tma_load_4d(&tmV, smem_u32(&v_full[st]), sV + st * Cfg::TILE_V + kb * 16384, kb * 64, j * 128, b, 0);
       }
     }
   } else if (warp == 1) {
     if (elect_one()) {
       constexpr uint32_t idesc_qk = make_idesc_bf16(128, 128, false, false);   // S = Q K^T : both K-major
-      constexpr uint32_t idesc_pv = make_idesc_bf16(128, D, false, true);      // O += P V  : A in TMEM, B MN-major
+      constexpr uint32_t idesc_pv = make_idesc_bf16(128, DV, false, true);     // O += P V  : A in TMEM, B MN-major
       auto issue_s = [&](int t, int j) {
-        const uint32_t kbase = sK + (j & 1) * Cfg::TILE;
-        const uint32_t qbase = sQ + t * Cfg::TILE;
+        const uint32_t kbase = sK + (j & 1) * Cfg::TILE_QK;
+        const uint32_t qbase = sQ + t * Cfg::TILE_QK;
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) {
+        for (int k = 0; k < DQK / 16; ++k) {
           const uint32_t off = (k >> 2) * 16384 + (k & 3) * 32;
           umma_f16(tmem + t * 128, make_sdesc(qbase + off, 16, 1024), make_sdesc(kbase + off, 16, 1024), idesc_qk,
                    k != 0 ? 1u : 0u);
@@ -224,7 +230,7 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
         const bool more = j + 1 < T;
         mbar_wait(smem_u32(&v_full[st]), ph);
         if (more) mbar_wait(smem_u32(&k_full[(j + 1) & 1]), static_cast<uint32_t>((j + 1) >> 1) & 1u);
-        const uint32_t vbase = sV + st * Cfg::TILE;
+        const uint32_t vbase = sV + st * Cfg::TILE_V;
         for (int t = 0; t < ntile; ++t) {
           mbar_wait(smem_u32(&p_full[t]), static_cast<uint32_t>(j) & 1u);   // P_t(j) is in TMEM, O_t rescaled
           tc_fence_after();
@@ -281,7 +287,7 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
             mbar_wait(smem_u32(&o_done[t]), static_cast<uint32_t>(j - 1) & 1u);   // P(j-1) V(j-1) has landed in O
             tc_fence_after();
 #pragma unroll 1
-            for (int c = 0; c < D / 32; ++c) {
+            for (int c = 0; c < DV / 32; ++c) {
               uint32_t v[32];
               tmem_ld_32x32(ocol + c * 32, v);
               tmem_ld_wait();
@@ -324,9 +330,9 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
       const float l = (l0 + l1) + (l2 + l3);
       const float inv = 1.f / l;
       const int grow = q0 + t * 128 + row;
-      bf16* yrow = Y + (static_cast<long long>(b) * N + grow) * D;
+      bf16* yrow = Y + (static_cast<long long>(b) * N + grow) * DV;
 #pragma unroll 1
-      for (int c = 0; c < D / 32; ++c) {
+      for (int c = 0; c < DV / 32; ++c) {
         uint32_t v[32];
         tmem_ld_32x32(ocol + c * 32, v);
         tmem_ld_wait();
@@ -361,22 +367,24 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
 // Pipelining: the 128 x 64 score / dP blocks are double-buffered in TMEM (stage = sub-tile parity) and the two compute
 // warpgroups alternate sub-tiles, so the tensor pipe computes sub-tile j+1's scores and sub-tile j-1's accumulation
 // while a warpgroup turns sub-tile j's scores into dS.
-//   dQ kernel TMEM   : stage s at [128 s, 128 s + 128): S [0,64) (dS bf16 over [0,32)), dP [64,128);  dQ at [256, 256+D)
-//   dK/dV kernel TMEM: dV [0,D), dK [128,128+D); stage s at [256 + 128 s, ..): S^T [0,64) (P^T bf16 over [0,32)),
+//   dQ kernel TMEM   : stage s at [128 s, 128 s + 128): S [0,64) (dS bf16 over [0,32)), dP [64,128);  dQ at [256, 256+DQK)
+//   dK/dV kernel TMEM: dV [0,DV), dK [128,128+DQK); stage s at [256 + 128 s, ..): S^T [0,64) (P^T bf16 over [0,32)),
 //                      dP^T [64,128) (dS^T bf16 over [64,96))
-template <int D>
+// dQ, dK and dV go to their own row-strided outputs (ld_* elements between rows).
+template <int DQK, int DV>
 __global__ void __launch_bounds__(FLASH_THREADS, 1)
     flash_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                         const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdY,
-                        const float* __restrict__ lse, const float* __restrict__ delta, bf16* __restrict__ dP3, int N,
-                        int q_tiles) {
-  using Cfg = FlashCfg<D>;
+                        const float* __restrict__ lse, const float* __restrict__ delta, bf16* __restrict__ dQ,
+                        long long ld_dq, int N, int q_tiles) {
+  using Cfg = FlashCfg<DQK, DV>;
   constexpr int RING = 4;
   extern __shared__ uint8_t fsm_raw[];
   __shared__ uint64_t q_full, kv_full[RING], kv_empty[RING], s_full[2], ds_full[2], dq_done;
   __shared__ uint32_t tmem_holder;
   const uint32_t base = (smem_u32(fsm_raw) + 1023u) & ~1023u;
-  const uint32_t sQ = base, sdY = base + Cfg::TILE, sRing = base + 2 * Cfg::TILE;   // ring slot: K_sub | V_sub
+  const uint32_t sQ = base, sdY = base + Cfg::TILE_QK, sRing = sdY + Cfg::TILE_V;   // ring slot: K_sub | V_sub
+  constexpr uint32_t SLOT = Cfg::SUB_QK + Cfg::SUB_V;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x / q_tiles, qt = blockIdx.x % q_tiles;
   const int q0 = qt * 128;
@@ -405,42 +413,42 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
 
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(smem_u32(&q_full), 2 * Cfg::TILE);
+      mbar_expect_tx(smem_u32(&q_full), Cfg::TILE_QK + Cfg::TILE_V);
 #pragma unroll
-      for (int kb = 0; kb < D / 64; ++kb) {
-        tma_load_4d(&tmQ, smem_u32(&q_full), sQ + kb * 16384, kb * 64, q0, b, 0);
-        tma_load_4d(&tmdY, smem_u32(&q_full), sdY + kb * 16384, kb * 64, q0, b, 0);
-      }
+      for (int kb = 0; kb < DQK / 64; ++kb) tma_load_4d(&tmQ, smem_u32(&q_full), sQ + kb * 16384, kb * 64, q0, b, 0);
+#pragma unroll
+      for (int kb = 0; kb < DV / 64; ++kb) tma_load_4d(&tmdY, smem_u32(&q_full), sdY + kb * 16384, kb * 64, q0, b, 0);
       for (int j = 0; j < T; ++j) {
         const int r = j % RING;
         const uint32_t ph = static_cast<uint32_t>(j / RING) & 1u;
         mbar_wait(smem_u32(&kv_empty[r]), ph ^ 1u);
-        mbar_expect_tx(smem_u32(&kv_full[r]), 2 * Cfg::SUB);
-        const uint32_t slot = sRing + r * 2 * Cfg::SUB;
+        mbar_expect_tx(smem_u32(&kv_full[r]), SLOT);
+        const uint32_t slot = sRing + r * SLOT;
 #pragma unroll
-        for (int kb = 0; kb < D / 64; ++kb) {
+        for (int kb = 0; kb < DQK / 64; ++kb)
           tma_load_4d(&tmK, smem_u32(&kv_full[r]), slot + kb * 8192, kb * 64, j * 64, b, 0);
-          tma_load_4d(&tmV, smem_u32(&kv_full[r]), slot + Cfg::SUB + kb * 8192, kb * 64, j * 64, b, 0);
-        }
+#pragma unroll
+        for (int kb = 0; kb < DV / 64; ++kb)
+          tma_load_4d(&tmV, smem_u32(&kv_full[r]), slot + Cfg::SUB_QK + kb * 8192, kb * 64, j * 64, b, 0);
       }
     }
   } else if (warp == 1) {
     if (elect_one()) {
       constexpr uint32_t idesc_s = make_idesc_bf16(128, 64, false, false);
-      constexpr uint32_t idesc_dq = make_idesc_bf16(128, D, false, true);
+      constexpr uint32_t idesc_dq = make_idesc_bf16(128, DQK, false, true);
       auto issue_sdp = [&](int j) {
         const int r = j % RING;
         mbar_wait(smem_u32(&kv_full[r]), static_cast<uint32_t>(j / RING) & 1u);
         tc_fence_after();
-        const uint32_t kb_ = sRing + r * 2 * Cfg::SUB, vb_ = kb_ + Cfg::SUB;
+        const uint32_t kb_ = sRing + r * SLOT, vb_ = kb_ + Cfg::SUB_QK;
         const uint32_t stage = tmem + (j & 1) * 128;
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) {   // S = Q K_sub^T
+        for (int k = 0; k < DQK / 16; ++k) {   // S = Q K_sub^T
           const uint32_t offa = (k >> 2) * 16384 + (k & 3) * 32, offb = (k >> 2) * 8192 + (k & 3) * 32;
           umma_f16(stage, make_sdesc(sQ + offa, 16, 1024), make_sdesc(kb_ + offb, 16, 1024), idesc_s, k != 0 ? 1u : 0u);
         }
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) {   // dP = dY V_sub^T
+        for (int k = 0; k < DV / 16; ++k) {   // dP = dY V_sub^T
           const uint32_t offa = (k >> 2) * 16384 + (k & 3) * 32, offb = (k >> 2) * 8192 + (k & 3) * 32;
           umma_f16(stage + 64, make_sdesc(sdY + offa, 16, 1024), make_sdesc(vb_ + offb, 16, 1024), idesc_s,
                    k != 0 ? 1u : 0u);
@@ -455,7 +463,7 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
         if (j + 1 < T) issue_sdp(j + 1);     // stage (j+1)&1 was drained by sub-tile j-1 (ordered behind its dQ product)
         mbar_wait(smem_u32(&ds_full[j & 1]), static_cast<uint32_t>(j >> 1) & 1u);   // dS (bf16) in stage columns [0,32)
         tc_fence_after();
-        const uint32_t kb_ = sRing + r * 2 * Cfg::SUB;
+        const uint32_t kb_ = sRing + r * SLOT;
 #pragma unroll
         for (int k = 0; k < 4; ++k)          // dQ += dS K_sub   (A from TMEM, K sub-tile read MN-major)
           umma_f16_ts(tmem + COL_DQ, tmem + (j & 1) * 128 + k * 8, make_sdesc(kb_ + k * 2048, 8192, 1024), idesc_dq,
@@ -506,10 +514,10 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
     }
     mbar_wait(smem_u32(&dq_done), 0);
     tc_fence_after();
-    bf16* orow = dP3 + (static_cast<long long>(b) * N + grow) * 3 * D;   // dTheta slot: columns [0, D)
-    // the two warpgroups split the D columns of dQ
+    bf16* orow = dQ + (static_cast<long long>(b) * N + grow) * ld_dq;
+    // the two warpgroups split the DQK columns of dQ
 #pragma unroll 1
-    for (int c = wg * (D / 64); c < (wg + 1) * (D / 64); ++c) {
+    for (int c = wg * (DQK / 64); c < (wg + 1) * (DQK / 64); ++c) {
       uint32_t v[32];
       tmem_ld_32x32(tmem + lane_addr + COL_DQ + c * 32, v);
       tmem_ld_wait();
@@ -530,20 +538,21 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
   if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
-template <int D>
+template <int DQK, int DV>
 __global__ void __launch_bounds__(FLASH_THREADS, 1)
     flash_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                          const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdY,
-                         const float* __restrict__ lse, const float* __restrict__ delta, bf16* __restrict__ dP3,
-                         int N, int kv_tiles) {
-  using Cfg = FlashCfg<D>;
+                         const float* __restrict__ lse, const float* __restrict__ delta, bf16* __restrict__ dK,
+                         long long ld_dk, bf16* __restrict__ dV, long long ld_dv, int N, int kv_tiles) {
+  using Cfg = FlashCfg<DQK, DV>;
   constexpr int RING = 4;
   extern __shared__ uint8_t fsm_raw[];
   __shared__ uint64_t kv_full, q_full[RING], q_empty[RING], s_full[2], p_full[2], acc_done;
   __shared__ uint32_t tmem_holder;
   __shared__ __align__(16) float lse_sm[2][2][64], del_sm[2][2][64];   // [warpgroup][buffer][query of the sub-tile]
   const uint32_t base = (smem_u32(fsm_raw) + 1023u) & ~1023u;
-  const uint32_t sK = base, sV = base + Cfg::TILE, sRing = base + 2 * Cfg::TILE;   // ring slot: Q_sub | dY_sub
+  const uint32_t sK = base, sV = base + Cfg::TILE_QK, sRing = sV + Cfg::TILE_V;   // ring slot: Q_sub | dY_sub
+  constexpr uint32_t SLOT = Cfg::SUB_QK + Cfg::SUB_V;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x / kv_tiles, kt = blockIdx.x % kv_tiles;
   const int k0 = kt * 128;
@@ -572,42 +581,43 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
 
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(smem_u32(&kv_full), 2 * Cfg::TILE);
+      mbar_expect_tx(smem_u32(&kv_full), Cfg::TILE_QK + Cfg::TILE_V);
 #pragma unroll
-      for (int kb = 0; kb < D / 64; ++kb) {
-        tma_load_4d(&tmK, smem_u32(&kv_full), sK + kb * 16384, kb * 64, k0, b, 0);
-        tma_load_4d(&tmV, smem_u32(&kv_full), sV + kb * 16384, kb * 64, k0, b, 0);
-      }
+      for (int kb = 0; kb < DQK / 64; ++kb) tma_load_4d(&tmK, smem_u32(&kv_full), sK + kb * 16384, kb * 64, k0, b, 0);
+#pragma unroll
+      for (int kb = 0; kb < DV / 64; ++kb) tma_load_4d(&tmV, smem_u32(&kv_full), sV + kb * 16384, kb * 64, k0, b, 0);
       for (int i = 0; i < T; ++i) {
         const int r = i % RING;
         const uint32_t ph = static_cast<uint32_t>(i / RING) & 1u;
         mbar_wait(smem_u32(&q_empty[r]), ph ^ 1u);
-        mbar_expect_tx(smem_u32(&q_full[r]), 2 * Cfg::SUB);
-        const uint32_t slot = sRing + r * 2 * Cfg::SUB;
+        mbar_expect_tx(smem_u32(&q_full[r]), SLOT);
+        const uint32_t slot = sRing + r * SLOT;
 #pragma unroll
-        for (int kb = 0; kb < D / 64; ++kb) {
+        for (int kb = 0; kb < DQK / 64; ++kb)
           tma_load_4d(&tmQ, smem_u32(&q_full[r]), slot + kb * 8192, kb * 64, i * 64, b, 0);
-          tma_load_4d(&tmdY, smem_u32(&q_full[r]), slot + Cfg::SUB + kb * 8192, kb * 64, i * 64, b, 0);
-        }
+#pragma unroll
+        for (int kb = 0; kb < DV / 64; ++kb)
+          tma_load_4d(&tmdY, smem_u32(&q_full[r]), slot + Cfg::SUB_QK + kb * 8192, kb * 64, i * 64, b, 0);
       }
     }
   } else if (warp == 1) {
     if (elect_one()) {
       constexpr uint32_t idesc_s = make_idesc_bf16(128, 64, false, false);
-      constexpr uint32_t idesc_acc = make_idesc_bf16(128, D, false, true);
+      constexpr uint32_t idesc_dv = make_idesc_bf16(128, DV, false, true);
+      constexpr uint32_t idesc_dk = make_idesc_bf16(128, DQK, false, true);
       auto issue_sdp = [&](int i) {
         const int r = i % RING;
         mbar_wait(smem_u32(&q_full[r]), static_cast<uint32_t>(i / RING) & 1u);
         tc_fence_after();
-        const uint32_t qb_ = sRing + r * 2 * Cfg::SUB, yb_ = qb_ + Cfg::SUB;
+        const uint32_t qb_ = sRing + r * SLOT, yb_ = qb_ + Cfg::SUB_QK;
         const uint32_t stage = tmem + COL_ST + (i & 1) * 128;
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) {   // S^T = K Q_sub^T
+        for (int k = 0; k < DQK / 16; ++k) {   // S^T = K Q_sub^T
           const uint32_t offa = (k >> 2) * 16384 + (k & 3) * 32, offb = (k >> 2) * 8192 + (k & 3) * 32;
           umma_f16(stage, make_sdesc(sK + offa, 16, 1024), make_sdesc(qb_ + offb, 16, 1024), idesc_s, k != 0 ? 1u : 0u);
         }
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) {   // dP^T = V dY_sub^T
+        for (int k = 0; k < DV / 16; ++k) {   // dP^T = V dY_sub^T
           const uint32_t offa = (k >> 2) * 16384 + (k & 3) * 32, offb = (k >> 2) * 8192 + (k & 3) * 32;
           umma_f16(stage + 64, make_sdesc(sV + offa, 16, 1024), make_sdesc(yb_ + offb, 16, 1024), idesc_s,
                    k != 0 ? 1u : 0u);
@@ -622,15 +632,15 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
         if (i + 1 < T) issue_sdp(i + 1);
         mbar_wait(smem_u32(&p_full[i & 1]), static_cast<uint32_t>(i >> 1) & 1u);   // P^T [0,32), dS^T [64,96) (bf16)
         tc_fence_after();
-        const uint32_t qb_ = sRing + r * 2 * Cfg::SUB, yb_ = qb_ + Cfg::SUB;
+        const uint32_t qb_ = sRing + r * SLOT, yb_ = qb_ + Cfg::SUB_QK;
         const uint32_t stage = tmem + COL_ST + (i & 1) * 128;
 #pragma unroll
         for (int k = 0; k < 4; ++k)          // dV += P^T dY_sub   (dY sub-tile read MN-major)
-          umma_f16_ts(tmem + COL_DV, stage + k * 8, make_sdesc(yb_ + k * 2048, 8192, 1024), idesc_acc,
+          umma_f16_ts(tmem + COL_DV, stage + k * 8, make_sdesc(yb_ + k * 2048, 8192, 1024), idesc_dv,
                       (i | k) != 0 ? 1u : 0u);
 #pragma unroll
         for (int k = 0; k < 4; ++k)          // dK += dS^T Q_sub   (Q sub-tile read MN-major)
-          umma_f16_ts(tmem + COL_DK, stage + 64 + k * 8, make_sdesc(qb_ + k * 2048, 8192, 1024), idesc_acc,
+          umma_f16_ts(tmem + COL_DK, stage + 64 + k * 8, make_sdesc(qb_ + k * 2048, 8192, 1024), idesc_dk,
                       (i | k) != 0 ? 1u : 0u);
         umma_commit(smem_u32(&q_empty[r]));
         if (i == T - 1) umma_commit(smem_u32(&acc_done));
@@ -700,11 +710,12 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
     }
     mbar_wait(smem_u32(&acc_done), 0);
     tc_fence_after();
-    // warpgroup 0 writes dK (dPhi slot), warpgroup 1 writes dV (dG slot)
-    bf16* orow = dP3 + (static_cast<long long>(b) * N + gkey) * 3 * D + (wg == 0 ? D : 2 * D);
+    // warpgroup 0 writes dK, warpgroup 1 writes dV
+    bf16* orow = wg == 0 ? dK + (static_cast<long long>(b) * N + gkey) * ld_dk
+                         : dV + (static_cast<long long>(b) * N + gkey) * ld_dv;
     const uint32_t acc = tmem + lane_addr + (wg == 0 ? COL_DK : COL_DV);
 #pragma unroll 1
-    for (int c = 0; c < D / 32; ++c) {
+    for (int c = 0; c < (wg == 0 ? DQK : DV) / 32; ++c) {
       uint32_t v[32];
       tmem_ld_32x32(acc + c * 32, v);
       tmem_ld_wait();
@@ -725,9 +736,10 @@ __global__ void __launch_bounds__(FLASH_THREADS, 1)
   if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
-// per-CTA partial column sums of a bf16 [rows, Ccols] matrix (bias gradients = column sums of dP): part [grid][2][Ccols]
+// per-CTA partial column sums of a bf16 [rows, Ccols] matrix with row stride ld (bias gradients = column sums of dP):
+// part [grid][2][Ccols]
 __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict__ A, float* __restrict__ part,
-                                                         long long rows, int Ccols) {
+                                                         long long rows, int Ccols, long long ld) {
   // thread = one 8-column group per pass; rows strided over (blockIdx, row lane)
   const int groups = Ccols / 8;
   for (int g0 = 0; g0 < groups; g0 += 64) {
@@ -738,7 +750,7 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict
     for (int t = 0; t < 8; ++t) s[t] = 0.f;
     if (g < groups) {
       for (long long r = static_cast<long long>(blockIdx.x) * 4 + ty; r < rows; r += static_cast<long long>(gridDim.x) * 4) {
-        const uint4 v = *reinterpret_cast<const uint4*>(A + r * Ccols + g * 8);
+        const uint4 v = *reinterpret_cast<const uint4*>(A + r * ld + g * 8);
         const uint32_t* u = reinterpret_cast<const uint32_t*>(&v);
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
@@ -761,61 +773,58 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict
   }
 }
 
-template <int D>
-static int launch_flash_bwd(const bf16* P3, const bf16* dY, const float* lse, const float* delta, bf16* dP3, int B,
-                            int N, cudaStream_t stream) {
-  using Cfg = FlashCfg<D>;
+template <int DQK, int DV>
+static int launch_flash_bwd(const AttnArgs& a, const bf16* dY, const float* lse, const float* delta, int B, int N,
+                            cudaStream_t stream) {
+  using Cfg = FlashCfg<DQK, DV>;
   // 128-row boxes for the operand that stays resident in a CTA, 64-row boxes for the streamed sub-tiles
   CUtensorMap tq128, tk128, tv128, ty128, tq64, tk64, tv64, ty64;
-  const long long seq = static_cast<long long>(N) * 3 * D;
-  const long long seqY = static_cast<long long>(N) * D;
+  const long long n = N;
   int rc;
-  if ((rc = make_tmap_bf16(&tq128, P3, D, N, B, 3 * D, seq, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tk128, P3 + D, D, N, B, 3 * D, seq, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tv128, P3 + 2 * D, D, N, B, 3 * D, seq, 128))) return rc;
-  if ((rc = make_tmap_bf16(&ty128, dY, D, N, B, D, seqY, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tq64, P3, D, N, B, 3 * D, seq, 64))) return rc;
-  if ((rc = make_tmap_bf16(&tk64, P3 + D, D, N, B, 3 * D, seq, 64))) return rc;
-  if ((rc = make_tmap_bf16(&tv64, P3 + 2 * D, D, N, B, 3 * D, seq, 64))) return rc;
-  if ((rc = make_tmap_bf16(&ty64, dY, D, N, B, D, seqY, 64))) return rc;
+  if ((rc = make_tmap_bf16(&tq128, a.q, DQK, N, B, a.ldq, n * a.ldq, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tk128, a.k, DQK, N, B, a.ldk, n * a.ldk, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tv128, a.v, DV, N, B, a.ldv, n * a.ldv, 128))) return rc;
+  if ((rc = make_tmap_bf16(&ty128, dY, DV, N, B, DV, n * DV, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tq64, a.q, DQK, N, B, a.ldq, n * a.ldq, 64))) return rc;
+  if ((rc = make_tmap_bf16(&tk64, a.k, DQK, N, B, a.ldk, n * a.ldk, 64))) return rc;
+  if ((rc = make_tmap_bf16(&tv64, a.v, DV, N, B, a.ldv, n * a.ldv, 64))) return rc;
+  if ((rc = make_tmap_bf16(&ty64, dY, DV, N, B, DV, n * DV, 64))) return rc;
   const uint32_t smem = Cfg::SMEM_BWD;
   const int tiles = (N + 127) / 128;
   {
-    auto kern = flash_bwd_dq_kernel<D>;
+    auto kern = flash_bwd_dq_kernel<DQK, DV>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(flash_bwd_dq)");
-    kern<<<B * tiles, FLASH_THREADS, smem, stream>>>(tq128, tk64, tv64, ty128, lse, delta, dP3, N, tiles);
+    kern<<<B * tiles, FLASH_THREADS, smem, stream>>>(tq128, tk64, tv64, ty128, lse, delta, a.dq, a.ld_dq, N, tiles);
     if ((rc = check_cuda(cudaGetLastError(), "flash_bwd_dq launch"))) return rc;
   }
   {
-    auto kern = flash_bwd_dkv_kernel<D>;
+    auto kern = flash_bwd_dkv_kernel<DQK, DV>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(flash_bwd_dkv)");
-    kern<<<B * tiles, FLASH_THREADS, smem, stream>>>(tq64, tk128, tv128, ty64, lse, delta, dP3, N, tiles);
+    kern<<<B * tiles, FLASH_THREADS, smem, stream>>>(tq64, tk128, tv128, ty64, lse, delta, a.dk, a.ld_dk, a.dvo,
+                                                     a.ld_dv, N, tiles);
     if ((rc = check_cuda(cudaGetLastError(), "flash_bwd_dkv launch"))) return rc;
   }
   return 0;
 }
 
-template <int D>
-static int launch_flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, cudaStream_t stream) {
-  using Cfg = FlashCfg<D>;
+template <int DQK, int DV>
+static int launch_flash_fwd(const AttnArgs& a, bf16* Y, float* lse, int B, int N, cudaStream_t stream) {
+  using Cfg = FlashCfg<DQK, DV>;
   CUtensorMap tq, tk, tv;
-  const long long seq = static_cast<long long>(N) * 3 * D;
+  const long long n = N;
   int rc;
-  if ((rc = make_tmap_bf16(&tq, P3, D, N, B, 3 * D, seq, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tk, P3 + D, D, N, B, 3 * D, seq, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tv, P3 + 2 * D, D, N, B, 3 * D, seq, 128))) return rc;
-  auto kern = flash_fwd_kernel<D>;
+  if ((rc = make_tmap_bf16(&tq, a.q, DQK, N, B, a.ldq, n * a.ldq, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tk, a.k, DQK, N, B, a.ldk, n * a.ldk, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tv, a.v, DV, N, B, a.ldv, n * a.ldv, 128))) return rc;
+  auto kern = flash_fwd_kernel<DQK, DV>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_FWD);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(flash_fwd)");
   const int q_pairs = (N + 255) / 256;
   kern<<<B * q_pairs, FLASH_THREADS, Cfg::SMEM_FWD, stream>>>(tq, tk, tv, Y, lse, N, q_pairs);
   return check_cuda(cudaGetLastError(), "flash_fwd launch");
 }
-
-namespace {
-}  // namespace
 
 int attn_ld(int N) { return (N + 7) & ~7; }
 
@@ -833,23 +842,53 @@ size_t attn_scratch_bytes(long long B, long long N, bool backward) {
   return nb * per * (backward ? 12 : 6) + 1024;
 }
 
-static int attn_fwd_materialized(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* scratch,
+AttnArgs attn_args_embedded(const bf16* P3, bf16* dP3, int Ci) {
+  AttnArgs a;
+  a.q = P3; a.k = P3 + Ci; a.v = P3 + 2 * Ci;
+  a.ldq = a.ldk = a.ldv = 3LL * Ci;
+  a.wqk = a.wv = Ci;
+  a.dq = dP3; a.dk = dP3 ? dP3 + Ci : nullptr; a.dvo = dP3 ? dP3 + 2 * Ci : nullptr;
+  a.ld_dq = a.ld_dk = a.ld_dv = 3LL * Ci;
+  a.bias_qkv = true;
+  return a;
+}
+
+AttnArgs attn_args_gaussian(const bf16* X, const bf16* G, bf16* dXa, bf16* dXb, bf16* dG, long long ld_dx,
+                            long long ld_dg, int C, int Ci) {
+  AttnArgs a;
+  a.q = a.k = X;
+  a.ldq = a.ldk = C;
+  a.v = G; a.ldv = Ci;
+  a.wqk = C; a.wv = Ci;
+  a.dq = dXa; a.dk = dXb; a.dvo = dG;
+  a.ld_dq = a.ld_dk = ld_dx; a.ld_dv = ld_dg;
+  a.bias_qkv = false;
+  return a;
+}
+
+bool attn_flash_supported(int wqk, int wv) {
+  return (wqk == 64 && wv == 64) || (wqk == 128 && wv == 64) || (wqk == 128 && wv == 128);
+}
+
+static int attn_fwd_materialized(const AttnArgs& a, bf16* Y, float* lse, int B, int N, void* scratch,
                                  cudaStream_t stream) {
   const int ld = attn_ld(N);
   const int nb = attn_chunk(B, N);
   const size_t per = static_cast<size_t>(ld) * N;
   float* S = reinterpret_cast<float*>(scratch);
   bf16* Pm = reinterpret_cast<bf16*>(S + nb * per);
-  const long long seqP = static_cast<long long>(N) * 3 * Ci;
+  const long long n = N;
   for (int b0 = 0; b0 < B; b0 += nb) {
     const int cb = (B - b0 < nb) ? (B - b0) : nb;
-    const bf16* Pb = P3 + b0 * seqP;
-    {  // S = Theta Phi^T   (columns [N, ld) come out as zeros: Phi rows beyond N are TMA out-of-bounds)
+    const bf16* Qb = a.q + b0 * n * a.ldq;
+    const bf16* Kb = a.k + b0 * n * a.ldk;
+    const bf16* Vb = a.v + b0 * n * a.ldv;
+    {  // S = Q K^T   (columns [N, ld) come out as zeros: K rows beyond N are TMA out-of-bounds)
       GemmArgs g;
-      g.A = op(Pb, 0, 3 * Ci, seqP);
-      g.B = op(Pb + Ci, 0, 3 * Ci, seqP);
+      g.A = op(Qb, 0, a.ldq, n * a.ldq);
+      g.B = op(Kb, 0, a.ldk, n * a.ldk);
       g.B.rows = N;
-      g.M = N; g.N = ld; g.K = Ci; g.batch = cb;
+      g.M = N; g.N = ld; g.K = a.wqk; g.batch = cb;
       g.out_kind = 1;
       g.D = S; g.ldd = ld; g.strideD = static_cast<long long>(per);
       int rc = gemm(g, stream);
@@ -859,12 +898,12 @@ static int attn_fwd_materialized(const bf16* P3, bf16* Y, float* lse, int B, int
         S, Pm, lse + static_cast<long long>(b0) * N, N, ld);
     int rc = check_cuda(cudaGetLastError(), "softmax_rows launch");
     if (rc) return rc;
-    {  // Y = P G
+    {  // Y = P V
       GemmArgs g;
       g.A = op(Pm, 0, ld, static_cast<long long>(per));
-      g.B = op(Pb + 2 * Ci, 1, 3 * Ci, seqP);
-      g.M = N; g.N = Ci; g.K = N; g.batch = cb;
-      g.D = Y + static_cast<long long>(b0) * N * Ci; g.ldd = Ci; g.strideD = static_cast<long long>(N) * Ci;
+      g.B = op(Vb, 1, a.ldv, n * a.ldv);
+      g.M = N; g.N = a.wv; g.K = N; g.batch = cb;
+      g.D = Y + b0 * n * a.wv; g.ldd = a.wv; g.strideD = n * a.wv;
       rc = gemm(g, stream);
       if (rc) return rc;
     }
@@ -872,15 +911,20 @@ static int attn_fwd_materialized(const bf16* P3, bf16* Y, float* lse, int B, int
   return 0;
 }
 
-int flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* scratch, cudaStream_t stream) {
-  if (Ci == 128) return launch_flash_fwd<128>(P3, Y, lse, B, N, stream);
-  if (Ci == 64) return launch_flash_fwd<64>(P3, Y, lse, B, N, stream);
-  return attn_fwd_materialized(P3, Y, lse, B, N, Ci, scratch, stream);   // other head widths: exact chunked path
+int attn_fwd(const AttnArgs& a, bf16* Y, float* lse, int B, int N, void* scratch, cudaStream_t stream) {
+  if (a.wqk == 128 && a.wv == 128) return launch_flash_fwd<128, 128>(a, Y, lse, B, N, stream);
+  if (a.wqk == 128 && a.wv == 64) return launch_flash_fwd<128, 64>(a, Y, lse, B, N, stream);
+  if (a.wqk == 64 && a.wv == 64) return launch_flash_fwd<64, 64>(a, Y, lse, B, N, stream);
+  return attn_fwd_materialized(a, Y, lse, B, N, scratch, stream);   // other widths: exact chunked path
 }
 
-static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3,
-                                 float* delta, float* cs_t, float* cs_p, float* cs_g, int cs_rows_out[3], int B, int N,
-                                 int Ci, void* scratch, cudaStream_t stream) {
+int flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* scratch, cudaStream_t stream) {
+  return attn_fwd(attn_args_embedded(P3, nullptr, Ci), Y, lse, B, N, scratch, stream);
+}
+
+static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta,
+                                 float* cs_t, float* cs_p, float* cs_g, int cs_rows_out[3], int B, int N,
+                                 void* scratch, cudaStream_t stream) {
   const int ld = attn_ld(N);
   const int nb = attn_chunk(B, N);
   const size_t per = static_cast<size_t>(ld) * N;
@@ -888,40 +932,44 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
   float* dPm = S + nb * per;
   bf16* Pm = reinterpret_cast<bf16*>(dPm + nb * per);
   bf16* dS = Pm + nb * per;
-  const long long seqP = static_cast<long long>(N) * 3 * Ci;
+  const long long n = N;
   const long long rows = static_cast<long long>(B) * N;
+  // bias sums: over all three outputs (mode='embedded': theta / phi / g biases), or over dV alone (mode='gaussian':
+  // Q = K = X carry no bias)
+  if (!a.bias_qkv) cs_t = cs_p = nullptr;
   // rows of each column-stat table written so far: the three products can leave different row counts per chunk (the
-  // dTheta GEMM runs 256-row super-tiles for N >= 1024, the other two do not), so each table has its own offset
+  // dQ GEMM runs 256-row super-tiles for N >= 1024, the other two do not), so each table has its own offset
   int cs_rows_total[3] = {0, 0, 0};
   {
     const long long threads = rows * 32;
-    rowdot_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, stream>>>(dY, Y, delta, rows, Ci);
+    rowdot_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, stream>>>(dY, Y, delta, rows, a.wv);
     int rc = check_cuda(cudaGetLastError(), "rowdot launch");
     if (rc) return rc;
   }
   for (int b0 = 0; b0 < B; b0 += nb) {
     const int cb = (B - b0 < nb) ? (B - b0) : nb;
-    const bf16* Pb = P3 + b0 * seqP;
-    const bf16* dYb = dY + static_cast<long long>(b0) * N * Ci;
-    bf16* dPb = dP3 + b0 * seqP;
+    const bf16* Qb = a.q + b0 * n * a.ldq;
+    const bf16* Kb = a.k + b0 * n * a.ldk;
+    const bf16* Vb = a.v + b0 * n * a.ldv;
+    const bf16* dYb = dY + b0 * n * a.wv;
     int r_t = 0, r_p = 0, r_g = 0;
     int rc;
-    {  // S = Theta Phi^T (recompute)
+    {  // S = Q K^T (recompute)
       GemmArgs g;
-      g.A = op(Pb, 0, 3 * Ci, seqP);
-      g.B = op(Pb + Ci, 0, 3 * Ci, seqP);
+      g.A = op(Qb, 0, a.ldq, n * a.ldq);
+      g.B = op(Kb, 0, a.ldk, n * a.ldk);
       g.B.rows = N;
-      g.M = N; g.N = ld; g.K = Ci; g.batch = cb;
+      g.M = N; g.N = ld; g.K = a.wqk; g.batch = cb;
       g.out_kind = 1;
       g.D = S; g.ldd = ld; g.strideD = static_cast<long long>(per);
       if ((rc = gemm(g, stream))) return rc;
     }
-    {  // dPm = dY G^T
+    {  // dPm = dY V^T
       GemmArgs g;
-      g.A = op(dYb, 0, Ci, static_cast<long long>(N) * Ci);
-      g.B = op(Pb + 2 * Ci, 0, 3 * Ci, seqP);
+      g.A = op(dYb, 0, a.wv, n * a.wv);
+      g.B = op(Vb, 0, a.ldv, n * a.ldv);
       g.B.rows = N;
-      g.M = N; g.N = ld; g.K = Ci; g.batch = cb;
+      g.M = N; g.N = ld; g.K = a.wv; g.batch = cb;
       g.out_kind = 1;
       g.D = dPm; g.ldd = ld; g.strideD = static_cast<long long>(per);
       if ((rc = gemm(g, stream))) return rc;
@@ -943,33 +991,37 @@ static int attn_bwd_materialized(const bf16* P3, const bf16* Y, const bf16* dY, 
       }
       if ((rc = check_cuda(cudaGetLastError(), "softmax_bwd launch"))) return rc;
     }
-    {  // dTheta = dS Phi
+    {  // dQ = dS K
       GemmArgs g;
       g.A = op(dS, 0, ld, static_cast<long long>(per));
-      g.B = op(Pb + Ci, 1, 3 * Ci, seqP);
-      g.M = N; g.N = Ci; g.K = N; g.batch = cb;
-      g.D = dPb; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_t + static_cast<long long>(cs_rows_total[0]) * 2 * Ci;
-      g.colstats_rows = &r_t;
+      g.B = op(Kb, 1, a.ldk, n * a.ldk);
+      g.M = N; g.N = a.wqk; g.K = N; g.batch = cb;
+      g.D = a.dq + b0 * n * a.ld_dq; g.ldd = a.ld_dq; g.strideD = n * a.ld_dq;
+      if (cs_t != nullptr) {
+        g.colstats = cs_t + static_cast<long long>(cs_rows_total[0]) * 2 * a.wqk;
+        g.colstats_rows = &r_t;
+      }
       if ((rc = gemm(g, stream))) return rc;
     }
-    {  // dPhi = dS^T Theta
+    {  // dK = dS^T Q
       GemmArgs g;
       g.A = op(dS, 1, ld, static_cast<long long>(per));
-      g.B = op(Pb, 1, 3 * Ci, seqP);
-      g.M = N; g.N = Ci; g.K = N; g.batch = cb;
-      g.D = dPb + Ci; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_p + static_cast<long long>(cs_rows_total[1]) * 2 * Ci;
-      g.colstats_rows = &r_p;
+      g.B = op(Qb, 1, a.ldq, n * a.ldq);
+      g.M = N; g.N = a.wqk; g.K = N; g.batch = cb;
+      g.D = a.dk + b0 * n * a.ld_dk; g.ldd = a.ld_dk; g.strideD = n * a.ld_dk;
+      if (cs_p != nullptr) {
+        g.colstats = cs_p + static_cast<long long>(cs_rows_total[1]) * 2 * a.wqk;
+        g.colstats_rows = &r_p;
+      }
       if ((rc = gemm(g, stream))) return rc;
     }
-    {  // dG = P^T dY
+    {  // dV = P^T dY
       GemmArgs g;
       g.A = op(Pm, 1, ld, static_cast<long long>(per));
-      g.B = op(dYb, 1, Ci, static_cast<long long>(N) * Ci);
-      g.M = N; g.N = Ci; g.K = N; g.batch = cb;
-      g.D = dPb + 2 * Ci; g.ldd = 3 * Ci; g.strideD = seqP;
-      g.colstats = cs_g + static_cast<long long>(cs_rows_total[2]) * 2 * Ci;
+      g.B = op(dYb, 1, a.wv, n * a.wv);
+      g.M = N; g.N = a.wv; g.K = N; g.batch = cb;
+      g.D = a.dvo + b0 * n * a.ld_dv; g.ldd = a.ld_dv; g.strideD = n * a.ld_dv;
+      g.colstats = cs_g + static_cast<long long>(cs_rows_total[2]) * 2 * a.wv;
       g.colstats_rows = &r_g;
       if ((rc = gemm(g, stream))) return rc;
     }
@@ -986,29 +1038,78 @@ int flash_bwd_colsum_blocks(long long rows) {
   return static_cast<int>(b < 1 ? 1 : (b > 148 * 4 ? 148 * 4 : b));
 }
 
-int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3, float* delta, float* cs_t,
-              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
-              cudaStream_t stream) {
-  if (Ci != 128 && Ci != 64)   // other head widths: exact chunked path
-    return attn_bwd_materialized(P3, Y, dY, lse, dP3, delta, cs_t, cs_p, cs_g, cs_rows_out, B, N, Ci, scratch, stream);
+int attn_bwd(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta, float* cs_t, float* cs_p,
+             float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, void* scratch, cudaStream_t stream) {
+  if (!attn_flash_supported(a.wqk, a.wv))   // other widths: exact chunked path
+    return attn_bwd_materialized(a, Y, dY, lse, delta, cs_t, cs_p, cs_g, cs_rows_out, B, N, scratch, stream);
   const long long rows = static_cast<long long>(B) * N;
   {
     const long long threads = rows * 32;
-    rowdot_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, stream>>>(dY, Y, delta, rows, Ci);
+    rowdot_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, stream>>>(dY, Y, delta, rows, a.wv);
     int rc = check_cuda(cudaGetLastError(), "rowdot launch");
     if (rc) return rc;
   }
-  int rc = (Ci == 128) ? launch_flash_bwd<128>(P3, dY, lse, delta, dP3, B, N, stream)
-                       : launch_flash_bwd<64>(P3, dY, lse, delta, dP3, B, N, stream);
+  int rc = (a.wqk == 128 && a.wv == 128) ? launch_flash_bwd<128, 128>(a, dY, lse, delta, B, N, stream)
+           : (a.wqk == 128)              ? launch_flash_bwd<128, 64>(a, dY, lse, delta, B, N, stream)
+                                         : launch_flash_bwd<64, 64>(a, dY, lse, delta, B, N, stream);
   if (rc) return rc;
-  // bias gradients: column sums of dP3 = [dTheta | dPhi | dG]; one table [grid][2][3Ci] written into cs_t, the caller's
-  // three reductions address it with a row stride of 2*3Ci through the offsets below (cs_p / cs_g are unused here)
   int grid = flash_bwd_colsum_blocks(rows);
-  if (grid > cs_cap_rows / 3) grid = cs_cap_rows / 3 > 0 ? cs_cap_rows / 3 : 1;   // cs_t holds cs_cap_rows x 2 x Ci floats
-  colsum_bf16_kernel<<<grid, 256, 0, stream>>>(dP3, cs_t, rows, 3 * Ci);
+  if (a.bias_qkv) {
+    // bias gradients: column sums of dP3 = [dTheta | dPhi | dG]; one table [grid][2][3Ci] written into cs_t, the
+    // caller's three reductions address it with a row stride of 2*3Ci through the offsets below (cs_p / cs_g are unused
+    // here)
+    if (grid > cs_cap_rows / 3) grid = cs_cap_rows / 3 > 0 ? cs_cap_rows / 3 : 1;   // cs_t holds cs_cap_rows x 2 x Ci floats
+    colsum_bf16_kernel<<<grid, 256, 0, stream>>>(a.dq, cs_t, rows, 3 * a.wv, 3LL * a.wv);
+    if ((rc = check_cuda(cudaGetLastError(), "colsum launch"))) return rc;
+    cs_rows_out[0] = cs_rows_out[1] = cs_rows_out[2] = -grid;   // negative: "single table of width 3Ci" (see glf_tpavi_bwd)
+    return 0;
+  }
+  // column sums of dV alone: a table [grid][2][DV] in cs_g
+  if (grid > cs_cap_rows) grid = cs_cap_rows > 0 ? cs_cap_rows : 1;
+  colsum_bf16_kernel<<<grid, 256, 0, stream>>>(a.dvo, cs_g, rows, a.wv, a.ld_dv);
   if ((rc = check_cuda(cudaGetLastError(), "colsum launch"))) return rc;
-  cs_rows_out[0] = cs_rows_out[1] = cs_rows_out[2] = -grid;   // negative: "single table of width 3Ci" (see glf_tpavi_bwd)
+  cs_rows_out[0] = cs_rows_out[1] = 0;
+  cs_rows_out[2] = grid;
   return 0;
+}
+
+int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3, float* delta, float* cs_t,
+              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
+              cudaStream_t stream) {
+  return attn_bwd(attn_args_embedded(P3, dP3, Ci), Y, dY, lse, delta, cs_t, cs_p, cs_g, cs_cap_rows, cs_rows_out, B, N,
+                  scratch, stream);
+}
+
+// out[r, c] = in[r, c] + in[r, C + c] over rows of 2C bf16 (fp32 sum, one rounding): dS X + dS^T X of mode='gaussian'
+__global__ void __launch_bounds__(256) sum_halves_kernel(const bf16* __restrict__ in, bf16* __restrict__ out,
+                                                        long long rows, int C) {
+  const long long nvec = rows * (C / 8);
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < nvec;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long r = i / (C / 8);
+    const int c = static_cast<int>(i % (C / 8)) * 8;
+    const uint4 a = *reinterpret_cast<const uint4*>(in + r * 2 * C + c);
+    const uint4 b = *reinterpret_cast<const uint4*>(in + r * 2 * C + C + c);
+    const uint32_t* ua = reinterpret_cast<const uint32_t*>(&a);
+    const uint32_t* ub = reinterpret_cast<const uint32_t*>(&b);
+    uint4 o;
+    uint32_t* uo = reinterpret_cast<uint32_t*>(&o);
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const float2 x = unpack_bf16(ua[t]), y = unpack_bf16(ub[t]);
+      uo[t] = pack_bf16(x.x + y.x, x.y + y.y);
+    }
+    *reinterpret_cast<uint4*>(out + r * C + c) = o;
+  }
+}
+
+int sum_halves(const bf16* in, bf16* out, long long rows, int C, cudaStream_t stream) {
+  const long long nvec = rows * (C / 8);
+  long long blocks = (nvec + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  if (blocks < 1) blocks = 1;
+  sum_halves_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(in, out, rows, C);
+  return check_cuda(cudaGetLastError(), "sum_halves launch");
 }
 
 }  // namespace glf

@@ -211,7 +211,8 @@ int spatial_sums(const void* x, int dtype, int B, int C, int T, long long sb, lo
                  cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------ softmax attention
-// mode='embedded' (ours.py:896-897,902): Y = softmax(Theta Phi^T) G, flash-style, per batch entry.
+// mode='embedded' (ours.py:896-897,902): Y = softmax(Theta Phi^T) G, flash-style, per batch entry;
+// mode='gaussian' (ours.py:869-873): Y = softmax(X X^T) G.
 // P: [B, N, 3Ci] bf16 (theta | phi | g); Y: [B, N, Ci] bf16; lse: [B, N] fp32 (natural-log-sum-exp per query row)
 int attn_ld(int N);
 int attn_chunk(long long B, long long N);
@@ -222,6 +223,32 @@ int flash_fwd(const bf16* P, bf16* Y, float* lse, int B, int N, int Ci, void* sc
 int flash_bwd(const bf16* P, const bf16* Y, const bf16* dY, const float* lse, bf16* dP, float* delta, float* cs_t,
               float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
               cudaStream_t stream);
+// The same attention with Q, K and V given separately: Y = softmax(Q K^T) V per sequence, Q / K of width wqk, V / Y / dY
+// of width wv, every operand token rows with its own leading dimension.  mode='embedded' is Q = Theta, K = Phi, V = G
+// (slots of one [Theta | Phi | G] row); mode='gaussian' (ours.py:869-873) is Q = K = X (wqk = C) and V = G (wv = C').
+// Flash kernels for (wqk, wv) in {(64, 64), (128, 64), (128, 128)}, the chunked exact path otherwise.
+struct AttnArgs {
+  const bf16 *q = nullptr, *k = nullptr, *v = nullptr;
+  long long ldq = 0, ldk = 0, ldv = 0;
+  int wqk = 0, wv = 0;
+  bf16 *dq = nullptr, *dk = nullptr, *dvo = nullptr;    // backward outputs dQ, dK, dV (no atomics: each is stored once)
+  long long ld_dq = 0, ld_dk = 0, ld_dv = 0;
+  bool bias_qkv = true;   // bias sums over [dQ | dK | dV] (adjacent slots of one row, 'embedded'), else over dV alone
+};
+AttnArgs attn_args_embedded(const bf16* P3, bf16* dP3, int Ci);
+AttnArgs attn_args_gaussian(const bf16* X, const bf16* G, bf16* dXa, bf16* dXb, bf16* dG, long long ld_dx,
+                            long long ld_dg, int C, int Ci);
+bool attn_flash_supported(int wqk, int wv);
+int attn_fwd(const AttnArgs& a, bf16* Y, float* lse, int B, int N, void* scratch, cudaStream_t stream);
+// bias_qkv: cs_rows_out as flash_bwd;  otherwise cs_rows_out[2] > 0 rows of one table [rows][2][wv] in cs_g
+int attn_bwd(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta, float* cs_t, float* cs_p,
+             float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, void* scratch, cudaStream_t stream);
+// out [rows, C] = in[:, :C] + in[:, C:2C] for in [rows, 2C] bf16 (fp32 sum, rounded once)
+int sum_halves(const bf16* in, bf16* out, long long rows, int C, cudaStream_t stream);
+// mode='gaussian' weights: wg [Ci, C] = bf16(g.weight), bg [Ci] = g.bias, wgT [C, 2C + Ci] = [I | I | g.weight^T] (the dX
+// product's B operand: dX = [dS X | dS^T X | dG] wgT^T), wz [C, Ci], wzT [Ci, C]
+int prep_weights_gaussian(const glf_weights* w, int C, int Ci, bf16* wg, bf16* wgT, float* bg, bf16* wz, bf16* wzT,
+                          cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------ P2P all-reduce (glf_p2p.cu)
 int p2p_grid(long long n_floats);

@@ -403,7 +403,7 @@ class _FusionFunction(torch.autograd.Function):
         out = [None, None, None, None, None] + list(df4) + list(dcls) + list(dctr)
         for mod, plist, gr in ((mg, pg, gg), (ml, pl, gl)):
             for name, p in zip(mod._plist_names(), plist):
-                if gr is None:
+                if gr is None or mod._grad_key(name) not in gr:    # (gaussian: theta / phi receive no gradient)
                     out.append(None)
                     continue
                 t = gr[mod._grad_key(name)].reshape(p.shape)

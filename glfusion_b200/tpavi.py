@@ -36,6 +36,10 @@ def set_default_precision(name: str) -> None:
 
 
 _PARAM_ORDER = ("theta_w", "theta_b", "phi_w", "phi_b", "g_w", "g_b", "wz_w", "wz_b", "bn_w", "bn_b", "ln_w", "ln_b")
+# mode='gaussian' scores the block input against itself (f = x x^T, ours.py:869-873): theta / phi are state_dict entries
+# that take no part, so the kernels neither read them nor write a gradient for them (their .grad stays None)
+_UNUSED_BY_MODE = {L.MODE_GAUSSIAN: frozenset(("theta_w", "theta_b", "phi_w", "phi_b"))}
+_MODE_IDS = {"dot": L.MODE_DOT, "embedded": L.MODE_EMBEDDED, "gaussian": L.MODE_GAUSSIAN}
 
 
 _IO_DTYPES = {torch.bfloat16: L.DTYPE_BF16, torch.float32: L.DTYPE_F32, torch.float16: L.DTYPE_F16}
@@ -170,7 +174,11 @@ def tpavi_backward_raw(dz: torch.Tensor, dz_layout: int, x: torch.Tensor, st: TP
     grads = {}
     gdt = params["ln_w"].dtype
     g = L.GlfGrads()
+    unused = _UNUSED_BY_MODE.get(d.mode, ())
     for name in _PARAM_ORDER:
+        if name in unused:
+            setattr(g, name, None)
+            continue
         ref = params.get(name)
         if ref is None:
             # bn_layer=False: no BN affine; the kernels still want a scratch target
@@ -260,6 +268,9 @@ class _TPAVIFunction(torch.autograd.Function):
         out = [dx, None]
         for name, p in zip(module._plist_names(), plist):
             gname = module._grad_key(name)
+            if gname not in grads:          # a parameter the mode does not use (gaussian: theta / phi)
+                out.append(None)
+                continue
             gr = grads[gname].reshape(p.shape)
             out.append(gr if gr.dtype == p.dtype else gr.to(p.dtype))
         return tuple(out)
@@ -276,9 +287,9 @@ class TPAVIModule(nn.Module):
         if dimension != 3:
             # ours.py:845-917 only works for dimension=3 (the LayerNorm permute is 5-D); 1/2 crash in the reference
             raise NotImplementedError("glfusion_b200.TPAVIModule supports dimension=3 (as the reference effectively does)")
-        if mode in ('gaussian', 'concatenate'):
-            raise NotImplementedError(f"mode='{mode}' is not built by any constructor site of the reference network; "
-                                      "supported: 'dot' (MGFM/MLFM) and 'embedded' (softmax)")
+        if mode == 'concatenate':
+            raise NotImplementedError("mode='concatenate' is not built by any constructor site of the reference network; "
+                                      "supported: 'dot' (MGFM/MLFM), 'embedded' and 'gaussian' (softmax)")
         self.mode = mode
         self.dimension = dimension
         self.in_channels = in_channels
@@ -305,7 +316,7 @@ class TPAVIModule(nn.Module):
         self.theta = nn.Conv3d(in_channels=self.in_channels, out_channels=self.inter_channels, kernel_size=1)
         self.phi = nn.Conv3d(in_channels=self.in_channels, out_channels=self.inter_channels, kernel_size=1)
         self._bn_layer = bool(bn_layer)
-        self._mode_id = L.MODE_DOT if mode == 'dot' else L.MODE_EMBEDDED
+        self._mode_id = _MODE_IDS[mode]
         # tensor-core operand precision (not a reference ctor argument; set the attribute after construction):
         #   'bf16' — bf16 operands, fp32 accumulate (throughput arm, 2e-2 tolerance)
         #   'fp32' — fp32-exact products via 3-limb bf16 split on the same tcgen05 kernel (1e-4 tolerance, mode='dot')

@@ -37,7 +37,9 @@ extern "C" {
 
 typedef void* glf_stream_t; /* cudaStream_t */
 
-enum { GLF_MODE_DOT = 0, GLF_MODE_EMBEDDED = 1 };         /* TPAVIModule(mode=...)  ours.py:896-900 */
+/* TPAVIModule(mode=...)  ours.py:869-900.  GLF_MODE_GAUSSIAN: f = X X^T on the block input itself (theta / phi take no
+ * part; their glf_weights / glf_grads pointers are ignored and may be NULL), y = softmax(f) g(x). */
+enum { GLF_MODE_DOT = 0, GLF_MODE_EMBEDDED = 1, GLF_MODE_GAUSSIAN = 2 };
 /* I/O dtypes of the activations a caller hands over.  GLF_DTYPE_F16 is an I/O type only (torch.autocast's default):
  * the boundary kernels convert it to bf16 where they read it and round to fp16 where they write; everything between
  * (tensor-core operands, statistics) is bf16 / fp32 as for bf16 input.  fp16 stores round to nearest, so a value
@@ -64,7 +66,7 @@ typedef struct glf_desc {
   int32_t x_layout;   /* physical layout of x and dx                   GLF_LAYOUT_* */
   int32_t dz_layout;  /* physical layout of dz (z itself is always GLF_LAYOUT_TOKEN, like the reference's
                          permuted LayerNorm output, ours.py:913-915) */
-  int32_t precision;  /* GLF_PRECISION_* (GLF_PRECISION_F32X3 takes fp32 or bf16 io_dtype, not fp16) */
+  int32_t precision;  /* GLF_PRECISION_* (GLF_PRECISION_F32X3: mode='dot' only; fp32 or bf16 io_dtype, not fp16) */
   int32_t training;   /* BatchNorm3d uses batch statistics and updates running stats (ours.py:822-825) */
   int32_t bn_layer;   /* 1: W_z = conv + BN ; 0: W_z = conv only (ours.py:829-833) */
   int32_t accumulate; /* fwd: z += result instead of z = result (fuses f4_global + f4_local, ours.py:1834) */
@@ -271,6 +273,22 @@ GLF_API size_t glf_attention_scratch_bytes(int B, int N, int Ci, int backward);
 GLF_API int glf_attention_fwd(const void* P3, void* Y, float* lse, int B, int N, int Ci, void* scratch, glf_stream_t s);
 GLF_API int glf_attention_bwd(const void* P3, const void* Y, const void* dY, const float* lse, void* dP3, float* bias_grad,
                       int B, int N, int Ci, void* scratch, glf_stream_t s);
+
+/* The softmax attention of mode='gaussian' on its own (unit tests): Q = K = X, no projection, no 1/sqrt(C) scale.
+ * Flash kernels for (C, Ci) = (64, 64), (128, 64) and (128, 128), the chunked exact path otherwise.
+ *   fwd: Y = softmax(X X^T) G per sequence;  lse = logsumexp of each score row (natural log).
+ *   bwd: with P = softmax(X X^T), delta = rowsum(dY o Y), dS = P o (dY G^T - delta):
+ *        dX = dS X + dS^T X  (each term rounded to bf16, then their fp32 sum rounded once),  dG = P^T dY;
+ *        bias_grad (optional, may be NULL): the Ci column sums of dG over all B * N rows (g.bias).
+ *   X, dX: [B, N, C] bf16;  G, Y, dY, dG: [B, N, Ci] bf16;  lse: [B, N] fp32.
+ *   B, N > 0;  C and Ci positive multiples of 8, at most 2048;  16-byte aligned pointers.
+ *   scratch: glf_attention_gaussian_scratch_bytes(B, N, C, Ci, backward) bytes, 256-byte aligned (0 = invalid). */
+GLF_API size_t glf_attention_gaussian_scratch_bytes(int B, int N, int C, int Ci, int backward);
+GLF_API int glf_attention_gaussian_fwd(const void* X, const void* G, void* Y, float* lse, int B, int N, int C, int Ci,
+                               void* scratch, glf_stream_t s);
+GLF_API int glf_attention_gaussian_bwd(const void* X, const void* G, const void* Y, const void* dY, const float* lse,
+                               void* dX, void* dG, float* bias_grad, int B, int N, int C, int Ci, void* scratch,
+                               glf_stream_t s);
 
 /* The two HBM-bound fused epilogues as standalone entry points (unit tests, roofline probes).
  *   fwd: Z = LayerNorm_C(bn_a * U + bn_b + X) * ln_w + ln_b   (ours.py:908-915 after the W_z GEMM); U, X bf16 [rows, C];
