@@ -47,35 +47,30 @@ int check_device_sm100() {
   return 0;
 }
 
+int pack_tokens(const Dims& m, const void* in, int in_dtype, bool ncthw, void* out, int out_dtype, cudaStream_t stream) {
+  if (ncthw)
+    return transpose_cast(in, out, static_cast<int>(m.B), m.C, static_cast<int>(m.N), in_dtype, out_dtype, stream);
+  return transpose_cast(in, out, 1, 1, static_cast<int>(m.rows * m.C), in_dtype, out_dtype, stream);   // cast only
+}
+
+int unpack_tokens(const Dims& m, const void* in, int in_dtype, void* out, bool ncthw, int out_dtype,
+                  cudaStream_t stream) {
+  if (ncthw)
+    return transpose_cast(in, out, static_cast<int>(m.B), static_cast<int>(m.N), m.C, in_dtype, out_dtype, stream);
+  return transpose_cast(in, out, 1, 1, static_cast<int>(m.rows * m.C), in_dtype, out_dtype, stream);
+}
+
+int scatter_proj_grads(const float* dwcat, const glf_grads* g, int C, int Ci, bool g_only, cudaStream_t stream) {
+  float* const dst[3] = {g->theta_w, g->phi_w, g->g_w};
+  const char* what[3] = {"copy dtheta", "copy dphi", "copy dg"};
+  const size_t n = static_cast<size_t>(Ci) * C;
+  for (int k = g_only ? 2 : 0, row = 0; k < 3; ++k, ++row)
+    GLF_TRY(check_cuda(cudaMemcpyAsync(dst[k], dwcat + row * n, sizeof(float) * n, cudaMemcpyDeviceToDevice, stream),
+                       what[k]));
+  return 0;
+}
+
 namespace {
-
-struct Carver {
-  uint8_t* base;
-  size_t off = 0;
-  explicit Carver(void* b) : base(reinterpret_cast<uint8_t*>(b)) {}
-  template <typename T>
-  T* take(size_t n) {
-    off = (off + 255) & ~static_cast<size_t>(255);
-    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-    off += n * sizeof(T);
-    return p;
-  }
-};
-
-struct Dims {
-  long long B, N, rows;
-  int C, Ci;
-  int tiles_seq;   // m-tiles per sequence (128 tokens)
-  int tiles_all;   // m-tiles over all rows
-  bool pack_x;     // x must be repacked to token-major bf16
-  bool pack_dz;
-  bool dot;
-  bool gauss;      // mode='gaussian': Q = K = X, only the g projection runs
-  bool gram;       // mode='dot' in its Gram form (channel-space products only)
-  int Ca;          // augmented width of the per-sequence matrices (gram)
-  int pdt;         // GLF_DTYPE_* of the glf_weights / glf_grads tensors (glf_desc.reserved[3])
-  bool half_params;   // bf16 / fp16 parameters: an fp32 shadow in `saved`, fp32 gradient staging in ws_bwd
-};
 
 int make_dims(const glf_desc* d, Dims* o) {
   if (d == nullptr) return set_error(GLF_ERR_INVALID, "null descriptor");
@@ -113,7 +108,8 @@ int make_dims(const glf_desc* d, Dims* o) {
   o->tiles_seq = gemm_tiles_m(static_cast<int>(o->N));
   o->tiles_all = gemm_tiles_m(static_cast<int>(o->rows > 0x7fffffff ? 0x7fffffff : o->rows));
   if (o->rows > 0x7fffff00LL) return set_error(GLF_ERR_INVALID, "too many tokens");
-  o->pack_x = !(d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_BF16);   // fp32 / fp16: a bf16 copy
+  const int work_dtype = d->precision == GLF_PRECISION_F32X3 ? GLF_DTYPE_F32 : GLF_DTYPE_BF16;
+  o->pack_x = !(d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == work_dtype);
   if (d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype != GLF_DTYPE_BF16 && o->rows * d->C > 0x7fffffffLL)
     return set_error(GLF_ERR_INVALID, "token-major fp32 / fp16 input too large for the cast kernel");
   o->pack_dz = d->dz_layout != GLF_LAYOUT_TOKEN;
@@ -152,21 +148,26 @@ void weight_list(const glf_weights* w, const void* p[NPARAMS]) {
                             w->wz_w,    w->wz_b,    w->bn_w,  w->bn_b,  w->ln_w, w->ln_b};
   for (int k = 0; k < NPARAMS; ++k) p[k] = v[k];
 }
-// `w` with its parameter tensors replaced by the fp32 shadow (running statistics untouched: bn_finalize reads and
-// updates them in their own dtype); an absent tensor (bn_layer = 0) stays absent
-glf_weights shadow_weights(const glf_weights* w, float* const sh[NPARAMS]) {
+// The parameters every kernel reads: the caller's tensors, or with bf16 / fp16 parameters their fp32 shadow `sh`
+// (running statistics untouched: bn_finalize reads and updates them in their own dtype); an absent tensor (bn_layer = 0)
+// stays absent
+glf_weights fp32_weights(const Dims& m, const glf_weights* w, float* const sh[NPARAMS]) {
   glf_weights o = *w;
+  if (!m.half_params) return o;
   const float** f[NPARAMS] = {&o.theta_w, &o.theta_b, &o.phi_w, &o.phi_b, &o.g_w, &o.g_b,
                               &o.wz_w,    &o.wz_b,    &o.bn_w,  &o.bn_b,  &o.ln_w, &o.ln_b};
   for (int k = 0; k < NPARAMS; ++k) *f[k] = *f[k] != nullptr ? sh[k] : nullptr;
   return o;
 }
-glf_grads grads_table(float* const st[NPARAMS]) {
-  glf_grads g;
-  float** f[NPARAMS] = {&g.theta_w, &g.theta_b, &g.phi_w, &g.phi_b, &g.g_w, &g.g_b,
-                        &g.wz_w,    &g.wz_b,    &g.bn_w,  &g.bn_b,  &g.ln_w, &g.ln_b};
+// The gradient targets every writer fills: the caller's tensors, or with bf16 / fp16 parameters the fp32 staging `st`
+// that emit_grads rounds into them
+glf_grads fp32_grads(const Dims& m, const glf_grads* g, float* const st[NPARAMS]) {
+  if (!m.half_params) return *g;
+  glf_grads o;
+  float** f[NPARAMS] = {&o.theta_w, &o.theta_b, &o.phi_w, &o.phi_b, &o.g_w, &o.g_b,
+                        &o.wz_w,    &o.wz_b,    &o.bn_w,  &o.bn_b,  &o.ln_w, &o.ln_b};
   for (int k = 0; k < NPARAMS; ++k) *f[k] = st[k];
-  return g;
+  return o;
 }
 // forward: the 2-byte masters into the fp32 shadow that every consumer reads
 int stage_params(const Dims& m, const glf_weights* w, float* const sh[NPARAMS], cudaStream_t stream) {
@@ -252,6 +253,32 @@ size_t carve_saved(const Dims& m, void* base, Saved* s) {
   s->ln_mu = c.take<float>(rows);
   s->ln_r = c.take<float>(rows);
   return (c.off + 255) & ~static_cast<size_t>(255);
+}
+
+// The two blocks' operands of the fused LayerNorm pass (index 0 = MGFM, 1 = MLFM) from their saved blobs, with ln_w /
+// ln_b as the kernels read them (the fp32 shadow of bf16 / fp16 parameters)
+struct LnPair {
+  const bf16 *U[2], *X[2];
+  const float *a[2], *b[2], *mean[2], *rstd[2], *lw[2], *lb[2];
+  float *mu[2], *r[2];
+};
+LnPair ln_pair(const Dims& m, const void* xg, const void* xl, const glf_weights* wg, const glf_weights* wl,
+               const void* saved_g, const void* saved_l) {
+  const void* x[2] = {xg, xl};
+  const glf_weights* w[2] = {wg, wl};
+  const void* saved[2] = {saved_g, saved_l};
+  LnPair p;
+  for (int k = 0; k < 2; ++k) {
+    Saved s;
+    carve_saved(m, const_cast<void*>(saved[k]), &s);
+    const glf_weights w32 = fp32_weights(m, w[k], s.pshadow);
+    p.U[k] = s.U;
+    p.X[k] = reinterpret_cast<const bf16*>(x[k]);
+    p.a[k] = s.bn_a; p.b[k] = s.bn_b; p.mean[k] = s.bn_mean; p.rstd[k] = s.bn_rstd;
+    p.lw[k] = w32.ln_w; p.lb[k] = w32.ln_b;
+    p.mu[k] = s.ln_mu; p.r[k] = s.ln_r;
+  }
+  return p;
 }
 
 struct WsFwd { float* colstats; float* red1; float* Mf; void* attn; void* saved_fallback; float* Sf; };
@@ -345,13 +372,22 @@ size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
-int pick_split(long long tiles, int K) {
-  const int kb = (K + 63) / 64;
-  if (tiles >= 96) return 1;  // enough CTAs already: write the result directly, no atomics
-  long long s = (2 * 148) / tiles;   // floor: tiles * s work items fill at most two full rounds of the 148 persistent CTAs
-  if (s < 1) s = 1;
-  if (s > kb) s = kb;
-  return static_cast<int>(s);
+// A per-sequence token contraction (K = N) of the token-space form into bf16 D [batch][M][N]: written directly when
+// there are enough output tiles, else split along K with fp32 red.add into `acc` (zeroed first), rounded once into D.
+int token_contraction(GemmArgs g, bf16* D, float* acc, cudaStream_t stream) {
+  const long long n = static_cast<long long>(g.batch) * g.M * g.N;
+  g.ldd = g.N; g.strideD = static_cast<long long>(g.M) * g.N;
+  g.split_k = pick_split(static_cast<long long>(g.batch) * ((g.M + 127) / 128) * ((g.N + 127) / 128), g.K);
+  if (g.split_k == 1) {
+    g.out_kind = 0;
+    g.D = D;
+    return gemm(g, stream);
+  }
+  GLF_TRY(check_cuda(cudaMemsetAsync(acc, 0, sizeof(float) * n, stream), "memset split-K accumulator"));
+  g.out_kind = 2;
+  g.D = acc;
+  GLF_TRY(gemm(g, stream));
+  return cast_bf16(acc, D, n, stream);
 }
 
 // Split of a long token contraction (K = all rows) whose output tiles alone leave the last round of the 148 persistent
@@ -371,18 +407,6 @@ int pick_split_rounds(long long M, long long N, long long batch, int K) {
   }
   return best;
 }
-
-GemmOperand opnd(const void* p, int mn, long long ld, long long bs) {
-  GemmOperand o;
-  o.ptr = p; o.mn_major = mn; o.ld = ld; o.batch_stride = bs;
-  return o;
-}
-
-#define GLF_TRY(expr)        \
-  do {                       \
-    int rc__ = (expr);       \
-    if (rc__ != 0) return rc__; \
-  } while (0)
 
 // reserved[0] = 1: the LayerNorm stage (forward epilogue / first backward kernel) is run for MGFM and MLFM together
 // by glf_fusion_ln_fwd / glf_fusion_ln_bwd instead of per block
@@ -480,6 +504,27 @@ int gemm_pair2(GemmArgs g, const bf16* A0, const bf16* A1, const bf16* B0, const
   return gemm(g, stream);
 }
 
+// The end of the forward from the U product on: its np rows of BatchNorm column statistics (shrunk by a stage-1
+// reduction when long) finalised into the affine, then Z = LN(BN(U) + X) unless the fused LayerNorm pair
+// (glf_fusion_ln_fwd) finishes both blocks in one pass
+int bn_ln_fwd(const glf_desc* d, const Dims& m, const bf16* X, const glf_weights* w, int np, void* z, const Saved& s,
+              const WsFwd& wf, cudaStream_t stream) {
+  const int C = m.C;
+  const float* bn_part = wf.colstats;
+  if (d->training && d->bn_layer && np > 4 * REDUCE_STAGE1_ROWS) {
+    long long rs = 2LL * C;
+    const int np_in[1] = {np};
+    GLF_TRY(reduce_stage1(wf.colstats, nullptr, nullptr, 1, np_in, &np, &rs, C, 2, C, wf.red1, stream));
+    bn_part = wf.red1;
+  }
+  GLF_TRY(bn_finalize(bn_part, np, C, static_cast<double>(m.rows), d, w, w->wz_b, s.bn_mean, s.bn_rstd, s.bn_a, s.bn_b,
+                      stream));
+  if (defer_ln(d)) return 0;
+  GLF_TRY(bn_res_ln_fwd(s.U, X, GLF_DTYPE_BF16, s.bn_a, s.bn_b, w->ln_w, w->ln_b, z, d->io_dtype, s.ln_mu, s.ln_r,
+                        m.rows, C, d->eps_ln, d->accumulate, stream));
+  return 0;
+}
+
 int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_weights* w, void* z, const Saved& s,
                    const WsFwd& wf, cudaStream_t stream) {
   const int C = m.C, Ci = m.Ci, Ca = m.Ca, C1 = m.C + 1;
@@ -489,10 +534,7 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
   const long long CCi = static_cast<long long>(C) * Ci;
   const bf16* X = reinterpret_cast<const bf16*>(x);
   if (m.pack_x) {
-    if (d->x_layout == GLF_LAYOUT_NCTHW)
-      GLF_TRY(transpose_cast(x, s.xtok, B, C, N, d->io_dtype, GLF_DTYPE_BF16, stream));
-    else
-      GLF_TRY(transpose_cast(x, s.xtok, 1, 1, static_cast<int>(m.rows * C), d->io_dtype, GLF_DTYPE_BF16, stream));
+    GLF_TRY(pack_tokens(m, x, d->io_dtype, d->x_layout == GLF_LAYOUT_NCTHW, s.xtok, GLF_DTYPE_BF16, stream));
     X = s.xtok;
   }
   // S_b = X_b^T X_b, s_b = X_b^T 1   ->   S~_b
@@ -561,19 +603,7 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
     g.colstats_rows = &np;
     GLF_TRY(gemm(g, stream));
   }
-  const float* bn_part = wf.colstats;
-  if (d->training && d->bn_layer && np > 4 * REDUCE_STAGE1_ROWS) {
-    long long rs = 2LL * C;
-    const int np_in[1] = {np};
-    GLF_TRY(reduce_stage1(wf.colstats, nullptr, nullptr, 1, np_in, &np, &rs, C, 2, C, wf.red1, stream));
-    bn_part = wf.red1;
-  }
-  GLF_TRY(bn_finalize(bn_part, np, C, static_cast<double>(m.rows), d, w, w->wz_b, s.bn_mean, s.bn_rstd, s.bn_a, s.bn_b,
-                      stream));
-  if (defer_ln(d)) return 0;
-  GLF_TRY(bn_res_ln_fwd(s.U, X, GLF_DTYPE_BF16, s.bn_a, s.bn_b, w->ln_w, w->ln_b, z, d->io_dtype, s.ln_mu, s.ln_r,
-                        m.rows, C, d->eps_ln, d->accumulate, stream));
-  return 0;
+  return bn_ln_fwd(d, m, X, w, np, z, s, wf, stream);
 }
 
 // Continues after the LayerNorm backward and bn_bwd_finalize: wb.dV, wb.k1..k3 are valid.
@@ -719,43 +749,26 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     GLF_TRY(gemm_pair2(g, wb.dV, X, wb.EF, wb.EF + CC, stream));
   }
   if (!chain) GLF_TRY(gram_unpack_grads(wb.dwaug, g_, C, Ci, Ca, stream));
-  if (m.pack_x) {
-    if (d->x_layout == GLF_LAYOUT_NCTHW)
-      GLF_TRY(transpose_cast(wb.dxtok, dx, B, N, C, GLF_DTYPE_BF16, d->io_dtype, stream));
-    else
-      GLF_TRY(transpose_cast(wb.dxtok, dx, 1, 1, static_cast<int>(m.rows * C), GLF_DTYPE_BF16, d->io_dtype, stream));
-  }
+  if (m.pack_x)
+    GLF_TRY(unpack_tokens(m, wb.dxtok, GLF_DTYPE_BF16, dx, d->x_layout == GLF_LAYOUT_NCTHW, d->io_dtype, stream));
   return 0;
 }
 
-// Bias gradients = column sums of dTheta / dPhi / dG, from the partial tables their producers wrote: the three GEMM
-// epilogues (np, np_p, np_g rows of [2][Ci] each; the row counts can differ, tile shape and grid differ per product),
-// or the flash backward (np < 0: one table of -np rows of [2][3Ci] in cs_t, the column sums of dP = [dTheta|dPhi|dG]).
-int reduce_bias_grads(const float* cs_t, const float* cs_p, const float* cs_g, int np, int np_p, int np_g, int Ci,
-                      float* red1, float* db_t, float* db_p, float* db_g, cudaStream_t stream) {
-  long long rs = 2LL * Ci;
-  const float *t0 = cs_t, *t1 = cs_p, *t2 = cs_g;
-  if (np < 0) {
-    np = np_p = np_g = -np;
-    rs = 2LL * 3 * Ci;
-    t1 = cs_t + Ci;
-    t2 = cs_t + 2 * Ci;
+// Bias gradients out[i] = column sums (the first n columns) of table i of `cs`: one fixed-order pass when the tables are
+// short (one row per CTA) and of one length, else a stage-1 reduction first
+int reduce_bias_grads(const ColTables& cs, int n, float* red1, float* const* out, cudaStream_t stream) {
+  int np = cs.rows[0];
+  long long rs = cs.stride;
+  bool one_pass = np <= 4 * REDUCE_STAGE1_ROWS;
+  for (int i = 1; i < cs.n; ++i) one_pass = one_pass && cs.rows[i] == np;
+  const float *t0 = cs.tab[0], *t1 = cs.tab[1], *t2 = cs.tab[2];
+  if (!one_pass) {
+    GLF_TRY(reduce_stage1(t0, t1, t2, cs.n, cs.rows, &np, &rs, 0, 1, n, red1, stream));
+    const long long pitch = static_cast<long long>(REDUCE_STAGE1_ROWS) * n;
+    t0 = red1; t1 = red1 + pitch; t2 = red1 + 2 * pitch;
   }
-  if (np == np_p && np == np_g && np <= 4 * REDUCE_STAGE1_ROWS)   // short tables (one row per CTA): one fixed-order pass
-    return reduce_partials3(t0, t1, t2, np, rs, Ci, db_t, db_p, db_g, stream);
-  const int np_in[3] = {np, np_p, np_g};
-  GLF_TRY(reduce_stage1(t0, t1, t2, 3, np_in, &np, &rs, 0, 1, Ci, red1, stream));
-  return reduce_partials3(red1, red1 + static_cast<long long>(REDUCE_STAGE1_ROWS) * Ci,
-                          red1 + 2LL * REDUCE_STAGE1_ROWS * Ci, np, rs, Ci, db_t, db_p, db_g, stream);
-}
-
-// The g bias gradient of mode='gaussian' from the one table of column sums of dG the attention backward left in cs
-int reduce_bias_grad1(const float* cs, int np, int Ci, float* red1, float* db, cudaStream_t stream) {
-  long long rs = 2LL * Ci;
-  if (np <= 4 * REDUCE_STAGE1_ROWS) return reduce_partials(cs, np, rs, Ci, 1.f, db, stream);
-  const int np_in[1] = {np};
-  GLF_TRY(reduce_stage1(cs, nullptr, nullptr, 1, np_in, &np, &rs, 0, 1, Ci, red1, stream));
-  return reduce_partials(red1, np, rs, Ci, 1.f, db, stream);
+  if (cs.n == 1) return reduce_partials(t0, np, rs, n, 1.f, out[0], stream);
+  return reduce_partials3(t0, t1, t2, np, rs, n, out[0], out[1], out[2], stream);
 }
 
 // Scratch of the standalone attention entry points: the same pieces, sized the same way, as ws_bwd / ws_fwd give the
@@ -809,7 +822,7 @@ GLF_API int glf_tpavi_sizes(const glf_desc* d, glf_sizes* out) {
   Dims m;
   GLF_TRY(make_dims(d, &m));
   if (out == nullptr) return set_error(GLF_ERR_INVALID, "out is NULL");
-  if (d->precision == GLF_PRECISION_F32X3) return tpavi_sizes_f32x3(d, out);
+  if (d->precision == GLF_PRECISION_F32X3) return tpavi_sizes_f32x3(d, m, out);
   Saved s; WsFwd wf; WsBwd wb;
   out->saved_bytes = carve_saved(m, nullptr, &s);
   out->ws_fwd_bytes = carve_ws_fwd(m, nullptr, &wf, out->saved_bytes);
@@ -829,17 +842,14 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
   if (w == nullptr) return set_error(GLF_ERR_INVALID, "weights is NULL");
   if ((reinterpret_cast<uintptr_t>(ws) & 255) != 0 || (saved && (reinterpret_cast<uintptr_t>(saved) & 255) != 0))
     return set_error(GLF_ERR_WORKSPACE, "saved/ws blobs must be 256-byte aligned");
-  if (d->precision == GLF_PRECISION_F32X3) return tpavi_fwd_f32x3(d, x, w, z, saved, ws, stream);
+  if (d->precision == GLF_PRECISION_F32X3) return tpavi_fwd_f32x3(d, m, x, w, z, saved, ws, stream);
   Saved s; WsFwd wf;
   const size_t saved_bytes = carve_saved(m, nullptr, &s);
   carve_ws_fwd(m, ws, &wf, saved_bytes);
   carve_saved(m, saved ? saved : wf.saved_fallback, &s);
-  glf_weights wh;
-  if (m.half_params) {
-    GLF_TRY(stage_params(m, w, s.pshadow, stream));
-    wh = shadow_weights(w, s.pshadow);
-    w = &wh;
-  }
+  if (m.half_params) GLF_TRY(stage_params(m, w, s.pshadow, stream));
+  const glf_weights w32 = fp32_weights(m, w, s.pshadow);
+  w = &w32;
   if (m.gram) return tpavi_fwd_gram(d, m, x, w, z, s, wf, stream);
   const int C = m.C, Ci = m.Ci;
   const int N = static_cast<int>(m.N), rows = static_cast<int>(m.rows), B = static_cast<int>(m.B);
@@ -850,10 +860,7 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
     GLF_TRY(prep_weights(w, C, Ci, s.wcat, s.wcatT, s.bcat, s.wz, s.wzT, stream));
   const bf16* X = reinterpret_cast<const bf16*>(x);
   if (m.pack_x) {
-    if (d->x_layout == GLF_LAYOUT_NCTHW)
-      GLF_TRY(transpose_cast(x, s.xtok, B, C, N, d->io_dtype, GLF_DTYPE_BF16, stream));
-    else
-      GLF_TRY(transpose_cast(x, s.xtok, 1, 1, static_cast<int>(m.rows * C), d->io_dtype, GLF_DTYPE_BF16, stream));  // cast only
+    GLF_TRY(pack_tokens(m, x, d->io_dtype, d->x_layout == GLF_LAYOUT_NCTHW, s.xtok, GLF_DTYPE_BF16, stream));
     X = s.xtok;
   }
   const int Pw = m.gauss ? Ci : 3 * Ci;
@@ -875,19 +882,7 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
       g.B = opnd(s.P + 2 * Ci, 1, 3 * Ci, static_cast<long long>(N) * 3 * Ci);
       g.M = Ci; g.N = Ci; g.K = N; g.batch = B;
       g.alpha = 1.f / static_cast<float>(N);
-      g.ldd = Ci; g.strideD = CiCi;
-      g.split_k = pick_split(static_cast<long long>(B) * ((Ci + 127) / 128) * ((Ci + 127) / 128), N);
-      if (g.split_k > 1) {
-        GLF_TRY(check_cuda(cudaMemsetAsync(wf.Mf, 0, sizeof(float) * B * CiCi, stream), "memset M"));
-        g.out_kind = 2;
-        g.D = wf.Mf;
-        GLF_TRY(gemm(g, stream));
-        GLF_TRY(cast_bf16(wf.Mf, s.Mb, B * CiCi, stream));
-      } else {
-        g.out_kind = 0;
-        g.D = s.Mb;
-        GLF_TRY(gemm(g, stream));
-      }
+      GLF_TRY(token_contraction(g, s.Mb, wf.Mf, stream));
     }
     {  // W'_b[c,i] = sum_j Wz[c,j] M_b[i,j]        (folds Y = Theta M and U = Y Wz^T into one product per token)
       GemmArgs g;
@@ -924,19 +919,7 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
       GLF_TRY(gemm(g, stream));
     }
   }
-  const float* bn_part = wf.colstats;
-  if (d->training && d->bn_layer && np > 4 * REDUCE_STAGE1_ROWS) {
-    long long rs = 2LL * C;
-    const int np_in[1] = {np};
-    GLF_TRY(reduce_stage1(wf.colstats, nullptr, nullptr, 1, np_in, &np, &rs, C, 2, C, wf.red1, stream));
-    bn_part = wf.red1;
-  }
-  GLF_TRY(bn_finalize(bn_part, np, C, static_cast<double>(m.rows), d, w, w->wz_b, s.bn_mean, s.bn_rstd, s.bn_a, s.bn_b,
-                      stream));
-  if (defer_ln(d)) return 0;   // the pair entry point glf_fusion_ln_fwd finishes both blocks in one pass
-  GLF_TRY(bn_res_ln_fwd(s.U, X, GLF_DTYPE_BF16, s.bn_a, s.bn_b, w->ln_w, w->ln_b, z, d->io_dtype, s.ln_mu, s.ln_r,
-                        m.rows, C, d->eps_ln, d->accumulate, stream));
-  return 0;
+  return bn_ln_fwd(d, m, X, w, np, z, s, wf, stream);
 }
 
 GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, const glf_weights* w, const void* saved, void* dx,
@@ -953,19 +936,15 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
   if (w == nullptr || g_ == nullptr) return set_error(GLF_ERR_INVALID, "weights/grads is NULL");
   if ((reinterpret_cast<uintptr_t>(ws) & 255) != 0 || (reinterpret_cast<uintptr_t>(saved) & 255) != 0)
     return set_error(GLF_ERR_WORKSPACE, "saved/ws blobs must be 256-byte aligned");
-  if (d->precision == GLF_PRECISION_F32X3) return tpavi_bwd_f32x3(d, dz, x, w, saved, dx, g_, ws, stream);
+  if (d->precision == GLF_PRECISION_F32X3) return tpavi_bwd_f32x3(d, m, dz, x, w, saved, dx, g_, ws, stream);
   Saved s; WsBwd wb;
   carve_saved(m, const_cast<void*>(saved), &s);
   carve_ws_bwd(d, m, ws, &wb);
   const glf_grads* g_out = g_;
-  glf_weights wh;
-  glf_grads gh;
-  if (m.half_params) {   // every consumer reads the forward's fp32 shadow, every writer fills the fp32 staging
-    wh = shadow_weights(w, s.pshadow);
-    w = &wh;
-    gh = grads_table(wb.gstage);
-    g_ = &gh;
-  }
+  const glf_weights w32 = fp32_weights(m, w, s.pshadow);
+  const glf_grads g32 = fp32_grads(m, g_, wb.gstage);
+  w = &w32;
+  g_ = &g32;
   const int C = m.C, Ci = m.Ci;
   const int N = static_cast<int>(m.N), rows = static_cast<int>(m.rows), B = static_cast<int>(m.B);
   const bf16* X = m.pack_x ? s.xtok : reinterpret_cast<const bf16*>(x);
@@ -974,7 +953,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
   const void* dZ = dz;
   int dz_dtype = d->io_dtype;
   if (m.pack_dz && !defer_ln(d)) {
-    GLF_TRY(transpose_cast(dz, wb.dztok, B, C, N, d->io_dtype, GLF_DTYPE_BF16, stream));
+    GLF_TRY(pack_tokens(m, dz, d->io_dtype, /*ncthw=*/true, wb.dztok, GLF_DTYPE_BF16, stream));
     dZ = wb.dztok;
     dz_dtype = GLF_DTYPE_BF16;
   }
@@ -997,8 +976,11 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     GLF_TRY(bn_bwd_apply(wb.dV, s.U, GLF_DTYPE_BF16, wb.k1, wb.k2, wb.k3, wb.dU, m.rows, C, stream));
     dU = wb.dU;
   }
-  int np = 0, np_p = 0, np_g = 0;
-  if (m.dot) {
+  ColTables cs;
+  if (m.dot) {   // three GEMM epilogues: their row counts can differ (tile shape and grid differ per product)
+    cs.n = 3;
+    cs.tab[0] = wb.cs_t; cs.tab[1] = wb.cs_p; cs.tab[2] = wb.cs_g;
+    cs.stride = 2LL * Ci;
     const long long CiCi = static_cast<long long>(Ci) * Ci;
     const long long CCi = static_cast<long long>(C) * Ci;
     {  // dTheta_b = dU_b W'_b          (B operand = W'_b read MN-major: stored [K=c][N=i])
@@ -1008,7 +990,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.M = N; g.N = Ci; g.K = C; g.batch = B;
       g.D = wb.dP; g.ldd = 3 * Ci; g.strideD = seqP;
       g.colstats = wb.cs_t;
-      g.colstats_rows = &np;
+      g.colstats_rows = &cs.rows[0];
       GLF_TRY(gemm(g, stream));
     }
     {  // dW'_b[c,i] = sum_n dU[n,c] Theta[n,i]
@@ -1016,19 +998,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.A = opnd(dU, 1, C, static_cast<long long>(N) * C);
       g.B = opnd(s.P, 1, 3 * Ci, seqP);
       g.M = C; g.N = Ci; g.K = N; g.batch = B;
-      g.ldd = Ci; g.strideD = CCi;
-      g.split_k = pick_split(static_cast<long long>(B) * ((C + 127) / 128) * ((Ci + 127) / 128), N);
-      if (g.split_k > 1) {
-        GLF_TRY(check_cuda(cudaMemsetAsync(wb.dWpf, 0, sizeof(float) * B * CCi, stream), "memset dW'"));
-        g.out_kind = 2;
-        g.D = wb.dWpf;
-        GLF_TRY(gemm(g, stream));
-        GLF_TRY(cast_bf16(wb.dWpf, wb.dWpb, B * CCi, stream));
-      } else {
-        g.out_kind = 0;
-        g.D = wb.dWpb;
-        GLF_TRY(gemm(g, stream));
-      }
+      GLF_TRY(token_contraction(g, wb.dWpb, wb.dWpf, stream));
     }
     GLF_TRY(check_cuda(cudaMemsetAsync(g_->wz_w, 0, sizeof(float) * CCi, stream), "memset dWz"));
     {  // dWz[c,j] = sum_b sum_i dW'_b[c,i] M_b[i,j]     (batch reduced by fp32 red.add into one output)
@@ -1056,7 +1026,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.alpha = 1.f / static_cast<float>(N);
       g.D = wb.dP + Ci; g.ldd = 3 * Ci; g.strideD = seqP;
       g.colstats = wb.cs_p;
-      g.colstats_rows = &np_p;
+      g.colstats_rows = &cs.rows[1];
       GLF_TRY(gemm(g, stream));
     }
     {  // dG_b = Phi_b dM_b / N          (B operand = dM_b read MN-major)
@@ -1067,7 +1037,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.alpha = 1.f / static_cast<float>(N);
       g.D = wb.dP + 2 * Ci; g.ldd = 3 * Ci; g.strideD = seqP;
       g.colstats = wb.cs_g;
-      g.colstats_rows = &np_g;
+      g.colstats_rows = &cs.rows[2];
       GLF_TRY(gemm(g, stream));
     }
   } else {
@@ -1090,19 +1060,15 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.split_k = pick_split_rounds(C, Ci, 1, rows);
       GLF_TRY(gemm(g, stream));
     }
-    int cs_rows[3];
     if (m.gauss) {   // dP = [dS X | dS^T X | dG]: the two attention terms of dX side by side, summed by the dX product
       const long long ldp = 2LL * C + Ci;
       const AttnArgs a = attn_args_gaussian(X, s.P, wb.dP, wb.dP + C, wb.dP + 2 * C, ldp, ldp, C, Ci);
-      GLF_TRY(attn_bwd(a, s.Y, wb.dY, s.lse, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows, B, N,
+      GLF_TRY(attn_bwd(a, s.Y, wb.dY, s.lse, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, &cs, B, N,
                        wb.attn, stream));
     } else {
-      GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, cs_rows,
+      GLF_TRY(flash_bwd(s.P, s.Y, wb.dY, s.lse, wb.dP, wb.delta, wb.cs_t, wb.cs_p, wb.cs_g, 4 * B * m.tiles_seq, &cs,
                         B, N, Ci, wb.attn, stream));
     }
-    np = cs_rows[0];
-    np_p = cs_rows[1];
-    np_g = cs_rows[2];
   }
   // dP columns [wrow, ldp) are the projection gradients (all three, or dG alone for gaussian)
   const int ldp = m.gauss ? 2 * C + Ci : 3 * Ci;
@@ -1119,14 +1085,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     g.split_k = pick_split_rounds(nproj, C, 1, rows);
     GLF_TRY(gemm(g, stream));
   }
-  const size_t wbytes = sizeof(float) * Ci * C;
-  if (m.gauss) {
-    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
-  } else {
-    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->theta_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dtheta"));
-    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->phi_w, wb.dwcat + static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dphi"));
-    GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat + 2 * static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
-  }
+  GLF_TRY(scatter_proj_grads(wb.dwcat, g_, C, Ci, m.gauss, stream));
   {  // dX = dP Wcat + dV   (gaussian: [dS X | dS^T X | dG] [I | I | Wg^T]^T + dV, each attention term rounded to bf16
      // once before this fp32 sum)
     GemmArgs g;
@@ -1137,17 +1096,10 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     g.D = m.pack_x ? static_cast<void*>(wb.dxtok) : dx; g.ldd = C;
     GLF_TRY(gemm(g, stream));
   }
-  if (m.gauss)
-    GLF_TRY(reduce_bias_grad1(wb.cs_g, np_g, Ci, wb.red1, g_->g_b, stream));
-  else
-    GLF_TRY(reduce_bias_grads(wb.cs_t, wb.cs_p, wb.cs_g, np, np_p, np_g, Ci, wb.red1, g_->theta_b, g_->phi_b, g_->g_b,
-                              stream));
-  if (m.pack_x) {
-    if (d->x_layout == GLF_LAYOUT_NCTHW)
-      GLF_TRY(transpose_cast(wb.dxtok, dx, B, N, C, GLF_DTYPE_BF16, d->io_dtype, stream));
-    else
-      GLF_TRY(transpose_cast(wb.dxtok, dx, 1, 1, static_cast<int>(m.rows * C), GLF_DTYPE_BF16, d->io_dtype, stream));
-  }
+  float* const db[3] = {g_->theta_b, g_->phi_b, g_->g_b};
+  GLF_TRY(reduce_bias_grads(cs, Ci, wb.red1, m.gauss ? db + 2 : db, stream));   // gaussian: the g bias alone
+  if (m.pack_x)
+    GLF_TRY(unpack_tokens(m, wb.dxtok, GLF_DTYPE_BF16, dx, d->x_layout == GLF_LAYOUT_NCTHW, d->io_dtype, stream));
   return emit_grads(m, wb.gstage, g_out, stream);
 }
 
@@ -1180,29 +1132,12 @@ GLF_API int glf_fusion_ln_fwd_parts(const glf_desc* d, const void* xg, const voi
   GLF_TRY(check_ptr(saved_g, "saved_g"));
   GLF_TRY(check_ptr(saved_l, "saved_l"));
   if (wg == nullptr || wl == nullptr) return set_error(GLF_ERR_INVALID, "weights is NULL");
-  Saved sg, sl;
-  carve_saved(m, saved_g, &sg);
-  carve_saved(m, saved_l, &sl);
-  glf_weights wgh, wlh;
-  if (m.half_params) {   // ln_w / ln_b from the fp32 shadows the blocks' forward left in their saved blobs
-    wgh = shadow_weights(wg, sg.pshadow);
-    wlh = shadow_weights(wl, sl.pshadow);
-    wg = &wgh;
-    wl = &wlh;
-  }
-  const bf16* U[2] = {sg.U, sl.U};
-  const bf16* X[2] = {reinterpret_cast<const bf16*>(xg), reinterpret_cast<const bf16*>(xl)};
-  const float* a[2] = {sg.bn_a, sl.bn_a};
-  const float* b[2] = {sg.bn_b, sl.bn_b};
-  const float* lw[2] = {wg->ln_w, wl->ln_w};
-  const float* lb[2] = {wg->ln_b, wl->ln_b};
-  float* mu[2] = {sg.ln_mu, sl.ln_mu};
-  float* r[2] = {sg.ln_r, sl.ln_r};
+  const LnPair p = ln_pair(m, xg, xl, wg, wl, saved_g, saved_l);
   if (!ln_tma_supported(m.C))     // wide rows (256 < C <= 2048): the sliced-row ring kernel, both blocks in one pass
-    return ln_pair_fwd_wide(U, X, a, b, lw, lb, mu, r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream, z_global,
-                            pair_z_dtype(d));
-  return ln_fwd_tma(2, U, X, a, b, lw, lb, mu, r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream, z_global,
-                    pair_z_dtype(d));
+    return ln_pair_fwd_wide(p.U, p.X, p.a, p.b, p.lw, p.lb, p.mu, p.r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream,
+                            z_global, pair_z_dtype(d));
+  return ln_fwd_tma(2, p.U, p.X, p.a, p.b, p.lw, p.lb, p.mu, p.r, z, m.rows, m.C, d->eps_ln, d->accumulate, stream,
+                    z_global, pair_z_dtype(d));
 }
 
 GLF_API int glf_fusion_ln_bwd(const glf_desc* d, const void* dz, const void* xg, const void* xl, const glf_weights* wg,
@@ -1236,28 +1171,10 @@ GLF_API int glf_fusion_ln_bwd_views(const glf_desc* d, const void* dz, const voi
   GLF_TRY(check_ptr(ws_g, "ws_g"));
   GLF_TRY(check_ptr(ws_l, "ws_l"));
   if (wg == nullptr || wl == nullptr) return set_error(GLF_ERR_INVALID, "weights is NULL");
-  Saved sg, sl;
+  const LnPair p = ln_pair(m, xg, xl, wg, wl, saved_g, saved_l);
   WsBwd bg, bl;
-  carve_saved(m, const_cast<void*>(saved_g), &sg);
-  carve_saved(m, const_cast<void*>(saved_l), &sl);
   carve_ws_bwd(d, m, ws_g, &bg);
   carve_ws_bwd(d, m, ws_l, &bl);
-  glf_weights wgh, wlh;
-  if (m.half_params) {
-    wgh = shadow_weights(wg, sg.pshadow);
-    wlh = shadow_weights(wl, sl.pshadow);
-    wg = &wgh;
-    wl = &wlh;
-  }
-  const bf16* U[2] = {sg.U, sl.U};
-  const bf16* X[2] = {reinterpret_cast<const bf16*>(xg), reinterpret_cast<const bf16*>(xl)};
-  const float* a[2] = {sg.bn_a, sl.bn_a};
-  const float* b[2] = {sg.bn_b, sl.bn_b};
-  const float* lw[2] = {wg->ln_w, wl->ln_w};
-  const float* mean[2] = {sg.bn_mean, sl.bn_mean};
-  const float* rstd[2] = {sg.bn_rstd, sl.bn_rstd};
-  const float* mu[2] = {sg.ln_mu, sl.ln_mu};
-  const float* r[2] = {sg.ln_r, sl.ln_r};
   bf16* dV[2] = {bg.dV, bl.dV};
   float* part[2] = {bg.part_ln, bl.part_ln};
   int nb = 0;
@@ -1267,12 +1184,12 @@ GLF_API int glf_fusion_ln_bwd_views(const glf_desc* d, const void* dz, const voi
     // the two blocks run the sliced-row ring kernel one after the other
     if (views) return set_error(GLF_ERR_UNSUPPORTED, "per-view dz needs C <= 256");
     for (int k = 0; k < 2; ++k)
-      GLF_TRY(bn_res_ln_bwd(dz, pair_z_dtype(d), U[k], X[k], GLF_DTYPE_BF16, a[k], b[k], mean[k], rstd[k], lw[k], mu[k],
-                            r[k], dV[k], part[k], m.rows, m.C, &nb, stream));
+      GLF_TRY(bn_res_ln_bwd(dz, pair_z_dtype(d), p.U[k], p.X[k], GLF_DTYPE_BF16, p.a[k], p.b[k], p.mean[k], p.rstd[k],
+                            p.lw[k], p.mu[k], p.r[k], dV[k], part[k], m.rows, m.C, &nb, stream));
     return 0;
   }
-  return ln_bwd_tma(2, dz, U, X, a, b, lw, mean, rstd, mu, r, dV, part, m.rows, m.C, &nb, stream, views ? d->T : 0,
-                    dz_views, reinterpret_cast<const long long*>(dz_stride_b), d->H * d->W, pair_z_dtype(d));
+  return ln_bwd_tma(2, dz, p.U, p.X, p.a, p.b, p.lw, p.mean, p.rstd, p.mu, p.r, dV, part, m.rows, m.C, &nb, stream,
+                    views ? d->T : 0, dz_views, reinterpret_cast<const long long*>(dz_stride_b), d->H * d->W, pair_z_dtype(d));
 }
 
 GLF_API int glf_gate_concat_fwd(int B, int C, int V, int h, int w, int ncls, float weight, int io_dtype, int x_dtype,
@@ -1465,13 +1382,13 @@ GLF_API int glf_attention_bwd(const void* P3, const void* Y, const void* dY, con
   GLF_TRY(check_device_sm100());
   WsAttn w;
   carve_ws_attn(B, N, Ci, true, scratch, &w);
-  int np[3];
+  ColTables cs;
   GLF_TRY(flash_bwd(reinterpret_cast<const bf16*>(P3), reinterpret_cast<const bf16*>(Y), reinterpret_cast<const bf16*>(dY),
-                    lse, reinterpret_cast<bf16*>(dP3), w.delta, w.cs_t, w.cs_p, w.cs_g, w.cs_cap_rows, np, B, N, Ci,
+                    lse, reinterpret_cast<bf16*>(dP3), w.delta, w.cs_t, w.cs_p, w.cs_g, w.cs_cap_rows, &cs, B, N, Ci,
                     w.attn, stream));
   if (bias_grad == nullptr) return 0;
-  return reduce_bias_grads(w.cs_t, w.cs_p, w.cs_g, np[0], np[1], np[2], Ci, w.red1, bias_grad, bias_grad + Ci,
-                           bias_grad + 2 * Ci, stream);
+  float* const db[3] = {bias_grad, bias_grad + Ci, bias_grad + 2 * Ci};
+  return reduce_bias_grads(cs, Ci, w.red1, db, stream);
 }
 
 GLF_API size_t glf_attention_gaussian_scratch_bytes(int B, int N, int C, int Ci, int backward) {
@@ -1517,12 +1434,12 @@ GLF_API int glf_attention_gaussian_bwd(const void* X, const void* G, const void*
   carve_ws_attn(B, N, Ci, true, scratch, &w, C);
   const AttnArgs a = attn_args_gaussian(reinterpret_cast<const bf16*>(X), reinterpret_cast<const bf16*>(G), w.dx2,
                                         w.dx2 + C, reinterpret_cast<bf16*>(dG), 2LL * C, Ci, C, Ci);
-  int np[3];
+  ColTables cs;
   GLF_TRY(attn_bwd(a, reinterpret_cast<const bf16*>(Y), reinterpret_cast<const bf16*>(dY), lse, w.delta, w.cs_t, w.cs_p,
-                   w.cs_g, w.cs_cap_rows, np, B, N, w.attn, stream));
+                   w.cs_g, w.cs_cap_rows, &cs, B, N, w.attn, stream));
   GLF_TRY(sum_halves(w.dx2, reinterpret_cast<bf16*>(dX), static_cast<long long>(B) * N, C, stream));
   if (bias_grad == nullptr) return 0;
-  return reduce_bias_grad1(w.cs_g, np[2], Ci, w.red1, bias_grad, stream);
+  return reduce_bias_grads(cs, Ci, w.red1, &bias_grad, stream);
 }
 
 GLF_API int glf_bn_res_ln_fwd(int64_t rows, int C, const void* U, const void* X, const float* bn_a, const float* bn_b,

@@ -11,54 +11,14 @@ namespace glf {
 
 namespace {
 
-struct Carver {
-  uint8_t* base;
-  size_t off = 0;
-  explicit Carver(void* b) : base(reinterpret_cast<uint8_t*>(b)) {}
-  template <typename T>
-  T* take(size_t n) {
-    off = (off + 255) & ~static_cast<size_t>(255);
-    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-    off += n * sizeof(T);
-    return p;
-  }
-};
-
-#define GLF_TRY(expr)           \
-  do {                          \
-    int rc__ = (expr);          \
-    if (rc__ != 0) return rc__; \
-  } while (0)
-
-struct D3 {
-  int B, N, rows, C, Ci, tiles;
-  bool x_direct;   // x is already fp32 token-major: no repacked copy
-  bool dz_direct;  // dz is fp32 token-major
-  bool dx_direct;  // dx can be written in place (fp32 token-major)
-};
-
-D3 dims(const glf_desc* d) {
-  D3 m;
-  m.B = d->B;
-  m.N = d->T * d->H * d->W;
-  m.rows = m.B * m.N;
-  m.C = d->C;
-  m.Ci = d->Ci;
-  m.tiles = gemm_tiles_m(m.N);
-  m.x_direct = d->x_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_F32;
-  m.dz_direct = d->dz_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_F32;
-  m.dx_direct = m.x_direct;
-  return m;
-}
-
 struct Saved3 {
   float *Xf, *Uf, *bcat, *bn_mean, *bn_rstd, *bn_a, *bn_b, *ln_mu, *ln_r;
   bf16 *Xl, *Pl, *Ml, *Wpl, *wcat_l, *wcatT_l, *wz_l;
 };
-size_t carve_saved3(const D3& m, void* base, Saved3* s) {
+size_t carve_saved3(const Dims& m, void* base, Saved3* s) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
-  s->Xf = m.x_direct ? nullptr : c.take<float>(rows * C);
+  s->Xf = m.pack_x ? c.take<float>(rows * C) : nullptr;
   s->Xl = c.take<bf16>(3 * rows * C);
   s->Pl = c.take<bf16>(3 * rows * 3 * Ci);
   s->Uf = c.take<float>(rows * C);
@@ -78,7 +38,7 @@ size_t carve_saved3(const D3& m, void* base, Saved3* s) {
 }
 
 struct WsF3 { float *wcat_f, *wcatT_f, *Pf, *Mf, *Wpf, *cs; void* saved_fallback; };
-size_t carve_wsf3(const D3& m, void* base, WsF3* w, size_t saved_bytes) {
+size_t carve_wsf3(const Dims& m, void* base, WsF3* w, size_t saved_bytes) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
   w->wcat_f = c.take<float>(3 * Ci * C);
@@ -95,10 +55,11 @@ struct WsB3 {
   float *dZf, *dVf, *dUf, *dPf, *dWpf, *dMf, *dXf, *part_ln, *k1, *k2, *k3, *cs, *dwcat;
   bf16 *dUl, *dPl, *dWpl, *dMl;
 };
-size_t carve_wsb3(const D3& m, void* base, WsB3* w) {
+size_t carve_wsb3(const glf_desc* d, const Dims& m, void* base, WsB3* w) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
-  w->dZf = m.dz_direct ? nullptr : c.take<float>(rows * C);
+  const bool dz_f32_tokens = d->dz_layout == GLF_LAYOUT_TOKEN && d->io_dtype == GLF_DTYPE_F32;   // read in place
+  w->dZf = dz_f32_tokens ? nullptr : c.take<float>(rows * C);
   w->dVf = c.take<float>(rows * C);
   w->dUf = c.take<float>(rows * C);
   w->dUl = c.take<bf16>(3 * rows * C);
@@ -108,7 +69,7 @@ size_t carve_wsb3(const D3& m, void* base, WsB3* w) {
   w->dWpl = c.take<bf16>(3 * B * C * Ci);
   w->dMf = c.take<float>(B * Ci * Ci);
   w->dMl = c.take<bf16>(3 * B * Ci * Ci);
-  w->dXf = m.dx_direct ? nullptr : c.take<float>(rows * C);
+  w->dXf = m.pack_x ? c.take<float>(rows * C) : nullptr;
   w->part_ln = c.take<float>(static_cast<size_t>(bn_res_ln_bwd_blocks(m.rows, m.C)) * 4 * C);
   w->k1 = c.take<float>(C);
   w->k2 = c.take<float>(C);
@@ -118,48 +79,29 @@ size_t carve_wsb3(const D3& m, void* base, WsB3* w) {
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
-// limb-plane operand: planes are `plane` elements apart
-GemmOperand lop(const bf16* p, int mn, long long ld, long long bs, long long plane) {
-  GemmOperand o;
-  o.ptr = p; o.mn_major = mn; o.ld = ld; o.batch_stride = bs; o.limb_stride = plane;
-  return o;
-}
 void six_pairs(GemmArgs& g) {
   static const int pa[6] = {0, 2, 1, 0, 1, 0};
   static const int pb[6] = {2, 0, 1, 1, 0, 0};
   g.npairs = 6;
   for (int i = 0; i < 6; ++i) { g.pairA[i] = pa[i]; g.pairB[i] = pb[i]; }
 }
-int pick_split3(long long tiles, int K) {
-  const int kb = (K + 63) / 64;
-  if (tiles >= 96) return 1;
-  long long s = (2 * 148) / tiles;   // floor: at most two full rounds of the 148 persistent CTAs
-  if (s < 1) s = 1;
-  if (s > kb) s = kb;
-  return static_cast<int>(s);
-}
-
 }  // namespace
 
-int tpavi_sizes_f32x3(const glf_desc* d, glf_sizes* out) {
-  if (d->mode != GLF_MODE_DOT) return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 is implemented for mode='dot'");
-  const D3 m = dims(d);
+int tpavi_sizes_f32x3(const glf_desc* d, const Dims& m, glf_sizes* out) {
   Saved3 s; WsF3 wf; WsB3 wb;
   out->saved_bytes = carve_saved3(m, nullptr, &s);
   out->ws_fwd_bytes = carve_wsf3(m, nullptr, &wf, out->saved_bytes);
-  out->ws_bwd_bytes = carve_wsb3(m, nullptr, &wb);
+  out->ws_bwd_bytes = carve_wsb3(d, m, nullptr, &wb);
   return 0;
 }
 
-int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void* z, void* saved, void* ws,
-                    cudaStream_t stream) {
-  if (d->mode != GLF_MODE_DOT) return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 is implemented for mode='dot'");
-  const D3 m = dims(d);
+int tpavi_fwd_f32x3(const glf_desc* d, const Dims& m, const void* x, const glf_weights* w, void* z, void* saved,
+                    void* ws, cudaStream_t stream) {
   Saved3 s; WsF3 wf;
   const size_t saved_bytes = carve_saved3(m, nullptr, &s);
   carve_wsf3(m, ws, &wf, saved_bytes);
   carve_saved3(m, saved ? saved : wf.saved_fallback, &s);
-  const int C = m.C, Ci = m.Ci, N = m.N, B = m.B, rows = m.rows;
+  const int C = m.C, Ci = m.Ci, N = static_cast<int>(m.N), B = static_cast<int>(m.B), rows = static_cast<int>(m.rows);
   const long long pX = static_cast<long long>(rows) * C, pP = static_cast<long long>(rows) * 3 * Ci;
   const long long pW = 3LL * Ci * C, pWz = static_cast<long long>(C) * Ci;
   const long long CiCi = static_cast<long long>(Ci) * Ci, CCi = pWz;
@@ -171,18 +113,15 @@ int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void
   GLF_TRY(split3(wf.wcatT_f, s.wcatT_l, pW, stream));
   GLF_TRY(split3(w->wz_w, s.wz_l, pWz, stream));
   const float* Xf = reinterpret_cast<const float*>(x);
-  if (!m.x_direct) {
-    if (d->x_layout == GLF_LAYOUT_NCTHW)
-      GLF_TRY(transpose_cast(x, s.Xf, B, C, N, d->io_dtype, GLF_DTYPE_F32, stream));
-    else
-      GLF_TRY(transpose_cast(x, s.Xf, 1, 1, static_cast<int>(pX), d->io_dtype, GLF_DTYPE_F32, stream));
+  if (m.pack_x) {
+    GLF_TRY(pack_tokens(m, x, d->io_dtype, d->x_layout == GLF_LAYOUT_NCTHW, s.Xf, GLF_DTYPE_F32, stream));
     Xf = s.Xf;
   }
   GLF_TRY(split3(Xf, s.Xl, pX, stream));
   {  // P = X Wcat^T + bcat
     GemmArgs g;
-    g.A = lop(s.Xl, 0, C, 0, pX);
-    g.B = lop(s.wcat_l, 0, C, 0, pW);
+    g.A = opnd(s.Xl, 0, C, 0, pX);
+    g.B = opnd(s.wcat_l, 0, C, 0, pW);
     six_pairs(g);
     g.M = rows; g.N = 3 * Ci; g.K = C;
     g.bias = s.bcat;
@@ -193,14 +132,14 @@ int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void
   GLF_TRY(split3(wf.Pf, s.Pl, pP, stream));
   {  // M_b = Phi_b^T G_b / N
     GemmArgs g;
-    g.A = lop(s.Pl + Ci, 1, 3 * Ci, seqP, pP);
-    g.B = lop(s.Pl + 2 * Ci, 1, 3 * Ci, seqP, pP);
+    g.A = opnd(s.Pl + Ci, 1, 3 * Ci, seqP, pP);
+    g.B = opnd(s.Pl + 2 * Ci, 1, 3 * Ci, seqP, pP);
     six_pairs(g);
     g.M = Ci; g.N = Ci; g.K = N; g.batch = B;
     g.alpha = 1.f / static_cast<float>(N);
     g.ldd = Ci; g.strideD = CiCi;
     g.D = wf.Mf;
-    g.split_k = pick_split3(static_cast<long long>(B) * ((Ci + 127) / 128) * ((Ci + 127) / 128), N);
+    g.split_k = pick_split(static_cast<long long>(B) * ((Ci + 127) / 128) * ((Ci + 127) / 128), N);
     if (g.split_k > 1) {
       GLF_TRY(check_cuda(cudaMemsetAsync(wf.Mf, 0, sizeof(float) * pM, stream), "memset M"));
       g.out_kind = 2;
@@ -212,8 +151,8 @@ int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void
   GLF_TRY(split3(wf.Mf, s.Ml, pM, stream));
   {  // W'_b = Wz M_b^T
     GemmArgs g;
-    g.A = lop(s.wz_l, 0, Ci, 0, pWz);
-    g.B = lop(s.Ml, 0, Ci, CiCi, pM);
+    g.A = opnd(s.wz_l, 0, Ci, 0, pWz);
+    g.B = opnd(s.Ml, 0, Ci, CiCi, pM);
     six_pairs(g);
     g.M = C; g.N = Ci; g.K = Ci; g.batch = B;
     g.out_kind = 1;
@@ -223,8 +162,8 @@ int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void
   GLF_TRY(split3(wf.Wpf, s.Wpl, pWp, stream));
   {  // U_b = Theta_b W'_b^T + bz
     GemmArgs g;
-    g.A = lop(s.Pl, 0, 3 * Ci, seqP, pP);
-    g.B = lop(s.Wpl, 0, Ci, CCi, pWp);
+    g.A = opnd(s.Pl, 0, 3 * Ci, seqP, pP);
+    g.B = opnd(s.Wpl, 0, Ci, CCi, pWp);
     six_pairs(g);
     g.M = N; g.N = C; g.K = Ci; g.batch = B;
     g.bias = w->wz_b;
@@ -243,25 +182,23 @@ int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void
   return 0;
 }
 
-int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_weights* w, const void* saved,
-                    void* dx, const glf_grads* g_, void* ws, cudaStream_t stream) {
-  if (d->mode != GLF_MODE_DOT) return set_error(GLF_ERR_UNSUPPORTED, "GLF_PRECISION_F32X3 is implemented for mode='dot'");
-  const D3 m = dims(d);
+int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void* x, const glf_weights* w,
+                    const void* saved, void* dx, const glf_grads* g_, void* ws, cudaStream_t stream) {
   Saved3 s; WsB3 wb;
   carve_saved3(m, const_cast<void*>(saved), &s);
-  carve_wsb3(m, ws, &wb);
-  const int C = m.C, Ci = m.Ci, N = m.N, B = m.B, rows = m.rows;
+  carve_wsb3(d, m, ws, &wb);
+  const int C = m.C, Ci = m.Ci, N = static_cast<int>(m.N), B = static_cast<int>(m.B), rows = static_cast<int>(m.rows);
   const long long pX = static_cast<long long>(rows) * C, pP = static_cast<long long>(rows) * 3 * Ci;
   const long long pW = 3LL * Ci * C, pWz = static_cast<long long>(C) * Ci;
   const long long CiCi = static_cast<long long>(Ci) * Ci, CCi = pWz;
   const long long pM = B * CiCi, pWp = B * CCi;
   const long long seqP = static_cast<long long>(N) * 3 * Ci;
-  const float* Xf = m.x_direct ? reinterpret_cast<const float*>(x) : s.Xf;
+  const float* Xf = m.pack_x ? s.Xf : reinterpret_cast<const float*>(x);
 
   const void* dZ = dz;
   int dz_dtype = d->io_dtype;
-  if (d->dz_layout != GLF_LAYOUT_TOKEN) {
-    GLF_TRY(transpose_cast(dz, wb.dZf, B, C, N, d->io_dtype, GLF_DTYPE_F32, stream));
+  if (m.pack_dz) {
+    GLF_TRY(pack_tokens(m, dz, d->io_dtype, /*ncthw=*/true, wb.dZf, GLF_DTYPE_F32, stream));
     dZ = wb.dZf;
     dz_dtype = GLF_DTYPE_F32;
   }
@@ -278,8 +215,8 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   GLF_TRY(split3(dUf, wb.dUl, pX, stream));
   {  // dTheta_b = dU_b W'_b
     GemmArgs g;
-    g.A = lop(wb.dUl, 0, C, static_cast<long long>(N) * C, pX);
-    g.B = lop(s.Wpl, 1, Ci, CCi, pWp);
+    g.A = opnd(wb.dUl, 0, C, static_cast<long long>(N) * C, pX);
+    g.B = opnd(s.Wpl, 1, Ci, CCi, pWp);
     six_pairs(g);
     g.M = N; g.N = Ci; g.K = C; g.batch = B;
     g.out_kind = 1;
@@ -288,13 +225,13 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   }
   {  // dW'_b = dU_b^T Theta_b
     GemmArgs g;
-    g.A = lop(wb.dUl, 1, C, static_cast<long long>(N) * C, pX);
-    g.B = lop(s.Pl, 1, 3 * Ci, seqP, pP);
+    g.A = opnd(wb.dUl, 1, C, static_cast<long long>(N) * C, pX);
+    g.B = opnd(s.Pl, 1, 3 * Ci, seqP, pP);
     six_pairs(g);
     g.M = C; g.N = Ci; g.K = N; g.batch = B;
     g.ldd = Ci; g.strideD = CCi;
     g.D = wb.dWpf;
-    g.split_k = pick_split3(static_cast<long long>(B) * ((C + 127) / 128) * ((Ci + 127) / 128), N);
+    g.split_k = pick_split(static_cast<long long>(B) * ((C + 127) / 128) * ((Ci + 127) / 128), N);
     if (g.split_k > 1) {
       GLF_TRY(check_cuda(cudaMemsetAsync(wb.dWpf, 0, sizeof(float) * pWp, stream), "memset dW'"));
       g.out_kind = 2;
@@ -307,8 +244,8 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   GLF_TRY(check_cuda(cudaMemsetAsync(g_->wz_w, 0, sizeof(float) * CCi, stream), "memset dWz"));
   {  // dWz = sum_b dW'_b M_b
     GemmArgs g;
-    g.A = lop(wb.dWpl, 0, Ci, CCi, pWp);
-    g.B = lop(s.Ml, 1, Ci, CiCi, pM);
+    g.A = opnd(wb.dWpl, 0, Ci, CCi, pWp);
+    g.B = opnd(s.Ml, 1, Ci, CiCi, pM);
     six_pairs(g);
     g.M = C; g.N = Ci; g.K = Ci; g.batch = B;
     g.out_kind = 2;
@@ -317,8 +254,8 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   }
   {  // dM_b = dW'_b^T Wz
     GemmArgs g;
-    g.A = lop(wb.dWpl, 1, Ci, CCi, pWp);
-    g.B = lop(s.wz_l, 1, Ci, 0, pWz);
+    g.A = opnd(wb.dWpl, 1, Ci, CCi, pWp);
+    g.B = opnd(s.wz_l, 1, Ci, 0, pWz);
     six_pairs(g);
     g.M = Ci; g.N = Ci; g.K = C; g.batch = B;
     g.out_kind = 1;
@@ -328,8 +265,8 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   GLF_TRY(split3(wb.dMf, wb.dMl, pM, stream));
   {  // dPhi_b = G_b dM_b^T / N
     GemmArgs g;
-    g.A = lop(s.Pl + 2 * Ci, 0, 3 * Ci, seqP, pP);
-    g.B = lop(wb.dMl, 0, Ci, CiCi, pM);
+    g.A = opnd(s.Pl + 2 * Ci, 0, 3 * Ci, seqP, pP);
+    g.B = opnd(wb.dMl, 0, Ci, CiCi, pM);
     six_pairs(g);
     g.M = N; g.N = Ci; g.K = Ci; g.batch = B;
     g.alpha = 1.f / static_cast<float>(N);
@@ -339,8 +276,8 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   }
   {  // dG_b = Phi_b dM_b / N
     GemmArgs g;
-    g.A = lop(s.Pl + Ci, 0, 3 * Ci, seqP, pP);
-    g.B = lop(wb.dMl, 1, Ci, CiCi, pM);
+    g.A = opnd(s.Pl + Ci, 0, 3 * Ci, seqP, pP);
+    g.B = opnd(wb.dMl, 1, Ci, CiCi, pM);
     six_pairs(g);
     g.M = N; g.N = Ci; g.K = Ci; g.batch = B;
     g.alpha = 1.f / static_cast<float>(N);
@@ -358,36 +295,29 @@ int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_
   GLF_TRY(check_cuda(cudaMemsetAsync(wb.dwcat, 0, sizeof(float) * pW, stream), "memset dWcat"));
   {  // dWcat = dP^T X
     GemmArgs g;
-    g.A = lop(wb.dPl, 1, 3 * Ci, 0, pP);
-    g.B = lop(s.Xl, 1, C, 0, pX);
+    g.A = opnd(wb.dPl, 1, 3 * Ci, 0, pP);
+    g.B = opnd(s.Xl, 1, C, 0, pX);
     six_pairs(g);
     g.M = 3 * Ci; g.N = C; g.K = rows;
     g.out_kind = 2;
     g.D = wb.dwcat; g.ldd = C;
-    g.split_k = pick_split3(static_cast<long long>((3 * Ci + 127) / 128) * ((C + 127) / 128), rows);
+    g.split_k = pick_split(static_cast<long long>((3 * Ci + 127) / 128) * ((C + 127) / 128), rows);
     GLF_TRY(gemm(g, stream));
   }
-  const size_t wbytes = sizeof(float) * Ci * C;
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->theta_w, wb.dwcat, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dtheta"));
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->phi_w, wb.dwcat + static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dphi"));
-  GLF_TRY(check_cuda(cudaMemcpyAsync(g_->g_w, wb.dwcat + 2 * static_cast<size_t>(Ci) * C, wbytes, cudaMemcpyDeviceToDevice, stream), "copy dg"));
+  GLF_TRY(scatter_proj_grads(wb.dwcat, g_, C, Ci, false, stream));
   {  // dX = dV + dP Wcat : the output is initialised with dV and the product is accumulated onto it (fp32 red.add)
-    float* dXf = m.dx_direct ? reinterpret_cast<float*>(dx) : wb.dXf;
+    float* dXf = m.pack_x ? wb.dXf : reinterpret_cast<float*>(dx);
     GLF_TRY(check_cuda(cudaMemcpyAsync(dXf, wb.dVf, sizeof(float) * pX, cudaMemcpyDeviceToDevice, stream), "copy dV"));
     GemmArgs g;
-    g.A = lop(wb.dPl, 0, 3 * Ci, 0, pP);
-    g.B = lop(s.wcatT_l, 0, 3 * Ci, 0, pW);
+    g.A = opnd(wb.dPl, 0, 3 * Ci, 0, pP);
+    g.B = opnd(s.wcatT_l, 0, 3 * Ci, 0, pW);
     six_pairs(g);
     g.M = rows; g.N = C; g.K = 3 * Ci;
     g.out_kind = 2;
     g.D = dXf; g.ldd = C;
     GLF_TRY(gemm(g, stream));
-    if (!m.dx_direct) {
-      if (d->x_layout == GLF_LAYOUT_NCTHW)
-        GLF_TRY(transpose_cast(dXf, dx, B, N, C, GLF_DTYPE_F32, d->io_dtype, stream));
-      else
-        GLF_TRY(transpose_cast(dXf, dx, 1, 1, static_cast<int>(pX), GLF_DTYPE_F32, d->io_dtype, stream));
-    }
+    if (m.pack_x)
+      GLF_TRY(unpack_tokens(m, dXf, GLF_DTYPE_F32, dx, d->x_layout == GLF_LAYOUT_NCTHW, d->io_dtype, stream));
   }
   return 0;
 }

@@ -31,12 +31,6 @@ namespace glf {
 
 namespace {
 
-#define GLF_TRY_RC(expr)        \
-  do {                          \
-    int rc__ = (expr);          \
-    if (rc__ != 0) return rc__; \
-  } while (0)
-
 constexpr int CC = 256;              // channels
 constexpr int CI = 128;              // inter channels
 constexpr int CA = 264;              // augmented leading dimension (gram_ca(256))
@@ -859,13 +853,13 @@ int gram_chain_fwd(const bf16* Sa, const float* sfv, const bf16* waug, const bf1
                    const float* bg, const float* bth, bf16* T, bf16* Mb, bf16* Wp, bf16* Qb, float* cvec, float* tv, int B,
                    int N, cudaStream_t stream) {
   CUtensorMap tmS, tmW, tmWz, tmT, tmM, tmWp, tmQ;
-  GLF_TRY_RC(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmW, waug, CC, 3 * CI, 1, CA, 0, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmWz, wz, CI, CC, 1, CI, 0, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmT, T, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmM, Mb, CI, CI, B, CI, static_cast<long long>(CI) * CI, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmWp, Wp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmQ, Qb, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmW, waug, CC, 3 * CI, 1, CA, 0, 128));
+  GLF_TRY(make_tmap_bf16(&tmWz, wz, CI, CC, 1, CI, 0, 128));
+  GLF_TRY(make_tmap_bf16(&tmT, T, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmM, Mb, CI, CI, B, CI, static_cast<long long>(CI) * CI, 128));
+  GLF_TRY(make_tmap_bf16(&tmWp, Wp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
+  GLF_TRY(make_tmap_bf16(&tmQ, Qb, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
   ChainFwdParams p;
   p.N = N;
   p.sfv = sfv; p.bphi = bphi; p.bg = bg; p.bth = bth;
@@ -881,17 +875,17 @@ int gram_chain_bwd(const bf16* Sa, const bf16* Qb, const bf16* waug, const bf16*
                    const float* bth, const float* bphi, const float* bg, int has_k2, bf16* dQa, bf16* dWp, bf16* dMn,
                    bf16* dT, bf16* EF, float* evec, float* dcv, float* dtv, int B, int N, cudaStream_t stream) {
   CUtensorMap tmS, tmQ, tmW, tmWz;
-  GLF_TRY_RC(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmQ, Qb, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmW, waug, CC, 3 * CI, 1, CA, 0, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmWz, wz, CI, CC, 1, CI, 0, 128));
+  GLF_TRY(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmQ, Qb, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmW, waug, CC, 3 * CI, 1, CA, 0, 128));
+  GLF_TRY(make_tmap_bf16(&tmWz, wz, CI, CC, 1, CI, 0, 128));
   CUtensorMap tmdQ, tmdWp, tmdM, tmdT, tmEF, tmR;
-  GLF_TRY_RC(make_tmap_bf16(&tmR, Rb, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmdQ, dQa, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmdWp, dWp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmdM, dMn, CI, CI, B, CI, static_cast<long long>(CI) * CI, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmdT, dT, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmEF, EF, CC, 2 * CC, B, CC, 2LL * CC * CC, 128));
+  GLF_TRY(make_tmap_bf16(&tmR, Rb, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmdQ, dQa, CC, CC, B, CA, static_cast<long long>(CC) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmdWp, dWp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
+  GLF_TRY(make_tmap_bf16(&tmdM, dMn, CI, CI, B, CI, static_cast<long long>(CI) * CI, 128));
+  GLF_TRY(make_tmap_bf16(&tmdT, dT, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmEF, EF, CC, 2 * CC, B, CC, 2LL * CC * CC, 128));
   ChainBwdParams p;
   p.N = N; p.has_k2 = has_k2;
   const char* tr = getenv("GLF_CHAIN_TRACE");

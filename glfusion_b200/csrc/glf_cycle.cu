@@ -14,12 +14,6 @@
 
 #include "glf_internal.h"
 
-#define GLF_TRY(expr)           \
-  do {                          \
-    int rc__ = (expr);          \
-    if (rc__ != 0) return rc__; \
-  } while (0)
-
 namespace glf {
 
 namespace {

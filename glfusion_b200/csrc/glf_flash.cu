@@ -90,12 +90,6 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-GemmOperand op(const void* p, int mn, long long ld, long long bs) {
-  GemmOperand o;
-  o.ptr = p; o.mn_major = mn; o.ld = ld; o.batch_stride = bs;
-  return o;
-}
-
 
 }  // namespace
 
@@ -885,8 +879,8 @@ static int attn_fwd_materialized(const AttnArgs& a, bf16* Y, float* lse, int B, 
     const bf16* Vb = a.v + b0 * n * a.ldv;
     {  // S = Q K^T   (columns [N, ld) come out as zeros: K rows beyond N are TMA out-of-bounds)
       GemmArgs g;
-      g.A = op(Qb, 0, a.ldq, n * a.ldq);
-      g.B = op(Kb, 0, a.ldk, n * a.ldk);
+      g.A = opnd(Qb, 0, a.ldq, n * a.ldq);
+      g.B = opnd(Kb, 0, a.ldk, n * a.ldk);
       g.B.rows = N;
       g.M = N; g.N = ld; g.K = a.wqk; g.batch = cb;
       g.out_kind = 1;
@@ -900,8 +894,8 @@ static int attn_fwd_materialized(const AttnArgs& a, bf16* Y, float* lse, int B, 
     if (rc) return rc;
     {  // Y = P V
       GemmArgs g;
-      g.A = op(Pm, 0, ld, static_cast<long long>(per));
-      g.B = op(Vb, 1, a.ldv, n * a.ldv);
+      g.A = opnd(Pm, 0, ld, static_cast<long long>(per));
+      g.B = opnd(Vb, 1, a.ldv, n * a.ldv);
       g.M = N; g.N = a.wv; g.K = N; g.batch = cb;
       g.D = Y + b0 * n * a.wv; g.ldd = a.wv; g.strideD = n * a.wv;
       rc = gemm(g, stream);
@@ -923,7 +917,7 @@ int flash_fwd(const bf16* P3, bf16* Y, float* lse, int B, int N, int Ci, void* s
 }
 
 static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta,
-                                 float* cs_t, float* cs_p, float* cs_g, int cs_rows_out[3], int B, int N,
+                                 float* cs_t, float* cs_p, float* cs_g, ColTables* cs, int B, int N,
                                  void* scratch, cudaStream_t stream) {
   const int ld = attn_ld(N);
   const int nb = attn_chunk(B, N);
@@ -956,8 +950,8 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     int rc;
     {  // S = Q K^T (recompute)
       GemmArgs g;
-      g.A = op(Qb, 0, a.ldq, n * a.ldq);
-      g.B = op(Kb, 0, a.ldk, n * a.ldk);
+      g.A = opnd(Qb, 0, a.ldq, n * a.ldq);
+      g.B = opnd(Kb, 0, a.ldk, n * a.ldk);
       g.B.rows = N;
       g.M = N; g.N = ld; g.K = a.wqk; g.batch = cb;
       g.out_kind = 1;
@@ -966,8 +960,8 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     }
     {  // dPm = dY V^T
       GemmArgs g;
-      g.A = op(dYb, 0, a.wv, n * a.wv);
-      g.B = op(Vb, 0, a.ldv, n * a.ldv);
+      g.A = opnd(dYb, 0, a.wv, n * a.wv);
+      g.B = opnd(Vb, 0, a.ldv, n * a.ldv);
       g.B.rows = N;
       g.M = N; g.N = ld; g.K = a.wv; g.batch = cb;
       g.out_kind = 1;
@@ -993,8 +987,8 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     }
     {  // dQ = dS K
       GemmArgs g;
-      g.A = op(dS, 0, ld, static_cast<long long>(per));
-      g.B = op(Kb, 1, a.ldk, n * a.ldk);
+      g.A = opnd(dS, 0, ld, static_cast<long long>(per));
+      g.B = opnd(Kb, 1, a.ldk, n * a.ldk);
       g.M = N; g.N = a.wqk; g.K = N; g.batch = cb;
       g.D = a.dq + b0 * n * a.ld_dq; g.ldd = a.ld_dq; g.strideD = n * a.ld_dq;
       if (cs_t != nullptr) {
@@ -1005,8 +999,8 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     }
     {  // dK = dS^T Q
       GemmArgs g;
-      g.A = op(dS, 1, ld, static_cast<long long>(per));
-      g.B = op(Qb, 1, a.ldq, n * a.ldq);
+      g.A = opnd(dS, 1, ld, static_cast<long long>(per));
+      g.B = opnd(Qb, 1, a.ldq, n * a.ldq);
       g.M = N; g.N = a.wqk; g.K = N; g.batch = cb;
       g.D = a.dk + b0 * n * a.ld_dk; g.ldd = a.ld_dk; g.strideD = n * a.ld_dk;
       if (cs_p != nullptr) {
@@ -1017,8 +1011,8 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     }
     {  // dV = P^T dY
       GemmArgs g;
-      g.A = op(Pm, 1, ld, static_cast<long long>(per));
-      g.B = op(dYb, 1, a.wv, n * a.wv);
+      g.A = opnd(Pm, 1, ld, static_cast<long long>(per));
+      g.B = opnd(dYb, 1, a.wv, n * a.wv);
       g.M = N; g.N = a.wv; g.K = N; g.batch = cb;
       g.D = a.dvo + b0 * n * a.ld_dv; g.ldd = a.ld_dv; g.strideD = n * a.ld_dv;
       g.colstats = cs_g + static_cast<long long>(cs_rows_total[2]) * 2 * a.wv;
@@ -1029,7 +1023,17 @@ static int attn_bwd_materialized(const AttnArgs& a, const bf16* Y, const bf16* d
     cs_rows_total[1] += r_p;
     cs_rows_total[2] += r_g;
   }
-  for (int i = 0; i < 3; ++i) cs_rows_out[i] = cs_rows_total[i];
+  // (embedded: wqk = wv, so the three tables share the row stride 2 wv)
+  if (a.bias_qkv) {
+    cs->n = 3;
+    cs->tab[0] = cs_t; cs->tab[1] = cs_p; cs->tab[2] = cs_g;
+    for (int i = 0; i < 3; ++i) cs->rows[i] = cs_rows_total[i];
+  } else {
+    cs->n = 1;
+    cs->tab[0] = cs_g;
+    cs->rows[0] = cs_rows_total[2];
+  }
+  cs->stride = 2LL * a.wv;
   return 0;
 }
 
@@ -1039,9 +1043,9 @@ int flash_bwd_colsum_blocks(long long rows) {
 }
 
 int attn_bwd(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta, float* cs_t, float* cs_p,
-             float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, void* scratch, cudaStream_t stream) {
+             float* cs_g, int cs_cap_rows, ColTables* cs, int B, int N, void* scratch, cudaStream_t stream) {
   if (!attn_flash_supported(a.wqk, a.wv))   // other widths: exact chunked path
-    return attn_bwd_materialized(a, Y, dY, lse, delta, cs_t, cs_p, cs_g, cs_rows_out, B, N, scratch, stream);
+    return attn_bwd_materialized(a, Y, dY, lse, delta, cs_t, cs_p, cs_g, cs, B, N, scratch, stream);
   const long long rows = static_cast<long long>(B) * N;
   {
     const long long threads = rows * 32;
@@ -1055,29 +1059,35 @@ int attn_bwd(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse,
   if (rc) return rc;
   int grid = flash_bwd_colsum_blocks(rows);
   if (a.bias_qkv) {
-    // bias gradients: column sums of dP3 = [dTheta | dPhi | dG]; one table [grid][2][3Ci] written into cs_t, the
-    // caller's three reductions address it with a row stride of 2*3Ci through the offsets below (cs_p / cs_g are unused
-    // here)
+    // bias gradients: column sums of dP3 = [dTheta | dPhi | dG] in one pass, a [grid][2][3Ci] table in cs_t whose
+    // column slices are the three tables (cs_p / cs_g are unused here)
     if (grid > cs_cap_rows / 3) grid = cs_cap_rows / 3 > 0 ? cs_cap_rows / 3 : 1;   // cs_t holds cs_cap_rows x 2 x Ci floats
     colsum_bf16_kernel<<<grid, 256, 0, stream>>>(a.dq, cs_t, rows, 3 * a.wv, 3LL * a.wv);
     if ((rc = check_cuda(cudaGetLastError(), "colsum launch"))) return rc;
-    cs_rows_out[0] = cs_rows_out[1] = cs_rows_out[2] = -grid;   // negative: "single table of width 3Ci" (see glf_tpavi_bwd)
+    cs->n = 3;
+    for (int i = 0; i < 3; ++i) {
+      cs->tab[i] = cs_t + i * a.wv;
+      cs->rows[i] = grid;
+    }
+    cs->stride = 2LL * 3 * a.wv;
     return 0;
   }
   // column sums of dV alone: a table [grid][2][DV] in cs_g
   if (grid > cs_cap_rows) grid = cs_cap_rows > 0 ? cs_cap_rows : 1;
   colsum_bf16_kernel<<<grid, 256, 0, stream>>>(a.dvo, cs_g, rows, a.wv, a.ld_dv);
   if ((rc = check_cuda(cudaGetLastError(), "colsum launch"))) return rc;
-  cs_rows_out[0] = cs_rows_out[1] = 0;
-  cs_rows_out[2] = grid;
+  cs->n = 1;
+  cs->tab[0] = cs_g;
+  cs->rows[0] = grid;
+  cs->stride = 2LL * a.wv;
   return 0;
 }
 
 int flash_bwd(const bf16* P3, const bf16* Y, const bf16* dY, const float* lse, bf16* dP3, float* delta, float* cs_t,
-              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
+              float* cs_p, float* cs_g, int cs_cap_rows, ColTables* cs, int B, int N, int Ci, void* scratch,
               cudaStream_t stream) {
-  return attn_bwd(attn_args_embedded(P3, dP3, Ci), Y, dY, lse, delta, cs_t, cs_p, cs_g, cs_cap_rows, cs_rows_out, B, N,
-                  scratch, stream);
+  return attn_bwd(attn_args_embedded(P3, dP3, Ci), Y, dY, lse, delta, cs_t, cs_p, cs_g, cs_cap_rows, cs, B, N, scratch,
+                  stream);
 }
 
 // out[r, c] = in[r, c] + in[r, C + c] over rows of 2C bf16 (fp32 sum, one rounding): dS X + dS^T X of mode='gaussian'

@@ -17,6 +17,27 @@ int check_device_sm100();                        // 0 or GLF_ERR_DEVICE
 using bf16 = __nv_bfloat16;
 using f16 = __half;        // I/O-only element type (GLF_DTYPE_F16): converted to bf16 / fp32 where it is read
 
+#define GLF_TRY(expr)           \
+  do {                          \
+    int rc__ = (expr);          \
+    if (rc__ != 0) return rc__; \
+  } while (0)
+
+// Hands out 256-byte aligned pieces of one caller-provided blob in a fixed order; with a NULL base every piece is NULL
+// and `off` ends as the blob's size.
+struct Carver {
+  uint8_t* base;
+  size_t off = 0;
+  explicit Carver(void* b) : base(reinterpret_cast<uint8_t*>(b)) {}
+  template <typename T>
+  T* take(size_t n) {
+    off = (off + 255) & ~static_cast<size_t>(255);
+    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off += n * sizeof(T);
+    return p;
+  }
+};
+
 // ------------------------------------------------------------------------------------------------ GEMM
 struct GemmOperand {
   const void* ptr = nullptr;
@@ -50,6 +71,20 @@ struct GemmArgs {
 };
 int gemm(const GemmArgs& a, cudaStream_t stream);
 inline int gemm_tiles_m(int M) { return (M + 127) / 128; }
+inline GemmOperand opnd(const void* p, int mn, long long ld, long long bs, long long limb_stride = 0) {
+  GemmOperand o;
+  o.ptr = p; o.mn_major = mn; o.ld = ld; o.batch_stride = bs; o.limb_stride = limb_stride;
+  return o;
+}
+// Split-K of a product with `tiles` output tiles and K = `K`
+inline int pick_split(long long tiles, int K) {
+  const int kb = (K + 63) / 64;
+  if (tiles >= 96) return 1;  // enough CTAs already: write the result directly, no atomics
+  long long s = (2 * 148) / tiles;   // floor: tiles * s work items fill at most two full rounds of the 148 persistent CTAs
+  if (s < 1) s = 1;
+  if (s > kb) s = kb;
+  return static_cast<int>(s);
+}
 // (glf_gemm.cu) operand map: K-major -> dims {K, rows, batch, limb}, MN-major -> {rows, K, batch, limb}; SWIZZLE_128B,
 // box {64, box_rows or 64}.  Output map: dims {N, M, batch}, box {32, 32}, SWIZZLE_64B (the epilogue's staging tile).
 int make_operand_tmap(CUtensorMap* tm, const GemmOperand& op, int rows, int K, int batch, int nlimbs, int box_rows);
@@ -218,10 +253,17 @@ int attn_ld(int N);
 int attn_chunk(long long B, long long N);
 size_t attn_scratch_bytes(long long B, long long N, bool backward);
 int flash_fwd(const bf16* P, bf16* Y, float* lse, int B, int N, int Ci, void* scratch, cudaStream_t stream);
-// cs_rows_out[i] > 0: rows of the three tables [rows][2][Ci] (cs_t, cs_p, cs_g);  < 0 (all three): one table
-// [-rows][2][3Ci] in cs_t
+// Partial column sums of the outputs that carry a bias: table i holds rows[i] rows of [2][width] floats at tab[i] (the
+// sums first), consecutive rows `stride` floats apart in every table of the set.
+struct ColTables {
+  int n = 0;
+  const float* tab[3] = {nullptr, nullptr, nullptr};
+  int rows[3] = {0, 0, 0};
+  long long stride = 0;
+};
+// cs: the column sums of dP = [dTheta | dPhi | dG], three tables
 int flash_bwd(const bf16* P, const bf16* Y, const bf16* dY, const float* lse, bf16* dP, float* delta, float* cs_t,
-              float* cs_p, float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, int Ci, void* scratch,
+              float* cs_p, float* cs_g, int cs_cap_rows, ColTables* cs, int B, int N, int Ci, void* scratch,
               cudaStream_t stream);
 // The same attention with Q, K and V given separately: Y = softmax(Q K^T) V per sequence, Q / K of width wqk, V / Y / dY
 // of width wv, every operand token rows with its own leading dimension.  mode='embedded' is Q = Theta, K = Phi, V = G
@@ -240,9 +282,10 @@ AttnArgs attn_args_gaussian(const bf16* X, const bf16* G, bf16* dXa, bf16* dXb, 
                             long long ld_dg, int C, int Ci);
 bool attn_flash_supported(int wqk, int wv);
 int attn_fwd(const AttnArgs& a, bf16* Y, float* lse, int B, int N, void* scratch, cudaStream_t stream);
-// bias_qkv: cs_rows_out as flash_bwd;  otherwise cs_rows_out[2] > 0 rows of one table [rows][2][wv] in cs_g
+// cs: the column sums of [dQ | dK | dV] (bias_qkv, three tables) or of dV alone (one table), written into the
+// cs_t / cs_p / cs_g scratch (cs_cap_rows rows of [2][width] each)
 int attn_bwd(const AttnArgs& a, const bf16* Y, const bf16* dY, const float* lse, float* delta, float* cs_t, float* cs_p,
-             float* cs_g, int cs_cap_rows, int cs_rows_out[3], int B, int N, void* scratch, cudaStream_t stream);
+             float* cs_g, int cs_cap_rows, ColTables* cs, int B, int N, void* scratch, cudaStream_t stream);
 // out [rows, C] = in[:, :C] + in[:, C:2C] for in [rows, 2C] bf16 (fp32 sum, rounded once)
 int sum_halves(const bf16* in, bf16* out, long long rows, int C, cudaStream_t stream);
 // mode='gaussian' weights: wg [Ci, C] = bf16(g.weight), bg [Ci] = g.bias, wgT [C, 2C + Ci] = [I | I | g.weight^T] (the dX
@@ -260,11 +303,35 @@ int p2p_export(const void* ptr, unsigned char handle[64], unsigned long long* of
 int p2p_open(const unsigned char handle[64], unsigned long long offset, void** out);
 int p2p_close(void* ptr, unsigned long long offset);
 
+// ------------------------------------------------------------------------------------------------ TPAVIModule (glf_api.cu)
+// One block's problem, validated and derived from its glf_desc by make_dims.
+struct Dims {
+  long long B, N, rows;
+  int C, Ci;
+  int tiles_seq;   // m-tiles per sequence (128 tokens)
+  int tiles_all;   // m-tiles over all rows
+  bool pack_x;     // x must be repacked to token-major in the working dtype (bf16, or fp32 under F32X3)
+  bool pack_dz;
+  bool dot;
+  bool gauss;      // mode='gaussian': Q = K = X, only the g projection runs
+  bool gram;       // mode='dot' in its Gram form (channel-space products only)
+  int Ca;          // augmented width of the per-sequence matrices (gram)
+  int pdt;         // GLF_DTYPE_* of the glf_weights / glf_grads tensors (glf_desc.reserved[3])
+  bool half_params;   // bf16 / fp16 parameters: an fp32 shadow in `saved`, fp32 gradient staging in ws_bwd
+};
+// x / dz (in_dtype, [B, C, N] when ncthw, else token-major) -> token-major [B * N, C] of out_dtype;
+// unpack_tokens is the way back for dx
+int pack_tokens(const Dims& m, const void* in, int in_dtype, bool ncthw, void* out, int out_dtype, cudaStream_t stream);
+int unpack_tokens(const Dims& m, const void* in, int in_dtype, void* out, bool ncthw, int out_dtype,
+                  cudaStream_t stream);
+// dWcat = [dtheta_w ; dphi_w ; dg_w] (Ci x C each), or dg_w alone (g_only), into the gradient tensors
+int scatter_proj_grads(const float* dwcat, const glf_grads* g, int C, int Ci, bool g_only, cudaStream_t stream);
+
 // ------------------------------------------------------------------------------------------------ F32X3 precision arm
-int tpavi_sizes_f32x3(const glf_desc* d, glf_sizes* out);
-int tpavi_fwd_f32x3(const glf_desc* d, const void* x, const glf_weights* w, void* z, void* saved, void* ws,
-                    cudaStream_t stream);
-int tpavi_bwd_f32x3(const glf_desc* d, const void* dz, const void* x, const glf_weights* w, const void* saved,
-                    void* dx, const glf_grads* g, void* ws, cudaStream_t stream);
+int tpavi_sizes_f32x3(const glf_desc* d, const Dims& m, glf_sizes* out);
+int tpavi_fwd_f32x3(const glf_desc* d, const Dims& m, const void* x, const glf_weights* w, void* z, void* saved,
+                    void* ws, cudaStream_t stream);
+int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void* x, const glf_weights* w,
+                    const void* saved, void* dx, const glf_grads* g, void* ws, cudaStream_t stream);
 
 }  // namespace glf

@@ -23,12 +23,6 @@ namespace glf {
 
 namespace {
 
-#define GLF_TRY_RC(expr)        \
-  do {                          \
-    int rc__ = (expr);          \
-    if (rc__ != 0) return rc__; \
-  } while (0)
-
 constexpr int CC = 256, CI = 128, CA = 264;
 constexpr int WG_THREADS = 64 + 256;           // warp 0 TMA, warp 1 MMA, warps 2..9 SIMT / epilogue
 constexpr int WG_STAGES = 4;
@@ -342,14 +336,14 @@ int gram_wgrad(const bf16* Wp, const bf16* dQa, const bf16* dWp, const bf16* Mb,
                const bf16* dT, const bf16* Sa, const float* dcv, const float* tv, const float* dtv, const float* sfv,
                float* part, const glf_grads* g, int B, int N, cudaStream_t stream) {
   CUtensorMap tmWp, tmdQ, tmdWp, tmM, tmdM, tmT, tmdT, tmS;
-  GLF_TRY_RC(make_tmap_bf16(&tmWp, Wp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 64));
-  GLF_TRY_RC(make_tmap_bf16(&tmdQ, dQa, CC, CC, B, CA, static_cast<long long>(CC) * CA, 64));
-  GLF_TRY_RC(make_tmap_bf16(&tmdWp, dWp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmM, Mb, CI, CI, B, CI, static_cast<long long>(CI) * CI, 64));
-  GLF_TRY_RC(make_tmap_bf16(&tmdM, dMn, CI, CI, B, CI, static_cast<long long>(CI) * CI, 64));
-  GLF_TRY_RC(make_tmap_bf16(&tmT, T, CC, CI, B, CA, static_cast<long long>(CI) * CA, 64));
-  GLF_TRY_RC(make_tmap_bf16(&tmdT, dT, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
-  GLF_TRY_RC(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmWp, Wp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 64));
+  GLF_TRY(make_tmap_bf16(&tmdQ, dQa, CC, CC, B, CA, static_cast<long long>(CC) * CA, 64));
+  GLF_TRY(make_tmap_bf16(&tmdWp, dWp, CI, CC, B, CI, static_cast<long long>(CC) * CI, 128));
+  GLF_TRY(make_tmap_bf16(&tmM, Mb, CI, CI, B, CI, static_cast<long long>(CI) * CI, 64));
+  GLF_TRY(make_tmap_bf16(&tmdM, dMn, CI, CI, B, CI, static_cast<long long>(CI) * CI, 64));
+  GLF_TRY(make_tmap_bf16(&tmT, T, CC, CI, B, CA, static_cast<long long>(CI) * CA, 64));
+  GLF_TRY(make_tmap_bf16(&tmdT, dT, CC, CI, B, CA, static_cast<long long>(CI) * CA, 128));
+  GLF_TRY(make_tmap_bf16(&tmS, Sa, CC, CC, B, CA, static_cast<long long>(CA) * CA, 128));
   int dev = 0, num_sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess ||
       cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || num_sms <= 0)
@@ -387,7 +381,7 @@ int gram_wgrad(const bf16* Wp, const bf16* dQa, const bf16* dWp, const bf16* Mb,
   cudaError_t e = cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(wgrad)");
   wgrad_kernel<<<p.cta0[4], WG_THREADS, WG_SMEM, stream>>>(tmWp, tmdQ, tmdWp, tmM, tmdM, tmT, tmdT, tmS, p);
-  GLF_TRY_RC(check_cuda(cudaGetLastError(), "wgrad launch"));
+  GLF_TRY(check_cuda(cudaGetLastError(), "wgrad launch"));
   if (p.trace) {
     long long t[4][8];
     cudaStreamSynchronize(stream);
