@@ -15,6 +15,7 @@ LAYOUT_NCTHW, LAYOUT_TOKEN = 0, 1
 PRECISION_BF16, PRECISION_F32X3 = 0, 1
 PRECISIONS = {"bf16": PRECISION_BF16, "fp32": PRECISION_F32X3}
 PARAMS_F32, PARAMS_BF16, PARAMS_F16 = 0, 1, 2      # glf_desc.reserved[3]: dtype of the parameter tensors
+DETERMINISTIC = 0x100      # ORed into glf_desc.reserved[1]: fixed-order split reductions (bitwise reproducible)
 
 EXPORTS = ("glf_version", "glf_last_error", "glf_tpavi_sizes", "glf_tpavi_fwd", "glf_tpavi_bwd",
            "glf_gate_concat_fwd", "glf_gate_concat_bwd", "glf_gate_concat_cl_fwd", "glf_gate_concat_cl_bwd",

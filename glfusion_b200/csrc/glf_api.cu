@@ -115,10 +115,14 @@ int make_dims(const glf_desc* d, Dims* o) {
   o->pack_dz = d->dz_layout != GLF_LAYOUT_TOKEN;
   o->dot = d->mode == GLF_MODE_DOT;
   o->gauss = d->mode == GLF_MODE_GAUSSIAN;
-  // reserved[1]: 0 = choose, 1 = token-space form (theta/phi/g per token), 2 = Gram form
-  if (d->reserved[1] < 0 || d->reserved[1] > 2) return set_error(GLF_ERR_INVALID, "reserved[1] (dot algorithm) must be 0, 1 or 2");
+  // reserved[1]: 0 = choose, 1 = token-space form (theta/phi/g per token), 2 = Gram form; | GLF_DETERMINISTIC
+  const int algo = d->reserved[1] & 0xff, flags = d->reserved[1] & ~0xff;
+  if (algo > 2 || (flags != 0 && flags != GLF_DETERMINISTIC))
+    return set_error(GLF_ERR_INVALID, "reserved[1] must be the dot algorithm 0, 1 or 2, optionally ORed with "
+                                      "GLF_DETERMINISTIC (0x100) (got 0x%x)", static_cast<unsigned>(d->reserved[1]));
+  o->det = flags == GLF_DETERMINISTIC;
   const bool gram_ok = o->dot && d->precision == GLF_PRECISION_BF16 && o->B <= 65535;
-  if (d->reserved[1] == 2 && !gram_ok)
+  if (algo == 2 && !gram_ok)
     return set_error(GLF_ERR_UNSUPPORTED, "the Gram form needs mode='dot', GLF_PRECISION_BF16 and B <= 65535");
   // per-sequence [C x C] products cost ~15 C^3 against 3.5 N C^2 of saved token-space FLOPs and 11 saved activation
   // passes.  Measured crossover on B200 (profiles/algo_crossover.py, r02_algo_crossover.txt): with the one-CTA-per-
@@ -126,7 +130,7 @@ int make_dims(const glf_desc* d, Dims* o) {
   // at C = 128 between 3 and 24; above C = 256 the token-space form (every GEMM on CTA pairs) still wins at N/C = 6
   // (C = 512: 1.37 vs 1.46 ms; C = 1024: 1.85 vs 1.96 ms).
   const long long thr = gram_chain_supported(d->C, d->Ci) ? 3 : (d->C > 256 ? 8 : 5);
-  o->gram = gram_ok && (d->reserved[1] == 2 || (d->reserved[1] == 0 && o->N >= thr * d->C));
+  o->gram = gram_ok && (algo == 2 || (algo == 0 && o->N >= thr * d->C));
   o->Ca = gram_ca(d->C);
   return 0;
 }
@@ -281,7 +285,51 @@ LnPair ln_pair(const Dims& m, const void* xg, const void* xl, const glf_weights*
   return p;
 }
 
-struct WsFwd { float* colstats; float* red1; float* Mf; void* attn; void* saved_fallback; float* Sf; };
+int pick_split_rounds(long long M, long long N, long long batch, int K);
+// K slices of the one-CTA-per-sequence token contraction: few long sequences are split to fill two rounds of the SMs
+int gram_ksplit(long long B) { return B < 96 ? ((2 * 148) / B < 1 ? 1 : static_cast<int>((2 * 148) / B)) : 1; }
+
+// Slab floats of the fixed-order split reductions (GLF_DETERMINISTIC): the largest need among the products of the
+// forward (or backward) that sum partials, with the splits those products pick
+long long det_slab_floats(const Dims& m, bool backward) {
+  const int B = static_cast<int>(m.B), C = m.C, Ci = m.Ci, N = static_cast<int>(m.N), rows = static_cast<int>(m.rows);
+  auto t = [](long long n) { return (n + 127) / 128; };
+  long long need = 0;
+  auto take = [&need](long long v) { need = v > need ? v : need; };
+  if (m.gram) {   // S = X^T X forward, R = dV^T X backward: the same shapes
+    if (gram_contraction_supported(C)) take(gram_slab_floats(B, N, C, gram_ksplit(B)));
+    else take(slab_need(C, C, B, N, pick_split(B * t(C) * t(C), N), false, true));
+    if (backward && !gram_chain_supported(C, Ci)) {   // dW~theta / dW~phi / dW~g and dWz summed over the sequences
+      take(slab_need(Ci, m.Ca, B, C, 1, true, false));
+      take(slab_need(C, Ci, B, Ci, 1, true, false));
+    }
+    return need;
+  }
+  if (m.dot) {
+    if (!backward) take(slab_need(Ci, Ci, B, N, pick_split(B * t(Ci) * t(Ci), N), false, false));     // M
+    else {
+      take(slab_need(C, Ci, B, N, pick_split(B * t(C) * t(Ci), N), false, false));                    // dW'
+      take(slab_need(C, Ci, B, Ci, 1, true, false));                                                  // dWz
+    }
+  } else if (backward) {
+    take(slab_need(C, Ci, 1, rows, pick_split_rounds(C, Ci, 1, rows), false, false));                 // dWz
+  }
+  if (backward) {
+    const int nproj = m.gauss ? Ci : 3 * Ci;
+    take(slab_need(nproj, C, 1, rows, pick_split_rounds(nproj, C, 1, rows), false, false));           // dWcat
+  }
+  return need;
+}
+// The slabs go last in ws, so that every other piece keeps its offset whether the flag is set or not
+void carve_slab(Carver& c, const Dims& m, bool backward, SplitSlab* s) {
+  *s = SplitSlab{};
+  if (!m.det) return;
+  s->on = true;
+  s->floats = det_slab_floats(m, backward);
+  if (s->floats > 0) s->p = c.take<float>(static_cast<size_t>(s->floats));
+}
+
+struct WsFwd { float* colstats; float* red1; float* Mf; void* attn; void* saved_fallback; float* Sf; SplitSlab det; };
 size_t carve_ws_fwd(const Dims& m, void* base, WsFwd* w, size_t saved_bytes) {
   Carver c(base);
   const size_t np = 4 * (m.dot ? static_cast<size_t>(m.B) * m.tiles_seq : static_cast<size_t>(m.tiles_all));
@@ -292,11 +340,13 @@ size_t carve_ws_fwd(const Dims& m, void* base, WsFwd* w, size_t saved_bytes) {
     w->Mf = nullptr; w->attn = nullptr;
     w->Sf = c.take<float>(static_cast<size_t>(m.B) * m.C * m.C);   // split-K accumulation target of S = X^T X
     w->saved_fallback = c.take<uint8_t>(saved_bytes);
+    carve_slab(c, m, false, &w->det);
     return (c.off + 255) & ~static_cast<size_t>(255);
   }
   w->Mf = m.dot ? c.take<float>(static_cast<size_t>(m.B) * m.Ci * m.Ci) : nullptr;  // split-K accumulation target
   w->attn = m.dot ? nullptr : c.take<uint8_t>(attn_scratch_bytes(m.B, m.N, false));
   w->saved_fallback = c.take<uint8_t>(saved_bytes);  // used when the caller passes saved == NULL (inference)
+  carve_slab(c, m, false, &w->det);
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
@@ -308,6 +358,7 @@ struct WsBwd {
   // Gram form
   float *Rf, *rv, *evec, *dwaug, *dcv, *dtv, *wpart;
   bf16 *Rb, *AK, *dQa, *dT, *EF, *G0, *Hf;
+  SplitSlab det;
 };
 size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
   Carver c(base);
@@ -343,6 +394,7 @@ size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
     w->dcv = c.take<float>(B * C);
     w->dtv = c.take<float>(B * Ci);
     w->wpart = gram_chain_supported(m.C, m.Ci) ? c.take<float>(gram_wgrad_scratch_floats()) : nullptr;
+    carve_slab(c, m, true, &w->det);
     return (c.off + 255) & ~static_cast<size_t>(255);
   }
   w->dU = d->bn_layer ? c.take<bf16>(rows * C) : nullptr;
@@ -369,6 +421,7 @@ size_t carve_ws_bwd(const glf_desc* d, const Dims& m, void* base, WsBwd* w) {
   w->cs_g = c.take<float>(np * 2 * Ci);
   w->red1 = c.take<float>(static_cast<size_t>(REDUCE_STAGE1_ROWS) * 3 * Ci);
   w->dwcat = c.take<float>(3 * Ci * C);
+  carve_slab(c, m, true, &w->det);
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
@@ -439,17 +492,14 @@ int check_ptr(const void* p, const char* name) {
 // [[S, colsum(A)], [rowv^T, corner]] of width Ca.  Enough sequences: the GEMM writes bf16 straight into it and a border
 // kernel adds the homogeneous row / column; few long sequences: split-K into fp32, then one assembling pass.
 int gram_token_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch, float* rowsum, const float* rowv,
-                           const float* rowscale, float corner, int B, int N, int C, int Ca, cudaStream_t stream,
-                           const GramPrep* prep = nullptr, bool* prep_done = nullptr) {
+                           const float* rowscale, float corner, int B, int N, int C, int Ca, const SplitSlab& det,
+                           cudaStream_t stream, const GramPrep* prep = nullptr, bool* prep_done = nullptr) {
   if (prep_done != nullptr) *prep_done = false;
   if (gram_contraction_supported(C)) {
     // one CTA per sequence; few long sequences are split along the tokens to fill two rounds of the SMs
-    int ks = 1;
-    if (B < 96) {
-      ks = (2 * 148) / B;
-      if (ks < 1) ks = 1;
-    }
-    GLF_TRY(gram_contraction(A, X, out_aug, scratch, rowsum, rowscale, rowv, corner, 1, B, N, C, Ca, ks, stream, prep));
+    const int ks = gram_ksplit(B);
+    GLF_TRY(gram_contraction(A, X, out_aug, scratch, rowsum, rowscale, rowv, corner, 1, B, N, C, Ca, ks, stream, prep,
+                             &det));
     if (prep != nullptr && prep_done != nullptr) *prep_done = true;
     const int kb = (N + 63) / 64;
     if ((ks > kb ? kb : ks) > 1)
@@ -462,6 +512,7 @@ int gram_token_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* s
   g.M = C; g.N = C; g.K = N; g.batch = B;
   g.bn_hint = 128;
   g.rowsum = rowsum; g.rowsum_stride = C;
+  g.det = det;
   g.split_k = pick_split(static_cast<long long>(B) * ((C + 127) / 128) * ((C + 127) / 128), N);
   if (g.split_k > 1 || rowscale != nullptr) {   // (a per-row scale needs the fp32 result: the GEMM's alpha is a scalar)
     if (g.split_k > 1) {
@@ -543,8 +594,8 @@ int tpavi_fwd_gram(const glf_desc* d, const Dims& m, const void* x, const glf_we
   prep.tw = w->theta_w; prep.tb = w->theta_b; prep.pw = w->phi_w; prep.pb = w->phi_b; prep.gw = w->g_w; prep.gb = w->g_b;
   prep.wz = w->wz_w; prep.waug = s.waug; prep.wzb = s.wz; prep.C = C; prep.Ci = Ci; prep.Ca = Ca;
   bool prep_done = false;
-  GLF_TRY(gram_token_contraction(X, X, s.Sa, wf.Sf, s.sfv, nullptr, nullptr, static_cast<float>(N), B, N, C, Ca, stream,
-                                 &prep, &prep_done));
+  GLF_TRY(gram_token_contraction(X, X, s.Sa, wf.Sf, s.sfv, nullptr, nullptr, static_cast<float>(N), B, N, C, Ca, wf.det,
+                                 stream, &prep, &prep_done));
   if (!prep_done) GLF_TRY(gram_prep_weights(w, C, Ci, Ca, s.waug, s.wz, stream));
   if (gram_chain_supported(C, Ci)) {
     // T~, M, W', Q~ and c of every sequence in one launch, one CTA per sequence (glf_chain.cu)
@@ -618,7 +669,8 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
   const bool bn_train = d->bn_layer && d->training;   // k2, k3 != 0 only then
   // k1 * [R_b | rv_b]  with R_b = dV_b^T X_b, rv_b = dV_b^T 1: the BatchNorm-backward scale k1 (per channel of dV =
   // row of R) is applied in fp32 by the contraction's epilogue
-  GLF_TRY(gram_token_contraction(wb.dV, X, wb.Rb, wb.Rf, wb.rv, s.sfv, wb.k1, static_cast<float>(N), B, N, C, Ca, stream));
+  GLF_TRY(gram_token_contraction(wb.dV, X, wb.Rb, wb.Rf, wb.rv, s.sfv, wb.k1, static_cast<float>(N), B, N, C, Ca, wb.det,
+                                 stream));
   // One CTA per sequence runs dQ~ -> dW' -> dM -> dT~ -> F (and E, e) in a single launch (glf_chain.cu); the four
   // weight-gradient sums over the sequences below then read its dQ~, dW', dM / N and dT~.
   const bool chain = gram_chain_supported(C, Ci);
@@ -659,6 +711,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.M = Ci; g.N = Ca; g.K = C; g.batch = B;
     g.bn_hint = 128;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = wb.dwaug; g.ldd = Ca; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
   }
@@ -669,6 +722,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.B = opnd(s.Mb, 1, Ci, CiCi);
     g.M = C; g.N = Ci; g.K = Ci; g.batch = B;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = g_->wz_w; g.ldd = Ci; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
   }
@@ -689,6 +743,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.bn_hint = 128;
     g.alpha = invN;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = wb.dwaug + 2 * CiCa; g.ldd = Ca; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
   }
@@ -711,6 +766,7 @@ int tpavi_bwd_gram(const glf_desc* d, const Dims& m, const bf16* X, const glf_we
     g.M = Ci; g.N = Ca; g.K = C1; g.batch = B;
     g.bn_hint = 128;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = wb.dwaug + CiCa; g.ldd = Ca; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
   }
@@ -882,6 +938,7 @@ GLF_API int glf_tpavi_fwd(const glf_desc* d, const void* x, const glf_weights* w
       g.B = opnd(s.P + 2 * Ci, 1, 3 * Ci, static_cast<long long>(N) * 3 * Ci);
       g.M = Ci; g.N = Ci; g.K = N; g.batch = B;
       g.alpha = 1.f / static_cast<float>(N);
+      g.det = wf.det;
       GLF_TRY(token_contraction(g, s.Mb, wf.Mf, stream));
     }
     {  // W'_b[c,i] = sum_j Wz[c,j] M_b[i,j]        (folds Y = Theta M and U = Y Wz^T into one product per token)
@@ -998,6 +1055,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.A = opnd(dU, 1, C, static_cast<long long>(N) * C);
       g.B = opnd(s.P, 1, 3 * Ci, seqP);
       g.M = C; g.N = Ci; g.K = N; g.batch = B;
+      g.det = wb.det;
       GLF_TRY(token_contraction(g, wb.dWpb, wb.dWpf, stream));
     }
     GLF_TRY(check_cuda(cudaMemsetAsync(g_->wz_w, 0, sizeof(float) * CCi, stream), "memset dWz"));
@@ -1007,6 +1065,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.B = opnd(s.Mb, 1, Ci, CiCi);
       g.M = C; g.N = Ci; g.K = Ci; g.batch = B;
       g.out_kind = 2;
+      g.det = wb.det;
       g.D = g_->wz_w; g.ldd = Ci; g.strideD = 0;
       GLF_TRY(gemm(g, stream));
     }
@@ -1056,6 +1115,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
       g.B = opnd(s.Y, 1, Ci, 0);
       g.M = C; g.N = Ci; g.K = rows;
       g.out_kind = 2;
+      g.det = wb.det;
       g.D = g_->wz_w; g.ldd = Ci;
       g.split_k = pick_split_rounds(C, Ci, 1, rows);
       GLF_TRY(gemm(g, stream));
@@ -1081,6 +1141,7 @@ GLF_API int glf_tpavi_bwd(const glf_desc* d, const void* dz, const void* x, cons
     g.B = opnd(X, 1, C, 0);
     g.M = nproj; g.N = C; g.K = rows;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = wb.dwcat; g.ldd = C;
     g.split_k = pick_split_rounds(nproj, C, 1, rows);
     GLF_TRY(gemm(g, stream));

@@ -37,7 +37,28 @@ size_t carve_saved3(const Dims& m, void* base, Saved3* s) {
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
-struct WsF3 { float *wcat_f, *wcatT_f, *Pf, *Mf, *Wpf, *cs; void* saved_fallback; };
+// Slab scratch of the fixed-order split reductions (GLF_DETERMINISTIC), last in ws: the largest need among the
+// products that sum partials (M forward; dW', dWz, dWcat backward)
+void carve_slab3(Carver& c, const Dims& m, bool backward, SplitSlab* s) {
+  *s = SplitSlab{};
+  if (!m.det) return;
+  const int B = static_cast<int>(m.B), C = m.C, Ci = m.Ci, N = static_cast<int>(m.N), rows = static_cast<int>(m.rows);
+  auto t = [](long long n) { return (n + 127) / 128; };
+  long long need = 0;
+  auto take = [&need](long long v) { need = v > need ? v : need; };
+  if (!backward) {
+    take(slab_need(Ci, Ci, B, N, pick_split(B * t(Ci) * t(Ci), N), false, false));
+  } else {
+    take(slab_need(C, Ci, B, N, pick_split(B * t(C) * t(Ci), N), false, false));
+    take(slab_need(C, Ci, B, Ci, 1, true, false));
+    take(slab_need(3 * Ci, C, 1, rows, pick_split(t(3 * Ci) * t(C), rows), false, false));
+  }
+  s->on = true;
+  s->floats = need;
+  if (need > 0) s->p = c.take<float>(static_cast<size_t>(need));
+}
+
+struct WsF3 { float *wcat_f, *wcatT_f, *Pf, *Mf, *Wpf, *cs; void* saved_fallback; SplitSlab det; };
 size_t carve_wsf3(const Dims& m, void* base, WsF3* w, size_t saved_bytes) {
   Carver c(base);
   const size_t rows = m.rows, C = m.C, Ci = m.Ci, B = m.B;
@@ -48,12 +69,14 @@ size_t carve_wsf3(const Dims& m, void* base, WsF3* w, size_t saved_bytes) {
   w->Wpf = c.take<float>(B * C * Ci);
   w->cs = c.take<float>(static_cast<size_t>(colstats_f32_blocks(m.rows)) * 2 * C);
   w->saved_fallback = c.take<uint8_t>(saved_bytes);
+  carve_slab3(c, m, false, &w->det);
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
 struct WsB3 {
   float *dZf, *dVf, *dUf, *dPf, *dWpf, *dMf, *dXf, *part_ln, *k1, *k2, *k3, *cs, *dwcat;
   bf16 *dUl, *dPl, *dWpl, *dMl;
+  SplitSlab det;
 };
 size_t carve_wsb3(const glf_desc* d, const Dims& m, void* base, WsB3* w) {
   Carver c(base);
@@ -76,6 +99,7 @@ size_t carve_wsb3(const glf_desc* d, const Dims& m, void* base, WsB3* w) {
   w->k3 = c.take<float>(C);
   w->cs = c.take<float>(static_cast<size_t>(colstats_f32_blocks(m.rows)) * 2 * 3 * Ci);
   w->dwcat = c.take<float>(3 * Ci * C);
+  carve_slab3(c, m, true, &w->det);
   return (c.off + 255) & ~static_cast<size_t>(255);
 }
 
@@ -139,6 +163,7 @@ int tpavi_fwd_f32x3(const glf_desc* d, const Dims& m, const void* x, const glf_w
     g.alpha = 1.f / static_cast<float>(N);
     g.ldd = Ci; g.strideD = CiCi;
     g.D = wf.Mf;
+    g.det = wf.det;
     g.split_k = pick_split(static_cast<long long>(B) * ((Ci + 127) / 128) * ((Ci + 127) / 128), N);
     if (g.split_k > 1) {
       GLF_TRY(check_cuda(cudaMemsetAsync(wf.Mf, 0, sizeof(float) * pM, stream), "memset M"));
@@ -231,6 +256,7 @@ int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void
     g.M = C; g.N = Ci; g.K = N; g.batch = B;
     g.ldd = Ci; g.strideD = CCi;
     g.D = wb.dWpf;
+    g.det = wb.det;
     g.split_k = pick_split(static_cast<long long>(B) * ((C + 127) / 128) * ((Ci + 127) / 128), N);
     if (g.split_k > 1) {
       GLF_TRY(check_cuda(cudaMemsetAsync(wb.dWpf, 0, sizeof(float) * pWp, stream), "memset dW'"));
@@ -249,6 +275,7 @@ int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void
     six_pairs(g);
     g.M = C; g.N = Ci; g.K = Ci; g.batch = B;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = g_->wz_w; g.ldd = Ci; g.strideD = 0;
     GLF_TRY(gemm(g, stream));
   }
@@ -300,6 +327,7 @@ int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void
     six_pairs(g);
     g.M = 3 * Ci; g.N = C; g.K = rows;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = wb.dwcat; g.ldd = C;
     g.split_k = pick_split(static_cast<long long>((3 * Ci + 127) / 128) * ((C + 127) / 128), rows);
     GLF_TRY(gemm(g, stream));
@@ -314,6 +342,7 @@ int tpavi_bwd_f32x3(const glf_desc* d, const Dims& m, const void* dz, const void
     six_pairs(g);
     g.M = rows; g.N = C; g.K = 3 * Ci;
     g.out_kind = 2;
+    g.det = wb.det;
     g.D = dXf; g.ldd = C;
     GLF_TRY(gemm(g, stream));
     if (m.pack_x)

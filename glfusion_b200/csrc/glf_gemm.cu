@@ -52,6 +52,7 @@ struct GemmKParams {
   long long bias_stride;         // elements between the bias vectors of consecutive batch entries (0 = shared)
   float* rowsum;                 // optional [batch][M] fp32: sum over K of the A operand's row (BN <= 128, npairs == 1)
   long long rowsum_stride;
+  long long split_stride, rs_split_stride;   // out_kind 1 slabs: K slice s stores at D / rowsum + s * stride
 };
 
 // MT = 128-row accumulators per CTA tile: MT = 2 computes a 256 x BN super-tile, so each k-block of the B operand is
@@ -323,8 +324,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
         tmem_ld_32x32(tmem_base + Cfg::RS_COL + acc * 16 + (static_cast<uint32_t>(q * 32) << 16), rv);
         tmem_ld_wait();
         if (grow < p.M) {
-          float* dst = p.rowsum + static_cast<long long>(b) * p.rowsum_stride + grow;
-          if (p.split_k > 1) atomicAdd(dst, __uint_as_float(rv[0]));
+          float* dst = p.rowsum + static_cast<long long>(b) * p.rowsum_stride + split * p.rs_split_stride + grow;
+          if (p.split_k > 1 && p.rs_split_stride == 0) atomicAdd(dst, __uint_as_float(rv[0]));
           else *dst = __uint_as_float(rv[0]);
         }
       }
@@ -363,7 +364,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
           }
         }
         if (p.out_kind != 0) {
-          float* Df = reinterpret_cast<float*>(p.D) + static_cast<long long>(b) * p.strideD +
+          float* Df = reinterpret_cast<float*>(p.D) + static_cast<long long>(b) * p.strideD + split * p.split_stride +
                       static_cast<long long>(grow) * p.ldd;
           if (grow < p.M) {
 #pragma unroll
@@ -536,6 +537,23 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
   if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
+// D[g] (+)= sum_j slab[g * nsum + j], j in order: one thread per output element, every slab read coalesced
+__global__ void slab_reduce_kernel(const float* __restrict__ slab, int nsum, long long sstride, float* D, int M, int N,
+                                   long long ldd, long long strideD, int groups, int accumulate) {
+  const long long mn = static_cast<long long>(M) * N;
+  const long long total = mn * groups;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long g = i / mn, e = i - g * mn;
+    const long long m = e / N, n = e - m * N;
+    const float* src = slab + g * nsum * sstride + e;
+    float acc = src[0];
+    for (int j = 1; j < nsum; ++j) acc += src[j * sstride];
+    float* dst = D + g * strideD + m * ldd + n;
+    *dst = accumulate ? *dst + acc : acc;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ host side
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -665,17 +683,73 @@ int launch_major(bool a_mn, bool b_mn, const CUtensorMap& tmA, const CUtensorMap
 
 }  // namespace
 
+int slab_reduce(const float* slab, int nsum, long long sstride, float* D, int M, int N, long long ldd, long long strideD,
+                int groups, int accumulate, cudaStream_t stream) {
+  const long long total = static_cast<long long>(M) * N * groups;
+  if (total <= 0 || nsum < 1) return set_error(GLF_ERR_INVALID, "slab_reduce: empty problem");
+  const long long blocks = (total + 255) / 256;
+  slab_reduce_kernel<<<static_cast<int>(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, stream>>>(
+      slab, nsum, sstride, D, M, N, ldd, strideD, groups, accumulate);
+  return check_cuda(cudaGetLastError(), "slab_reduce launch");
+}
+
+namespace {
+
+// GLF_DETERMINISTIC form of an out_kind-2 product: each (batch entry, K slice) stores its fp32 tile into a slab of
+// a.det, then the slabs are added onto D in entry / slice order.  The batch runs in groups when all slabs at once would
+// exceed the scratch (slab_need caps it); D then receives one fixed-order sum per group, groups in order.
+int gemm_slabs(const GemmArgs& a, cudaStream_t stream) {
+  const bool batch_reduced = a.strideD == 0 && a.batch > 1;
+  int s = effective_split(a.K, a.split_k);
+  const long long mn = static_cast<long long>(a.M) * a.N, per = mn + (a.rowsum != nullptr ? a.M : 0);
+  if (s * per > a.det.floats) s = static_cast<int>(a.det.floats / per);
+  if (s < 1 && !batch_reduced) s = 1;
+  if (s == 1 && !batch_reduced) {   // one add per element onto the zeroed output: already in a fixed order
+    GemmArgs g = a;
+    g.det = SplitSlab{};
+    g.split_k = 1;
+    return gemm(g, stream);
+  }
+  if (s < 1 || a.det.p == nullptr) return set_error(GLF_ERR_WORKSPACE, "gemm: deterministic slab scratch too small");
+  const int chunk = static_cast<int>(a.det.floats / (s * per) < a.batch ? a.det.floats / (s * per) : a.batch);
+  for (int b0 = 0; b0 < a.batch; b0 += chunk) {
+    const int nb = a.batch - b0 < chunk ? a.batch - b0 : chunk;
+    GemmArgs g = a;
+    g.det = SplitSlab{};
+    g.batch = nb;
+    g.A.ptr = static_cast<const bf16*>(a.A.ptr) + b0 * a.A.batch_stride;
+    g.B.ptr = static_cast<const bf16*>(a.B.ptr) + b0 * a.B.batch_stride;
+    if (a.bias != nullptr) g.bias = a.bias + b0 * a.bias_stride;
+    g.split_k = s;
+    g.out_kind = 1;
+    g.D = a.det.p; g.ldd = a.N; g.strideD = s * mn; g.split_stride = mn;
+    float* rs = a.det.p + static_cast<long long>(nb) * s * mn;
+    if (a.rowsum != nullptr) { g.rowsum = rs; g.rowsum_stride = static_cast<long long>(s) * a.M; g.rowsum_split_stride = a.M; }
+    GLF_TRY(gemm(g, stream));
+    float* D = static_cast<float*>(a.D) + b0 * a.strideD;
+    const int nsum = batch_reduced ? nb * s : s, groups = batch_reduced ? 1 : nb;
+    GLF_TRY(slab_reduce(a.det.p, nsum, mn, D, a.M, a.N, a.ldd, a.strideD, groups, 1, stream));
+    if (a.rowsum != nullptr)
+      GLF_TRY(slab_reduce(rs, nsum, a.M, a.rowsum + b0 * a.rowsum_stride, 1, a.M, a.M, a.rowsum_stride, groups, 1, stream));
+  }
+  return 0;
+}
+
+}  // namespace
+
 int gemm(const GemmArgs& a, cudaStream_t stream) {
   if (a.M <= 0 || a.N <= 0 || a.K <= 0 || a.batch <= 0) return set_error(GLF_ERR_INVALID, "gemm: empty problem");
   if (a.N % 8 != 0) return set_error(GLF_ERR_INVALID, "gemm: N must be a multiple of 8 (got %d)", a.N);
   if (a.out_kind < 0 || a.out_kind > 2) return set_error(GLF_ERR_INVALID, "gemm: bad out_kind");
-  if (a.split_k > 1 && a.out_kind != 2) return set_error(GLF_ERR_INVALID, "gemm: split_k needs atomic output");
+  if (a.split_k > 1 && a.out_kind != 2 && !(a.out_kind == 1 && a.split_stride != 0))
+    return set_error(GLF_ERR_INVALID, "gemm: split_k needs atomic output");
   if (a.out_kind != 0 && (a.addend != nullptr || a.colstats != nullptr))
     return set_error(GLF_ERR_INVALID, "gemm: addend/colstats only with bf16 output");
   if (a.ldd % 8 != 0 || (reinterpret_cast<uintptr_t>(a.D) & 15) != 0)
     return set_error(GLF_ERR_INVALID, "gemm: output must be 16-byte aligned with ldd %% 8 == 0");
   if (a.npairs < 1 || a.npairs > 6) return set_error(GLF_ERR_INVALID, "gemm: npairs out of range");
   if (a.rowsum != nullptr && a.npairs != 1) return set_error(GLF_ERR_INVALID, "gemm: rowsum needs a single operand pair");
+  if (a.det.on && a.out_kind == 2) return gemm_slabs(a, stream);
 
   // Small-K products are HBM-bound: 128-wide tiles keep 2 CTAs per SM so one CTA's epilogue overlaps the other's
   // loads.  Large-K (tensor-bound, e.g. C=2048) products take the 128x256 tile.
@@ -730,6 +804,8 @@ int gemm(const GemmArgs& a, cudaStream_t stream) {
   p.bias_stride = a.bias != nullptr ? a.bias_stride : 0;
   p.rowsum = a.rowsum;
   p.rowsum_stride = a.rowsum_stride;
+  p.split_stride = a.split_stride;
+  p.rs_split_stride = a.rowsum_split_stride;
   p.cs_accum = 0;
   p.tiles_m = gemm_tiles_m(a.M);
   p.tiles_n = 0;  // set per tile shape in launch()

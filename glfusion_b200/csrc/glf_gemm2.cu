@@ -53,6 +53,7 @@ struct Gemm2Params {
   int split_k, kb_per_split;   // K slices per tile (fp32 atomic output only)
   float* Df;               // out_kind 2: fp32 output, red.global.add (split-K slices / batch-reduced products)
   long long ldd, strideD;
+  long long split_stride;  // != 0 (out_kind 1 slabs): K slice s stores its tile at Df + s * split_stride, no atomics
 };
 
 __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
@@ -231,8 +232,15 @@ __global__ void __launch_bounds__(G2_THREADS, 1)
         if (p.Df != nullptr) {                                // fp32 atomic output: no staging, no bulk store
           if (lane < rows_valid) {
             float* dr = p.Df + static_cast<long long>(b) * p.strideD + static_cast<long long>(m0 + q * 32 + lane) * p.ldd + gc0;
+            if (p.split_stride != 0) {
+              dr += (item % p.split_k) * p.split_stride;
 #pragma unroll
-            for (int j = 0; j < 16; j += 2) red_add_v4(dr + 2 * j, f[j].x, f[j].y, f[j + 1].x, f[j + 1].y);
+              for (int j = 0; j < 16; j += 2)
+                *reinterpret_cast<float4*>(dr + 2 * j) = make_float4(f[j].x, f[j].y, f[j + 1].x, f[j + 1].y);
+            } else {
+#pragma unroll
+              for (int j = 0; j < 16; j += 2) red_add_v4(dr + 2 * j, f[j].x, f[j].y, f[j + 1].x, f[j + 1].y);
+            }
           }
           __syncwarp();
           continue;
@@ -334,10 +342,10 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
 }  // namespace
 
 bool gemm_pair_applicable(const GemmArgs& a, int num_sms) {
-  if (a.N % BN2 != 0 || a.M < 1024 || a.out_kind == 1 || a.rowsum != nullptr) return false;
+  if (a.N % BN2 != 0 || a.M < 1024 || (a.out_kind == 1 && a.split_stride == 0) || a.rowsum != nullptr) return false;
   if (a.npairs > 6 || num_sms < 2) return false;
   if (a.out_kind == 0 && (a.split_k > 1 || a.strideD % 8 != 0)) return false;
-  if (a.out_kind == 2 && (a.bias != nullptr || a.addend != nullptr || a.colstats != nullptr || a.ldd % 4 != 0 ||
+  if (a.out_kind != 0 && (a.split_stride % 4 != 0 || a.bias != nullptr || a.addend != nullptr || a.colstats != nullptr || a.ldd % 4 != 0 ||
                           a.strideD % 4 != 0 || (reinterpret_cast<uintptr_t>(a.D) & 15) != 0))
     return false;
   // MN-major A is the token contraction of the token-space path (K = tokens): worth a pair only when tensor-bound
@@ -380,9 +388,10 @@ int gemm_pair(const GemmArgs& a, int num_sms, cudaStream_t stream) {
     p.kb_per_split = (p.kb_total + sk - 1) / sk;
     p.split_k = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
   }
-  p.Df = a.out_kind == 2 ? reinterpret_cast<float*>(a.D) : nullptr;
+  p.Df = a.out_kind != 0 ? reinterpret_cast<float*>(a.D) : nullptr;
   p.ldd = a.ldd;
   p.strideD = a.strideD;
+  p.split_stride = a.out_kind == 1 ? a.split_stride : 0;
   p.npairs = a.npairs;
   for (int i = 0; i < 6; ++i) { p.pairA[i] = a.pairA[i]; p.pairB[i] = a.pairB[i]; }
   p.a_batched = a.A.batch_stride != 0;

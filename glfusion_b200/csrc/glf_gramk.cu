@@ -44,6 +44,7 @@ struct GramKParams {
   bf16* out;       // ksplit == 1: [B][Ca][Ca] bf16, rows/cols < C written
   float* outf;     // ksplit  > 1: [B][C][C] fp32, atomically accumulated (zeroed by the caller)
   float* rowsum;   // [B][C] column sums of A (stored, or atomically accumulated when ksplit > 1)
+  int slabs;       // ksplit > 1: split s stores into slab s (outf + s [B][C][C], rowsum + s [B][C]) instead of atomics
   const float* rowscale;   // optional [C]: bf16 output row r is scaled by rowscale[r] (ksplit == 1 path)
   // ksplit == 1: the homogeneous border of the augmented matrix is written here as well (no separate launch):
   //   column C = rowscale * column sums of A, row C = rowv (or the column sums when rowv is null), corner, zero padding
@@ -194,7 +195,8 @@ __global__ void __launch_bounds__(GK_THREADS, 1)
     auto emit_colsum = [&](int ch, float cs) {
       float* dst = p.rowsum + static_cast<long long>(b) * p.C + ch;
       if (p.ksplit > 1) {
-        atomicAdd(dst, cs);
+        if (p.slabs) dst[static_cast<long long>(split) * p.B * p.C] = cs;
+        else atomicAdd(dst, cs);
         return;
       }
       *dst = cs;
@@ -272,11 +274,19 @@ __global__ void __launch_bounds__(GK_THREADS, 1)
         tmem_ld_wait();
         if (p.ksplit > 1) {
           float* dst = p.outf + (static_cast<long long>(b) * p.C + row) * p.C + c * 32;
+          if (p.slabs) {
+            dst += static_cast<long long>(split) * p.B * p.C * p.C;
 #pragma unroll
-          for (int j = 0; j < 32; j += 4)
-            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(__uint_as_float(v[j])),
-                         "f"(__uint_as_float(v[j + 1])), "f"(__uint_as_float(v[j + 2])), "f"(__uint_as_float(v[j + 3]))
-                         : "memory");
+            for (int j = 0; j < 32; j += 4)
+              *reinterpret_cast<float4*>(dst + j) = make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]),
+                                                                __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
+          } else {
+#pragma unroll
+            for (int j = 0; j < 32; j += 4)
+              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(__uint_as_float(v[j])),
+                           "f"(__uint_as_float(v[j + 1])), "f"(__uint_as_float(v[j + 2])), "f"(__uint_as_float(v[j + 3]))
+                           : "memory");
+          }
         } else {
           uint8_t* dst = stg + static_cast<uint32_t>(row) * STG_PITCH + c * 64;
 #pragma unroll
@@ -336,7 +346,7 @@ bool gram_contraction_supported(int C) { return C == 128 || C == 256; }
 // rowsum = column sums of A (unscaled).
 int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch, float* rowsum, const float* rowscale,
                      const float* rowv, float corner, int border, int B, int N, int C, int Ca, int ksplit,
-                     cudaStream_t stream, const GramPrep* prep) {
+                     cudaStream_t stream, const GramPrep* prep, const SplitSlab* slab) {
   if (!gram_contraction_supported(C)) return set_error(GLF_ERR_UNSUPPORTED, "gram_contraction: C must be 128 or 256");
   CUtensorMap tmA, tmX;
   int rc = make_tmap_bf16(&tmA, A, C, N, B, C, static_cast<long long>(N) * C, 64);
@@ -355,7 +365,14 @@ int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch
   p.out = out_aug; p.outf = scratch; p.rowsum = rowsum; p.rowscale = rowscale;
   p.rowv = rowv; p.corner = corner;
   p.border = (border && Ca > C) ? 1 : 0;
-  if (p.ksplit > 1) {
+  p.slabs = (slab != nullptr && slab->on && p.ksplit > 1) ? 1 : 0;
+  const long long BCC = static_cast<long long>(B) * C * C;
+  if (p.slabs) {
+    if (slab->p == nullptr || slab->floats < gram_slab_floats(B, N, C, ksplit))
+      return set_error(GLF_ERR_WORKSPACE, "gram_contraction: deterministic slab scratch too small");
+    p.outf = slab->p;
+    p.rowsum = slab->p + p.ksplit * BCC;
+  } else if (p.ksplit > 1) {
     rc = check_cuda(cudaMemsetAsync(scratch, 0, sizeof(float) * B * C * C, stream), "memset S");
     if (rc) return rc;
     rc = check_cuda(cudaMemsetAsync(rowsum, 0, sizeof(float) * B * C, stream), "memset s");
@@ -378,6 +395,10 @@ int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch
   }
   gram_kernel<<<static_cast<int>(grid) + p.nprep, GK_THREADS, GK_SMEM, stream>>>(tmA, tmX, p);
   rc = check_cuda(cudaGetLastError(), "gram_contraction launch");
+  if (rc == 0 && p.slabs) {   // the split slabs summed in split order: S into scratch, the column sums into rowsum
+    rc = slab_reduce(p.outf, p.ksplit, BCC, scratch, B * C, C, C, 0, 1, 0, stream);
+    if (rc == 0) rc = slab_reduce(p.rowsum, p.ksplit, static_cast<long long>(B) * C, rowsum, B, C, C, 0, 1, 0, stream);
+  }
   if (rc == 0 && p.trace) {      // debug only: synchronises the stream
     long long t[8] = {0};
     cudaStreamSynchronize(stream);

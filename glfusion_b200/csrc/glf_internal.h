@@ -48,6 +48,15 @@ struct GemmOperand {
   int rows = 0;              // valid rows of the operand (0 = the GEMM's M / N); smaller values are zero-filled by TMA
 };
 
+// fp32 scratch of the fixed-order split reductions (GLF_DETERMINISTIC).  on: a product with out_kind 2 whose output
+// elements would receive more than one atomic add (K slices, or a batch summed into one output) stores every partial
+// into its own slab of `p` instead and sums the slabs in slice / batch order onto D.
+struct SplitSlab {
+  bool on = false;
+  float* p = nullptr;
+  long long floats = 0;
+};
+
 struct GemmArgs {
   GemmOperand A, B;
   int M = 0, N = 0, K = 0, batch = 1;
@@ -59,6 +68,9 @@ struct GemmArgs {
   int out_kind = 0;                 // 0 bf16 store, 1 f32 store, 2 f32 atomic add
   void* D = nullptr;
   int64_t ldd = 0, strideD = 0;
+  int64_t split_stride = 0;         // out_kind 1 with split_k > 1: K slice s stores at D + s * split_stride (slabs)
+  int64_t rowsum_split_stride = 0;  //   and its row sums at rowsum + s * rowsum_split_stride
+  SplitSlab det;                    // fixed-order split reductions (out_kind 2 only; gemm() routes them)
   const bf16* addend = nullptr;     // optional bf16 [M, N] added in the epilogue (out_kind 0 only)
   int64_t ld_add = 0, stride_add = 0;
   float* colstats = nullptr;        // partial table, sized for [batch*tiles_m*4][2][N]; rows actually written:
@@ -85,6 +97,29 @@ inline int pick_split(long long tiles, int K) {
   if (s > kb) s = kb;
   return static_cast<int>(s);
 }
+// K slices the kernels actually run for a requested split: clamped to the k-blocks, and no slice left empty
+inline int effective_split(int K, int split) {
+  const int kb = (K + 63) / 64;
+  int s = split < 1 ? 1 : (split > kb ? kb : split);
+  const int per = (kb + s - 1) / s;
+  return (kb + per - 1) / per;
+}
+// Slab space of one deterministic out_kind-2 product is capped here (128 MB): a product that would need more runs its
+// batch entries in groups, or fewer K slices, so that each group's slabs fit.
+constexpr long long SLAB_CAP_FLOATS = 32LL << 20;
+// fp32 slab floats a deterministic out_kind-2 product uses (0: every output element receives a single add)
+inline long long slab_need(long long M, long long N, int batch, int K, int split, bool batch_reduced, bool rowsum) {
+  const int s = effective_split(K, split);
+  if (s == 1 && !(batch_reduced && batch > 1)) return 0;
+  const long long per = (M * N + (rowsum ? M : 0)) * s;
+  const long long full = per * batch;
+  if (full <= SLAB_CAP_FLOATS) return full;
+  return per > SLAB_CAP_FLOATS ? per : (SLAB_CAP_FLOATS / per) * per;
+}
+// D[g] (+)= sum_{j < nsum} slab[g * nsum + j] for g < groups, in slab order (fp32): D[g] is [M][N] with row pitch ldd
+// and group stride strideD, slab j is [M][N] dense, consecutive slabs `sstride` floats apart
+int slab_reduce(const float* slab, int nsum, long long sstride, float* D, int M, int N, long long ldd, long long strideD,
+                int groups, int accumulate, cudaStream_t stream);
 // (glf_gemm.cu) operand map: K-major -> dims {K, rows, batch, limb}, MN-major -> {rows, K, batch, limb}; SWIZZLE_128B,
 // box {64, box_rows or 64}.  Output map: dims {N, M, batch}, box {32, 32}, SWIZZLE_64B (the epilogue's staging tile).
 int make_operand_tmap(CUtensorMap* tm, const GemmOperand& op, int rows, int K, int batch, int nlimbs, int box_rows);
@@ -191,9 +226,15 @@ int gram_assemble_F(const bf16* G0, const bf16* Hf, const bf16* dT, const bf16* 
                     int C, int Ci, int Ca, cudaStream_t stream);
 // One CTA per sequence (glf_gramk.cu): D_b = A_b^T X_b for C = 128 / 256, operands streamed once
 bool gram_contraction_supported(int C);
+// slab (optional): with a token split, each split stores its S and column sums into its own slab there
+// (gram_slab_floats) and the slabs are summed in split order into scratch / rowsum, instead of atomics
 int gram_contraction(const bf16* A, const bf16* X, bf16* out_aug, float* scratch, float* rowsum, const float* rowscale,
                      const float* rowv, float corner, int border, int B, int N, int C, int Ca, int ksplit,
-                     cudaStream_t stream, const GramPrep* prep = nullptr);
+                     cudaStream_t stream, const GramPrep* prep = nullptr, const SplitSlab* slab = nullptr);
+inline long long gram_slab_floats(int B, int N, int C, int ksplit) {
+  const int s = effective_split(N, ksplit);
+  return s > 1 ? static_cast<long long>(s) * B * (static_cast<long long>(C) * C + C) : 0;
+}
 int gram_unpack_grads(const float* dwaug, const glf_grads* g, int C, int Ci, int Ca, cudaStream_t stream);
 // One CTA per sequence runs the whole [C x C] chain between the token-sized products (glf_chain.cu), C = 256, C' = 128
 bool gram_chain_supported(int C, int Ci);
@@ -318,6 +359,7 @@ struct Dims {
   int Ca;          // augmented width of the per-sequence matrices (gram)
   int pdt;         // GLF_DTYPE_* of the glf_weights / glf_grads tensors (glf_desc.reserved[3])
   bool half_params;   // bf16 / fp16 parameters: an fp32 shadow in `saved`, fp32 gradient staging in ws_bwd
+  bool det;           // GLF_DETERMINISTIC: fixed-order split reductions (slabs in ws)
 };
 // x / dz (in_dtype, [B, C, N] when ncthw, else token-major) -> token-major [B * N, C] of out_dtype;
 // unpack_tokens is the way back for dx

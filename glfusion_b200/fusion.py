@@ -341,6 +341,8 @@ class _FusionFunction(torch.autograd.Function):
         n_in = 5 + 3 * V + 2 * ng
         if dout is None and dglob is None:
             return (None,) * n_in
+        stg.refresh_deterministic()                 # (the ws blobs below are sized from the backward's flag)
+        stl.refresh_deterministic()
         tg, tl = mg._param_table(pg, ctx.pdt), ml._param_table(pl, ctx.pdt)
         bg, bl = mg._buffer_table(ctx.pdt), ml._buffer_table(ctx.pdt)
         gl = None

@@ -87,6 +87,13 @@ def _blob(nbytes: int, device) -> torch.Tensor:
 DOT_ALGO = int(os.environ.get("GLF_DOT_ALGO", "0"))
 
 
+def _deterministic_bit() -> int:
+    # torch.use_deterministic_algorithms(True) is the switch: the blocks then sum split products in a fixed order
+    # (GLF_DETERMINISTIC) and give bitwise identical results from run to run.  warn_only changes nothing: the
+    # deterministic implementation always exists.
+    return L.DETERMINISTIC if torch.are_deterministic_algorithms_enabled() else 0
+
+
 class TPAVIState:
     """Everything one forward/backward pair shares: descriptor, weights table, saved blob."""
 
@@ -105,12 +112,23 @@ class TPAVIState:
         d.accumulate = int(accumulate)
         d.eps_bn, d.eps_ln, d.momentum = eps_bn, eps_ln, momentum
         d.reserved[0] = 1 if defer_ln else 0     # LayerNorm stage run for MGFM + MLFM together (glf_fusion_ln_*)
-        d.reserved[1] = DOT_ALGO                 # 0 = library chooses, 1 = token-space form, 2 = Gram form
+        d.reserved[1] = DOT_ALGO | _deterministic_bit()   # dot algorithm (0 / 1 / 2) | GLF_DETERMINISTIC
         d.reserved[3] = param_dtype              # dtype of the parameter tensors, gradients and running statistics
         self.desc = d
+        self._resize()
+
+    def _resize(self):
         sz = L.GlfSizes()
-        L.check(L.load().glf_tpavi_sizes(C.byref(d), C.byref(sz)))
+        L.check(L.load().glf_tpavi_sizes(C.byref(self.desc), C.byref(sz)))
         self.sizes = sz
+
+    def refresh_deterministic(self):
+        """Backward reads torch.are_deterministic_algorithms_enabled() again, as forward did: the flag only changes
+        workspace sizes and reduction order, never the saved blob, so it may differ between the two."""
+        bit = _deterministic_bit()
+        if (self.desc.reserved[1] & L.DETERMINISTIC) != bit:
+            self.desc.reserved[1] = (self.desc.reserved[1] & 0xFF) | bit
+            self._resize()
 
 
 def _weights_struct(p, buffers) -> L.GlfWeights:
@@ -169,6 +187,7 @@ def tpavi_backward_raw(dz: torch.Tensor, dz_layout: int, x: torch.Tensor, st: TP
     a data-parallel all-reduce bucket, dp.GradBucket.bind): the returned gradient then aliases it."""
     lib = L.load()
     dev = x.device
+    st.refresh_deterministic()
     d = st.desc
     d.dz_layout = dz_layout
     grads = {}

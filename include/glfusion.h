@@ -77,6 +77,7 @@ typedef struct glf_desc {
                           reserved[1]: algorithm of mode='dot' (both are exact reassociations of ours.py:881-902):
                           0 = the library chooses (Gram form when N >= 5 C), 1 = token-space form (theta/phi/g formed
                           per token), 2 = Gram form (S = X~^T X~ per sequence, channel-space products only).
+                          reserved[1] | GLF_DETERMINISTIC: bitwise run-to-run reproducible results (below).
                           reserved[2]: dtype of z / z_global / dz of the fused LayerNorm pass (GLF_DTYPE_BF16 or F16).
                           reserved[3]: GLF_PARAMS_* — element type of every glf_weights / glf_grads tensor, the running
                           statistics included (bn_num_batches_tracked stays int64).  With GLF_PARAMS_BF16 / F16 the block
@@ -85,6 +86,14 @@ typedef struct glf_desc {
                           rounds the fp32 gradients to nearest into glf_grads backward (fp16 overflow: +-inf); the running
                           statistics are updated in place, rounded once.  GLF_PRECISION_F32X3 needs GLF_PARAMS_F32. */
 } glf_desc;
+
+/* Flag ORed into glf_desc.reserved[1] (the low byte keeps the mode='dot' algorithm): every product that would sum the
+ * partial results of several K slices or batch entries with fp32 atomics instead stores each partial into its own slab
+ * of ws and sums the slabs in a fixed order, so glf_tpavi_fwd / glf_tpavi_bwd give bitwise identical outputs and
+ * gradients from run to run (same descriptor, device and build).  Everything else already reduces in a fixed order.
+ * glf_tpavi_sizes counts the slabs in ws_fwd_bytes / ws_bwd_bytes only when the flag is set and a split occurs; the
+ * glf_fusion_ln_* entry points accept the flag and ignore it. */
+#define GLF_DETERMINISTIC 0x100
 
 /* Master parameters, same shapes as the reference state_dict (SURVEY.md §8b): fp32, or the bf16 / fp16 element type
  * glf_desc.reserved[3] names (the pointers are then read as that type). */
